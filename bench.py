@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — front-end frames/s of the B200-native PL-VIWO visual front end (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload at every N: BASELINE.json configs[4] — 64 independent camera streams, each the configs[1] front end
 (synthetic KAIST-shaped 1280x560 mono, point + line front end, 400 points, 5x5 grid, maxLevel 4, 15x15 window),
@@ -18,6 +18,9 @@ frame's copies, kernels and result read-back happen inside it (pipeline fill and
   e2e    : the same from pinned HOST frames through the C ABI: H2D of every frame and D2H of every result row inside
            the timed region
   roofline / cpu_baseline / clocks : see DESIGN.md "Measurement"
+--dump-outputs DIR writes, after the timed steps, the rows the resident pass returned for the last frame of every stream
+(engine_rows / dump_outputs below).  The inputs are seeded, so two builds run with the same arguments can be compared
+file by file.
 --impl reference times the reference's CPU path on the host cores: the oracle's restatement of TrackKLT / TrackLSD
 driving the real OpenCV kernels (cv2), one process per core group over independent streams (the reference itself needs
 OpenCV C++ / Eigen / ROS headers and cannot be compiled in this image).
@@ -419,6 +422,42 @@ def timed_pass(torch, dist, eng, first, n_frames, ptrs, pitch, on_device):
     return dict(ms=float(ev0.elapsed_time(ev1)), wall_ms=1e3 * wall, frames=frames, counters=c)
 
 
+def engine_rows(eng):
+    """Per stream (point rows, line rows, points on lines) of the last frame the engine played: what a caller of
+    plviwo_fe_play / plviwo_fe_group_play reads once the call returns."""
+    if eng.name == "group":
+        return [(eng.g.point_rows(s),) + eng.g.line_rows(s) for s in range(eng.g.n)]
+    return [(h.point_rows(),) + h.line_rows() for h in eng.h]
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, streams, rows, suffix=""):
+    """Writes `rows` (engine_rows) as out_dir/<name><suffix>.npy.  Ids and counts go to float64 arrays (exact below 2^53) whose
+    column 0 is the stream index, coordinates to float32 arrays with the same row order, so that ids can be compared exactly
+    and coordinates with a tolerance."""
+    def stream_col(parts):
+        return np.concatenate([np.full(len(p), s, np.float64) for s, p in zip(streams, parts)])
+
+    pts, lines, lpts = ([r[k] for r in rows] for k in range(3))
+    P, L, Q = np.concatenate(pts), np.concatenate(lines), np.concatenate(lpts)
+    out = {
+        "point_ids": np.stack([stream_col(pts), P["id"].astype(np.float64)], 1),
+        "point_uv": np.stack([P["u"], P["v"], P["un"], P["vn"]], 1).astype(np.float32),
+        "line_ids": np.stack([stream_col(lines)] + [L[k].astype(np.float64) for k in ("id", "D", "n_pts", "pt_offset", "matched")], 1),
+        "line_endpoints": np.concatenate([L["line"], L["line_n"]], 1).astype(np.float32),
+        "line_point_ids": np.stack([stream_col(lpts), Q["pid"].astype(np.float64)], 1),
+        "line_point_uv": np.stack([Q["dist"], Q["u"], Q["v"]], 1).astype(np.float32),
+    }
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes, more than %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def parity_against(fe_mod, dev, data, meta, rows_cpu):
     """BASELINE.json's third metric ("KLT px err").  The oracle is the checker here, nothing of it is timed.
     (a) teacher forced over 40 frames: the GPU tracker is loaded with the oracle's state before every frame, so each frame
@@ -518,7 +557,11 @@ def main():
     ap.add_argument("--engine", default=os.environ.get("PLVIWO_BENCH_ENGINE", "auto"), choices=["auto", "group", "handles"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the single-stream / synchronous / stereo extras")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the rows of the last frame of every stream as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path, not of --impl reference")
     args.warmup = max(args.warmup, 3)
     # exactly ONE line on stdout: libraries that print banners there (NCCL's version line) are sent to stderr
     real_stdout = os.dup(1)
@@ -535,7 +578,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        steps = min(args.steps, 20)
+        steps = args.steps
         warm = min(args.warmup, 4) * 4
         # a step of the reference arm = FRAMES_PER_STEP frames on each stream of its bounded sample (one stream per process)
         r, sweep, cores = run_cpu_arm(steps * FRAMES_PER_STEP, warm, 24)
@@ -601,10 +644,14 @@ def main():
     eng.run(0, n_warm, d_ptrs, W, True, frame_index=frame_index)                       # untimed: graph capture, clocks, then DRAINED (run returns when
     torch.cuda.synchronize()                                   # every frame is collected)
     sampler = ClockSampler(dev) if rank == 0 else None
-    res = timed_pass(torch, dist, eng, n_warm, n_timed, d_ptrs, W, True)
-    clocks = sampler.stop() if sampler else {}
+    try:
+        res = timed_pass(torch, dist, eng, n_warm, n_timed, d_ptrs, W, True)
+    finally:   # the sampler is a child process: never leave it running
+        clocks = sampler.stop() if sampler else {}
     if res["counters"]["kernel_launches_total"] == 0 or res["frames"] != n_timed * S:
         raise SystemExit("bench.py: the timed region launched no kernel or lost frames (%r)" % (res,))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, streams, engine_rows(eng), "" if world == 1 else "_rank%d" % rank)
     # ---- per-kernel durations: a short pass with CUDA-event stage timing on
     stage = None
     try:
