@@ -27,9 +27,8 @@ SOURCES = [
     ("fe_capi.cu", []),
     ("ransac.cpp", []),
     ("host_simd.cpp", []),
-    ("sm_partition.cpp", []),
 ]
-HEADERS = ["fe_kernels.h", "fe_group_dev.h", "fe_group.h", "ransac_core.h", "fe_context.h", "fe_stereo.h", "sm_partition.h", "tma_bulk.h", "introsort.h", os.path.join("..", "..", "include", "plviwo_fe.h")]
+HEADERS = ["fe_kernels.h", "fe_group_dev.h", "fe_group.h", "ransac_core.h", "fe_context.h", "fe_stereo.h", "tma_bulk.h", "introsort.h", os.path.join("..", "..", "include", "plviwo_fe.h")]
 
 
 def _nvcc() -> str:

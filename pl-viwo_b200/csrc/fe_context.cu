@@ -9,7 +9,6 @@
 // submit() on its own streams; collect() runs the state-dependent chain (top-off detection on the previous
 // image, LK, RANSAC gate, line association) in frame order.
 #include "fe_context.h"
-#include "sm_partition.h"
 
 #include <algorithm>
 #include <chrono>
@@ -153,7 +152,7 @@ int FeContext::init() {
   FE_CUDA(cudaSetDevice(device_));
   int lo = 0, hi = 0;
   FE_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-  FE_CUDA(create_stream_on_partition(device_, SmPart::Tracking, hi, &s_pt_));
+  FE_CUDA(cudaStreamCreateWithPriority(&s_pt_, cudaStreamNonBlocking, hi));
   init_device_constants();
   use_graphs_ = std::getenv("PLVIWO_NO_GRAPHS") == nullptr;
   // Line-path batching: the segment extraction of a frame is > 2 ms of kernel TIME (the sequential chain walk), and the
@@ -196,30 +195,12 @@ int FeContext::init() {
       FE_CUDA(cudaMallocHost(&s.h_fld_counts, 2 * sizeof(int)));
     }
     FE_CUDA(cudaMallocHost(&s.h_raw, (size_t)Win_ * Hin_));
-    // One stream per slot and path by default; PLVIWO_LINE_STREAMS / _IMAGE_STREAMS / _FAST_STREAMS = n > 0 share n streams
-    // between the slots instead (slot i uses entry i mod n).  Measured on B200 (profiles/experiments_r1.md): sharing
+    // One stream per slot and path.  Measured on B200 (profiles/experiments_r1.md): sharing streams between the slots
     // LOWERS single-stream throughput — the line path needs ~2.5 ms of kernel time per frame, so its throughput is
     // (streams in flight) / 2.5 ms: 12 line streams 5.7k frames/s, 16: 7.3k, 24: 8.0k, one per slot (26): 9.3k.
-    {
-      auto pool_size = [&](const char *env, int dflt) {
-        const char *e = std::getenv(env);
-        int v = e ? std::atoi(e) : dflt;
-        if (v <= 0) v = nslots;   // 0: one stream per slot (no sharing)
-        return std::min(v, nslots);
-      };
-      const int nl = cfg_.use_lines ? pool_size("PLVIWO_LINE_STREAMS", 0) : 0, na = pool_size("PLVIWO_IMAGE_STREAMS", 0),
-                nb = pool_size("PLVIWO_FAST_STREAMS", 0);
-      const int i = s.index;
-      if (i < nl) FE_CUDA(create_stream_on_partition(device_, SmPart::Rest, lo, &s.s_line));
-      if (i < na) FE_CUDA(create_stream_on_partition(device_, SmPart::Rest, lo, &s.s_a));
-      if (i < nb) FE_CUDA(create_stream_on_partition(device_, SmPart::Rest, lo, &s.s_b));
-      s.owns_line = i < nl;
-      s.owns_a = i < na;
-      s.owns_b = i < nb;
-      if (!s.owns_line && nl > 0) s.s_line = slots_[i % nl].s_line;
-      if (!s.owns_a) s.s_a = slots_[i % na].s_a;
-      if (!s.owns_b) s.s_b = slots_[i % nb].s_b;
-    }
+    if (cfg_.use_lines) FE_CUDA(cudaStreamCreateWithPriority(&s.s_line, cudaStreamNonBlocking, lo));
+    FE_CUDA(cudaStreamCreateWithPriority(&s.s_a, cudaStreamNonBlocking, lo));
+    FE_CUDA(cudaStreamCreateWithPriority(&s.s_b, cudaStreamNonBlocking, lo));
     FE_CUDA(cudaMalloc(&s.d_hist, 256 * sizeof(unsigned)));
     FE_CUDA(cudaMemset(s.d_hist, 0, 256 * sizeof(unsigned)));
     FE_CUDA(cudaMalloc(&s.d_clahe, 64 * 256));
@@ -294,17 +275,12 @@ int FeContext::init() {
     FE_CUDA(cudaMalloc(&s.d_sc_done, sizeof(unsigned)));
     FE_CUDA(cudaMemset(s.d_sc_done, 0, sizeof(unsigned)));
   }
-  // Speculative tracking is on whenever frames are pipelined (PLVIWO_SPECULATION=0 switches it off): it takes RANSAC and
-  // the detection glue off the point tracker's dependent chain (100 -> 67 us per frame) at ~40 % more LK work.  It only
-  // pays when the line path keeps up — which it does since consecutive frames share their line-path launches
-  // (line_batch_) and the lookahead is deep enough (profiles/experiments_r1.md: 9.3 k -> 12.4 k frames/s).  Results are
-  // bit-identical either way (tests/test_frontend_gpu.py).  A synchronous handle (lookahead 0) never has a next frame to
-  // speculate into.
-  {
-    const char *e = std::getenv("PLVIWO_SPECULATION");
-    use_spec_ = e ? std::atoi(e) != 0 : cfg_.lookahead >= 1;
-  }
-  use_spec_cand_ = std::getenv("PLVIWO_NO_CANDIDATE_SPECULATION") == nullptr;
+  // Speculative tracking is on whenever frames are pipelined: it takes RANSAC and the detection glue off the point
+  // tracker's dependent chain (100 -> 67 us per frame) at ~40 % more LK work.  It only pays when the line path keeps up —
+  // which it does since consecutive frames share their line-path launches (line_batch_) and the lookahead is deep enough
+  // (profiles/experiments_r1.md: 9.3 k -> 12.4 k frames/s).  Results are bit-identical to the synchronous handle's
+  // (tests/test_frontend_gpu.py), which (lookahead 0) never has a next frame to speculate into.
+  use_spec_ = cfg_.lookahead >= 1;
   FE_CUDA(cudaMallocHost(&h_pts0_, (size_t)max_pts_ * sizeof(float2)));
   FE_CUDA(cudaMallocHost(&h_pts1_, (size_t)max_pts_ * sizeof(float2)));
   FE_CUDA(cudaMallocHost(&h_p0n_, (size_t)max_pts_ * sizeof(float2)));
@@ -340,9 +316,9 @@ FeContext::~FeContext() {
     for (auto &e : s.ev_sp_t) if (e) cudaEventDestroy(e);
     destroy_graphs(s);
     cudaFree(s.d_hist); cudaFree(s.d_counters); cudaFree(s.d_seq); cudaFree(s.d_clahe);
-    if (s.s_a && s.owns_a) cudaStreamDestroy(s.s_a);
-    if (s.s_b && s.owns_b) cudaStreamDestroy(s.s_b);
-    if (s.s_line && s.owns_line) cudaStreamDestroy(s.s_line);
+    if (s.s_a) cudaStreamDestroy(s.s_a);
+    if (s.s_b) cudaStreamDestroy(s.s_b);
+    if (s.s_line) cudaStreamDestroy(s.s_line);
     if (s.ev_pyr) cudaEventDestroy(s.ev_pyr);
     if (s.ev_lines) cudaEventDestroy(s.ev_lines);
     for (auto &e : s.ev_t) if (e) cudaEventDestroy(e);
@@ -690,7 +666,7 @@ int FeContext::flush_line_batch() {
 // reads the few results that belong to candidates the detection really adds.
 int FeContext::track_candidates(FrameSlot &prev, FrameSlot &s) {
   s.sc_prev = -1;
-  if (!use_spec_ || !use_spec_cand_ || cfg_.line_samples > 0) return FE_OK;
+  if (!use_spec_ || cfg_.line_samples > 0) return FE_OK;
   LkParams prm;
   prm.win = cfg_.win_size;
   prm.max_level = cfg_.pyr_levels;

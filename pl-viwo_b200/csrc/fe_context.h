@@ -102,7 +102,6 @@ struct FrameSlot {
   cudaEvent_t ev_pyr = nullptr, ev_lines = nullptr;
   cudaStream_t s_line = nullptr;   // per-slot streams: the frame-independent work of different frames overlaps
   cudaStream_t s_a = nullptr, s_b = nullptr;
-  bool owns_line = false, owns_a = false, owns_b = false;   // streams are pooled: only the first slots of a pool own theirs
   unsigned *d_hist = nullptr, *d_counters = nullptr;
   uint8_t *d_clahe = nullptr;      // CLAHE: 64 tile LUTs of this frame
   int *d_seq = nullptr;            // device-side sequence numbers of the completion signals [fast, -, lines]
@@ -288,7 +287,6 @@ class FeContext {
   static constexpr int kCandBase = 1 << 24;   // src >= kCandBase: result of candidate table slot (src - kCandBase)
   int prev_submit_slot_ = -1;                 // caller's thread: slot of the frame submitted last
   int spec_n_ = 0, seq_sp_ = 0;
-  bool use_spec_cand_ = true;
   int spec_prev_slot_ = -1, spec_next_slot_ = -1;
   bool spec_valid_ = false, spec_timed_ = false, use_spec_ = true;
   std::vector<int> spec_of_lk_;     // per point of this frame's LK arrays: its index in the speculative launch, or -1

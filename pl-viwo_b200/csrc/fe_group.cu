@@ -173,7 +173,6 @@ int FeGroup::init() {
     FG_CUDA(dev_alloc(dev_allocs_, &sl.band_off, std::max(ncell * cells_nb_, 1)));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.band_cnt, std::max(ncell * cells_nb_, 1)));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.cand, g_.cand_cap));
-    FG_CUDA(dev_alloc(dev_allocs_, &sl.cand_ref, g_.cand_cap));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.cand_cnt, std::max(ncell, 1)));
     if (cfg_.use_lines) {
       rc = alloc_image(sl.half, W_ / 2, H_ / 2);

@@ -1,11 +1,12 @@
 // Stream group: many camera streams of one device tracked together (BASELINE.json configs[4], "multi-session batch
 // throughput").  Each stream is what one FeContext is — one ov_core::TrackKLT + one viw::TrackLSD for one camera, same
 // results bit for bit — but
-//   * the state-independent work of a frame of EVERY stream (equalise, pyramid, FAST on every grid cell + std::sort / top-k +
-//     cornerSubPix, Canny, connected components, chain walk, segments) is one set of launches per tick (grid.z = stream), and
+//   * the state-independent work of a frame of EVERY stream (equalise, pyramid, Canny, connected components, chain walk,
+//     segments) is one set of launches per tick (grid.z = stream), and
 //   * the tracker state (pts_last / ids_last / currid, lines_last / point_on_lines_last) lives in device memory and the
-//     state machine of a frame (top-off detection on the previous image, LK, RANSAC gate, row filter, line association)
-//     is four launches per tick for all streams (kernels_glue.cu, k_lk15_g) — no host thread sees a feature before the
+//     state machine of a frame (top-off detection on the previous image, with FAST + std::sort / top-k + cornerSubPix on
+//     the cells it leaves open, LK, RANSAC gate, row filter, line association) is one set of launches per tick for all
+//     streams (kernels_glue.cu, kernels_fast.cu, k_lk15w_g) — no host thread sees a feature before the
 //     rows of the frame are complete in pinned host memory.
 // The caller's thread only enqueues launches (submit) and waits for a tick's completion event (collect).
 #pragma once

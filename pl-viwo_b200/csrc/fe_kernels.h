@@ -188,7 +188,7 @@ struct SlotRec {
   unsigned *fast_total;          // [0] corners [1] scratch cursor
   unsigned *kps, *sort_scratch;
   int *band_off, *band_cnt;
-  float2 *cand, *cand_ref;       // per-cell candidate table before / after cornerSubPix (cell c at c * nfg)
+  float2 *cand;                  // per-cell candidate table (cell c at c * nfg)
   int *cand_cnt;
   FldBuffers fld;
 };
@@ -204,14 +204,13 @@ struct FrontGeom {               // the same for every stream of a group
   int n_cells, max_bands, max_cell_w, fast_threshold, kps_cap, nfg;
   const FastCell *cells;
 };
-// State-independent work of n_jobs frames: equalise + pyramid, FAST on every grid cell + std::sort/top-k + cornerSubPix.
+// State-independent work of n_jobs frames: histogram (+ CLAHE tile LUTs), equalise + pyramid (+ the half-resolution
+// line input).  FAST, its per-cell selection and cornerSubPix run later, on demand, on the cells the tracker leaves
+// open (fe_group_dev.h).
 void launch_hist_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, int *slot_flags, cudaStream_t s);
 void launch_clahe_lut_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, cudaStream_t s);
 void launch_eq_pyr1_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, bool want_half, cudaStream_t s);
 void launch_pyr_level_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, int level, int dw, int dh, cudaStream_t s);
-void launch_fast_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, cudaStream_t s);
-void launch_fast_select_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, cudaStream_t s);
-void launch_corner_subpix_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, cudaStream_t s);
 // The line kernels take either a FldBatch by value (a few frames of one handle) or this view of the slot table
 // (entry k of the launch = slot idx[k]); same kernel bodies, instantiated for both.
 struct FldTable {

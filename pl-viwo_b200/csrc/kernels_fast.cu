@@ -339,13 +339,6 @@ __global__ void __launch_bounds__(kFastThreads)
            unsigned *__restrict__ kps, int kps_cap, int smem_w) {
   fast_body(blockIdx.y, img, pitch, cells, max_bands, threshold, total, band_off, band_cnt, kps, kps_cap, smem_w);
 }
-// grid = (band, cell, job)
-__global__ void __launch_bounds__(kFastThreads, 4)
-    k_fast_b(const SlotRec *__restrict__ slots, const FrontJob *__restrict__ jobs, FrontGeom g, int smem_w) {
-  const SlotRec &sl = slots[jobs[blockIdx.z].slot];
-  fast_body(blockIdx.y, sl.lvl[0].p, sl.lvl[0].pitch, g.cells, g.max_bands, g.fast_threshold, sl.fast_total, sl.band_off, sl.band_cnt,
-            sl.kps, g.kps_cap, smem_w);
-}
 // Stream group, FAST on demand: grid = (band, index into the stream's valid-cell list, job).  The reference runs cv::FAST on the
 // valid cells only (Grider_GRID.h:108-125); which cells are valid is known once k_group_detect has counted the tracked points
 // per cell, so the detector runs between the two halves of the detection, on the image the detection is about.
@@ -420,14 +413,7 @@ __global__ void __launch_bounds__(kSelThreads)
                   int *__restrict__ cand_cnt) {
   fast_select_body(blockIdx.x, cells, max_bands, total, band_off, band_cnt, kps, kps_cap, scratch, nfg, cand_sel, cand_cnt);
 }
-// grid = (cell, job)
-__global__ void __launch_bounds__(kSelThreads)
-    k_fast_select_b(const SlotRec *__restrict__ slots, const FrontJob *__restrict__ jobs, FrontGeom g) {
-  const SlotRec &sl = slots[jobs[blockIdx.y].slot];
-  fast_select_body(blockIdx.x, g.cells, g.max_bands, sl.fast_total, sl.band_off, sl.band_cnt, sl.kps, g.kps_cap, sl.sort_scratch, g.nfg,
-                   sl.cand, sl.cand_cnt);
-}
-// grid = (index into the stream's valid-cell list, job)
+// grid =(index into the stream's valid-cell list, job)
 __global__ void __launch_bounds__(kSelThreads)
     k_fast_select_g(const __grid_constant__ GroupDev gd, const TrackJob *__restrict__ jobs, FrontGeom g) {
   const TrackJob &job = jobs[blockIdx.y];
@@ -439,21 +425,6 @@ __global__ void __launch_bounds__(kSelThreads)
   const SlotRec &sl = gd.slots[gd.wmode[s] == 1 ? job.cur_slot : job.prev_slot];
   fast_select_body(c, g.cells, g.max_bands, sl.fast_total, sl.band_off, sl.band_cnt, sl.kps, g.kps_cap, sl.sort_scratch, g.nfg, sl.cand,
                    sl.cand_cnt);
-}
-
-void launch_fast_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, cudaStream_t s) {
-  if (n_jobs <= 0 || g.n_cells <= 0) return;
-  const int smem_w = (g.max_cell_w + 15) & ~15;
-  const size_t smem = (size_t)(2 * kBH + 10) * smem_w + 3 * kFastPad + (size_t)(kBH + 2) * smem_w * 4;
-  static SmemOptIn optin;
-  optin.ensure(k_fast_b, smem);
-  PLVIWO_CARVEOUT(k_fast_b);
-  k_fast_b<<<dim3(g.max_bands, g.n_cells, n_jobs), kFastThreads, smem, s>>>(slots, jobs, g, smem_w);
-}
-void launch_fast_select_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, cudaStream_t s) {
-  if (n_jobs <= 0 || g.n_cells <= 0 || g.max_bands > kSelMaxBands) return;
-  PLVIWO_CARVEOUT(k_fast_select_b);
-  k_fast_select_b<<<dim3(g.n_cells, n_jobs), kSelThreads, 0, s>>>(slots, jobs, g);
 }
 
 void launch_group_fast(const GroupDev &gd, const TrackJob *jobs, int n_jobs, const FrontGeom &g, cudaStream_t s) {

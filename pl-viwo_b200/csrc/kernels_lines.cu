@@ -12,8 +12,10 @@
 // the sequential algorithm is exactly "for every connected component, run the raster-order walk on that component
 // alone; then list all chains by the raster index of their seed".  So
 //   1. connected components of the edge map by union-find (label = smallest raster index = the component's first seed),
-//   2. one warp per component with >= length_threshold + 1 pixels: it copies the component's pixels into a private
-//      bit map in shared memory, its lanes scan for the next seed together and lane 0 walks the chain,
+//   2. every component with >= length_threshold + 1 pixels is copied into a private bit map in shared memory and walked
+//      there: the small ones of a launch over many frames by one thread each (k_fld_walk_thread, one 64-bit word per
+//      row), the others by one warp each (k_fld_walk_cc: its lanes scan for the next seed together and fetch the 5 x 5
+//      window of every step together); both walks take their steps from the same two decision tables,
 //   3. chains are ranked by seed index, segments are fitted by one thread per chain (running double-precision sums,
 //      identical to refitting from scratch) and an ordered compaction restores the reference's output order.
 // The first version walked the whole frame with a single thread: 14.6 ms per 640x280 frame.
@@ -22,6 +24,7 @@
 #include <cstdlib>
 
 #include <algorithm>
+#include <type_traits>
 #include <mutex>
 #include <cstdio>
 #include <cmath>
@@ -246,9 +249,12 @@ __global__ void k_ccl_reset(const __grid_constant__ B b) {
 // ------------------------------------------------------------------------------------------------ Canny
 constexpr int kCnW = 64, kCnH = 16, kCnThreads = 256;
 
-// kFuse: the CTA goes on to label its tile (the Canny tile IS the connected-component tile: same 64 x 16 pixels, same 256
-// threads), so the edge bits never make the trip through global memory before the first labelling step and the frame's
-// tiles are launched once instead of twice.  k_ccl_reset must have run before the launch.
+// Stream group (FldTable): the Canny CTA goes on to label its tile (the Canny tile IS the connected-component tile: same
+// 64 x 16 pixels, same 256 threads), so the edge bits never make the trip through global memory before the first labelling
+// step and the frame's tiles are launched once instead of twice; k_ccl_reset runs ahead of that Canny launch.  A handle's
+// frames (FldBatch) are labelled by k_ccl_tile, at the start of the line launches.
+template <class B>
+constexpr bool kFusedLabels = std::is_same<B, FldTable>::value;
 static_assert(kCnW == kTileW && kCnH == kTileH && kCnThreads == kTileThreads, "Canny tile = connected-component tile");
 struct CannySmem {
   uint8_t pix[kCnH + 4][kCnW + 4];
@@ -256,9 +262,10 @@ struct CannySmem {
   short sdy[kCnH + 2][kCnW + 2];
   unsigned short mag[kCnH + 2][kCnW + 2];
 };
-template <class B, bool kFuse>
+template <class B>
 __global__ void __launch_bounds__(kCnThreads)
     k_canny(const __grid_constant__ B b, int low) {
+  constexpr bool kFuse = kFusedLabels<B>;
   const uint8_t *__restrict__ img = b.half_of(blockIdx.z).p;
   const int w = b.half_of(blockIdx.z).w, h = b.half_of(blockIdx.z).h, pitch = b.half_of(blockIdx.z).pitch;
   unsigned *__restrict__ edges = b.fld_of(blockIdx.z).edges;
@@ -331,7 +338,7 @@ __global__ void __launch_bounds__(kCnThreads)
     if (lane == 0 && gy < h && (tx0 + (q & 1) * 32) < w) edges[(size_t)gy * words_per_row + ((tx0 + (q & 1) * 32) >> 5)] = bits;
     if (kFuse && lane == 0) s_bits[r][q & 1] = bits;   // pixels beyond the frame are not edges: the same bits k_ccl_tile would read
   }
-  if (kFuse) {
+  if constexpr (kFuse) {
     __syncthreads();   // every warp is done with the gradient planes; the tile's bits are complete
     CclTileSmem &ts = *reinterpret_cast<CclTileSmem *>(smem_raw);
     if (tid < kCnH * 2) ts.bits[tid >> 1][tid & 1] = s_bits[tid >> 1][tid & 1];
@@ -341,17 +348,14 @@ __global__ void __launch_bounds__(kCnThreads)
 }
 
 template <class B>
-static void launch_canny_any(const B &b, int n, int w, int h, float th_low, cudaStream_t s, bool fuse_labels = false) {
+static void launch_canny_any(const B &b, int n, int w, int h, float th_low, cudaStream_t s) {
   dim3 grid((w + kCnW - 1) / kCnW, (h + kCnH - 1) / kCnH, n);
-  if (fuse_labels) {   // Canny + the tile-local labelling of the connected components; launch_fld_any(..., tiles_done = true) follows
+  if constexpr (kFusedLabels<B>) {
     PLVIWO_CARVEOUT(k_ccl_reset<B>);
     k_ccl_reset<B><<<n, 32, 0, s>>>(b);
-    PLVIWO_CARVEOUT((k_canny<B, true>));
-    k_canny<B, true><<<grid, kCnThreads, 0, s>>>(b, (int)floorf(th_low));
-    return;
   }
-  PLVIWO_CARVEOUT((k_canny<B, false>));
-  k_canny<B, false><<<grid, kCnThreads, 0, s>>>(b, (int)floorf(th_low));
+  PLVIWO_CARVEOUT(k_canny<B>);
+  k_canny<B><<<grid, kCnThreads, 0, s>>>(b, (int)floorf(th_low));
 }
 void launch_canny_batch(const FldBatch &b, float th_low, float th_high, cudaStream_t s) {
   (void)th_high;  // low == high is enforced at create time (no hysteresis pass is implemented)
@@ -359,7 +363,7 @@ void launch_canny_batch(const FldBatch &b, float th_low, float th_high, cudaStre
 }
 void launch_canny_table(const SlotRec *slots, const int *line_slots, int n_jobs, int w, int h, float th_low, cudaStream_t s) {
   if (n_jobs <= 0) return;
-  launch_canny_any(FldTable{slots, line_slots}, n_jobs, w, h, th_low, s, true);
+  launch_canny_any(FldTable{slots, line_slots}, n_jobs, w, h, th_low, s);
 }
 void launch_canny(const DevImage &half, float th_low, float th_high, FldBuffers &fb, cudaStream_t s) {
   FldBatch b;
@@ -710,72 +714,13 @@ __device__ __forceinline__ void walk_component(const WalkCtx &c, unsigned *bm, u
   }
 }
 
-// The same walk by ONE lane of the warp (the others wait at the __syncwarp that follows): no ballots, no warp synchronisation
-// inside the step, about half the instructions per step of the cooperative form (a warp instruction costs an issue slot whether
-// one lane or 25 take part), at a similar latency per step — the step is a chain of dependent shared-memory accesses either
-// way.  The 3 x 3 neighbourhood comes from two adjacent words of each of the three rows (funnel shift), the tables are the
-// cooperative walk's, so are the seeds (raster order) and the consumption order: identical chains.
-__device__ __forceinline__ void walk_component_single(const WalkCtx &c, unsigned *bm, const uint8_t *lut, int root, int y0, int g0,
-                                                      int groups, int bh, int ws) {
-  int npts = atomicAdd(c.counters + 2, c.cnt[root]);   // this component's slice of the chain-point pool
-  const int xbase = (g0 << 5) - 32;                    // global x of bit 0 of a private row
-  int sy = 0, sg = 0;                                  // scan position (row, word): everything before it is consumed
-  while (sy < bh) {
-    const int rbs = (sy + kPadRows) * ws;
-    unsigned wv = 0;
-    while (sg < groups && (wv = bm[rbs + 1 + sg]) == 0u) sg++;
-    if (sg >= groups) {
-      sg = 0;
-      sy++;
-      continue;
-    }
-    int p = ((sg + 1) << 5) + __ffs((int)wv) - 1, cy = sy;
-    int rb = rbs;
-    const int start = npts;
-    const int seed = (y0 + cy) * c.w + xbase + p;
-    int step = 0;
-    unsigned dsel = 0;
-    const uint8_t *tb = lut + kKeys * 8;     // first-step half of the table
-    bm[rb + (p >> 5)] = wv & ~(1u << (p & 31));   // the seed is consumed
-    while (true) {
-      c.chain_pts[npts++] = make_int2(xbase + p, y0 + cy);
-      const int q = p - 1, wi = q >> 5, sh = q & 31;
-      const unsigned *r0 = bm + rb + wi;
-      const unsigned t3 = __funnelshift_r(r0[-ws], r0[-ws + 1], sh) & 7u;
-      const unsigned c3 = __funnelshift_r(r0[0], r0[1], sh) & 7u;
-      const unsigned b3 = __funnelshift_r(r0[ws], r0[ws + 1], sh) & 7u;
-      const unsigned key = t3 | ((c3 & 1u) << 3) | ((c3 >> 2) << 4) | (b3 << 5);
-      const unsigned e = tb[key * 8u + dsel];
-      const unsigned i = e & 15u;
-      if (i == 8u) break;
-      dsel = lut[kLut1 + ((unsigned)min(step, 7) * 8u + dsel) * 8u + i];
-      step++;
-      tb = lut;
-      const int dr = (int)((e >> 4) & 3u) - 1, dc = (int)((e >> 6) & 3u) - 1;
-      p += dc;
-      cy += dr;
-      rb += dr * ws;
-      bm[rb + (p >> 5)] &= ~(1u << (p & 31));   // the new pixel is consumed
-    }
-    if (npts - start < c.length_threshold + 1) {
-      npts = start;  // chain too short: dropped (its pixels stay consumed)
-    } else {
-      const int k = atomicAdd(c.counters + 3, 1);
-      if (k < c.max_chains) {
-        c.chain_seed[k] = seed;
-        c.chain_off[k] = start;
-        c.chain_len[k] = npts - start;
-      }
-    }
-  }
-}
-
 // grid = (walkers, frame).  Phase 1: the CTA takes BIG components one at a time (all warps gather into the whole arena,
 // warp 0 walks).  Phase 2: every warp takes components of its own from the common queue (B then C) and works in its slice
-// of the arena; no block-wide synchronisation any more.
+// of the arena; no block-wide synchronisation any more.  The 8 CTAs per SM of the launch bounds hold the kernel to 64
+// registers without spills (up to 72 otherwise); its ~31 KB of shared memory allow 7 per SM anyway.
 template <class B>
-__global__ void __launch_bounds__(kWalkThreads)
-    k_fld_walk_cc(const __grid_constant__ B b, int w, int h, int length_threshold, int coop) {
+__global__ void __launch_bounds__(kWalkThreads, 8)
+    k_fld_walk_cc(const __grid_constant__ B b, int w, int h, int length_threshold) {
   const FldBuffers &fb = b.fld_of(blockIdx.y);
   WalkCtx c;
   c.edges = fb.edges;
@@ -822,10 +767,7 @@ __global__ void __launch_bounds__(kWalkThreads)
     __syncthreads();
     walk_gather(c, arena, root, y0, g0, groups, bh, ws, warp, kWalkWarps, lane);
     __syncthreads();
-    if (warp == 0) {
-      if (coop) walk_component(c, arena, lut_addr, root, y0, g0, groups, bh, ws, lane);
-      else if (lane == 0) walk_component_single(c, arena, lut, root, y0, g0, groups, bh, ws);
-    }
+    if (warp == 0) walk_component(c, arena, lut_addr, root, y0, g0, groups, bh, ws, lane);
   }
   // ---- phase 2
   unsigned *bm = arena + warp * kSliceWords;
@@ -842,8 +784,7 @@ __global__ void __launch_bounds__(kWalkThreads)
     __syncwarp();
     walk_gather(c, bm, root, y0, g0, groups, bh, ws, 0, 1, lane);
     __syncwarp();
-    if (coop) walk_component(c, bm, lut_addr, root, y0, g0, groups, bh, ws, lane);
-    else if (lane == 0) walk_component_single(c, bm, lut, root, y0, g0, groups, bh, ws);
+    walk_component(c, bm, lut_addr, root, y0, g0, groups, bh, ws, lane);
     __syncwarp();
   }
 }
@@ -1198,11 +1139,11 @@ void FldBuffers::release() {
 
 template <class B>
 static void launch_fld_any(const B &b, int nb_frames, int w, int h, int max_chains, int length_threshold, float distance_threshold,
-                           cudaStream_t s, cudaEvent_t *ev, bool tiles_done = false) {
+                           cudaStream_t s, cudaEvent_t *ev) {
   const int n = w * h;
   const int tpb = 256;
   const int lroot_cap = n / 4 + 1;
-  if (!tiles_done) {   // (the stream group's Canny launch has labelled the tiles already: launch_canny_table)
+  if constexpr (!kFusedLabels<B>) {
     PLVIWO_CARVEOUT(k_ccl_reset<B>);
     k_ccl_reset<B><<<nb_frames, 32, 0, s>>>(b);
     PLVIWO_CARVEOUT(k_ccl_tile<B>);
@@ -1253,11 +1194,7 @@ static void launch_fld_any(const B &b, int nb_frames, int w, int h, int max_chai
     k_fld_walk_thread<B><<<dim3(walk_t, nb_frames), kTLanes, 0, s>>>(b, w, h, length_threshold);
   }
   PLVIWO_CARVEOUT(k_fld_walk_cc<B>);
-  // PLVIWO_WALK_SINGLE=1: the single-lane step instead of the warp-cooperative one (25 lanes fetch the 5 x 5 window).  Same
-  // chains, same throughput in the 64-stream pipeline (55.3 k vs 55.4 k frames/s) and the same launch duration: the step is a
-  // chain of dependent shared-memory accesses either way.  The cooperative form is the one compute-sanitizer has seen.
-  static const int coop = [] { const char *e = std::getenv("PLVIWO_WALK_SINGLE"); return (e && std::atoi(e)) ? 0 : 1; }();
-  k_fld_walk_cc<B><<<dim3(walk_ctas, nb_frames), kWalkThreads, smem, s>>>(b, w, h, length_threshold, coop);
+  k_fld_walk_cc<B><<<dim3(walk_ctas, nb_frames), kWalkThreads, smem, s>>>(b, w, h, length_threshold);
   if (ev) cudaEventRecord(ev[1], s);
   PLVIWO_CARVEOUT(k_fld_order<B>);
   k_fld_order<B><<<dim3((max_chains + 127) / 128, nb_frames), 128, 0, s>>>(b);
@@ -1272,7 +1209,7 @@ void launch_fld_batch(const FldBatch &b, int length_threshold, float distance_th
 void launch_fld_table(const SlotRec *slots, const int *line_slots, int n_jobs, int w, int h, int max_chains, int length_threshold,
                       float distance_threshold, cudaStream_t s, cudaEvent_t *ev) {
   if (n_jobs <= 0) return;
-  launch_fld_any(FldTable{slots, line_slots}, n_jobs, w, h, max_chains, length_threshold, distance_threshold, s, ev, true);
+  launch_fld_any(FldTable{slots, line_slots}, n_jobs, w, h, max_chains, length_threshold, distance_threshold, s, ev);
 }
 
 void launch_fld(const DevImage &half, int length_threshold, float distance_threshold, FldBuffers &fb, cudaStream_t s,

@@ -566,12 +566,11 @@ def test_downsample_prestep(fe, synth, size, lines):
 
 
 @pytest.mark.parametrize("kw,lookahead", [(CFG2, 6), (CFG_KAIST, 3)])
-def test_speculative_tracking_equals_synchronous(fe, synth, kw, lookahead, monkeypatch):
-    """With frames queued ahead and PLVIWO_SPECULATION=1, LK(t -> t+1) is launched speculatively for every trackable
-    point before frame t's RANSAC gate (FeContext::speculate, track_candidates).  Rows, ids and line rows must be
-    IDENTICAL (bitwise) to feeding frame by frame, where nothing is speculated, over a sequence long enough to contain
-    detections, losses and occluders."""
-    monkeypatch.setenv("PLVIWO_SPECULATION", "1")
+def test_speculative_tracking_equals_synchronous(fe, synth, kw, lookahead):
+    """With frames queued ahead (lookahead >= 1), LK(t -> t+1) is launched speculatively for every trackable point
+    before frame t's RANSAC gate (FeContext::speculate, track_candidates).  Rows, ids and line rows must be IDENTICAL
+    (bitwise) to feeding frame by frame (lookahead 0), where nothing is speculated, over a sequence long enough to
+    contain detections, losses and occluders."""
     n = 40
     seq = synth.SynthSequence(seed=1015, n_frames=n)
     cfg = dict(width=1280, height=560, K=seq.K, D=seq.D, **kw)
