@@ -367,6 +367,9 @@ int plviwo_op_sort_corners(int device, const uint32_t *packed, int n, int nfg, u
 int plviwo_op_corner_subpix(int device, const uint8_t *img, int w, int h, float *pts /* in/out 2 per point */, int n);
 int plviwo_op_lk(int device, const uint8_t *img0, const uint8_t *img1, int w, int h, int win, int max_level,
                  const float *pts0, float *pts1 /* in: initial flow, out */, uint8_t *status, int n);
+/* The same tracking by the stream group's one-warp-per-feature kernel (win 15 and maxLevel <= 5 only): bit-identical results */
+int plviwo_op_lk_warp(int device, const uint8_t *img0, const uint8_t *img1, int w, int h, int win, int max_level,
+                      const float *pts0, float *pts1 /* in: initial flow, out */, uint8_t *status, int n);
 int plviwo_op_undistort(int device, const float *pts, int n, const double K[4], const double D[4], float *out);
 int plviwo_op_canny_half(int device, const uint8_t *img, int w, int h, float th, uint8_t *edges /* w*h bytes */);
 int plviwo_op_fld(int device, const uint8_t *img, int w, int h, int length_threshold, float distance_threshold,

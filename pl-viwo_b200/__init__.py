@@ -110,7 +110,7 @@ EXPORTS = [
     "plviwo_fe_feed_device", "plviwo_fe_submit", "plviwo_fe_collect", "plviwo_fe_play", "plviwo_fe_get_point_rows", "plviwo_fe_get_last_obs",
     "plviwo_fe_get_line_rows", "plviwo_fe_get_line_points", "plviwo_fe_get_line_samples", "plviwo_fe_get_state",
     "plviwo_fe_set_state", "plviwo_fe_enable_taps", "plviwo_fe_tap", "plviwo_fe_enable_timing", "plviwo_fe_get_stage_times",
-    "plviwo_op_equalize_pyramid", "plviwo_op_clahe", "plviwo_op_fast_cell", "plviwo_op_sort_corners", "plviwo_op_corner_subpix", "plviwo_op_lk", "plviwo_op_undistort",
+    "plviwo_op_equalize_pyramid", "plviwo_op_clahe", "plviwo_op_fast_cell", "plviwo_op_sort_corners", "plviwo_op_corner_subpix", "plviwo_op_lk", "plviwo_op_lk_warp", "plviwo_op_undistort",
     "plviwo_op_canny_half", "plviwo_op_fld", "plviwo_op_image_kernels_time", "plviwo_op_ransac_fundamental",
     "plviwo_fe_stereo_create", "plviwo_fe_stereo_destroy", "plviwo_fe_stereo_last_error", "plviwo_fe_stereo_set_calib",
     "plviwo_fe_stereo_set_num_features", "plviwo_fe_stereo_change_feat_id", "plviwo_fe_stereo_feed", "plviwo_fe_stereo_submit",
@@ -195,6 +195,7 @@ def lib() -> C.CDLL:
         L.plviwo_op_sort_corners.argtypes = [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]
         L.plviwo_op_lk.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_int]
+        L.plviwo_op_lk_warp.argtypes = L.plviwo_op_lk.argtypes
         L.plviwo_op_undistort.argtypes = [C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_void_p]
         L.plviwo_op_canny_half.argtypes = [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_void_p]
         L.plviwo_op_fld.argtypes = [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_void_p, C.c_int,
@@ -1041,14 +1042,19 @@ def op_corner_subpix(img: np.ndarray, pts: np.ndarray, device: int = 0) -> np.nd
     return p
 
 
-def op_lk(img0, img1, pts0, pts1_init, win: int = 15, max_level: int = 5, device: int = 0):
+def op_lk(img0, img1, pts0, pts1_init, win: int = 15, max_level: int = 5, device: int = 0, form: str = "cta"):
+    """calcOpticalFlowPyrLK with an initial flow.  form "cta": the single-handle kernels (k_lk15 for win 15); "warp": the
+    stream group's one-warp-per-feature kernel (win 15, max_level <= 5), which gives the same results bit for bit."""
+    if form not in ("cta", "warp"):
+        raise ValueError("form must be 'cta' or 'warp', not %r" % (form,))
     img0 = np.ascontiguousarray(img0, np.uint8)
     img1 = np.ascontiguousarray(img1, np.uint8)
     p0 = np.ascontiguousarray(pts0, np.float32).reshape(-1, 2)
     p1 = np.ascontiguousarray(pts1_init, np.float32).reshape(-1, 2).copy()
     st = np.zeros((len(p0),), np.uint8)
-    _check(lib().plviwo_op_lk(device, img0.ctypes.data, img1.ctypes.data, img0.shape[1], img0.shape[0], win, max_level,
-                              p0.ctypes.data, p1.ctypes.data, st.ctypes.data, len(p0)))
+    fn = lib().plviwo_op_lk if form == "cta" else lib().plviwo_op_lk_warp
+    _check(fn(device, img0.ctypes.data, img1.ctypes.data, img0.shape[1], img0.shape[0], win, max_level,
+              p0.ctypes.data, p1.ctypes.data, st.ctypes.data, len(p0)))
     return p1, st
 
 

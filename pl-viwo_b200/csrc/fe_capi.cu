@@ -511,8 +511,8 @@ int plviwo_op_corner_subpix(int device, const uint8_t *img, int w, int h, float 
   API_END
 }
 
-int plviwo_op_lk(int device, const uint8_t *img0, const uint8_t *img1, int w, int h, int win, int max_level,
-                 const float *pts0, float *pts1, uint8_t *status, int n) {
+static int op_lk(int device, const uint8_t *img0, const uint8_t *img1, int w, int h, int win, int max_level, const float *pts0,
+                 float *pts1, uint8_t *status, int n, bool warp) {
   API_BEGIN
   if (!img0 || !img1 || !pts0 || !pts1 || !status || n < 0 || win < 3 || win > kMaxWin || !(win & 1) || max_level < 0 ||
       max_level >= kMaxLevels)
@@ -537,12 +537,23 @@ int plviwo_op_lk(int device, const uint8_t *img0, const uint8_t *img1, int w, in
   prm.min_eig = 1e-4f;
   prm.undistort = 0;
   for (int i = 0; i < 4; i++) prm.K[i] = prm.D[i] = 0;
-  launch_lk(p0.pyr, p1.pyr, d0.p, d1.p, ds.p, dn0.p, dn1.p, n, prm, 0);
+  if (!warp) launch_lk(p0.pyr, p1.pyr, d0.p, d1.p, ds.p, dn0.p, dn1.p, n, prm, 0);
+  else if (!launch_lk_warp(p0.pyr, p1.pyr, d0.p, d1.p, ds.p, n, prm, 0)) return FE_BAD_ARG;
   OP_CUDA(cudaDeviceSynchronize());
   OP_CUDA(cudaMemcpy(pts1, d1.p, (size_t)n * sizeof(float2), cudaMemcpyDeviceToHost));
   OP_CUDA(cudaMemcpy(status, ds.p, (size_t)n, cudaMemcpyDeviceToHost));
   return FE_OK;
   API_END
+}
+
+int plviwo_op_lk(int device, const uint8_t *img0, const uint8_t *img1, int w, int h, int win, int max_level,
+                 const float *pts0, float *pts1, uint8_t *status, int n) {
+  return op_lk(device, img0, img1, w, h, win, max_level, pts0, pts1, status, n, false);
+}
+
+int plviwo_op_lk_warp(int device, const uint8_t *img0, const uint8_t *img1, int w, int h, int win, int max_level,
+                      const float *pts0, float *pts1, uint8_t *status, int n) {
+  return op_lk(device, img0, img1, w, h, win, max_level, pts0, pts1, status, n, true);
 }
 
 int plviwo_op_undistort(int device, const float *pts, int n, const double K[4], const double D[4], float *out) {

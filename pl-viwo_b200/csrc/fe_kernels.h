@@ -129,6 +129,10 @@ bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, f
 // belongs to cell i / tab_stride, live iff i % tab_stride < d_tab_cnt[cell]); flow_is_zero: the initial guess is the
 // previous position, d_pts1 is written only; cell_mask (8 words, optional): only cells whose bit is set are tracked.
 bool lk_table_mode_ok(const LkParams &prm, int pyramid_images);
+// k_lk15w_g's one-warp-per-feature body on n points over one pyramid pair (15 x 15 window, <= 6 pyramid images, no
+// undistortion; false otherwise): the same results as launch_lk's k_lk15, bit for bit
+bool launch_lk_warp(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status, int n,
+                    const LkParams &prm, cudaStream_t s);
 void launch_undistort(const float2 *d_pts, float2 *d_out, int n, const double K[4], const double D[4], cudaStream_t s);
 
 // ---- lines (kernels_lines.cu) -------------------------------------------------------------------------------

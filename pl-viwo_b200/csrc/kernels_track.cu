@@ -746,9 +746,10 @@ __global__ void __launch_bounds__(kLk15MaxLevels * 32)
 // compares a group, which runs this kernel, with single handles, which run k_lk15).  An SM holds 32+ features.
 constexpr int kLkwWarps = 4;
 // Staged rows of the previous image (18 x 18 pixels) and of the region of the next image (25 x 25) are kept with a row
-// stride that is a multiple of 4 bytes and their first word aligned like the image's: a neighbourhood that lies inside the
-// image is staged with 32-bit loads (4 + 6 per lane instead of 11 + 20 single bytes with reflected indices); the bytes
-// that end up in shared memory are the same either way.
+// stride that is a multiple of 4 bytes and their first word aligned like the image's (it holds the region's first column,
+// x0 & 3 bytes in).  Rows are reflected through their row pointer; a word that lies inside the image row is one 32-bit
+// load, and only the words that cross or lie beyond its left or right edge are assembled from REFLECT_101 columns byte by
+// byte.  Interior and border neighbourhoods take the same path, and the bytes in shared memory are the reference's.
 constexpr int kRawStride = 24;   // >= 18 + 3
 constexpr int kJStride = 28;     // >= 25 + 3
 // One buffer per warp, used three ways in turn (each hand-over is separated by a __syncwarp): the staged rows of the previous
@@ -764,12 +765,54 @@ struct LkwSmem {
   __align__(16) uint8_t buf[kLkwBytes];
 };
 
+// kRows staged rows of kStride bytes: image rows y0.., columns from the word that holds column x0 (see above).  `aligned`:
+// the image pointer and pitch are multiples of 4 (group pyramids are 256-byte aligned); otherwise every word is assembled
+// byte by byte.
+template <int kRows, int kStride>
+__device__ __forceinline__ void lkw_stage(uint8_t *dst, const uint8_t *__restrict__ img, int pitch, int cols, int rows, int x0,
+                                          int y0, bool aligned, int lane) {
+  constexpr int kW = kStride / 4, kN = kRows * kW, kL = (kN + 31) / 32;
+  const int xw = x0 & ~3;
+  unsigned v[kL];
+#pragma unroll
+  for (int j = 0; j < kL; j++) {
+    const int i = lane + 32 * j;
+    v[j] = 0;
+    if (i < kN) {
+      const int r = i / kW, x = xw + 4 * (i - r * kW);
+      const uint8_t *row = img + (size_t)reflect101(y0 + r, rows) * pitch;
+      if (aligned && x >= 0 && x + 4 <= cols) {
+        v[j] = __ldg(reinterpret_cast<const unsigned *>(row + x));
+      } else {
+#pragma unroll
+        for (int k = 0; k < 4; k++) v[j] |= (unsigned)__ldg(row + reflect101(x + k, cols)) << (8 * k);
+      }
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < kL; j++)
+    if (lane + 32 * j < kN) reinterpret_cast<unsigned *>(dst)[lane + 32 * j] = v[j];
+}
+
+// Bilinear taps as 2-way dot products: w holds two signed 16-bit weights, px four unsigned 8-bit pixels, of which the low
+// (dp2a_lo) or high (dp2a_hi) pair is used: c + w.h0 * px.b0 + w.h1 * px.b1.  Exact in int32 (|weight| <= 16384).
+__device__ __forceinline__ int dp2a_lo(int w, unsigned px, int c) {
+  int d;
+  asm("dp2a.lo.s32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(w), "r"(px), "r"(c));
+  return d;
+}
+__device__ __forceinline__ int dp2a_hi(int w, unsigned px, int c) {
+  int d;
+  asm("dp2a.hi.s32.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(w), "r"(px), "r"(c));
+  return d;
+}
+__device__ __forceinline__ int pack_w16(int lo, int hi) { return (int)(((unsigned)lo & 0xffffu) | ((unsigned)hi << 16)); }
+
 template <class Args>
 __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restrict__ pts0, float2 *__restrict__ pts1,
                                            uint8_t *__restrict__ status, float2 *__restrict__ p0n, float2 *__restrict__ p1n, int pi,
                                            LkwSmem &sm) {
   constexpr int win = kW15, np = win + 3, nd = win + 1;
-  constexpr int kRawLoads = (np * np + 31) / 32;   // 11
   const int lane = threadIdx.x & 31;
   const int r0 = (lane >> 2) * 2, c0 = (lane & 3) * 4;   // set-up: this lane's 2 x 4 block of window pixels
   const int wy = lane >> 1, wx = (lane & 1) * 8;         // chain: this lane's row and its 8 adjacent pixels
@@ -790,7 +833,8 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
       next.x = next.x * 2.f;
       next.y = next.y * 2.f;
     }
-    // ---- set-up of this level (k_lk15's, verbatim): raw neighbourhood, Scharr derivatives, fixed-point patches, A
+    // ---- set-up of this level (k_lk15's integers and float sums): raw neighbourhood, Scharr derivatives, fixed-point
+    // patches, A
     const float px = prev_in.x * lscale - half, py = prev_in.y * lscale - half;
     const int ipx = __float2int_rd(px), ipy = __float2int_rd(py);
     const bool in_range = !(ipx < -win || ipx >= cols || ipy < -win || ipy >= rows);
@@ -802,71 +846,31 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
     __syncwarp();   // the previous level's patches have been read by every lane
     {
       uint8_t *const raw_s = sm.buf;
-      const uint8_t *raw = raw_s;
       short *ddx = reinterpret_cast<short *>(sm.buf + kLkwDdxOff), *ddy = reinterpret_cast<short *>(sm.buf + kLkwDdyOff);
-      bool interior = false;
-      int roff_b = 0;
-      {
-        const uint8_t *I = a.p0[level];
-        const int pitchI = a.pitch0[level];
-        const int rx0 = ipx - 1, ry0 = ipy - 1;
-        if (rx0 >= 0 && ry0 >= 0 && rx0 + np <= cols && ry0 + np <= rows && ((((size_t)I) | (size_t)pitchI) & 3) == 0) {
-          // inside the image: 18 rows x 6 aligned words (the staged row starts at the word that holds column rx0)
-          const int roff = rx0 & 3;
-          const uint8_t *base = I + (size_t)ry0 * pitchI + (rx0 - roff);
-          constexpr int kWords = np * (kRawStride / 4);   // 108
-          unsigned v[(kWords + 31) / 32];
-#pragma unroll
-          for (int j = 0; j < (kWords + 31) / 32; j++) {
-            const int i = lane + 32 * j;
-            v[j] = 0;
-            if (i < kWords) {
-              const int r = i / (kRawStride / 4), c = i - r * (kRawStride / 4);
-              v[j] = __ldg(reinterpret_cast<const unsigned *>(base + (size_t)r * pitchI) + c);
-            }
-          }
-#pragma unroll
-          for (int j = 0; j < (kWords + 31) / 32; j++)
-            if (lane + 32 * j < kWords) reinterpret_cast<unsigned *>(raw_s)[lane + 32 * j] = v[j];
-          raw = raw_s + roff;
-          interior = true;
-          roff_b = 8 * roff;
-        } else {
-          uint8_t v[kRawLoads];
-#pragma unroll
-          for (int j = 0; j < kRawLoads; j++) {
-            const int i = lane + 32 * j;
-            v[j] = 0;
-            if (i < np * np) {
-              const int r = i / np, c = i - r * np;
-              v[j] = I[(size_t)reflect101(ry0 + r, rows) * pitchI + reflect101(rx0 + c, cols)];
-            }
-          }
-#pragma unroll
-          for (int j = 0; j < kRawLoads; j++) {
-            const int i = lane + 32 * j;
-            if (i < np * np) raw_s[(i / np) * kRawStride + (i % np)] = v[j];
-          }
-        }
-      }
+      // raw neighbourhood, origin (ipx - 1, ipy - 1): 18 rows x 6 words, column ipx - 1 at byte roff of each row
+      const uint8_t *I = a.p0[level];
+      const int pitchI = a.pitch0[level];
+      const int roff = (ipx - 1) & 3;
+      lkw_stage<np, kRawStride>(raw_s, I, pitchI, cols, rows, ipx - 1, ipy - 1, ((((size_t)I) | (size_t)pitchI) & 3) == 0, lane);
       const float fa = px - ipx, fb = py - ipy;
       const int iw00 = __float2int_rn((1.f - fa) * (1.f - fb) * 16384.f);
       const int iw01 = __float2int_rn(fa * (1.f - fb) * 16384.f);
       const int iw10 = __float2int_rn((1.f - fa) * fb * 16384.f);
       const int iw11 = 16384 - iw00 - iw01 - iw10;
       __syncwarp();
-      if (interior) {
-        // Scharr derivatives of the 16 x 16 positions, all inside the image: this lane's row r and 8 adjacent columns from
-        // three staged rows of 10 pixels, each taken as four aligned words and shifted into place
+      {
+        // Scharr derivatives of the 16 x 16 positions (ipx + c, ipy + r): this lane's row r and 8 adjacent columns from
+        // three staged rows of 10 pixels, each taken as four aligned words and shifted into place; zero outside the frame,
+        // which is what the reference's zero-padded derivative planes hold
         const int r = lane >> 1, cb = (lane & 1) * 8;
         unsigned X[3][3];
 #pragma unroll
         for (int k = 0; k < 3; k++) {
           const uint2 *rp = reinterpret_cast<const uint2 *>(raw_s + (r + k) * kRawStride + cb);   // 8-byte aligned (stride 24)
           const uint2 wa = rp[0], wb = rp[1];
-          X[k][0] = __funnelshift_r(wa.x, wa.y, roff_b);
-          X[k][1] = __funnelshift_r(wa.y, wb.x, roff_b);
-          X[k][2] = __funnelshift_r(wb.x, wb.y, roff_b);
+          X[k][0] = __funnelshift_r(wa.x, wa.y, 8 * roff);
+          X[k][1] = __funnelshift_r(wa.y, wb.x, 8 * roff);
+          X[k][2] = __funnelshift_r(wb.x, wb.y, 8 * roff);
         }
         int S[10], Dv[10];   // column smoothing 3 t + 10 m + 3 b and column difference b - t
 #pragma unroll
@@ -876,51 +880,72 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
           S[c] = 3 * (t + bb) + 10 * m;
           Dv[c] = bb - t;
         }
-        unsigned px[4], py[4];
+        const int gy = ipy + r, gx = ipx + cb;
+        const bool inside = gy >= 0 && gy < rows && gx >= 0 && gx + 8 <= cols;
+        unsigned qx[4], qy[4];
 #pragma unroll
         for (int c = 0; c < 8; c += 2) {
-          const int vx0 = S[c + 2] - S[c], vx1 = S[c + 3] - S[c + 1];
-          const int vy0 = 3 * (Dv[c] + Dv[c + 2]) + 10 * Dv[c + 1], vy1 = 3 * (Dv[c + 1] + Dv[c + 3]) + 10 * Dv[c + 2];
-          px[c >> 1] = ((unsigned)vx0 & 0xffffu) | ((unsigned)vx1 << 16);
-          py[c >> 1] = ((unsigned)vy0 & 0xffffu) | ((unsigned)vy1 << 16);
+          int vx0 = S[c + 2] - S[c], vx1 = S[c + 3] - S[c + 1];
+          int vy0 = 3 * (Dv[c] + Dv[c + 2]) + 10 * Dv[c + 1], vy1 = 3 * (Dv[c + 1] + Dv[c + 3]) + 10 * Dv[c + 2];
+          if (!inside) {
+            const bool row_in = gy >= 0 && gy < rows;
+            if (!(row_in && (unsigned)(gx + c) < (unsigned)cols)) vx0 = vy0 = 0;
+            if (!(row_in && (unsigned)(gx + c + 1) < (unsigned)cols)) vx1 = vy1 = 0;
+          }
+          qx[c >> 1] = ((unsigned)vx0 & 0xffffu) | ((unsigned)vx1 << 16);
+          qy[c >> 1] = ((unsigned)vy0 & 0xffffu) | ((unsigned)vy1 << 16);
         }
-        *reinterpret_cast<uint4 *>(&ddx[r * nd + cb]) = make_uint4(px[0], px[1], px[2], px[3]);
-        *reinterpret_cast<uint4 *>(&ddy[r * nd + cb]) = make_uint4(py[0], py[1], py[2], py[3]);
-      } else
-      for (int i = lane; i < nd * nd; i += 32) {
-        int r = i / nd, c = i - r * nd;
-        int gx = ipx + c, gy = ipy + r;
-        int vx = 0, vy = 0;
-        if (gx >= 0 && gx < cols && gy >= 0 && gy < rows) {
-          const uint8_t *q = raw + (r + 1) * kRawStride + (c + 1);
-          int tl = q[-kRawStride - 1], tc = q[-kRawStride], tr = q[-kRawStride + 1];
-          int ml = q[-1], mr = q[1];
-          int bl = q[kRawStride - 1], bc = q[kRawStride], br = q[kRawStride + 1];
-          vx = 3 * (tr + br) + 10 * mr - 3 * (tl + bl) - 10 * ml;
-          vy = 3 * (bl + br) + 10 * bc - 3 * (tl + tr) - 10 * tc;
-        }
-        ddx[i] = (short)vx;
-        ddy[i] = (short)vy;
+        *reinterpret_cast<uint4 *>(&ddx[r * nd + cb]) = make_uint4(qx[0], qx[1], qx[2], qx[3]);
+        *reinterpret_cast<uint4 *>(&ddy[r * nd + cb]) = make_uint4(qy[0], qy[1], qy[2], qy[3]);
       }
       __syncwarp();
       short pv[3][8];   // this lane's 2 x 4 block of I, Ix, Iy: stored once every lane is done with the rows and planes
+      {
+        // bilinear taps of I: staged rows r0 + 1 .. r0 + 3 from column c0 + 1 on, P = bytes 0..3 and Q = bytes 1..4 of it
+        const int wI0 = pack_w16(iw00, iw01), wI1 = pack_w16(iw10, iw11);
+        const int off = roff + c0 + 1;
+        unsigned P[3], Q[3];
 #pragma unroll
-      for (int k = 0; k < 8; k++) {
-        const int y = r0 + (k >> 2), x = c0 + (k & 3);
-        int ival = 0, ixval = 0, iyval = 0;
-        if (y < win && x < win) {
-          const uint8_t *q = raw + (y + 1) * kRawStride + (x + 1);
-          ival = (q[0] * iw00 + q[1] * iw01 + q[kRawStride] * iw10 + q[kRawStride + 1] * iw11 + (1 << 8)) >> 9;
-          const int di = y * nd + x;
-          ixval = (ddx[di] * iw00 + ddx[di + 1] * iw01 + ddx[di + nd] * iw10 + ddx[di + nd + 1] * iw11 + (1 << 13)) >> 14;
-          iyval = (ddy[di] * iw00 + ddy[di + 1] * iw01 + ddy[di + nd] * iw10 + ddy[di + nd + 1] * iw11 + (1 << 13)) >> 14;
+        for (int k = 0; k < 3; k++) {
+          const unsigned *rp = reinterpret_cast<const unsigned *>(raw_s + (r0 + 1 + k) * kRawStride) + (off >> 2);
+          const unsigned w0 = rp[0], w1 = rp[1];
+          P[k] = __funnelshift_r(w0, w1, 8 * (off & 3));
+          Q[k] = __funnelshift_rc(w0, w1, 8 * (off & 3) + 8);   // clamped: a shift of 32 yields w1
         }
-        pv[0][k] = (short)ival;
-        pv[1][k] = (short)ixval;
-        pv[2][k] = (short)iyval;
-        A11 += (float)(ixval * ixval);
-        A12 += (float)(ixval * iyval);
-        A22 += (float)(iyval * iyval);
+        // derivative rows r0 .. r0 + 2 (clamped to the plane), columns c0 .. c0 + 4, read as int16 pairs
+        int dx[3][5], dy[3][5];
+#pragma unroll
+        for (int k = 0; k < 3; k++) {
+          const int rr = min(r0 + k, nd - 1);
+          const uint2 xa = *reinterpret_cast<const uint2 *>(&ddx[rr * nd + c0]);
+          const uint2 ya = *reinterpret_cast<const uint2 *>(&ddy[rr * nd + c0]);
+          const unsigned xe = *reinterpret_cast<const unsigned *>(&ddx[rr * nd + min(c0 + 4, nd - 2)]);
+          const unsigned ye = *reinterpret_cast<const unsigned *>(&ddy[rr * nd + min(c0 + 4, nd - 2)]);
+          dx[k][0] = (short)(xa.x & 0xffffu); dx[k][1] = (int)xa.x >> 16;
+          dx[k][2] = (short)(xa.y & 0xffffu); dx[k][3] = (int)xa.y >> 16;
+          dx[k][4] = (short)(xe & 0xffffu);
+          dy[k][0] = (short)(ya.x & 0xffffu); dy[k][1] = (int)ya.x >> 16;
+          dy[k][2] = (short)(ya.y & 0xffffu); dy[k][3] = (int)ya.y >> 16;
+          dy[k][4] = (short)(ye & 0xffffu);
+        }
+#pragma unroll
+        for (int k = 0; k < 8; k++) {
+          const int t = k >> 2, m = k & 3;
+          const int y = r0 + t, x = c0 + m;
+          int ival = 0, ixval = 0, iyval = 0;
+          if (y < win && x < win) {
+            const unsigned top = (m & 1) ? Q[t] : P[t], bot = (m & 1) ? Q[t + 1] : P[t + 1];
+            ival = ((m & 2) ? dp2a_hi(wI0, top, dp2a_hi(wI1, bot, 1 << 8)) : dp2a_lo(wI0, top, dp2a_lo(wI1, bot, 1 << 8))) >> 9;
+            ixval = (dx[t][m] * iw00 + dx[t][m + 1] * iw01 + dx[t + 1][m] * iw10 + dx[t + 1][m + 1] * iw11 + (1 << 13)) >> 14;
+            iyval = (dy[t][m] * iw00 + dy[t][m + 1] * iw01 + dy[t + 1][m] * iw10 + dy[t + 1][m + 1] * iw11 + (1 << 13)) >> 14;
+          }
+          pv[0][k] = (short)ival;
+          pv[1][k] = (short)ixval;
+          pv[2][k] = (short)iyval;
+          A11 += (float)(ixval * ixval);
+          A12 += (float)(ixval * iyval);
+          A22 += (float)(iyval * iyval);
+        }
       }
       __syncwarp();   // the patches take the place of the rows and planes they were computed from
       {
@@ -949,8 +974,9 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
       continue;
     }
     Dt = 1.f / Dt;
-    // ---- this lane's 8 window pixels: I, Ix, Iy (int16 pairs, one 16-byte load per patch)
-    int Iw[8], Ix[8], Iy[8];
+    // ---- this lane's 8 window pixels: Ix, Iy (int16 pairs, one 16-byte load per patch) and the constant part of the
+    // mismatch sums, ci1 = sum I * Ix and ci2 = sum I * Iy
+    int Ix[8], Iy[8], ci1 = 0, ci2 = 0;
     {
       uint4 q0 = make_uint4(0, 0, 0, 0), q1 = q0, q2 = q0;
       if (own) {
@@ -962,12 +988,13 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
       const unsigned w0[4] = {q0.x, q0.y, q0.z, q0.w}, w1[4] = {q1.x, q1.y, q1.z, q1.w}, w2[4] = {q2.x, q2.y, q2.z, q2.w};
 #pragma unroll
       for (int k = 0; k < 4; k++) {
-        Iw[2 * k] = (short)(w0[k] & 0xffffu);
-        Iw[2 * k + 1] = (short)(w0[k] >> 16);
         Ix[2 * k] = (short)(w1[k] & 0xffffu);
         Ix[2 * k + 1] = (short)(w1[k] >> 16);
         Iy[2 * k] = (short)(w2[k] & 0xffffu);
         Iy[2 * k + 1] = (short)(w2[k] >> 16);
+        const int i0 = (short)(w0[k] & 0xffffu), i1 = (short)(w0[k] >> 16);
+        ci1 += i0 * Ix[2 * k] + i1 * Ix[2 * k + 1];
+        ci2 += i0 * Iy[2 * k] + i1 * Iy[2 * k + 1];
       }
     }
     float2 result = next;   // nextPts[ptidx] as stored by OpenCV; only rewritten after an update step
@@ -976,12 +1003,11 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
     float2 prevDelta = make_float2(0.f, 0.f);
     const uint8_t *J = a.p1[level];
     const int pitchJ = a.pitch1[level];
-    int jt[9], jb[9];   // the 2 x 9 block of the next image under this lane's pixels
-#pragma unroll
-    for (int k = 0; k < 9; k++) jt[k] = jb[k] = 0;
+    const bool alignedJ = ((((size_t)J) | (size_t)pitchJ) & 3) == 0;
+    // the 2 x 9 block of the next image under this lane's pixels, byte-packed: per row, columns 0..3, 1..4, 4..7, 5..8
+    unsigned jt[4] = {0, 0, 0, 0}, jb[4] = {0, 0, 0, 0};
     int cached_x = INT_MIN, cached_y = INT_MIN;
     int reg_x0 = INT_MIN / 2, reg_y0 = INT_MIN / 2;   // origin of the staged region (none yet)
-    int joff = 0;                                     // byte offset of the region's first column inside its staged rows
     for (int j = 0; j < a.max_count; j++) {
       const int inx = __float2int_rd(next.x), iny = __float2int_rd(next.y);
       if (inx < -win || inx >= cols || iny < -win || iny >= rows) {
@@ -1001,65 +1027,40 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
           reg_x0 = inx - kJMargin;
           reg_y0 = iny - kJMargin;
           __syncwarp();   // every lane is done reading the old region
-          if (reg_x0 >= 0 && reg_y0 >= 0 && reg_x0 + kJR <= cols && reg_y0 + kJR <= rows && ((((size_t)J) | (size_t)pitchJ) & 3) == 0) {
-            // inside the image: 25 rows x 7 aligned words
-            joff = reg_x0 & 3;
-            const uint8_t *base = J + (size_t)reg_y0 * pitchJ + (reg_x0 - joff);
-            constexpr int kWords = kJR * (kJStride / 4);   // 175
-            unsigned t[(kWords + 31) / 32];
-#pragma unroll
-            for (int q = 0; q < (kWords + 31) / 32; q++) {
-              const int i = lane + 32 * q;
-              t[q] = 0;
-              if (i < kWords) {
-                const int ry = i / (kJStride / 4), cw = i - ry * (kJStride / 4);
-                t[q] = __ldg(reinterpret_cast<const unsigned *>(base + (size_t)ry * pitchJ) + cw);
-              }
-            }
-#pragma unroll
-            for (int q = 0; q < (kWords + 31) / 32; q++)
-              if (lane + 32 * q < kWords) reinterpret_cast<unsigned *>(sm.buf)[lane + 32 * q] = t[q];
-          } else {
-            joff = 0;
-            constexpr int kJLoads = (kJR * kJR + 31) / 32;   // 20, in two rounds of 10 loads in flight
-#pragma unroll 1
-            for (int q0 = 0; q0 < kJLoads; q0 += kJLoads / 2) {
-              uint8_t t[kJLoads / 2];
-#pragma unroll
-              for (int q = 0; q < kJLoads / 2; q++) {
-                const int i = lane + 32 * (q0 + q);
-                const int ry = i / kJR, rx = i - ry * kJR;
-                t[q] = 0;
-                if (i < kJR * kJR) t[q] = J[(size_t)reflect101(reg_y0 + ry, rows) * pitchJ + reflect101(reg_x0 + rx, cols)];
-              }
-#pragma unroll
-              for (int q = 0; q < kJLoads / 2; q++) {
-                const int i = lane + 32 * (q0 + q);
-                if (i < kJR * kJR) sm.buf[(i / kJR) * kJStride + (i % kJR)] = t[q];
-              }
-            }
-          }
+          lkw_stage<kJR, kJStride>(sm.buf, J, pitchJ, cols, rows, reg_x0, reg_y0, alignedJ, lane);
           __syncwarp();
         }
         if (own) {
-          const uint8_t *Jp = sm.buf + (iny - reg_y0 + wy) * kJStride + (inx - reg_x0 + joff + wx);
-#pragma unroll
-          for (int k = 0; k < 9; k++) {
-            jt[k] = Jp[k];
-            jb[k] = Jp[kJStride + k];
-          }
+          const int o = inx - reg_x0 + (reg_x0 & 3) + wx;   // byte of this lane's first pixel in its staged row
+          const unsigned *rp = reinterpret_cast<const unsigned *>(sm.buf + (iny - reg_y0 + wy) * kJStride) + (o >> 2);
+          const int sh = 8 * (o & 3);
+          unsigned w0 = rp[0], w1 = rp[1], w2 = rp[2];
+          jt[0] = __funnelshift_r(w0, w1, sh);
+          jt[1] = __funnelshift_rc(w0, w1, sh + 8);   // clamped: a shift of 32 yields w1
+          jt[2] = __funnelshift_r(w1, w2, sh);
+          jt[3] = __funnelshift_rc(w1, w2, sh + 8);
+          w0 = rp[kJStride / 4];
+          w1 = rp[kJStride / 4 + 1];
+          w2 = rp[kJStride / 4 + 2];
+          jb[0] = __funnelshift_r(w0, w1, sh);
+          jb[1] = __funnelshift_rc(w0, w1, sh + 8);
+          jb[2] = __funnelshift_r(w1, w2, sh);
+          jb[3] = __funnelshift_rc(w1, w2, sh + 8);
         }
       }
-      // mismatch vector: exact integer sums (the pixels a lane does not own have I = Ix = Iy = 0 and contribute 0)
-      // |jv - Iw| <= 255 * 32 and |Ix|, |Iy| <= 16 * 255 (Scharr of 8-bit pixels, bilinear weights summing to 1), so a
-      // lane's eight products stay below 2^29: 32-bit per lane, the warp total through 16-bit halves as in k_lk15
-      int s1 = 0, s2 = 0;
+      // mismatch vector b = sum (J - I) * (Ix, Iy) = sum J * (Ix, Iy) - (ci1, ci2), in exact integers (the pixels a lane
+      // does not own have Ix = Iy = 0 and I = 0).  Bounds: the four bilinear weights sum to 16384 and none is below -2,
+      // so |J|, |I| <= 8161 and |Ix|, |Iy| <= 16 * 255 = 4080 (Scharr of 8-bit pixels); every product is below 2^25, a
+      // lane's eight-term sums below 2^28 and their difference below 2^29: 32-bit per lane, the warp total through 16-bit
+      // halves as in k_lk15
+      const int wJ0 = pack_w16(jw00, jw01), wJ1 = pack_w16(jw10, jw11);
+      int s1 = -ci1, s2 = -ci2;
 #pragma unroll
       for (int k = 0; k < 8; k++) {
-        const int jv = (jt[k] * jw00 + jt[k + 1] * jw01 + jb[k] * jw10 + jb[k + 1] * jw11 + (1 << 8)) >> 9;
-        const int dv = jv - Iw[k];   // lanes without pixels hold I = Ix = Iy = 0 and J = 0: dv = 0
-        s1 += dv * Ix[k];
-        s2 += dv * Iy[k];
+        const int q = ((k >> 2) << 1) | (k & 1);   // pixel k's pair (k, k + 1): low or high half of jt[q] / jb[q]
+        const int jv = ((k & 2) ? dp2a_hi(wJ0, jt[q], dp2a_hi(wJ1, jb[q], 1 << 8)) : dp2a_lo(wJ0, jt[q], dp2a_lo(wJ1, jb[q], 1 << 8))) >> 9;
+        s1 += jv * Ix[k];
+        s2 += jv * Iy[k];
       }
       const long long t1 = ((long long)__reduce_add_sync(0xffffffffu, s1 >> 16) << 16) + (long long)__reduce_add_sync(0xffffffffu, s1 & 0xffff);
       const long long t2 = ((long long)__reduce_add_sync(0xffffffffu, s2 >> 16) << 16) + (long long)__reduce_add_sync(0xffffffffu, s2 & 0xffff);
@@ -1180,10 +1181,7 @@ bool lk_table_mode_ok(const LkParams &prm, int pyramid_images) {
   return prm.win == kW15 && std::min(prm.max_level + 1, pyramid_images) <= kLk15MaxLevels;
 }
 
-bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status,
-               float2 *d_p0n, float2 *d_p1n, int n, const LkParams &prm, cudaStream_t s, int *host_flag, int flag_value,
-               unsigned *d_done_counter, const int *d_tab_cnt, int tab_stride, bool flow_is_zero, const unsigned *cell_mask) {
-  if (n <= 0) return false;
+static LkArgs lk_args(const Pyramid &prev, const Pyramid &next, const LkParams &prm, bool flow_is_zero, const unsigned *cell_mask) {
   LkArgs a;
   int levels = prm.max_level + 1;
   if (levels > prev.n) levels = prev.n;
@@ -1204,6 +1202,15 @@ bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, f
   a.flow_is_zero = flow_is_zero ? 1 : 0;
   for (int i = 0; i < 8; i++) a.cell_mask[i] = cell_mask ? cell_mask[i] : 0xffffffffu;
   for (int i = 0; i < 4; i++) { a.calib.K[i] = prm.K[i]; a.calib.D[i] = prm.D[i]; }
+  return a;
+}
+
+bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status,
+               float2 *d_p0n, float2 *d_p1n, int n, const LkParams &prm, cudaStream_t s, int *host_flag, int flag_value,
+               unsigned *d_done_counter, const int *d_tab_cnt, int tab_stride, bool flow_is_zero, const unsigned *cell_mask) {
+  if (n <= 0) return false;
+  const LkArgs a = lk_args(prev, next, prm, flow_is_zero, cell_mask);
+  const int levels = a.max_level + 1;
   if (prm.win == kW15 && levels <= kLk15MaxLevels) {   // one CTA per feature, one warp per level
     PLVIWO_CARVEOUT(k_lk15);
     k_lk15<<<n, std::max(levels, kChainWarps) * 32, 0, s>>>(a, d_pts0, d_pts1, d_status, d_p0n, d_p1n, n, host_flag, flag_value, d_done_counter,
@@ -1219,6 +1226,28 @@ bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, f
   PLVIWO_CARVEOUT(k_lk);
   k_lk<<<(n + kLkWarps - 1) / kLkWarps, kLkWarps * 32, smem, s>>>(a, d_pts0, d_pts1, d_status, d_p0n, d_p1n, n);
   return false;
+}
+
+
+// k_lk15w_g's per-feature body (one warp per feature) on arbitrary points over one image pair: lets tests reach the border
+// paths of the group kernel with points a tracker would not produce
+__global__ void __launch_bounds__(kLkwWarps * 32, 5)
+    k_lk15w(const __grid_constant__ LkArgs a, const float2 *__restrict__ pts0, float2 *__restrict__ pts1,
+            uint8_t *__restrict__ status, int n) {
+  __shared__ LkwSmem sm[kLkwWarps];
+  const int pi = blockIdx.x * kLkwWarps + (threadIdx.x >> 5);
+  if (pi >= n) return;
+  lk15w_body(a, pts0, pts1, status, nullptr, nullptr, pi, sm[threadIdx.x >> 5]);
+}
+
+bool launch_lk_warp(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status, int n,
+                    const LkParams &prm, cudaStream_t s) {
+  if (prm.win != kW15 || std::min(prm.max_level + 1, prev.n) > kLk15MaxLevels || prm.undistort) return false;
+  if (n <= 0) return true;
+  const LkArgs a = lk_args(prev, next, prm, false, nullptr);
+  PLVIWO_CARVEOUT(k_lk15w);
+  k_lk15w<<<(n + kLkwWarps - 1) / kLkwWarps, kLkwWarps * 32, 0, s>>>(a, d_pts0, d_pts1, d_status, n);
+  return true;
 }
 
 }  // namespace plviwo
