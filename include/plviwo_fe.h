@@ -306,7 +306,10 @@ int plviwo_fe_stereo_get_stage_times(FeStereoHandle *h, FeStageTimes *out, int r
  * one FeHandle is — its rows are bit-identical to those of a handle fed the same frames — but the frames of all streams
  * of a tick share their kernel launches and the tracker state lives on the device (csrc/fe_group.h).  All streams share
  * the FeConfig (image size, knobs); the calibration is per stream.  cfg->lookahead = ticks that submit may run ahead of
- * collect.  Not supported in a group: cfg->downsample, cfg->line_samples, set_num_features / change_feat_id.
+ * collect.  Not supported in a group: cfg->downsample, set_num_features / change_feat_id.
+ * cfg->line_samples > 0 (with use_lines): each stream's samples come back through plviwo_fe_group_get_line_samples, equal to a
+ * handle's; every output record then holds a sample region of min(line_samples * 1024, max(4096, 8 * num_features) + 32768)
+ * samples (17 bytes each: at line_samples = 10, 170 KB per record, n_streams * (lookahead + 2) records of pinned memory).
  */
 typedef struct FeGroupHandle FeGroupHandle;
 enum FeGroupKernel {
@@ -345,6 +348,9 @@ int plviwo_fe_group_get_point_rows(FeGroupHandle *g, int stream, FePointRow *out
 int plviwo_fe_group_get_last_obs(FeGroupHandle *g, int stream, uint64_t *ids, float *uv, int cap, int *n_out);
 int plviwo_fe_group_get_line_rows(FeGroupHandle *g, int stream, FeLineRow *out, int cap, int *n_out);
 int plviwo_fe_group_get_line_points(FeGroupHandle *g, int stream, FeLinePoint *out, int cap, int *n_out);
+/* as plviwo_fe_get_line_samples, for stream `stream` of the last collected tick */
+int plviwo_fe_group_get_line_samples(FeGroupHandle *g, int stream, float *uv01 /* 4 per sample */, uint8_t *status, int cap,
+                                     int *n_out);
 /* per-stream tracker state, same blob as plviwo_fe_get_state / _set_state (teacher forcing, checkpoint / resume) */
 int plviwo_fe_group_get_state(FeGroupHandle *g, int stream, void *buf, size_t cap, size_t *n_bytes);
 int plviwo_fe_group_set_state(FeGroupHandle *g, int stream, const void *buf, size_t n_bytes);

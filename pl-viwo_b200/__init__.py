@@ -121,6 +121,7 @@ EXPORTS = [
     "plviwo_fe_group_create", "plviwo_fe_group_destroy", "plviwo_fe_group_last_error", "plviwo_fe_group_set_calib", "plviwo_fe_group_set_camera",
     "plviwo_fe_group_submit", "plviwo_fe_group_collect", "plviwo_fe_group_play", "plviwo_fe_group_get_point_rows",
     "plviwo_fe_group_get_last_obs", "plviwo_fe_group_get_line_rows", "plviwo_fe_group_get_line_points",
+    "plviwo_fe_group_get_line_samples",
     "plviwo_fe_group_get_state", "plviwo_fe_group_set_state", "plviwo_fe_group_tap", "plviwo_fe_group_enable_timing",
     "plviwo_fe_group_get_times", "plviwo_fe_set_camera", "plviwo_fe_get_currid", "plviwo_fe_set_currid",
     "plviwo_fe_stereo_set_camera",
@@ -217,6 +218,7 @@ def lib() -> C.CDLL:
         for name in ("plviwo_fe_group_get_point_rows", "plviwo_fe_group_get_line_rows", "plviwo_fe_group_get_line_points"):
             getattr(L, name).argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
         L.plviwo_fe_group_get_last_obs.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
+        L.plviwo_fe_group_get_line_samples.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
         L.plviwo_fe_group_get_state.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
         L.plviwo_fe_group_set_state.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]
         L.plviwo_fe_group_tap.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
@@ -663,6 +665,18 @@ class GroupFrontEnd:
         if n.value:
             self._check(self._lib.plviwo_fe_group_get_last_obs(self._h, stream, ids.ctypes.data, uv.ctypes.data, n.value, C.byref(n)))
         return ids, uv
+
+    def line_samples(self, stream: int):
+        """cfg.line_samples: the samples of stream `stream` in the last collected tick, as FrontEnd.line_samples():
+        uv (n, 4) float32 = u0 v0 (previous image) u1 v1 (current image), status (n,) uint8."""
+        n = C.c_int(0)
+        self._check(self._lib.plviwo_fe_group_get_line_samples(self._h, stream, None, None, 0, C.byref(n)))
+        uv = np.zeros((n.value, 4), np.float32)
+        st = np.zeros((n.value,), np.uint8)
+        if n.value:
+            self._check(self._lib.plviwo_fe_group_get_line_samples(self._h, stream, uv.ctypes.data, st.ctypes.data, n.value,
+                                                                   C.byref(n)))
+        return uv, st
 
     def get_state(self, stream: int) -> bytes:
         n = C.c_size_t(0)

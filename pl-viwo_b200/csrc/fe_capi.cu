@@ -777,7 +777,6 @@ int plviwo_fe_group_create(const FeConfig *cfg, int n_streams, int device, FeGro
   if (cfg->histogram_method != FE_HIST_NONE && cfg->histogram_method != FE_HIST_HISTOGRAM && cfg->histogram_method != FE_HIST_CLAHE)
     return bad("bad histogram_method");
   if (cfg->downsample) return bad("cfg.downsample is not supported in a stream group");
-  if (cfg->line_samples) return bad("cfg.line_samples is not supported in a stream group");
   if (cfg->use_lines) {
     if ((cfg->width & 1) || (cfg->height & 1)) return bad("line tracker needs even image dimensions (exact 2x decimation)");
     if (cfg->canny_th1 != cfg->canny_th2) return bad("canny_th1 != canny_th2: hysteresis pass is not implemented");
@@ -879,6 +878,10 @@ int plviwo_fe_group_get_line_points(FeGroupHandle *g, int stream, FeLinePoint *o
   const GroupOutHeader *h = g->grp->header(stream);
   if (!h) return FE_BAD_ARG;
   return copy_rows(g->grp->line_points(stream), h->info.n_line_rows > 0 ? h->n_line_points : 0, sizeof(FeLinePoint), out, cap, n_out);
+}
+int plviwo_fe_group_get_line_samples(FeGroupHandle *g, int stream, float *uv01, uint8_t *status, int cap, int *n_out) {
+  if (!g) return FE_BAD_ARG;
+  return g->grp->line_samples(stream, uv01, status, cap, n_out);
 }
 int plviwo_fe_group_get_state(FeGroupHandle *g, int stream, void *buf, size_t cap, size_t *n_bytes) {
   API_BEGIN

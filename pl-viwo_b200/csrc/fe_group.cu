@@ -223,6 +223,7 @@ int FeGroup::init() {
     FG_CUDA(dev_alloc(dev_allocs_, &g_.line_buf, S_));
     FG_CUDA(dev_alloc(dev_allocs_, &g_.line_currid, S_));
     FG_CUDA(dev_alloc(dev_allocs_, &g_.lnew, (size_t)S_ * g_.lines_cap));
+    FG_CUDA(dev_alloc(dev_allocs_, &g_.n_lnew, S_));   // zero: no segments before the first frame fed with vanishing points
     FG_CUDA(dev_alloc(dev_allocs_, &g_.lcnt, (size_t)S_ * (g_.lines_cap + 1)));
     FG_CUDA(dev_alloc(dev_allocs_, &g_.loff, (size_t)S_ * (g_.lines_cap + 1)));
     FG_CUDA(dev_alloc(dev_allocs_, &g_.lpos, (size_t)S_ * g_.pol_cap));
@@ -232,12 +233,26 @@ int FeGroup::init() {
   }
 
   // ---- output ring (pinned, device-mapped): header | point rows | obs ids | obs uv | line rows | line points
+  //      [| sample p0 | sample p1 | sample status: cfg.line_samples only]
   g_.off_rows = align_up_sz(sizeof(GroupOutHeader), 64);
   g_.off_obs_ids = align_up_sz(g_.off_rows + (size_t)g_.pts_cap * sizeof(FePointRow), 64);
   g_.off_obs_uv = align_up_sz(g_.off_obs_ids + (size_t)g_.pts_cap * sizeof(uint64_t), 64);
   g_.off_lrows = align_up_sz(g_.off_obs_uv + (size_t)g_.pts_cap * sizeof(float2), 64);
   g_.off_lpts = align_up_sz(g_.off_lrows + (size_t)(cfg_.use_lines ? g_.lines_cap : 0) * sizeof(FeLineRow), 64);
-  g_.out_stride = align_up_sz(g_.off_lpts + (size_t)(cfg_.use_lines ? g_.pol_cap : 0) * sizeof(FeLinePoint), 256);
+  const size_t end_lpts = g_.off_lpts + (size_t)(cfg_.use_lines ? g_.pol_cap : 0) * sizeof(FeLinePoint);
+  if (cfg_.use_lines && cfg_.line_samples > 0) {
+    // a handle tracks its samples in its LK buffer, after the n points: ns = min(S * L, max_pts - n) (fe_context.cu init /
+    // perform_matching); L <= lines_cap here.  At S = 10: 10240 samples, 170 KB per record.
+    g_.line_samples = cfg_.line_samples;
+    g_.sample_max_pts = std::max(4096, 8 * cfg_.num_features) + 4096 * 8;
+    g_.sample_cap = (int)std::min<long long>((long long)cfg_.line_samples * g_.lines_cap, g_.sample_max_pts);
+    g_.off_sp0 = align_up_sz(end_lpts, 64);
+    g_.off_sp1 = g_.off_sp0 + (size_t)g_.sample_cap * sizeof(float2);
+    g_.off_sst = g_.off_sp1 + (size_t)g_.sample_cap * sizeof(float2);
+    g_.out_stride = align_up_sz(g_.off_sst + (size_t)g_.sample_cap, 256);
+  } else {
+    g_.out_stride = align_up_sz(end_lpts, 256);
+  }
   FG_CUDA(cudaHostAlloc((void **)&h_out_, g_.out_stride * (size_t)RB_ * S_, cudaHostAllocMapped));
   host_allocs_.push_back(h_out_);
   std::memset(h_out_, 0, g_.out_stride * (size_t)RB_ * S_);
@@ -693,8 +708,15 @@ int FeGroup::launch_track(int tick) {
           sl = s_lines_[l];
           FG_CUDA(cudaEventRecord(ev_gate_[(size_t)ring * lanes_ + l], st));
           FG_CUDA(cudaStreamWaitEvent(sl, ev_gate_[(size_t)ring * lanes_ + l], 0));
-          FG_CUDA(cudaStreamWaitEvent(sl, ev_front_[tr.batch], 0));   // the frame's segments (chain walk + fit of the batch)
         }
+        if (g_.sample_cap > 0) {
+          // cfg.line_samples: needs the gate's header and the segments the previous association left in lnew, which this
+          // tick's association rewrites next on the same stream; the point chain never waits for it, collect does (ev_done_)
+          launch_group_line_samples(g_, dj + j0, n, prm, sl);
+          launches_++;
+          step(FE_GK_LK);
+        }
+        if (!tm) FG_CUDA(cudaStreamWaitEvent(sl, ev_front_[tr.batch], 0));   // the frame's segments (chain walk + fit of the batch)
         launch_group_lines(g_, dj + j0, n, sl);
         launches_++;
         step(FE_GK_LINES);
@@ -735,7 +757,7 @@ int FeGroup::collect(FeFrameInfo *infos) {
     frames_done_++;
     d2h_bytes_ += sizeof(GroupOutHeader) + (size_t)h->info.n_point_rows * sizeof(FePointRow) +
                   (size_t)h->n_obs * (sizeof(uint64_t) + sizeof(float2)) + (size_t)h->info.n_line_rows * sizeof(FeLineRow) +
-                  (size_t)h->n_line_points * sizeof(FeLinePoint);
+                  (size_t)h->n_line_points * sizeof(FeLinePoint) + (size_t)h->n_samples * (2 * sizeof(float2) + 1);
     if (h->status != FE_OK && status == FE_OK) {
       status = h->status;
       static const char *what[] = {"?", "points", "lines", "point / line pairs", "candidates"};
@@ -773,6 +795,27 @@ const FeLineRow *FeGroup::line_rows(int s) const {
 const FeLinePoint *FeGroup::line_points(int s) const {
   const uint8_t *r = reinterpret_cast<const uint8_t *>(header(s));
   return r ? reinterpret_cast<const FeLinePoint *>(r + g_.off_lpts) : nullptr;
+}
+int FeGroup::line_samples(int s, float *uv01, uint8_t *status, int cap, int *n_out) const {
+  const GroupOutHeader *h = header(s);
+  if (!h) return FE_BAD_ARG;
+  const int n = h->n_samples;
+  if (n_out) *n_out = n;
+  if (!uv01 && !status) return FE_OK;
+  if (cap < n) return FE_OVERFLOW;
+  if (n == 0) return FE_OK;
+  const uint8_t *r = reinterpret_cast<const uint8_t *>(h);
+  if (uv01) {
+    const float2 *p0 = reinterpret_cast<const float2 *>(r + g_.off_sp0), *p1 = reinterpret_cast<const float2 *>(r + g_.off_sp1);
+    for (int k = 0; k < n; k++) {
+      uv01[4 * k + 0] = p0[k].x;
+      uv01[4 * k + 1] = p0[k].y;
+      uv01[4 * k + 2] = p1[k].x;
+      uv01[4 * k + 3] = p1[k].y;
+    }
+  }
+  if (status) std::memcpy(status, r + g_.off_sst, (size_t)n);
+  return FE_OK;
 }
 
 // Whole-sequence playback of every stream (run_bag.cpp:272-340 feeds the cameras in time order): images[t * S + s].

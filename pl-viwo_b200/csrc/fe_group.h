@@ -46,6 +46,8 @@ class FeGroup {
   const float *obs_uv(int stream) const;
   const FeLineRow *line_rows(int stream) const;
   const FeLinePoint *line_points(int stream) const;
+  // cfg.line_samples: u0 v0 u1 v1 and status per sample, as plviwo_fe_get_line_samples
+  int line_samples(int stream, float *uv01, uint8_t *status, int cap, int *n_out) const;
 
   int get_state(int stream, void *buf, size_t cap, size_t *n_bytes);
   int set_state(int stream, const void *buf, size_t n_bytes);

@@ -30,7 +30,8 @@ struct GroupOutHeader {
   int32_t n_line_points;
   int32_t status;            // FE_OK or FE_INTERNAL (a capacity was exceeded: the message says which)
   int32_t overflow_what;     // 1 points, 2 lines, 3 point/line pairs, 4 candidates
-  int32_t reserved[12];
+  int32_t n_samples;         // cfg.line_samples: samples tracked in this frame (0 when the frame made no LK call)
+  int32_t reserved[11];
 };
 
 constexpr int kValidStride = 260;
@@ -82,6 +83,7 @@ struct GroupDev {
   uint64_t *line_currid;
   // scratch of the line association, per stream
   float4 *lnew;                  // lines_cap: detected lines longer than line_min_length (full-res)
+  int *n_lnew;                   // per stream: lines in lnew, written with it (the segments the next frame's samples lie on)
   int *lcnt, *loff;              // lines_cap (+1): points per line, entry offsets
   float2 *lpos;                  // pol_cap: point_position entries (detection order)
   int *lmatch;                   // lines_cap
@@ -89,6 +91,10 @@ struct GroupDev {
   uint8_t *out;
   size_t out_stride;
   size_t off_rows, off_obs_ids, off_obs_uv, off_lrows, off_lpts;   // byte offsets inside a record
+  // cfg.line_samples (0: off, no region): samples per segment, the handle's LK buffer size (max_pts, fe_context.cu) that
+  // truncates them, and the record's sample region: sample_cap positions p0, p1 (float2) and status bytes
+  int line_samples, sample_max_pts, sample_cap;
+  size_t off_sp0, off_sp1, off_sst;
 };
 
 // tracking launches (kernels_glue.cu, kernels_track.cu)
@@ -103,6 +109,9 @@ void launch_group_subpix(const GroupDev &g, const TrackJob *jobs, int n_jobs, cu
 void launch_group_accept(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
 void launch_group_lk(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s);
 void launch_group_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
+// cfg.line_samples: LK of the samples along the stream's last detected segments (lnew), previous -> current pyramid, for the
+// frames whose point LK ran; reads the header the gate wrote and lnew before this tick's k_group_lines rewrites it
+void launch_group_line_samples(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s);
 void launch_group_lines(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
 
 }  // namespace plviwo

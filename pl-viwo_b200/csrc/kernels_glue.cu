@@ -763,6 +763,7 @@ __global__ void __launch_bounds__(kGT)
   const bool over_pairs = ne > PC;
   if (tid == 0) {
     g.line_currid[s] = lcurr + (uint64_t)L;
+    g.n_lnew[s] = L;   // lines_det_last_ of a handle (fe_context.cu lsd_feed): cfg.line_samples samples the next frame along these
     hdr->info.n_lines_detected = L;
     if (s_over) {
       hdr->status = FE_INTERNAL;

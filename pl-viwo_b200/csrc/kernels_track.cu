@@ -222,13 +222,12 @@ struct LkArgs {
   CalibArgs calib;
 };
 
+// feature pi of the warp's launch; the warp's shared memory is its slice of the dynamic buffer
 template <class Args>
 __device__ __forceinline__ void lk_body(const Args &a, const float2 *__restrict__ pts0, float2 *__restrict__ pts1,
-                                        uint8_t *__restrict__ status, float2 *__restrict__ p0n, float2 *__restrict__ p1n, int n) {
+                                        uint8_t *__restrict__ status, float2 *__restrict__ p0n, float2 *__restrict__ p1n, int pi) {
   extern __shared__ __align__(16) uint8_t lk_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int pi = blockIdx.x * kLkWarps + warp;
-  if (pi >= n) return;
   const int win = a.win;
   const int np = win + 3;        // raw patch side
   const int nd = win + 1;        // derivative grid side
@@ -404,7 +403,9 @@ __device__ __forceinline__ void lk_body(const Args &a, const float2 *__restrict_
 __global__ void __launch_bounds__(kLkWarps * 32)
     k_lk(LkArgs a, const float2 *__restrict__ pts0, float2 *__restrict__ pts1, uint8_t *__restrict__ status,
          float2 *__restrict__ p0n, float2 *__restrict__ p1n, int n) {
-  lk_body(a, pts0, pts1, status, p0n, p1n, n);
+  const int pi = blockIdx.x * kLkWarps + (threadIdx.x >> 5);
+  if (pi >= n) return;
+  lk_body(a, pts0, pts1, status, p0n, p1n, pi);
 }
 
 // ------------------------------------------------------------------------------------------ LK, 15 x 15 window
@@ -1139,8 +1140,10 @@ __global__ void __launch_bounds__(kLkWarps * 32)
   if (g.wmode[s] != 0 || n < 10 || (int)blockIdx.x * kLkWarps >= n) return;
   if (threadIdx.x == 0) group_lk_args(sa, g, job, prm);
   __syncthreads();
+  const int pi = blockIdx.x * kLkWarps + (threadIdx.x >> 5);
+  if (pi >= n) return;
   const size_t o = (size_t)s * g.pts_cap;
-  lk_body(sa, g.wpts + o, g.lk_pts1 + o, g.lk_status + o, g.lk_p0n + o, g.lk_p1n + o, n);
+  lk_body(sa, g.wpts + o, g.lk_pts1 + o, g.lk_status + o, g.lk_p0n + o, g.lk_p1n + o, pi);
 }
 
 // 5 resident CTAs per SM: 94 registers, no spills
@@ -1175,6 +1178,97 @@ void launch_group_lk(const GroupDev &g, const TrackJob *jobs, int n_jobs, const 
   optin.ensure(k_lk_g, smem);
   PLVIWO_CARVEOUT(k_lk_g);
   k_lk_g<<<dim3((g.pts_cap + kLkWarps - 1) / kLkWarps, n_jobs), kLkWarps * 32, smem, s>>>(g, jobs, prm);
+}
+
+// ---- stream group, cfg.line_samples: the samples a handle appends to its point LK launch (fe_context.cu perform_matching),
+// one warp per sample, grid.y = job.  Samples exist when the frame's point LK ran — the gate then wrote n_lk_in = n >= 10
+// into the frame's header, 0 otherwise — and lie along the stream's last detected segments (lnew, n_lnew: k_group_lines of
+// the latest frame fed with vanishing points), k = 0..S-1 per segment, cut where the handle's LK buffer ends:
+// ns = min(S * L, max_pts - n).  Same LK parameters and pyramids as the points, initial guess = the sample itself.
+// Thread 0 of a CTA: the job's sample count (CTAs past it read nothing but n_lnew) and the job's LK arguments.
+__device__ __forceinline__ int group_samples_setup(LkArgs &sa, const GroupDev &g, const TrackJob &job, const LkParams &prm,
+                                                   int first) {
+  const long long all = (long long)g.line_samples * g.n_lnew[job.stream];
+  if (first >= all) return 0;
+  GroupOutHeader *hdr = reinterpret_cast<GroupOutHeader *>(g.out + (size_t)job.out * g.out_stride);
+  const int n = hdr->info.n_lk_in;
+  if (n < 10) return 0;
+  const int ns = (int)max(0ll, min(all, (long long)(g.sample_max_pts - n)));
+  if (blockIdx.x == 0) hdr->n_samples = ns;
+  if (first < ns) {
+    group_lk_args(sa, g, job, prm);
+    sa.undistort = 0;   // the handle computes the samples' undistorted positions and discards them
+  }
+  return ns;
+}
+
+// sample pi of the job: a = k / (S - 1) (0.5 for S = 1) along segment pi / S, rounded as the host rounds it (no contraction)
+__device__ __forceinline__ float2 group_sample_pos(const GroupDev &g, const TrackJob &job, int pi) {
+  const int S = g.line_samples, k = pi % S;
+  const float4 l = g.lnew[(size_t)job.stream * g.lines_cap + pi / S];
+  const float a = S > 1 ? (float)k / (float)(S - 1) : 0.5f;
+  return make_float2(l.x + (l.z - l.x) * a, l.y + (l.w - l.y) * a);
+}
+
+__global__ void __launch_bounds__(kLkwWarps * 32, 5)
+    k_lk15w_samples_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
+  __shared__ LkArgs sa;
+  __shared__ LkwSmem sm[kLkwWarps];
+  __shared__ float2 s_p1[kLkwWarps];   // the body's result, stored to the record afterwards (no record pointer held through it)
+  __shared__ uint8_t s_st[kLkwWarps];
+  __shared__ int s_ns;
+  const TrackJob &job = jobs[blockIdx.y];
+  const int warp = threadIdx.x >> 5;
+  if (threadIdx.x == 0) s_ns = group_samples_setup(sa, g, job, prm, (int)blockIdx.x * kLkwWarps);
+  __syncthreads();
+  const int pi = blockIdx.x * kLkwWarps + warp;
+  if (pi >= s_ns) return;
+  const float2 p0 = group_sample_pos(g, job, pi);
+  lk15w_body(sa, &p0, &s_p1[warp], &s_st[warp], nullptr, nullptr, 0, sm[warp]);
+  if ((threadIdx.x & 31) == 0) {   // the lane that wrote the result
+    uint8_t *const rec = g.out + (size_t)jobs[blockIdx.y].out * g.out_stride;
+    reinterpret_cast<float2 *>(rec + g.off_sp0)[pi] = p0;
+    reinterpret_cast<float2 *>(rec + g.off_sp1)[pi] = s_p1[warp];
+    rec[g.off_sst + pi] = s_st[warp];
+  }
+}
+
+__global__ void __launch_bounds__(kLkWarps * 32)
+    k_lk_samples_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
+  __shared__ LkArgs sa;
+  __shared__ float2 s_p1[kLkWarps];
+  __shared__ uint8_t s_st[kLkWarps];
+  __shared__ int s_ns;
+  const TrackJob &job = jobs[blockIdx.y];
+  const int warp = threadIdx.x >> 5;
+  if (threadIdx.x == 0) s_ns = group_samples_setup(sa, g, job, prm, (int)blockIdx.x * kLkWarps);
+  __syncthreads();
+  const int pi = blockIdx.x * kLkWarps + warp;
+  if (pi >= s_ns) return;
+  const float2 p0 = group_sample_pos(g, job, pi);
+  lk_body(sa, &p0, &s_p1[warp], &s_st[warp], nullptr, nullptr, 0);
+  if ((threadIdx.x & 31) == 0) {
+    uint8_t *const rec = g.out + (size_t)jobs[blockIdx.y].out * g.out_stride;
+    reinterpret_cast<float2 *>(rec + g.off_sp0)[pi] = p0;
+    reinterpret_cast<float2 *>(rec + g.off_sp1)[pi] = s_p1[warp];
+    rec[g.off_sst + pi] = s_st[warp];
+  }
+}
+
+void launch_group_line_samples(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s) {
+  if (n_jobs <= 0 || g.sample_cap <= 0) return;
+  if (prm.win == kW15 && prm.max_level + 1 <= kLk15MaxLevels) {
+    PLVIWO_CARVEOUT(k_lk15w_samples_g);
+    k_lk15w_samples_g<<<dim3((g.sample_cap + kLkwWarps - 1) / kLkwWarps, n_jobs), kLkwWarps * 32, 0, s>>>(g, jobs, prm);
+    return;
+  }
+  const int win = prm.win, np = win + 3, nd = win + 1, nw = win * win;
+  const int per_warp = ((np * np + 15) & ~15) + 2 * ((nd * nd * 2 + 15) & ~15) + 3 * ((nw * 2 + 15) & ~15);
+  const size_t smem = (size_t)per_warp * kLkWarps;
+  static SmemOptIn optin;
+  optin.ensure(k_lk_samples_g, smem);
+  PLVIWO_CARVEOUT(k_lk_samples_g);
+  k_lk_samples_g<<<dim3((g.sample_cap + kLkWarps - 1) / kLkWarps, n_jobs), kLkWarps * 32, smem, s>>>(g, jobs, prm);
 }
 
 bool lk_table_mode_ok(const LkParams &prm, int pyramid_images) {
