@@ -378,6 +378,13 @@ int plviwo_op_lk_warp(int device, const uint8_t *img0, const uint8_t *img1, int 
                       const float *pts0, float *pts1 /* in: initial flow, out */, uint8_t *status, int n);
 int plviwo_op_undistort(int device, const float *pts, int n, const double K[4], const double D[4], float *out);
 int plviwo_op_canny_half(int device, const uint8_t *img, int w, int h, float th, uint8_t *edges /* w*h bytes */);
+/* Connected components (8-connected) of every 64 x 16 tile of a bit-packed edge map on its own, as the line detector's first
+   labelling step computes them.  edge_words: (w + 31) / 32 words per row, bit x % 32 of word x / 32 = pixel x.  For every
+   edge pixel, label = raster index of the smallest pixel of its component inside the tile (other entries: -1).  At those
+   roots: cnt = pixels, bbox[0|1|2][root] = max y, min x, max x (planes of w*h ints; other entries undefined).  roots: the
+   tile-local roots in any order, *n_roots of them (FE_OVERFLOW if more than cap). */
+int plviwo_op_ccl_tiles(int device, const uint32_t *edge_words, int w, int h, int32_t *label /* w*h */, int32_t *cnt /* w*h */,
+                        int32_t *bbox /* 3*w*h */, int32_t *roots, int cap, int *n_roots);
 int plviwo_op_fld(int device, const uint8_t *img, int w, int h, int length_threshold, float distance_threshold,
                   float canny_th, float *lines /* 4 per segment */, int cap, int *n_out);
 /* Micro-benchmark of the image-domain kernels on a DEVICE-resident synthetic image of any size (w, h multiples of 4):

@@ -111,7 +111,7 @@ EXPORTS = [
     "plviwo_fe_get_line_rows", "plviwo_fe_get_line_points", "plviwo_fe_get_line_samples", "plviwo_fe_get_state",
     "plviwo_fe_set_state", "plviwo_fe_enable_taps", "plviwo_fe_tap", "plviwo_fe_enable_timing", "plviwo_fe_get_stage_times",
     "plviwo_op_equalize_pyramid", "plviwo_op_clahe", "plviwo_op_fast_cell", "plviwo_op_sort_corners", "plviwo_op_corner_subpix", "plviwo_op_lk", "plviwo_op_lk_warp", "plviwo_op_undistort",
-    "plviwo_op_canny_half", "plviwo_op_fld", "plviwo_op_image_kernels_time", "plviwo_op_ransac_fundamental",
+    "plviwo_op_canny_half", "plviwo_op_ccl_tiles", "plviwo_op_fld", "plviwo_op_image_kernels_time", "plviwo_op_ransac_fundamental",
     "plviwo_fe_stereo_create", "plviwo_fe_stereo_destroy", "plviwo_fe_stereo_last_error", "plviwo_fe_stereo_set_calib",
     "plviwo_fe_stereo_set_num_features", "plviwo_fe_stereo_change_feat_id", "plviwo_fe_stereo_feed", "plviwo_fe_stereo_submit",
     "plviwo_fe_stereo_collect", "plviwo_fe_stereo_get_point_rows", "plviwo_fe_stereo_get_last_obs", "plviwo_fe_stereo_get_state",
@@ -199,6 +199,8 @@ def lib() -> C.CDLL:
         L.plviwo_op_lk_warp.argtypes = L.plviwo_op_lk.argtypes
         L.plviwo_op_undistort.argtypes = [C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_void_p]
         L.plviwo_op_canny_half.argtypes = [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_void_p]
+        L.plviwo_op_ccl_tiles.argtypes = [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_int, C.POINTER(C.c_int)]
         L.plviwo_op_fld.argtypes = [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_void_p, C.c_int,
                                     C.POINTER(C.c_int)]
         L.plviwo_op_image_kernels_time.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float)]
@@ -1084,6 +1086,27 @@ def op_canny(img: np.ndarray, th: float = 50.0, device: int = 0) -> np.ndarray:
     out = np.zeros_like(img)
     _check(lib().plviwo_op_canny_half(device, img.ctypes.data, img.shape[1], img.shape[0], th, out.ctypes.data))
     return out
+
+
+def op_ccl_tiles(edges: np.ndarray, device: int = 0) -> Dict[str, np.ndarray]:
+    """Connected components of every 64 x 16 tile of an edge map (h x w, nonzero = edge) on their own: label (h x w,
+    raster index of the tile-local root, -1 off the edges), cnt and bbox (3 x h x w; meaningful at the roots) and the
+    sorted tile-local roots."""
+    e = np.ascontiguousarray(edges) != 0
+    h, w = e.shape
+    wpr = (w + 31) // 32
+    padded = np.zeros((h, wpr * 32), bool)
+    padded[:, :w] = e
+    words = np.ascontiguousarray(np.packbits(padded, axis=1, bitorder="little").view("<u4"))
+    label = np.empty((h, w), np.int32)
+    cnt = np.empty((h, w), np.int32)
+    bbox = np.empty((3, h, w), np.int32)
+    cap = w * h // 4 + 1
+    roots = np.empty(cap, np.int32)
+    n = C.c_int(0)
+    _check(lib().plviwo_op_ccl_tiles(device, words.ctypes.data, w, h, label.ctypes.data, cnt.ctypes.data, bbox.ctypes.data,
+                                     roots.ctypes.data, cap, C.byref(n)))
+    return {"label": label, "cnt": cnt, "bbox": bbox, "roots": np.sort(roots[:n.value])}
 
 
 def op_fld(img: np.ndarray, length_threshold: int = 20, distance_threshold: float = 1.414213562, canny_th: float = 50.0,

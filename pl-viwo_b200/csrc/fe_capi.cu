@@ -594,6 +594,32 @@ int plviwo_op_canny_half(int device, const uint8_t *img, int w, int h, float th,
   API_END
 }
 
+int plviwo_op_ccl_tiles(int device, const uint32_t *edge_words, int w, int h, int32_t *label, int32_t *cnt, int32_t *bbox,
+                        int32_t *roots, int cap, int *n_roots) {
+  API_BEGIN
+  if (!edge_words || !label || !cnt || !bbox || !n_roots || (cap > 0 && !roots) || cap < 0 || w < 1 || h < 1 ||
+      (size_t)w * h > (size_t)1 << 28)
+    return FE_BAD_ARG;
+  OP_CUDA(cudaSetDevice(device));
+  TmpFld f;
+  if (f.alloc(w, h, 20, 16)) return FE_CUDA_ERROR;
+  const size_t n = (size_t)w * h;
+  OP_CUDA(cudaMemcpy(f.fb.edges, edge_words, (size_t)f.fb.words_per_row * h * sizeof(unsigned), cudaMemcpyHostToDevice));
+  OP_CUDA(cudaMemset(f.fb.label, 0xff, n * sizeof(int)));
+  launch_ccl_tiles(f.fb, w, h, 0);
+  OP_CUDA(cudaDeviceSynchronize());
+  int nr = 0;
+  OP_CUDA(cudaMemcpy(&nr, f.fb.lroot_n, sizeof(int), cudaMemcpyDeviceToHost));
+  OP_CUDA(cudaMemcpy(label, f.fb.label, n * sizeof(int), cudaMemcpyDeviceToHost));
+  OP_CUDA(cudaMemcpy(cnt, f.fb.cnt, n * sizeof(int), cudaMemcpyDeviceToHost));
+  OP_CUDA(cudaMemcpy(bbox, f.fb.bbox, 3 * n * sizeof(int), cudaMemcpyDeviceToHost));
+  *n_roots = nr;
+  if (nr > cap) return FE_OVERFLOW;
+  if (nr) OP_CUDA(cudaMemcpy(roots, f.fb.lroots, (size_t)nr * sizeof(int), cudaMemcpyDeviceToHost));
+  return FE_OK;
+  API_END
+}
+
 int plviwo_op_fld(int device, const uint8_t *img, int w, int h, int length_threshold, float distance_threshold,
                   float canny_th, float *lines, int cap, int *n_out) {
   API_BEGIN

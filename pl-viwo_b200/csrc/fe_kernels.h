@@ -176,6 +176,8 @@ void launch_canny(const DevImage &half, float th_low, float th_high, FldBuffers 
 void launch_fld(const DevImage &half, int length_threshold, float distance_threshold, FldBuffers &fb, cudaStream_t s,
                 cudaEvent_t *ev = nullptr);
 void launch_unpack_edges(const FldBuffers &fb, int w, int h, uint8_t *d_out, cudaStream_t s);
+// connected components of every 64 x 16 tile of fb.edges alone (label / cnt / bbox / lroots), no border pass
+void launch_ccl_tiles(FldBuffers &fb, int w, int h, cudaStream_t s);
 
 // ---- batched multi-stream launches (FeGroup, fe_group.cu) ------------------------------------------------------
 // A stream group processes one frame of MANY camera streams per launch (grid.z = job).  Every frame slot of every

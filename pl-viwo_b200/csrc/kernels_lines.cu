@@ -68,10 +68,9 @@ __device__ __forceinline__ bool edge_at(const unsigned *__restrict__ edges, int 
 }
 
 // Connected components in three steps:
-//   k_ccl_tile     every 64 x 16 tile labels ITS pixels in shared memory (union-find with shared-memory atomics) and counts
-//                  pixels / bounding boxes per tile-local component: the label written out for a pixel is the raster index of
-//                  its tile-local root, the aggregates go to the root's slot of the cnt / bbox planes (other edge pixels of
-//                  the tile get cnt = 0);
+//   k_ccl_tile     every 64 x 16 tile labels ITS pixels in shared memory (union-find over the tile's horizontal runs) and
+//                  counts pixels / bounding boxes per tile-local component: the label written out for a pixel is the raster
+//                  index of its tile-local root, the aggregates go to the root's slot of the cnt / bbox planes;
 //   k_ccl_border   unions across tile borders on the global label array (only border pixels: ~8 % of the frame);
 //   k_ccl_link     tile-local roots that are not global roots point straight at their global root and hand it their
 //                  aggregates (a pixel reaches its global root in two loads: label[label[p]]).
@@ -79,6 +78,8 @@ __device__ __forceinline__ bool edge_at(const unsigned *__restrict__ edges, int 
 // planes are written for the ~5-10 % of the pixels that are edges, and the hot global atomics of a large component are one
 // per TILE it crosses instead of one per few pixels.
 constexpr int kTileW = 64, kTileH = 16, kTilePx = kTileW * kTileH, kTileThreads = 256;
+constexpr int kTileRuns = kTilePx / 2;                  // a 64-pixel row holds at most 32 runs
+constexpr int kRunsPer = kTileRuns / kTileThreads;      // 2
 
 __device__ __forceinline__ int sm_find(const int *lab, int i) {
   int p = lab[i];
@@ -100,120 +101,138 @@ __device__ __forceinline__ void sm_union(int *lab, int a, int b) {
   }
 }
 
+// Shared memory of the tile labelling, indexed by run id: the tile's horizontal runs numbered in raster order of their
+// first pixels.  The first pixel of a component is the first pixel of a run, so the smallest run id of a component is the
+// run of its smallest raster index.
 struct CclTileSmem {
-  unsigned bits[kTileH][2];
-  int pref[kTileH * 2 + 1];      // exclusive prefix of the words' population counts
-  int lab[kTilePx];
-  int a_cnt[kTilePx], a_ymax[kTilePx], a_xmin[kTilePx], a_xmax[kTilePx];
+  unsigned start[kTileH * 2];    // first pixels of the runs, in the words of the edge bits
+  int rpref[kTileH * 2 + 1];     // runs starting before word f (exclusive prefix); [32] = all runs of the tile
+  int nroot, base;               // tile-local roots; their first slot in lroots
+  int rpix[kTileRuns];           // run -> tile pixel index of its first pixel
+  int lab[kTileRuns];            // union-find over the runs
+  int glab[kTileRuns];           // run -> global raster index of its component's root pixel
+  int a_cnt[kTileRuns], a_ymax[kTileRuns], a_xmin[kTileRuns], a_xmax[kTileRuns];
 };
 
-// Labels one 64 x 16 tile whose edge bits are in sm.bits (block-wide call, kTileThreads threads, bits visible to all).
-// The work is per EDGE pixel and edge pixels are a fraction of the tile, so they are enumerated densely: thread t takes the
-// t-th, (t + 256)-th ... set bit of the tile's 32 words (prefix of the population counts, then the n-th set bit of the word) —
-// every lane of a warp has a pixel in hand in every step instead of one lane in four.  The result does not depend on the
-// order the pixels are processed in (roots are minima, aggregates are sums / minima / maxima).
-__device__ __forceinline__ void ccl_tile_body(const FldBuffers &fb, CclTileSmem &sm, int x0, int y0, int w, int h) {
+// Labels one 64 x 16 tile whose edge bits are bits[row][half] (block-wide call, kTileThreads threads, bits visible to all).
+// The nodes of the union-find are the horizontal runs (~146 per tile on the bench scenes against ~247 edge pixels):
+//   1. warp 0 numbers the runs in raster order (the first-pixel bits of each word, a scan of their population counts);
+//   2. thread t takes run t (and t + 256): its length, and the aggregates of the run alone;
+//   3. a run is 8-adjacent to every run of the row above that meets its pixels dilated by one; those are consecutive ids;
+//   4. every run finds its root, adds its aggregates there and records the root's global index;
+//   5. one lane per pixel writes the labels (a pixel's run id is a population count of the first-pixel bits before it),
+//      the roots write cnt / bbox and take their lroots slots from one reservation per tile.
+// Nothing depends on the order the runs are processed in (roots are minima, aggregates are sums / minima / maxima).
+__device__ __forceinline__ void ccl_tile_body(const FldBuffers &fb, CclTileSmem &sm, const unsigned (*bits)[2], int x0, int y0,
+                                              int w, int h) {
   int *__restrict__ label = fb.label, *__restrict__ cnt = fb.cnt, *__restrict__ bbox = fb.bbox /* maxy, minx, maxx planes */;
-  auto &bits = sm.bits;
   int *lab = sm.lab, *a_cnt = sm.a_cnt, *a_ymax = sm.a_ymax, *a_xmin = sm.a_xmin, *a_xmax = sm.a_xmax;
-  const int tid = threadIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, wv = tid >> 5;
   const unsigned *flat = &bits[0][0];   // word f = row f / 2, half f % 2: pixel index = 32 f + bit
-  if (tid < 32) {
-    const int c = __popc(flat[tid]);
+  auto row_of = [&](const unsigned *v, int y) -> unsigned long long { return (unsigned long long)v[2 * y + 1] << 32 | v[2 * y]; };
+  if (wv == 0) {
+    const unsigned b = flat[lane];
+    const unsigned lo = __shfl_sync(0xffffffffu, b, lane & ~1);   // a run of the high half may start in the low half
+    const unsigned st = b & ~(b << 1 | ((lane & 1) ? lo >> 31 : 0u));
+    const int c = __popc(st);
     int incl = c;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
       const int t = __shfl_up_sync(0xffffffffu, incl, d);
-      if (tid >= d) incl += t;
+      if (lane >= d) incl += t;
     }
-    sm.pref[tid] = incl - c;
-    if (tid == 31) sm.pref[32] = incl;
+    sm.start[lane] = st;
+    sm.rpref[lane] = incl - c;
+    if (lane == 31) sm.rpref[32] = incl;
+    if (lane == 0) sm.nroot = 0;
+    int q = incl - c;
+    for (unsigned m = st; m; m &= m - 1) sm.rpix[q++] = 32 * lane + __ffs((int)m) - 1;
   }
   __syncthreads();
-  const int total = sm.pref[32];
-  if (total == 0) return;   // no edge pixel in this tile
-  auto edge = [&](int lx, int ly) -> bool { return (bits[ly][lx >> 5] >> (lx & 31)) & 1u; };
-  constexpr int kMaxPer = kTilePx / kTileThreads;   // 4
-  int px[kMaxPer];
+  const int nruns = sm.rpref[32];
+  if (nruns == 0) return;   // no edge pixel in this tile
+  int ry[kRunsPer], rx[kRunsPer], rlen[kRunsPer];
 #pragma unroll
-  for (int k = 0; k < kMaxPer; k++) {
-    const int e = tid + k * kTileThreads;
-    px[k] = -1;
-    if (e < total) {
-      int f = 0;   // largest f with pref[f] <= e
-#pragma unroll
-      for (int step = 16; step >= 1; step >>= 1)
-        if (sm.pref[f + step] <= e) f += step;
-      unsigned m = flat[f];
-      for (int r = e - sm.pref[f]; r > 0; r--) m &= m - 1;   // drop the r lowest set bits
-      px[k] = 32 * f + __ffs((int)m) - 1;
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < kMaxPer; k++) {
-    const int p = px[k];
-    if (p < 0) continue;
-    lab[p] = p;
-    a_cnt[p] = 0;
-    a_ymax[p] = 0;
-    a_xmin[p] = kTileW;
-    a_xmax[p] = -1;
-  }
-  __syncthreads();
-  // backward half of the 8-neighbourhood inside the tile: W, NW, N, NE.  N is 8-adjacent to the other three (and they are
-  // merged with it when THEY are processed), so a set N needs one union; otherwise W (or, without W, NW — W's own N) and NE
-  // are independent.
-#pragma unroll
-  for (int k = 0; k < kMaxPer; k++) {
-    const int p = px[k];
-    if (p < 0) continue;
-    const int ly = p >> 6, lx = p & (kTileW - 1);
-    const bool eW = lx > 0 && edge(lx - 1, ly);
-    if (ly > 0) {
-      if (edge(lx, ly - 1)) {
-        sm_union(lab, p, p - kTileW);
-        continue;
-      }
-      if (eW) sm_union(lab, p, p - 1);
-      else if (lx > 0 && edge(lx - 1, ly - 1)) sm_union(lab, p, p - kTileW - 1);
-      if (lx < kTileW - 1 && edge(lx + 1, ly - 1)) sm_union(lab, p, p - kTileW + 1);
-    } else if (eW) {
-      sm_union(lab, p, p - 1);
+  for (int k = 0; k < kRunsPer; k++) {
+    const int t = tid + k * kTileThreads;
+    rlen[k] = 0;
+    if (t < nruns) {
+      const int p = sm.rpix[t];
+      ry[k] = p >> 6;
+      rx[k] = p & (kTileW - 1);
+      rlen[k] = __clzll(__brevll(~(row_of(flat, ry[k]) >> rx[k])));   // trailing ones from the first pixel
+      lab[t] = t;
+      a_cnt[t] = rlen[k];
+      a_ymax[t] = ry[k];
+      a_xmin[t] = rx[k];
+      a_xmax[t] = rx[k] + rlen[k] - 1;
     }
   }
   __syncthreads();
-  int root[kMaxPer];
+  // run id of the pixel at (x, y): the runs before row y, plus the runs of row y starting at or before x, minus one
+  auto run_at = [&](int x, int y) -> int {
+    return sm.rpref[2 * y] + __popcll(row_of(sm.start, y) & (~0ull >> (63 - x))) - 1;
+  };
 #pragma unroll
-  for (int k = 0; k < kMaxPer; k++) {
-    root[k] = -1;
-    const int p = px[k];
-    if (p < 0) continue;
-    const int ly = p >> 6, lx = p & (kTileW - 1);
-    const int r = sm_find(lab, p);
-    root[k] = r;
-    atomicAdd(&a_cnt[r], 1);
-    atomicMax(&a_ymax[r], ly);
-    atomicMin(&a_xmin[r], lx);
-    atomicMax(&a_xmax[r], lx);
+  for (int k = 0; k < kRunsPer; k++) {
+    if (rlen[k] == 0 || ry[k] == 0) continue;
+    const int lo = max(rx[k] - 1, 0), hi = min(rx[k] + rlen[k], kTileW - 1);
+    const unsigned long long touch = row_of(flat, ry[k] - 1) & (~0ull >> (63 - hi)) & (~0ull << lo);
+    if (touch == 0) continue;
+    const int t = tid + k * kTileThreads;
+    const int first = run_at(__clzll(__brevll(touch)), ry[k] - 1), last = run_at(63 - __clzll(touch), ry[k] - 1);
+    for (int j = first; j <= last; j++) sm_union(lab, t, j);
+  }
+  __syncthreads();
+  bool is_root[kRunsPer];
+#pragma unroll
+  for (int k = 0; k < kRunsPer; k++) {
+    const int t = tid + k * kTileThreads;
+    is_root[k] = false;
+    if (rlen[k] == 0) continue;
+    const int r = sm_find(lab, t);
+    is_root[k] = r == t;
+    if (!is_root[k]) {
+      atomicAdd(&a_cnt[r], rlen[k]);
+      atomicMax(&a_ymax[r], ry[k]);
+      atomicMin(&a_xmin[r], rx[k]);
+      atomicMax(&a_xmax[r], rx[k] + rlen[k] - 1);
+    }
+    const int rp = sm.rpix[r];
+    sm.glab[t] = (y0 + (rp >> 6)) * w + x0 + (rp & (kTileW - 1));
+  }
+  int slot[kRunsPer];   // the root's place among the tile's roots
+#pragma unroll
+  for (int k = 0; k < kRunsPer; k++) {
+    const unsigned m = __ballot_sync(0xffffffffu, is_root[k]);
+    int q = 0;
+    if (lane == 0 && m) q = atomicAdd(&sm.nroot, __popc(m));
+    slot[k] = __shfl_sync(0xffffffffu, q, 0) + __popc(m & ((1u << lane) - 1));
+  }
+  __syncthreads();
+  if (tid == 0) sm.base = atomicAdd(fb.lroot_n, sm.nroot);   // tile-local roots, for k_ccl_link
+  // labels: warp wv writes rows 2 wv and 2 wv + 1, one lane per pixel, so a warp's stores are one row segment
+#pragma unroll
+  for (int j = 0; j < 4; j++) {
+    const int f = 4 * wv + j;
+    if ((flat[f] >> lane) & 1u) {
+      const int id = sm.rpref[f] + __popc(sm.start[f] & (0xffffffffu >> (31 - lane))) - 1;
+      label[(y0 + (f >> 1)) * w + x0 + 32 * (f & 1) + lane] = sm.glab[id];
+    }
   }
   __syncthreads();
   const int n = w * h;
 #pragma unroll
-  for (int k = 0; k < kMaxPer; k++) {
-    if (root[k] < 0) continue;
-    const int p = px[k];
-    const int ly = p >> 6, lx = p & (kTileW - 1);
-    const int gi = (y0 + ly) * w + x0 + lx;
-    const int r = root[k];
-    label[gi] = (y0 + (r >> 6)) * w + x0 + (r & (kTileW - 1));
-    if (r == p) {
-      cnt[gi] = a_cnt[p];
-      bbox[gi] = y0 + a_ymax[p];
-      bbox[n + gi] = x0 + a_xmin[p];
-      bbox[2 * n + gi] = x0 + a_xmax[p];
-      const int q = atomicAdd(fb.lroot_n, 1);   // tile-local roots, for k_ccl_link
-      if (q < fb.lroot_cap) fb.lroots[q] = gi;
-    }
+  for (int k = 0; k < kRunsPer; k++) {
+    if (!is_root[k]) continue;
+    const int t = tid + k * kTileThreads;
+    const int gi = sm.glab[t];
+    cnt[gi] = a_cnt[t];
+    bbox[gi] = y0 + a_ymax[t];
+    bbox[n + gi] = x0 + a_xmin[t];
+    bbox[2 * n + gi] = x0 + a_xmax[t];
+    const int q = sm.base + slot[k];
+    if (q < fb.lroot_cap) fb.lroots[q] = gi;
   }
 }
 
@@ -224,6 +243,7 @@ __global__ void __launch_bounds__(kTileThreads)
   const unsigned *__restrict__ edges = fb.edges;
   const int words_per_row = fb.words_per_row;
   __shared__ CclTileSmem sm;
+  __shared__ unsigned s_bits[kTileH][2];
   const int tid = threadIdx.x;
   const int x0 = blockIdx.x * kTileW, y0 = blockIdx.y * kTileH;
   // (counters and the local-root count are zeroed by k_ccl_reset, ahead of this launch)
@@ -233,10 +253,10 @@ __global__ void __launch_bounds__(kTileThreads)
     unsigned v = 0;
     if (gy < h && gw < words_per_row) v = edges[(size_t)gy * words_per_row + gw];
     if (gy < h && (gw << 5) + 32 > w) v &= (gw << 5) < w ? (0xffffffffu >> (32 - (w - (gw << 5)))) : 0u;   // beyond the frame
-    sm.bits[r][k] = v;
+    s_bits[r][k] = v;
   }
   __syncthreads();
-  ccl_tile_body(fb, sm, x0, y0, w, h);
+  ccl_tile_body(fb, sm, s_bits, x0, y0, w, h);
 }
 
 template <class B>
@@ -256,8 +276,9 @@ constexpr int kCnW = 64, kCnH = 16, kCnThreads = 256;
 template <class B>
 constexpr bool kFusedLabels = std::is_same<B, FldTable>::value;
 static_assert(kCnW == kTileW && kCnH == kTileH && kCnThreads == kTileThreads, "Canny tile = connected-component tile");
+constexpr int kCnPixW = kCnW + 8;   // staged columns: x0 - 4 ... x0 + 67, whole aligned words (the Sobel halo is x0 - 2 ... x0 + 65)
 struct CannySmem {
-  uint8_t pix[kCnH + 4][kCnW + 4];
+  uint8_t pix[kCnH + 4][kCnPixW];
   short sdx[kCnH + 2][kCnW + 2];
   short sdy[kCnH + 2][kCnW + 2];
   unsigned short mag[kCnH + 2][kCnW + 2];
@@ -281,11 +302,22 @@ __global__ void __launch_bounds__(kCnThreads)
   auto &mag = cs.mag;
   const int tx0 = blockIdx.x * kCnW, ty0 = blockIdx.y * kCnH;
   const int tid = threadIdx.x;
-  // pixels with a halo of 2, BORDER_REPLICATE
-  for (int i = tid; i < (kCnH + 4) * (kCnW + 4); i += kCnThreads) {
-    int r = i / (kCnW + 4), c = i - r * (kCnW + 4);
-    int gx = min(max(tx0 - 2 + c, 0), w - 1), gy = min(max(ty0 - 2 + r, 0), h - 1);
-    pix[r][c] = img[(size_t)gy * pitch + gx];
+  // pixels with a halo of 2, BORDER_REPLICATE: one 32-bit word per thread and step; a word that reaches beyond the frame
+  // (or an unaligned image) is read byte by byte with the coordinates clamped
+  const bool aligned = ((pitch | (int)(size_t)img) & 3) == 0;
+  for (int i = tid; i < (kCnH + 4) * (kCnPixW / 4); i += kCnThreads) {
+    const int r = i / (kCnPixW / 4), k = i - r * (kCnPixW / 4);
+    const int gy = min(max(ty0 - 2 + r, 0), h - 1), gx = tx0 - 4 + 4 * k;
+    const uint8_t *src = img + (size_t)gy * pitch;
+    unsigned v;
+    if (aligned && gx >= 0 && gx + 3 < w) {
+      v = __ldg(reinterpret_cast<const unsigned *>(src + gx));
+    } else {
+      v = 0;
+#pragma unroll
+      for (int j = 0; j < 4; j++) v |= (unsigned)src[min(max(gx + j, 0), w - 1)] << (8 * j);
+    }
+    *reinterpret_cast<unsigned *>(&pix[r][4 * k]) = v;
   }
   __syncthreads();
   // Sobel + L1 magnitude with a halo of 1; zero outside the image
@@ -294,8 +326,8 @@ __global__ void __launch_bounds__(kCnThreads)
     int gx = tx0 - 1 + c, gy = ty0 - 1 + r;
     int dx = 0, dy = 0, m = 0;
     if (gx >= 0 && gx < w && gy >= 0 && gy < h) {
-      const uint8_t *p = &pix[r + 1][c + 1];
-      const int s = kCnW + 4;
+      const uint8_t *p = &pix[r + 1][c + 3];
+      const int s = kCnPixW;
       dx = (p[-s + 1] + 2 * p[1] + p[s + 1]) - (p[-s - 1] + 2 * p[-1] + p[s - 1]);
       dy = (p[s - 1] + 2 * p[s] + p[s + 1]) - (p[-s - 1] + 2 * p[-s] + p[-s + 1]);
       m = abs(dx) + abs(dy);
@@ -340,11 +372,19 @@ __global__ void __launch_bounds__(kCnThreads)
   }
   if constexpr (kFuse) {
     __syncthreads();   // every warp is done with the gradient planes; the tile's bits are complete
-    CclTileSmem &ts = *reinterpret_cast<CclTileSmem *>(smem_raw);
-    if (tid < kCnH * 2) ts.bits[tid >> 1][tid & 1] = s_bits[tid >> 1][tid & 1];
-    __syncthreads();
-    ccl_tile_body(b.fld_of(blockIdx.z), ts, tx0, ty0, w, h);
+    ccl_tile_body(b.fld_of(blockIdx.z), *reinterpret_cast<CclTileSmem *>(smem_raw), s_bits, tx0, ty0, w, h);
   }
+}
+
+// Tile labelling of one frame's edge bits (fb.edges), as the line launches start it; for tests.
+void launch_ccl_tiles(FldBuffers &fb, int w, int h, cudaStream_t s) {
+  FldBatch b;
+  b.n = 1;
+  b.f[0] = fb;
+  PLVIWO_CARVEOUT(k_ccl_reset<FldBatch>);
+  k_ccl_reset<FldBatch><<<1, 32, 0, s>>>(b);
+  PLVIWO_CARVEOUT(k_ccl_tile<FldBatch>);
+  k_ccl_tile<FldBatch><<<dim3((w + kTileW - 1) / kTileW, (h + kTileH - 1) / kTileH, 1), kTileThreads, 0, s>>>(b, w, h);
 }
 
 template <class B>
