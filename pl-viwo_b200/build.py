@@ -26,9 +26,11 @@ SOURCES = [
     ("kernels_glue.cu", ["--fmad=false"]),
     ("fe_capi.cu", []),
     ("ransac.cpp", []),
+    ("state_blob.cpp", []),
     ("host_simd.cpp", []),
 ]
-HEADERS = ["fe_kernels.h", "fe_group_dev.h", "fe_group.h", "ransac_core.h", "fe_context.h", "fe_stereo.h", "tma_bulk.h", "introsort.h", os.path.join("..", "..", "include", "plviwo_fe.h")]
+HEADERS = ["fe_kernels.h", "fe_group_dev.h", "fe_group.h", "ransac_core.h", "tracker_core.h", "state_blob.h", "fe_context.h", "fe_stereo.h",
+           "tma_bulk.h", "introsort.h", os.path.join("..", "..", "include", "plviwo_fe.h")]
 
 
 def _nvcc() -> str:

@@ -43,6 +43,40 @@ struct EnvInit {
     return FE_INTERNAL;                           \
   }
 
+// Creation errors: the reason goes to plviwo_*_last_error(NULL).
+static int create_error(int code, const char *why) {
+  g_create_error = why;
+  return code;
+}
+
+// The config rules of every creator; tw x th is the size the tracker runs at (the handle's downsampled size, the raw size
+// elsewhere).  nullptr when they hold, otherwise the reason.
+static const char *check_config(const FeConfig &c, int tw, int th) {
+  if (c.width < 64 || c.height < 64 || c.width > 4095 || c.height > 4095) return "image size must be in [64, 4095]";
+  if (c.win_size < 3 || c.win_size > kMaxWin || (c.win_size & 1) == 0) return "win_size must be odd and in [3, 31]";
+  if (c.pyr_levels < 0 || c.pyr_levels >= kMaxLevels) return "pyr_levels must be in [0, 7]";
+  if (c.grid_x < 1 || c.grid_y < 1 || c.min_px_dist < 1 || c.num_features < 1) return "bad grid / distance / feature count";
+  if (c.histogram_method != FE_HIST_NONE && c.histogram_method != FE_HIST_HISTOGRAM && c.histogram_method != FE_HIST_CLAHE)
+    return "bad histogram_method";
+  if (c.use_lines) {
+    if ((tw & 1) || (th & 1)) return "line tracker needs even (tracking) image dimensions (exact 2x decimation)";
+    if (c.canny_th1 != c.canny_th2) return "canny_th1 != canny_th2: hysteresis pass is not implemented";
+    if (c.fld_length_threshold < 2) return "bad fld_length_threshold";
+  }
+  return nullptr;
+}
+
+// After the config checks: the device a creator is asked for exists.
+static int check_device(int device) {
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
+    cudaGetLastError();
+    return create_error(FE_NO_DEVICE, "no CUDA device: this front end has no CPU fallback");
+  }
+  if (device < 0 || device >= ndev) return create_error(FE_BAD_ARG, "device index out of range");
+  return FE_OK;
+}
+
 static int copy_rows(const void *src, int n, size_t elem, void *out, int cap, int *n_out) {
   if (n_out) *n_out = n;
   if (!out) return FE_OK;
@@ -100,30 +134,10 @@ int plviwo_fe_create(const FeConfig *cfg, int device, FeHandle **out) {
   API_BEGIN
   if (!cfg || !out) return FE_BAD_ARG;
   *out = nullptr;
-  auto bad = [&](const char *why) {
-    g_create_error = why;
-    return FE_BAD_ARG;
-  };
-  if (cfg->width < 64 || cfg->height < 64 || cfg->width > 4095 || cfg->height > 4095) return bad("image size must be in [64, 4095]");
-  if (cfg->win_size < 3 || cfg->win_size > kMaxWin || (cfg->win_size & 1) == 0) return bad("win_size must be odd and in [3, 31]");
-  if (cfg->pyr_levels < 0 || cfg->pyr_levels >= kMaxLevels) return bad("pyr_levels must be in [0, 7]");
-  if (cfg->grid_x < 1 || cfg->grid_y < 1 || cfg->min_px_dist < 1 || cfg->num_features < 1) return bad("bad grid / distance / feature count");
-  if (cfg->histogram_method != FE_HIST_NONE && cfg->histogram_method != FE_HIST_HISTOGRAM && cfg->histogram_method != FE_HIST_CLAHE)
-    return bad("bad histogram_method");
   const int tw = cfg->downsample ? (int)(cfg->width / 2.0) : cfg->width, th = cfg->downsample ? (int)(cfg->height / 2.0) : cfg->height;
-  if (cfg->downsample && (tw < 64 || th < 64)) return bad("downsampled image would be smaller than 64 pixels");
-  if (cfg->use_lines) {
-    if ((tw & 1) || (th & 1)) return bad("line tracker needs even (tracking) image dimensions (exact 2x decimation)");
-    if (cfg->canny_th1 != cfg->canny_th2) return bad("canny_th1 != canny_th2: hysteresis pass is not implemented");
-    if (cfg->fld_length_threshold < 2) return bad("bad fld_length_threshold");
-  }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-    cudaGetLastError();
-    g_create_error = "no CUDA device: this front end has no CPU fallback";
-    return FE_NO_DEVICE;
-  }
-  if (device < 0 || device >= ndev) return bad("device index out of range");
+  if (cfg->downsample && (tw < 64 || th < 64)) return create_error(FE_BAD_ARG, "downsampled image would be smaller than 64 pixels");
+  if (const char *why = check_config(*cfg, tw, th)) return create_error(FE_BAD_ARG, why);
+  if (int rc = check_device(device)) return rc;
   FeContext *ctx = new FeContext(*cfg, device);
   int rc = ctx->init();
   if (rc != FE_OK) {
@@ -790,31 +804,11 @@ int plviwo_fe_group_create(const FeConfig *cfg, int n_streams, int device, FeGro
   API_BEGIN
   if (!cfg || !out) return FE_BAD_ARG;
   *out = nullptr;
-  auto bad = [&](const char *why) {
-    g_create_error = why;
-    return FE_BAD_ARG;
-  };
-  if (n_streams < 1 || n_streams > 4096) return bad("n_streams must be in [1, 4096]");
-  if (cfg->width < 64 || cfg->height < 64 || cfg->width > 4095 || cfg->height > 4095) return bad("image size must be in [64, 4095]");
-  if (cfg->win_size < 3 || cfg->win_size > kMaxWin || (cfg->win_size & 1) == 0) return bad("win_size must be odd and in [3, 31]");
-  if (cfg->pyr_levels < 0 || cfg->pyr_levels >= kMaxLevels) return bad("pyr_levels must be in [0, 7]");
-  if (cfg->grid_x < 1 || cfg->grid_y < 1 || cfg->min_px_dist < 1 || cfg->num_features < 1) return bad("bad grid / distance / feature count");
-  if (cfg->grid_x * cfg->grid_y > 256) return bad("a stream group supports at most 256 grid cells");
-  if (cfg->histogram_method != FE_HIST_NONE && cfg->histogram_method != FE_HIST_HISTOGRAM && cfg->histogram_method != FE_HIST_CLAHE)
-    return bad("bad histogram_method");
-  if (cfg->downsample) return bad("cfg.downsample is not supported in a stream group");
-  if (cfg->use_lines) {
-    if ((cfg->width & 1) || (cfg->height & 1)) return bad("line tracker needs even image dimensions (exact 2x decimation)");
-    if (cfg->canny_th1 != cfg->canny_th2) return bad("canny_th1 != canny_th2: hysteresis pass is not implemented");
-    if (cfg->fld_length_threshold < 2) return bad("bad fld_length_threshold");
-  }
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-    cudaGetLastError();
-    g_create_error = "no CUDA device: this front end has no CPU fallback";
-    return FE_NO_DEVICE;
-  }
-  if (device < 0 || device >= ndev) return bad("device index out of range");
+  if (n_streams < 1 || n_streams > 4096) return create_error(FE_BAD_ARG, "n_streams must be in [1, 4096]");
+  if (cfg->downsample) return create_error(FE_BAD_ARG, "cfg.downsample is not supported in a stream group");
+  if (const char *why = check_config(*cfg, cfg->width, cfg->height)) return create_error(FE_BAD_ARG, why);
+  if (cfg->grid_x * cfg->grid_y > 256) return create_error(FE_BAD_ARG, "a stream group supports at most 256 grid cells");
+  if (int rc = check_device(device)) return rc;
   FeGroup *grp = new FeGroup(*cfg, n_streams, device);
   int rc = grp->init();
   if (rc != FE_OK) {
@@ -944,28 +938,9 @@ int plviwo_fe_stereo_create(const FeConfig *cfg, const double K_right[4], const 
   API_BEGIN
   if (!cfg || !out) return FE_BAD_ARG;
   *out = nullptr;
-  auto bad = [&](const char *why) {
-    g_create_error = why;
-    return FE_BAD_ARG;
-  };
-  if (cfg->width < 64 || cfg->height < 64 || cfg->width > 4095 || cfg->height > 4095) return bad("image size must be in [64, 4095]");
-  if (cfg->win_size < 3 || cfg->win_size > kMaxWin || (cfg->win_size & 1) == 0) return bad("win_size must be odd and in [3, 31]");
-  if (cfg->pyr_levels < 0 || cfg->pyr_levels >= kMaxLevels) return bad("pyr_levels must be in [0, 7]");
-  if (cfg->grid_x < 1 || cfg->grid_y < 1 || cfg->min_px_dist < 1 || cfg->num_features < 1) return bad("bad grid / distance / feature count");
-  if (cfg->histogram_method != FE_HIST_NONE && cfg->histogram_method != FE_HIST_HISTOGRAM && cfg->histogram_method != FE_HIST_CLAHE)
-    return bad("bad histogram_method");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-    cudaGetLastError();
-    g_create_error = "no CUDA device: this front end has no CPU fallback";
-    return FE_NO_DEVICE;
-  }
-  if (device < 0 || device >= ndev) return bad("device index out of range");
-  if (cfg->use_lines) {
-    if ((cfg->width & 1) || (cfg->height & 1)) return bad("line tracker needs even image dimensions (exact 2x decimation)");
-    if (cfg->canny_th1 != cfg->canny_th2) return bad("canny_th1 != canny_th2: hysteresis pass is not implemented");
-    if (cfg->fld_length_threshold < 2) return bad("bad fld_length_threshold");
-  }
+  // the rig tracks at the raw size: it zeroes cfg.downsample
+  if (const char *why = check_config(*cfg, cfg->width, cfg->height)) return create_error(FE_BAD_ARG, why);
+  if (int rc = check_device(device)) return rc;
   FeStereo *st = new FeStereo(*cfg, K_right, D_right, device);
   int rc = st->init();
   if (rc != FE_OK) {

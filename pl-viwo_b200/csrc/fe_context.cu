@@ -9,6 +9,7 @@
 // submit() on its own streams; collect() runs the state-dependent chain (top-off detection on the previous
 // image, LK, RANSAC gate, line association) in frame order.
 #include "fe_context.h"
+#include "state_blob.h"
 
 #include <algorithm>
 #include <chrono>
@@ -23,8 +24,6 @@ namespace plviwo {
     cudaError_t e__ = (call);                          \
     if (e__ != cudaSuccess) return fail(e__, #call);   \
   } while (0)
-
-static inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
 
 namespace {
 struct HostTimer {  // accumulates wall time into FeStageTimes::host_ms[idx]
@@ -139,15 +138,6 @@ void FeContext::reset_times() {
   times_ = FeStageTimes{};
 }
 
-int FeContext::alloc_image(DevImage &im, int w, int h) {
-  im.w = w;
-  im.h = h;
-  im.pitch = align_up(w, 256);
-  FE_CUDA(cudaMalloc(&im.p, (size_t)im.pitch * h + 256));
-  FE_CUDA(cudaMemset(im.p, 0, (size_t)im.pitch * h + 256));
-  return FE_OK;
-}
-
 int FeContext::init() {
   FE_CUDA(cudaSetDevice(device_));
   int lo = 0, hi = 0;
@@ -169,26 +159,20 @@ int FeContext::init() {
   slots_.resize(nslots);
   for (int i = 0; i < nslots; i++) slots_[i].index = i;
   for (FrameSlot &s : slots_) {
-    int rc = alloc_image(s.raw, W_, H_);
-    if (rc) return rc;
-    if (cfg_.downsample) {
-      rc = alloc_image(s.raw_in, Win_, Hin_);
-      if (rc) return rc;
-    }
+    FE_CUDA(alloc_image(s.raw, W_, H_));
+    if (cfg_.downsample) FE_CUDA(alloc_image(s.raw_in, Win_, Hin_));
     // cv::buildOpticalFlowPyramid: a level is kept while both sides stay > winSize
     int w = W_, h = H_;
     s.pyr.n = 0;
     for (int l = 0; l <= cfg_.pyr_levels && l < kMaxLevels; l++) {
-      rc = alloc_image(s.pyr.lvl[l], w, h);
-      if (rc) return rc;
+      FE_CUDA(alloc_image(s.pyr.lvl[l], w, h));
       s.pyr.n = l + 1;
       w = (w + 1) / 2;
       h = (h + 1) / 2;
       if (w <= cfg_.win_size || h <= cfg_.win_size) break;
     }
     if (cfg_.use_lines) {
-      rc = alloc_image(s.half, W_ / 2, H_ / 2);
-      if (rc) return rc;
+      FE_CUDA(alloc_image(s.half, W_ / 2, H_ / 2));
       FldBuffers &fb = s.fld;
       if (fb.alloc(W_ / 2, H_ / 2, cfg_.fld_length_threshold, 4096)) return fail(cudaGetLastError(), "FldBuffers::alloc");
       FE_CUDA(cudaMallocHost(&s.h_segs, (size_t)fb.out_cap * sizeof(float4)));
@@ -415,21 +399,8 @@ int FeContext::set_num_features(int n) {
 
 // cells x num_features_grid of the Grider_GRID layout for a feature count (layout_cells)
 int FeContext::cand_table_size(int num_features) const {
-  const int gx = cfg_.grid_x, gy = cfg_.grid_y;
-  int ggx = gx, ggy = gy;
-  if (num_features < ggx * ggy) {
-    double ratio = (double)ggx / (double)ggy;
-    ggy = (int)std::ceil(std::sqrt(num_features / ratio));
-    ggx = (int)std::ceil(ggy * ratio);
-  }
-  const int nfg = (int)((double)num_features / (double)(ggx * ggy)) + 1;
-  const int csx = W_ / ggx, csy = H_ / ggy;
-  int ncell = 0;
-  if (csx > 0 && csy > 0)
-    for (int x = 0; x < gx; x++)
-      for (int y = 0; y < gy; y++)
-        if (x * csx + csx <= W_ && y * csy + csy <= H_) ncell++;
-  return ncell * nfg;
+  const GriderLayout L = grider_layout(W_, H_, cfg_.grid_x, cfg_.grid_y, num_features);
+  return (int)L.cells.size() * L.nfg;
 }
 
 int FeContext::set_currid(uint64_t id) {
@@ -439,22 +410,6 @@ int FeContext::set_currid(uint64_t id) {
   }
   currid_ = id;
   return FE_OK;
-}
-
-// cv::undistortPoints on one point (Appendix A6) — only for the two endpoints of each line row
-void FeContext::undistort_host(const double K[4], const double D[4], float u, float v, float &un, float &vn) {
-  double x0 = ((double)u - K[2]) / K[0], y0 = ((double)v - K[3]) / K[1];
-  double x = x0, y = y0;
-  for (int j = 0; j < 5; j++) {
-    double r2 = x * x + y * y;
-    double icdist = 1.0 / (1.0 + (D[1] * r2 + D[0]) * r2);
-    double dx = 2 * D[2] * x * y + D[3] * (r2 + 2 * x * x);
-    double dy = D[2] * (r2 + 2 * y * y) + 2 * D[3] * x * y;
-    x = (x0 - dx) * icdist;
-    y = (y0 - dy) * icdist;
-  }
-  un = (float)x;
-  vn = (float)y;
 }
 
 // ------------------------------------------------------------------------------------------------ submit
@@ -477,12 +432,12 @@ int FeContext::record_image_path(FrameSlot &s, cudaStream_t st) {
 }
 
 int FeContext::record_fast_path(FrameSlot &s, cudaStream_t st) {
-  const int ncell = (int)cells_.size(), nb = cells_nb_;
+  const int ncell = (int)cells_.cells.size(), nb = cells_.n_bands;
   if (ncell > 0) {
-    const int nfg = cells_nfg_, ntab_c = ncell * nfg;
+    const int nfg = cells_.nfg, ntab_c = ncell * nfg;
     FE_CUDA(cudaMemsetAsync(s.d_fast_total, 0, 2 * sizeof(unsigned), st));
     if (timing) cudaEventRecord(s.ev_fast_t[0], st);
-    launch_fast(s.pyr.lvl[0], d_cells_, ncell, nb, cells_csx_, cfg_.fast_threshold, s.d_fast_total, s.d_band_off, s.d_band_cnt,
+    launch_fast(s.pyr.lvl[0], d_cells_, ncell, nb, cells_.csx, cfg_.fast_threshold, s.d_fast_total, s.d_band_off, s.d_band_cnt,
                 s.d_kps, kps_cap_, st);
     // Grider_GRID.h:128-133 and :163-179 on the device: per-cell std::sort + top num_features_grid, then cornerSubPix of
     // every survivor.  Only the candidate table (a few KB) goes back to the host.
@@ -613,11 +568,11 @@ int FeContext::enqueue_frame_independent(FrameSlot &s) {
   }
   s.warmed = true;
   // bookkeeping (identical for both ways of issuing the work)
-  const int ncell = (int)cells_.size(), ntab = ncell * cells_nb_;
+  const int ncell = (int)cells_.cells.size(), ntab = ncell * cells_.n_bands;
   mst_.kernel_launches_total += (cfg_.histogram_method != FE_HIST_NONE ? 1 : 0) + 1 + std::max(s.pyr.n - 2, 0) +
                                  (ncell > 0 ? 3 : 0) + 1 + (lines && !batched ? 13 : 0);
   (void)ntab;
-  if (ncell > 0) mst_.d2h_bytes += (size_t)ncell * sizeof(int) + (size_t)2 * ncell * cells_nfg_ * sizeof(float2);
+  if (ncell > 0) mst_.d2h_bytes += (size_t)ncell * sizeof(int) + (size_t)2 * ncell * cells_.nfg * sizeof(float2);
   if (lines) mst_.d2h_bytes += 2 * sizeof(int) + 1024 * sizeof(float4);
   return FE_OK;
 }
@@ -789,31 +744,7 @@ int FeContext::submit_impl(double t, const uint8_t *image, int stride, bool on_d
 
 // ------------------------------------------------------------------------------------------ pre-detection
 void FeContext::layout_cells() {
-  // Grider_GRID geometry (Grider_GRID.h:88-100): the grider may shrink ITS grid when num_features < grid_x * grid_y
-  // while the cell indices still come from the caller's grid; cells that leave the image are skipped (:117-118)
-  const int gx = cfg_.grid_x, gy = cfg_.grid_y;
-  int ggx = gx, ggy = gy;
-  if (cfg_.num_features < ggx * ggy) {
-    double ratio = (double)ggx / (double)ggy;
-    ggy = (int)std::ceil(std::sqrt(cfg_.num_features / ratio));
-    ggx = (int)std::ceil(ggy * ratio);
-  }
-  cells_nfg_ = (int)((double)cfg_.num_features / (double)(ggx * ggy)) + 1;
-  cells_csx_ = W_ / ggx;
-  cells_csy_ = H_ / ggy;
-  cells_.clear();
-  cell_of_loc_.assign((size_t)gx * gy, -1);
-  if (cells_csx_ > 0 && cells_csy_ > 0) {
-    for (int x = 0; x < gx; x++)
-      for (int y = 0; y < gy; y++) {
-        int px = x * cells_csx_, py = y * cells_csy_;
-        if (px + cells_csx_ > W_ || py + cells_csy_ > H_) continue;
-        if ((int)cells_.size() >= max_cells_) continue;
-        cell_of_loc_[(size_t)x * gy + y] = (int)cells_.size();
-        cells_.push_back(FastCell{px, py, cells_csx_, cells_csy_});
-      }
-  }
-  cells_nb_ = cells_csy_ > 0 ? (cells_csy_ + kFastBandRows - 1) / kFastBandRows : 0;
+  cells_ = grider_layout(W_, H_, cfg_.grid_x, cfg_.grid_y, cfg_.num_features);
   cells_num_features_ = cfg_.num_features;
   cells_uploaded_ = false;
 }
@@ -826,15 +757,15 @@ int FeContext::enqueue_fast_all_cells(FrameSlot &s) {
     layout_cells();
     layout_version_++;
   }
-  if (!cells_uploaded_ && !cells_.empty()) {
-    FE_CUDA(cudaMemcpy(d_cells_, cells_.data(), cells_.size() * sizeof(FastCell), cudaMemcpyHostToDevice));
+  if (!cells_uploaded_ && !cells_.cells.empty()) {
+    FE_CUDA(cudaMemcpy(d_cells_, cells_.cells.data(), cells_.cells.size() * sizeof(FastCell), cudaMemcpyHostToDevice));
     cells_uploaded_ = true;
   }
-  s.cells = cells_;
-  s.cell_of_loc = cell_of_loc_;
-  s.predet_ncell = (int)cells_.size();
-  s.predet_nb = cells_nb_;
-  s.predet_nfg = cells_nfg_;
+  s.cells = cells_.cells;
+  s.cell_of_loc = cells_.cell_of_loc;
+  s.predet_ncell = (int)cells_.cells.size();
+  s.predet_nb = cells_.n_bands;
+  s.predet_nfg = cells_.nfg;
   s.predet_num_features = cfg_.num_features;
   s.predet_state.store(1);
   return FE_OK;
@@ -1528,44 +1459,6 @@ int FeContext::perform_matching(const FrameSlot &f0, FrameSlot &f1, std::vector<
 }
 
 // -------------------------------------------------------------------------------------------- TrackLSD
-namespace {
-// TrackLSD::PointLineDistance (TrackLSD.cpp:794-814): float arithmetic, std::pow(float,int) promotes to double
-float point_line_distance(const float4 &line, float x0, float y0) {
-  float x1 = line.x, y1 = line.y, x2 = line.z, y2 = line.w;
-  float cross = (x2 - x1) * (x0 - x1) + (y2 - y1) * (y0 - y1);
-  if (cross <= 0) return std::sqrt((x0 - x1) * (x0 - x1) + (y0 - y1) * (y0 - y1));
-  float d = (x2 - x1) * (x2 - x1) + (y2 - y1) * (y2 - y1);
-  if (cross > d) return std::sqrt((x0 - x2) * (x0 - x2) + (y0 - y2) * (y0 - y2));
-  return (float)std::abs(std::fabs((y2 - y1) * x0 + (x1 - x2) * y0 + ((x2 * y1) - (x1 * y2))) /
-                         (std::sqrt(std::pow((double)(y2 - y1), 2) + std::pow((double)(x1 - x2), 2))));
-}
-// TrackLSD::LineSimilar (:816-830)
-bool line_similar(const float4 &line2, const float4 &line1) {
-  float mx = (line1.x + line1.z) / 2, my = (line1.y + line1.w) / 2;
-  return point_line_distance(line2, mx, my) <= 6;
-}
-// TrackLSD::LineClass (:335-366), including atan(dy) / dx at :350-351
-bool line_class(const float4 &line, double vx, double vy) {
-  double s[3] = {line.x, line.y, 1}, e[3] = {line.z, line.w, 1};
-  double mid[3] = {(s[0] + e[0]) / 2, (s[1] + e[1]) / 2, (s[2] + e[2]) / 2};
-  double v3[3] = {vx, vy, 1};
-  double ln[3] = {mid[1] * v3[2] - mid[2] * v3[1], mid[2] * v3[0] - mid[0] * v3[2], mid[0] * v3[1] - mid[1] * v3[0]};
-  double dis_error = (std::abs(ln[0] * s[0] + ln[1] * s[1] + ln[2] * s[2]) + std::abs(ln[0] * e[0] + ln[1] * e[1] + ln[2] * e[2])) /
-                     (2 * std::sqrt(ln[0] * ln[0] + ln[1] * ln[1]));
-  dis_error = std::abs(dis_error);
-  double angle1 = std::atan(line.y - line.w) / (line.x - line.z);   // float arithmetic, as written in the reference
-  double angle2 = std::atan(mid[1] - vy) / (mid[0] - vx);
-  double angle_error = std::abs(angle1 - angle2);
-  return dis_error <= 5.0 && angle_error <= 0.35;
-}
-int line_classification(const float4 &line, const double vp[6]) {  // :318-333
-  if (line_class(line, vp[4], vp[5])) return 3;
-  if (line_class(line, vp[2], vp[3])) return 2;
-  if (line_class(line, vp[0], vp[1])) return 1;
-  return 0;
-}
-}  // namespace
-
 // TrackLSD::AssignPointToLines (:744-792): per line the points inside its (mis-indexed, :754-757) bounding box and within
 // 5 px of the SEGMENT; lines without a point are dropped.  The candidate test of one line against all points is
 // vectorised (line_candidates, host_simd.cpp); survivors go through the exact PointLineDistance.
@@ -1721,8 +1614,8 @@ int FeContext::lsd_feed(FrameSlot &cur) {
     r.id = good_ids[i];
     const float4 &l = filt_lines[i];
     r.line[0] = l.x; r.line[1] = l.y; r.line[2] = l.z; r.line[3] = l.w;
-    undistort_host(cur.K, cur.D, l.x, l.y, r.line_n[0], r.line_n[1]);
-    undistort_host(cur.K, cur.D, l.z, l.w, r.line_n[2], r.line_n[3]);
+    const float2 n0 = undistort_radtan(make_float2(l.x, l.y), cur.K, cur.D), n1 = undistort_radtan(make_float2(l.z, l.w), cur.K, cur.D);
+    r.line_n[0] = n0.x; r.line_n[1] = n0.y; r.line_n[2] = n1.x; r.line_n[3] = n1.y;
     r.D = line_classification(l, cur.vp);
     r.n_pts = (int)pol_new[i].size();
     r.pt_offset = (int)line_points.size();
@@ -1752,16 +1645,6 @@ int FeContext::classify_lines(const double vp[6]) {
 }
 
 // ------------------------------------------------------------------------------------------ state / taps
-namespace {
-struct StateHeader {
-  uint32_t magic, version;
-  int32_t w, h;
-  uint64_t currid, line_currid;
-  int32_t n_pts, n_lines, has_image, has_mask;
-  int32_t n_pol_entries, reserved;
-};
-}  // namespace
-
 // Both are only legal between frames (nothing in flight): the tracker threads are idle then and their state is visible
 // to the caller's thread through the release/acquire pair on FrameSlot::stage.
 int FeContext::get_state(void *buf, size_t cap, size_t *n_bytes) {
@@ -1772,43 +1655,19 @@ int FeContext::get_state(void *buf, size_t cap, size_t *n_bytes) {
   int rc = [&]() -> int {
   FE_CUDA(cudaSetDevice(device_));
   const int last_slot_ = klt_last_slot_;
-  StateHeader hd;
-  std::memset(&hd, 0, sizeof(hd));
-  hd.magic = 0x504c5657u;
-  hd.version = 1;
-  hd.w = W_;
-  hd.h = H_;
-  hd.currid = currid_;
-  hd.line_currid = line_currid_;
-  hd.n_pts = (int)pts_last_.size();
-  hd.n_lines = (int)lines_last_.size();
-  hd.has_image = last_slot_ >= 0 ? 1 : 0;
-  hd.has_mask = (last_slot_ >= 0 && !slots_[last_slot_].mask.empty()) ? 1 : 0;
-  int npol = 0;
-  for (auto &m : pol_last_) npol += (int)m.size();
-  hd.n_pol_entries = npol;
-  size_t need = sizeof(hd) + (size_t)hd.n_pts * (sizeof(Pt) + sizeof(uint64_t)) +
-                (size_t)hd.n_lines * (sizeof(float4) + sizeof(uint64_t) + sizeof(int32_t)) +
-                (size_t)npol * (sizeof(int32_t) + sizeof(double)) + (hd.has_image ? (size_t)W_ * H_ : 0) +
-                (hd.has_mask ? (size_t)W_ * H_ : 0);
-  if (n_bytes) *n_bytes = need;
-  if (!buf || cap < need) return buf ? FE_OVERFLOW : FE_OK;
+  const bool has_image = last_slot_ >= 0;
+  const StateHeader hd = state_header(W_, H_, currid_, line_currid_, (int)pts_last_.size(), (int)lines_last_.size(), pol_last_,
+                                      has_image, has_image && !slots_[last_slot_].mask.empty());
+  const StateLayout at = state_layout(hd);
+  if (n_bytes) *n_bytes = at.size;
+  if (!buf || cap < at.size) return buf ? FE_OVERFLOW : FE_OK;
   uint8_t *p = static_cast<uint8_t *>(buf);
-  auto put = [&](const void *src, size_t n) { std::memcpy(p, src, n); p += n; };
-  put(&hd, sizeof(hd));
-  put(pts_last_.data(), pts_last_.size() * sizeof(Pt));
-  put(ids_last_.data(), ids_last_.size() * sizeof(uint64_t));
-  put(lines_last_.data(), lines_last_.size() * sizeof(float4));
-  put(line_ids_last_.data(), line_ids_last_.size() * sizeof(uint64_t));
-  for (auto &m : pol_last_) { int32_t k = (int32_t)m.size(); put(&k, sizeof(k)); }
-  for (auto &m : pol_last_)
-    for (auto &kv : m) { int32_t k = kv.first; put(&k, sizeof(k)); put(&kv.second, sizeof(double)); }
+  state_write(p, hd, pts_last_.data(), ids_last_.data(), lines_last_.data(), line_ids_last_.data(), pol_last_);
   if (hd.has_image) {
     const DevImage &l0 = slots_[last_slot_].pyr.lvl[0];
-    FE_CUDA(cudaMemcpy2D(p, W_, l0.p, l0.pitch, W_, H_, cudaMemcpyDeviceToHost));
-    p += (size_t)W_ * H_;
+    FE_CUDA(cudaMemcpy2D(p + at.image, W_, l0.p, l0.pitch, W_, H_, cudaMemcpyDeviceToHost));
   }
-  if (hd.has_mask) put(slots_[last_slot_].mask.data(), (size_t)W_ * H_);
+  if (hd.has_mask) std::memcpy(p + at.mask, slots_[last_slot_].mask.data(), (size_t)W_ * H_);
   return FE_OK;
   }();
   if (rc == FE_CUDA_ERROR) last_error = t_err;
@@ -1816,56 +1675,30 @@ int FeContext::get_state(void *buf, size_t cap, size_t *n_bytes) {
 }
 
 int FeContext::set_state(const void *buf, size_t n_bytes) {
-  if (!buf || n_bytes < sizeof(StateHeader) || !queue_.empty()) return FE_BAD_ARG;
+  if (!queue_.empty()) {
+    last_error = "set_state: collect the pending frames first";
+    return FE_BAD_ARG;
+  }
+  // parse into temporaries: the tracker state is only replaced once the whole blob has been checked
+  StateView v;
+  if (const char *why = state_read(buf, n_bytes, W_, H_, v)) {
+    last_error = why;
+    return FE_BAD_ARG;
+  }
+  const StateHeader &hd = v.hd;
   int rc = [&]() -> int {
   FE_CUDA(cudaSetDevice(device_));
-  const uint8_t *p = static_cast<const uint8_t *>(buf);
-  StateHeader hd;
-  std::memcpy(&hd, p, sizeof(hd));
-  p += sizeof(hd);
-  if (hd.magic != 0x504c5657u || hd.version != 1 || hd.w != W_ || hd.h != H_) return FE_BAD_ARG;
-  if (hd.n_pts < 0 || hd.n_lines < 0 || hd.n_pol_entries < 0) return FE_BAD_ARG;
-  {   // the blob must hold everything its header announces (a truncated or foreign buffer is rejected, not read past)
-    const size_t need = sizeof(hd) + (size_t)hd.n_pts * (sizeof(Pt) + sizeof(uint64_t)) +
-                        (size_t)hd.n_lines * (sizeof(float4) + sizeof(uint64_t) + sizeof(int32_t)) +
-                        (size_t)hd.n_pol_entries * (sizeof(int32_t) + sizeof(double)) + (hd.has_image ? (size_t)W_ * H_ : 0) +
-                        (hd.has_image && hd.has_mask ? (size_t)W_ * H_ : 0);
-    if (n_bytes < need) return FE_BAD_ARG;
-  }
-  auto get = [&](void *dst, size_t n) { std::memcpy(dst, p, n); p += n; };
-  // parse into temporaries: the tracker state is only replaced once the whole blob has been checked
-  std::vector<Pt> t_pts(hd.n_pts);
-  std::vector<uint64_t> t_ids(hd.n_pts);
-  get(t_pts.data(), (size_t)hd.n_pts * sizeof(Pt));
-  get(t_ids.data(), (size_t)hd.n_pts * sizeof(uint64_t));
-  std::vector<float4> t_lines(hd.n_lines);
-  std::vector<uint64_t> t_lids(hd.n_lines);
-  get(t_lines.data(), (size_t)hd.n_lines * sizeof(float4));
-  get(t_lids.data(), (size_t)hd.n_lines * sizeof(uint64_t));
-  std::vector<int32_t> sizes(hd.n_lines);
-  get(sizes.data(), (size_t)hd.n_lines * sizeof(int32_t));
-  long long tot = 0;
-  for (int32_t v : sizes) {
-    if (v < 0) return FE_BAD_ARG;
-    tot += v;
-  }
-  if (tot != hd.n_pol_entries) return FE_BAD_ARG;   // the entries the lines announce are the entries the blob holds
-  std::vector<std::map<int, double>> t_pol(hd.n_lines);
-  for (int i = 0; i < hd.n_lines; i++)
-    for (int k = 0; k < sizes[i]; k++) {
-      int32_t key;
-      double val;
-      get(&key, sizeof(key));
-      get(&val, sizeof(val));
-      t_pol[i][key] = val;
-    }
   currid_ = hd.currid;
   line_currid_ = hd.line_currid;
-  pts_last_.swap(t_pts);
-  ids_last_.swap(t_ids);
-  lines_last_.swap(t_lines);
-  line_ids_last_.swap(t_lids);
-  pol_last_.swap(t_pol);
+  pts_last_.resize(hd.n_pts);
+  ids_last_.resize(hd.n_pts);
+  lines_last_.resize(hd.n_lines);
+  line_ids_last_.resize(hd.n_lines);
+  std::memcpy(pts_last_.data(), v.base + v.at.pts, (size_t)hd.n_pts * sizeof(Pt));
+  std::memcpy(ids_last_.data(), v.base + v.at.ids, (size_t)hd.n_pts * sizeof(uint64_t));
+  std::memcpy(lines_last_.data(), v.base + v.at.lines, (size_t)hd.n_lines * sizeof(float4));
+  std::memcpy(line_ids_last_.data(), v.base + v.at.line_ids, (size_t)hd.n_lines * sizeof(uint64_t));
+  pol_last_.swap(v.pol);
   for (FrameSlot &s : slots_) {
     s.busy = false;
   }
@@ -1883,8 +1716,7 @@ int FeContext::set_state(const void *buf, size_t n_bytes) {
   if (hd.has_image) {
     FrameSlot &s = slots_[0];
     s.busy = true;
-    FE_CUDA(cudaMemcpy2DAsync(s.raw.p, s.raw.pitch, p, W_, W_, H_, cudaMemcpyHostToDevice, s.s_a));
-    p += (size_t)W_ * H_;
+    FE_CUDA(cudaMemcpy2DAsync(s.raw.p, s.raw.pitch, v.base + v.at.image, W_, W_, H_, cudaMemcpyHostToDevice, s.s_a));
     // the stored image is already equalised: rebuild the pyramid from it without a LUT
     launch_eq_pyr1(s.raw, s.d_hist, s.d_counters, 0, s.pyr.lvl[0], s.pyr.n > 1 ? s.pyr.lvl[1] : DevImage(),
                    cfg_.use_lines ? s.half : DevImage(), s.s_a);
@@ -1900,12 +1732,8 @@ int FeContext::set_state(const void *buf, size_t n_bytes) {
       s.seq_fast++;
       FE_CUDA(cudaEventRecord(s.ev_fast, s.s_b));
     }
-    if (hd.has_mask) {
-      s.mask.resize((size_t)W_ * H_);
-      get(s.mask.data(), (size_t)W_ * H_);
-    } else {
-      s.mask.clear();
-    }
+    if (hd.has_mask) s.mask.assign(v.base + v.at.mask, v.base + v.at.mask + (size_t)W_ * H_);
+    else s.mask.clear();
     last_slot_ = 0;
     klt_last_slot_ = 0;
     prev_submit_slot_ = 0;
@@ -1934,29 +1762,14 @@ int FeContext::tap(int what, void *buf, size_t cap, size_t *n_bytes) {
   if (what == FE_TAP_SUBPIX_LAST) return copy_vec(tap_subpix_.data(), tap_subpix_.size() * sizeof(float));
   if (what == FE_TAP_FLD_LAST) return copy_vec(tap_fld_.data(), tap_fld_.size() * sizeof(float));
   if (si < 0) return FE_BAD_ARG;
-  FrameSlot &s = slots_[si];
+  const FrameSlot &s = slots_[si];
   FE_CUDA(cudaDeviceSynchronize());
-  if (what >= FE_TAP_PYR_LEVEL0 && what < FE_TAP_PYR_LEVEL0 + kMaxLevels) {
-    int l = what - FE_TAP_PYR_LEVEL0;
-    if (l >= s.pyr.n) return FE_BAD_ARG;
-    const DevImage &im = s.pyr.lvl[l];
-    size_t n = (size_t)im.w * im.h;
-    if (n_bytes) *n_bytes = n;
-    if (!buf) return FE_OK;
-    if (cap < n) return FE_OVERFLOW;
-    FE_CUDA(cudaMemcpy2D(buf, im.w, im.p, im.pitch, im.w, im.h, cudaMemcpyDeviceToHost));
-    return FE_OK;
-  }
-  if (what == FE_TAP_HALF && cfg_.use_lines) {
-    const DevImage &im = s.half;
-    size_t n = (size_t)im.w * im.h;
-    if (n_bytes) *n_bytes = n;
-    if (!buf) return FE_OK;
-    if (cap < n) return FE_OVERFLOW;
-    FE_CUDA(cudaMemcpy2D(buf, im.w, im.p, im.pitch, im.w, im.h, cudaMemcpyDeviceToHost));
-    return FE_OK;
-  }
-  return FE_BAD_ARG;
+  const DevImage *im = nullptr;
+  if (what >= FE_TAP_PYR_LEVEL0 && what < FE_TAP_PYR_LEVEL0 + kMaxLevels && what - FE_TAP_PYR_LEVEL0 < s.pyr.n) im = &s.pyr.lvl[what - FE_TAP_PYR_LEVEL0];
+  if (what == FE_TAP_HALF && cfg_.use_lines) im = &s.half;
+  if (!im) return FE_BAD_ARG;
+  const int rc = tap_image(*im, buf, cap, n_bytes);
+  return rc == FE_CUDA_ERROR ? fail(cudaGetLastError(), "tap: cudaMemcpy2D") : rc;
 }
 
 }  // namespace plviwo

@@ -16,6 +16,7 @@
 
 #include "../../include/plviwo_fe.h"
 #include "fe_kernels.h"
+#include "tracker_core.h"
 
 namespace plviwo {
 
@@ -200,7 +201,6 @@ class FeContext {
   void line_main();
   int spin_sync(cudaStream_t st);
   int wait_flag(volatile int *flag, int value, cudaStream_t st, std::string *err);
-  int alloc_image(DevImage &im, int w, int h);
   int enqueue_frame_independent(FrameSlot &s);
   int record_image_path(FrameSlot &s, cudaStream_t st);
   int record_fast_path(FrameSlot &s, cudaStream_t st);
@@ -226,7 +226,6 @@ class FeContext {
   int track_candidates(FrameSlot &prev, FrameSlot &s);
   // TrackLSD
   int lsd_feed(FrameSlot &cur);
-  static void undistort_host(const double K[4], const double D[4], float u, float v, float &un, float &vn);
 
   FeConfig cfg_;
   bool external_ = false;   // the frame-independent pipeline only: a FeStereo owns the tracker state and the slots
@@ -260,9 +259,8 @@ class FeContext {
 
   // ---- detection: static cell layout + worker
   FastCell *d_cells_ = nullptr;
-  std::vector<FastCell> cells_;            // every in-image cell, x-major like valid_locs
-  std::vector<int> cell_of_loc_;           // caller-grid (x * grid_y + y) -> index into cells_ or -1
-  int cells_nfg_ = 0, cells_nb_ = 0, cells_csx_ = 0, cells_csy_ = 0, cells_num_features_ = -1;
+  GriderLayout cells_;                     // the layout of cells_num_features_
+  int cells_num_features_ = -1;
   int max_cells_ = 0, max_bands_ = 0, kps_cap_ = 0, cand_cap_ = 0;
   bool cells_uploaded_ = false;
   int layout_version_ = 0;

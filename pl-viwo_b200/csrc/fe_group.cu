@@ -3,6 +3,7 @@
 //   viw::TrackLSD::feed_new_camera / feed_monocular          PL-VIWO/src/update/cam/TrackLSD.cpp:39-192
 //   the bag loop feeding every camera in time order           PL-VIWO/src/run_bag.cpp:272-340
 #include "fe_group.h"
+#include "state_blob.h"
 
 #include <algorithm>
 #include <chrono>
@@ -34,41 +35,12 @@ int FeGroup::err(int code, const std::string &msg) {
   return code;
 }
 
-int FeGroup::alloc_image(DevImage &im, int w, int h) {
-  im.w = w;
-  im.h = h;
-  im.pitch = align_up(w, 256);
-  FG_CUDA(cudaMalloc(&im.p, (size_t)im.pitch * h + 256));
-  FG_CUDA(cudaMemset(im.p, 0, (size_t)im.pitch * h + 256));
-  dev_allocs_.push_back(im.p);
-  return FE_OK;
-}
-
-// Grider_GRID geometry (Grider_GRID.h:88-100), as FeContext::layout_cells
 void FeGroup::layout_cells() {
-  const int gx = cfg_.grid_x, gy = cfg_.grid_y;
-  int ggx = gx, ggy = gy;
-  if (cfg_.num_features < ggx * ggy) {
-    double ratio = (double)ggx / (double)ggy;
-    ggy = (int)std::ceil(std::sqrt(cfg_.num_features / ratio));
-    ggx = (int)std::ceil(ggy * ratio);
-  }
-  g_.nfg = (int)((double)cfg_.num_features / (double)(ggx * ggy)) + 1;
-  cells_csx_ = W_ / ggx;
-  cells_csy_ = H_ / ggy;
-  cells_.clear();
+  cells_ = grider_layout(W_, H_, cfg_.grid_x, cfg_.grid_y, cfg_.num_features);
+  g_.nfg = cells_.nfg;
+  g_.n_cells = (int)cells_.cells.size();
   for (int i = 0; i < 256; i++) g_.cell_of_loc[i] = -1;
-  if (cells_csx_ > 0 && cells_csy_ > 0) {
-    for (int x = 0; x < gx; x++)
-      for (int y = 0; y < gy; y++) {
-        int px = x * cells_csx_, py = y * cells_csy_;
-        if (px + cells_csx_ > W_ || py + cells_csy_ > H_) continue;
-        g_.cell_of_loc[x * gy + y] = (int)cells_.size();
-        cells_.push_back(FastCell{px, py, cells_csx_, cells_csy_});
-      }
-  }
-  cells_nb_ = cells_csy_ > 0 ? (cells_csy_ + kFastBandRows - 1) / kFastBandRows : 0;
-  g_.n_cells = (int)cells_.size();
+  std::copy(cells_.cell_of_loc.begin(), cells_.cell_of_loc.end(), g_.cell_of_loc);   // grid_x * grid_y <= 256
 }
 
 template <class T>
@@ -132,12 +104,12 @@ int FeGroup::init() {
   const int kps_cap = W_ * H_ / 4 + 1024;
   const int max_bands = (H_ + kFastBandRows - 1) / kFastBandRows;
   FG_CUDA(dev_alloc(dev_allocs_, &d_cells_, std::max(ncell, 1)));
-  if (ncell) FG_CUDA(cudaMemcpy(d_cells_, cells_.data(), ncell * sizeof(FastCell), cudaMemcpyHostToDevice));
+  if (ncell) FG_CUDA(cudaMemcpy(d_cells_, cells_.cells.data(), ncell * sizeof(FastCell), cudaMemcpyHostToDevice));
   fg_.w = W_;
   fg_.h = H_;
   fg_.n_cells = ncell;
-  fg_.max_bands = cells_nb_;
-  fg_.max_cell_w = cells_csx_;
+  fg_.max_bands = cells_.n_bands;
+  fg_.max_cell_w = cells_.csx;
   fg_.fast_threshold = cfg_.fast_threshold;
   fg_.kps_cap = kps_cap;
   fg_.nfg = nfg;
@@ -151,13 +123,13 @@ int FeGroup::init() {
   h_mask_.assign(nslots, nullptr);
   for (int i = 0; i < nslots; i++) {
     SlotRec &sl = slots_[i];
-    int rc = alloc_image(sl.raw, W_, H_);
-    if (rc) return rc;
+    FG_CUDA(alloc_image(sl.raw, W_, H_));
+    dev_allocs_.push_back(sl.raw.p);
     int w = W_, h = H_;
     sl.n_lvl = 0;
     for (int l = 0; l <= cfg_.pyr_levels && l < kMaxLevels; l++) {   // cv::buildOpticalFlowPyramid: a level is kept while both sides stay > winSize
-      rc = alloc_image(sl.lvl[l], w, h);
-      if (rc) return rc;
+      FG_CUDA(alloc_image(sl.lvl[l], w, h));
+      dev_allocs_.push_back(sl.lvl[l].p);
       sl.n_lvl = l + 1;
       w = (w + 1) / 2;
       h = (h + 1) / 2;
@@ -170,13 +142,13 @@ int FeGroup::init() {
     FG_CUDA(dev_alloc(dev_allocs_, &sl.fast_total, 2));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.kps, kps_cap, false));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.sort_scratch, kps_cap, false));
-    FG_CUDA(dev_alloc(dev_allocs_, &sl.band_off, std::max(ncell * cells_nb_, 1)));
-    FG_CUDA(dev_alloc(dev_allocs_, &sl.band_cnt, std::max(ncell * cells_nb_, 1)));
+    FG_CUDA(dev_alloc(dev_allocs_, &sl.band_off, std::max(ncell * cells_.n_bands, 1)));
+    FG_CUDA(dev_alloc(dev_allocs_, &sl.band_cnt, std::max(ncell * cells_.n_bands, 1)));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.cand, g_.cand_cap));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.cand_cnt, std::max(ncell, 1)));
     if (cfg_.use_lines) {
-      rc = alloc_image(sl.half, W_ / 2, H_ / 2);
-      if (rc) return rc;
+      FG_CUDA(alloc_image(sl.half, W_ / 2, H_ / 2));
+      dev_allocs_.push_back(sl.half.p);
       if (sl.fld.alloc(W_ / 2, H_ / 2, cfg_.fld_length_threshold, g_.segs_cap)) return fail(cudaGetLastError(), "FldBuffers::alloc");
     }
   }
@@ -854,162 +826,89 @@ int FeGroup::play(int n_ticks, const uint8_t *const *images, int stride, bool on
 }
 
 // ------------------------------------------------------------------------------------------ state / taps
-namespace {
-struct StateHeader {   // the blob layout of plviwo_fe_get_state / _set_state (fe_context.cu)
-  uint32_t magic, version;
-  int32_t w, h;
-  uint64_t currid, line_currid;
-  int32_t n_pts, n_lines, has_image, has_mask;
-  int32_t n_pol_entries, reserved;
-};
-}  // namespace
-
+// One stream's blob, in the format of a single handle's (state_blob.h): the device's per-line point lists (CSR, float
+// distances) go through the handle's point maps.
 int FeGroup::get_state(int s, void *buf, size_t cap, size_t *n_bytes) {
   FG_CUDA(cudaSetDevice(device_));
   if (s < 0 || s >= S_) return err(FE_BAD_ARG, "get_state: bad stream");
   if (submitted_ != collected_) return err(FE_BAD_ARG, "get_state: collect the pending ticks first");
   FG_CUDA(cudaDeviceSynchronize());
-  StateHeader hd;
-  std::memset(&hd, 0, sizeof(hd));
-  hd.magic = 0x504c5657u;
-  hd.version = 1;
-  hd.w = W_;
-  hd.h = H_;
   int n_pts = 0, lb = 0, n_lines = 0;
+  uint64_t currid = 0, line_currid = 1;
   const size_t rec = (size_t)prev_rec_[s];   // the stream's current state record
   FG_CUDA(cudaMemcpy(&n_pts, g_.n_pts + rec, sizeof(int), cudaMemcpyDeviceToHost));
-  FG_CUDA(cudaMemcpy(&hd.currid, g_.currid + s, sizeof(uint64_t), cudaMemcpyDeviceToHost));
-  hd.line_currid = 1;
+  FG_CUDA(cudaMemcpy(&currid, g_.currid + s, sizeof(uint64_t), cudaMemcpyDeviceToHost));
   std::vector<float4> lines;
   std::vector<uint64_t> lids;
-  std::vector<int> poff(1, 0), ppid;
-  std::vector<float> pdist;
+  PointsOnLines pol;
   if (cfg_.use_lines) {
     FG_CUDA(cudaMemcpy(&lb, g_.line_buf + s, sizeof(int), cudaMemcpyDeviceToHost));
     FG_CUDA(cudaMemcpy(&n_lines, g_.n_lines + 2 * s + lb, sizeof(int), cudaMemcpyDeviceToHost));
-    FG_CUDA(cudaMemcpy(&hd.line_currid, g_.line_currid + s, sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    FG_CUDA(cudaMemcpy(&line_currid, g_.line_currid + s, sizeof(uint64_t), cudaMemcpyDeviceToHost));
     const size_t b = (size_t)(2 * s + lb);
     lines.resize(n_lines);
     lids.resize(n_lines);
-    poff.resize(n_lines + 1);
+    std::vector<int> poff(n_lines + 1);
     FG_CUDA(cudaMemcpy(lines.data(), g_.lines + b * g_.lines_cap, n_lines * sizeof(float4), cudaMemcpyDeviceToHost));
     FG_CUDA(cudaMemcpy(lids.data(), g_.line_ids + b * g_.lines_cap, n_lines * sizeof(uint64_t), cudaMemcpyDeviceToHost));
     FG_CUDA(cudaMemcpy(poff.data(), g_.pol_off + b * (g_.lines_cap + 1), (n_lines + 1) * sizeof(int), cudaMemcpyDeviceToHost));
     if (n_lines == 0) poff[0] = 0;
     const int ne = poff[n_lines];
-    ppid.resize(ne);
-    pdist.resize(ne);
+    std::vector<int> ppid(ne);
+    std::vector<float> pdist(ne);
     FG_CUDA(cudaMemcpy(ppid.data(), g_.pol_pid + b * g_.pol_cap, ne * sizeof(int), cudaMemcpyDeviceToHost));
     FG_CUDA(cudaMemcpy(pdist.data(), g_.pol_dist + b * g_.pol_cap, ne * sizeof(float), cudaMemcpyDeviceToHost));
+    pol.resize(n_lines);
+    for (int i = 0; i < n_lines; i++)
+      for (int e = poff[i]; e < poff[i + 1]; e++) pol[i][ppid[e]] = (double)pdist[e];
   }
-  hd.n_pts = n_pts;
-  hd.n_lines = n_lines;
   const int ps = prev_slot_[s];
   int flags = 0;
   if (ps >= 0) FG_CUDA(cudaMemcpy(&flags, d_slot_flags_ + ps, sizeof(int), cudaMemcpyDeviceToHost));
-  hd.has_image = ps >= 0 ? 1 : 0;
-  hd.has_mask = (ps >= 0 && (flags & 1)) ? 1 : 0;
-  hd.n_pol_entries = poff[n_lines];
-  const size_t need = sizeof(hd) + (size_t)n_pts * (sizeof(float2) + sizeof(uint64_t)) +
-                      (size_t)n_lines * (sizeof(float4) + sizeof(uint64_t) + sizeof(int32_t)) +
-                      (size_t)hd.n_pol_entries * (sizeof(int32_t) + sizeof(double)) + (hd.has_image ? (size_t)W_ * H_ : 0) +
-                      (hd.has_mask ? (size_t)W_ * H_ : 0);
-  if (n_bytes) *n_bytes = need;
-  if (!buf || cap < need) return buf ? FE_OVERFLOW : FE_OK;
+  const StateHeader hd = state_header(W_, H_, currid, line_currid, n_pts, n_lines, pol, ps >= 0, (flags & 1) != 0);
+  const StateLayout at = state_layout(hd);
+  if (n_bytes) *n_bytes = at.size;
+  if (!buf || cap < at.size) return buf ? FE_OVERFLOW : FE_OK;
+  std::vector<float2> pts(n_pts);
+  std::vector<uint64_t> ids(n_pts);
+  FG_CUDA(cudaMemcpy(pts.data(), g_.pts + rec * g_.pts_cap, n_pts * sizeof(float2), cudaMemcpyDeviceToHost));
+  FG_CUDA(cudaMemcpy(ids.data(), g_.ids + rec * g_.pts_cap, n_pts * sizeof(uint64_t), cudaMemcpyDeviceToHost));
   uint8_t *p = static_cast<uint8_t *>(buf);
-  auto put = [&](const void *src, size_t n) { std::memcpy(p, src, n); p += n; };
-  put(&hd, sizeof(hd));
-  FG_CUDA(cudaMemcpy(p, g_.pts + rec * g_.pts_cap, n_pts * sizeof(float2), cudaMemcpyDeviceToHost));
-  p += n_pts * sizeof(float2);
-  FG_CUDA(cudaMemcpy(p, g_.ids + rec * g_.pts_cap, n_pts * sizeof(uint64_t), cudaMemcpyDeviceToHost));
-  p += n_pts * sizeof(uint64_t);
-  put(lines.data(), lines.size() * sizeof(float4));
-  put(lids.data(), lids.size() * sizeof(uint64_t));
-  for (int i = 0; i < n_lines; i++) { int32_t k = poff[i + 1] - poff[i]; put(&k, sizeof(k)); }
-  for (int e = 0; e < hd.n_pol_entries; e++) {
-    int32_t k = ppid[e];
-    double v = (double)pdist[e];
-    put(&k, sizeof(k));
-    put(&v, sizeof(v));
-  }
+  state_write(p, hd, pts.data(), ids.data(), lines.data(), lids.data(), pol);
   if (hd.has_image) {
     const DevImage &l0 = slots_[ps].lvl[0];
-    FG_CUDA(cudaMemcpy2D(p, W_, l0.p, l0.pitch, W_, H_, cudaMemcpyDeviceToHost));
-    p += (size_t)W_ * H_;
+    FG_CUDA(cudaMemcpy2D(p + at.image, W_, l0.p, l0.pitch, W_, H_, cudaMemcpyDeviceToHost));
   }
-  if (hd.has_mask) {
-    FG_CUDA(cudaMemcpy(p, slots_[ps].mask, (size_t)W_ * H_, cudaMemcpyDeviceToHost));
-    p += (size_t)W_ * H_;
-  }
+  if (hd.has_mask) FG_CUDA(cudaMemcpy(p + at.mask, slots_[ps].mask, (size_t)W_ * H_, cudaMemcpyDeviceToHost));
   return FE_OK;
 }
 
 int FeGroup::set_state(int s, const void *buf, size_t n_bytes) {
   FG_CUDA(cudaSetDevice(device_));
-  if (s < 0 || s >= S_ || !buf || n_bytes < sizeof(StateHeader)) return err(FE_BAD_ARG, "set_state: bad arguments");
+  if (s < 0 || s >= S_) return err(FE_BAD_ARG, "set_state: bad stream");
   if (submitted_ != collected_) return err(FE_BAD_ARG, "set_state: collect the pending ticks first");
   // ---- parse and validate everything before any of it is applied
-  const uint8_t *p = static_cast<const uint8_t *>(buf);
-  StateHeader hd;
-  std::memcpy(&hd, p, sizeof(hd));
-  p += sizeof(hd);
-  if (hd.magic != 0x504c5657u || hd.version != 1 || hd.w != W_ || hd.h != H_) return err(FE_BAD_ARG, "set_state: foreign blob");
-  if (hd.n_pts < 0 || hd.n_lines < 0 || hd.n_pol_entries < 0) return err(FE_BAD_ARG, "set_state: negative counts");
+  StateView v;
+  if (const char *why = state_read(buf, n_bytes, W_, H_, v)) return err(FE_BAD_ARG, why);
+  const StateHeader &hd = v.hd;
   if (hd.n_pts > g_.pts_cap || hd.n_lines > g_.lines_cap || hd.n_pol_entries > g_.pol_cap)
     return err(FE_BAD_ARG, "set_state: more points / lines than the group's buffers hold");
-  const size_t need = sizeof(hd) + (size_t)hd.n_pts * (sizeof(float2) + sizeof(uint64_t)) +
-                      (size_t)hd.n_lines * (sizeof(float4) + sizeof(uint64_t) + sizeof(int32_t)) +
-                      (size_t)hd.n_pol_entries * (sizeof(int32_t) + sizeof(double)) + (hd.has_image ? (size_t)W_ * H_ : 0) +
-                      (hd.has_image && hd.has_mask ? (size_t)W_ * H_ : 0);
-  if (n_bytes < need) return err(FE_BAD_ARG, "set_state: blob shorter than its header announces");
-  const uint8_t *p_pts = p;
-  p += (size_t)hd.n_pts * sizeof(float2);
-  const uint8_t *p_ids = p;
-  p += (size_t)hd.n_pts * sizeof(uint64_t);
-  const uint8_t *p_lines = p;
-  p += (size_t)hd.n_lines * sizeof(float4);
-  const uint8_t *p_lids = p;
-  p += (size_t)hd.n_lines * sizeof(uint64_t);
-  std::vector<int32_t> sizes(hd.n_lines);
-  std::memcpy(sizes.data(), p, (size_t)hd.n_lines * sizeof(int32_t));
-  p += (size_t)hd.n_lines * sizeof(int32_t);
-  long long tot = 0;
-  for (int32_t v : sizes) {
-    if (v < 0) return err(FE_BAD_ARG, "set_state: negative line size");
-    tot += v;
-  }
-  if (tot != hd.n_pol_entries) return err(FE_BAD_ARG, "set_state: line sizes do not add up to the header's entry count");
-  std::vector<int> poff(hd.n_lines + 1, 0), ppid(hd.n_pol_entries);
-  std::vector<float> pdist(hd.n_pol_entries);
-  {
-    int e = 0;
-    for (int i = 0; i < hd.n_lines; i++) {
-      std::map<int, double> m;   // the reference's container: ascending keys, one value per key
-      for (int k = 0; k < sizes[i]; k++) {
-        int32_t key;
-        double val;
-        std::memcpy(&key, p, sizeof(key));
-        p += sizeof(key);
-        std::memcpy(&val, p, sizeof(val));
-        p += sizeof(val);
-        m[key] = val;
-      }
-      poff[i] = e;
-      for (auto &kv : m) {
-        ppid[e] = kv.first;
-        pdist[e] = (float)kv.second;
-        e++;
-      }
+  std::vector<int> poff(hd.n_lines + 1, 0), ppid;
+  std::vector<float> pdist;
+  for (int i = 0; i < hd.n_lines; i++) {
+    poff[i] = (int)ppid.size();
+    for (const auto &kv : v.pol[i]) {
+      ppid.push_back(kv.first);
+      pdist.push_back((float)kv.second);
     }
-    poff[hd.n_lines] = e;
   }
-  const uint8_t *p_img = p;
+  poff[hd.n_lines] = (int)ppid.size();
   // ---- apply
   FG_CUDA(cudaDeviceSynchronize());
   const int n = hd.n_pts;
   const size_t rec = (size_t)prev_rec_[s];   // nothing is in flight: the stream's current state record is rewritten in place
-  FG_CUDA(cudaMemcpy(g_.pts + rec * g_.pts_cap, p_pts, n * sizeof(float2), cudaMemcpyHostToDevice));
-  FG_CUDA(cudaMemcpy(g_.ids + rec * g_.pts_cap, p_ids, n * sizeof(uint64_t), cudaMemcpyHostToDevice));
+  FG_CUDA(cudaMemcpy(g_.pts + rec * g_.pts_cap, v.base + v.at.pts, n * sizeof(float2), cudaMemcpyHostToDevice));
+  FG_CUDA(cudaMemcpy(g_.ids + rec * g_.pts_cap, v.base + v.at.ids, n * sizeof(uint64_t), cudaMemcpyHostToDevice));
   FG_CUDA(cudaMemcpy(g_.n_pts + rec, &n, sizeof(int), cudaMemcpyHostToDevice));
   FG_CUDA(cudaMemcpy(g_.currid + s, &hd.currid, sizeof(uint64_t), cudaMemcpyHostToDevice));
   if (cfg_.use_lines) {
@@ -1018,8 +917,8 @@ int FeGroup::set_state(int s, const void *buf, size_t n_bytes) {
     FG_CUDA(cudaMemcpy(g_.line_buf + s, &lb, sizeof(int), cudaMemcpyHostToDevice));
     FG_CUDA(cudaMemcpy(g_.n_lines + 2 * s + lb, &hd.n_lines, sizeof(int), cudaMemcpyHostToDevice));
     FG_CUDA(cudaMemcpy(g_.line_currid + s, &hd.line_currid, sizeof(uint64_t), cudaMemcpyHostToDevice));
-    FG_CUDA(cudaMemcpy(g_.lines + b * g_.lines_cap, p_lines, hd.n_lines * sizeof(float4), cudaMemcpyHostToDevice));
-    FG_CUDA(cudaMemcpy(g_.line_ids + b * g_.lines_cap, p_lids, hd.n_lines * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    FG_CUDA(cudaMemcpy(g_.lines + b * g_.lines_cap, v.base + v.at.lines, hd.n_lines * sizeof(float4), cudaMemcpyHostToDevice));
+    FG_CUDA(cudaMemcpy(g_.line_ids + b * g_.lines_cap, v.base + v.at.line_ids, hd.n_lines * sizeof(uint64_t), cudaMemcpyHostToDevice));
     FG_CUDA(cudaMemcpy(g_.pol_off + b * (g_.lines_cap + 1), poff.data(), (hd.n_lines + 1) * sizeof(int), cudaMemcpyHostToDevice));
     FG_CUDA(cudaMemcpy(g_.pol_pid + b * g_.pol_cap, ppid.data(), ppid.size() * sizeof(int), cudaMemcpyHostToDevice));
     FG_CUDA(cudaMemcpy(g_.pol_dist + b * g_.pol_cap, pdist.data(), pdist.size() * sizeof(float), cudaMemcpyHostToDevice));
@@ -1028,7 +927,7 @@ int FeGroup::set_state(int s, const void *buf, size_t n_bytes) {
   if (hd.has_image) {   // the stored image is already equalised: rebuild its pyramid and candidate table without a LUT
     const int slot = s * R_ + (int)(frame_count_[s] % R_);
     SlotRec &sl = slots_[slot];
-    FG_CUDA(cudaMemcpy2D(sl.raw.p, sl.raw.pitch, p_img, W_, W_, H_, cudaMemcpyHostToDevice));
+    FG_CUDA(cudaMemcpy2D(sl.raw.p, sl.raw.pitch, v.base + v.at.image, W_, W_, H_, cudaMemcpyHostToDevice));
     FrontJob fj;
     fj.src = sl.raw.p;
     fj.src_pitch = sl.raw.pitch;
@@ -1038,7 +937,7 @@ int FeGroup::set_state(int s, const void *buf, size_t n_bytes) {
     if (hd.has_mask) {
       int rc = ensure_mask_buffer(slot);
       if (rc) return rc;
-      FG_CUDA(cudaMemcpy(slots_[slot].mask, p_img + (size_t)W_ * H_, (size_t)W_ * H_, cudaMemcpyHostToDevice));
+      FG_CUDA(cudaMemcpy(slots_[slot].mask, v.base + v.at.mask, (size_t)W_ * H_, cudaMemcpyHostToDevice));
       fj.flags |= 1;
     }
     cudaStream_t st = s_front_[0];
@@ -1064,12 +963,8 @@ int FeGroup::tap(int s, int what, void *buf, size_t cap, size_t *n_bytes) {
   if (what >= FE_TAP_PYR_LEVEL0 && what < FE_TAP_PYR_LEVEL0 + kMaxLevels && what - FE_TAP_PYR_LEVEL0 < sl.n_lvl) im = &sl.lvl[what - FE_TAP_PYR_LEVEL0];
   if (what == FE_TAP_HALF && cfg_.use_lines) im = &sl.half;
   if (!im) return err(FE_BAD_ARG, "tap: not available");
-  const size_t n = (size_t)im->w * im->h;
-  if (n_bytes) *n_bytes = n;
-  if (!buf) return FE_OK;
-  if (cap < n) return FE_OVERFLOW;
-  FG_CUDA(cudaMemcpy2D(buf, im->w, im->p, im->pitch, im->w, im->h, cudaMemcpyDeviceToHost));
-  return FE_OK;
+  const int rc = tap_image(*im, buf, cap, n_bytes);
+  return rc == FE_CUDA_ERROR ? fail(cudaGetLastError(), "tap: cudaMemcpy2D") : rc;
 }
 
 }  // namespace plviwo

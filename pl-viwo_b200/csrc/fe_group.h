@@ -18,6 +18,7 @@
 
 #include "../../include/plviwo_fe.h"
 #include "fe_group_dev.h"
+#include "tracker_core.h"
 
 namespace plviwo {
 
@@ -72,7 +73,6 @@ class FeGroup {
   };
   int fail(cudaError_t e, const char *what);
   int err(int code, const std::string &msg);
-  int alloc_image(DevImage &im, int w, int h);
   void layout_cells();
   int flush_front();                     // launches the pending front batch and the tracking of its ticks
   int launch_front(FrontBatch &b, int buf);
@@ -91,8 +91,7 @@ class FeGroup {
   SlotRec *d_slots_ = nullptr;
   int *d_slot_flags_ = nullptr;
   FastCell *d_cells_ = nullptr;
-  std::vector<FastCell> cells_;
-  int cells_nb_ = 0, cells_csx_ = 0, cells_csy_ = 0;
+  GriderLayout cells_;
   std::vector<void *> dev_allocs_, host_allocs_;
   std::vector<uint8_t *> h_raw_;         // pinned staging per slot for pageable host frames (lazy)
   std::vector<uint8_t *> h_mask_;        // pinned staging per slot (lazy)

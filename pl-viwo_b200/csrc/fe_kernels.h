@@ -4,6 +4,8 @@
 #include <atomic>
 #include <cstdint>
 
+#include "../../include/plviwo_fe.h"
+
 namespace plviwo {
 
 // Opt-in to more than 48 KB of dynamic shared memory.  The attribute is per DEVICE (handles of one process may live on
@@ -55,6 +57,23 @@ struct DevImage {
   uint8_t *p = nullptr;
   int w = 0, h = 0, pitch = 0;
 };
+// Rows padded to 256 bytes and 256 bytes of slack after the last row (vectorised kernels read past the row end), zeroed.
+inline cudaError_t alloc_image(DevImage &im, int w, int h) {
+  im.w = w;
+  im.h = h;
+  im.pitch = (w + 255) / 256 * 256;
+  const cudaError_t e = cudaMalloc(&im.p, (size_t)im.pitch * h + 256);
+  return e != cudaSuccess ? e : cudaMemset(im.p, 0, (size_t)im.pitch * h + 256);
+}
+// The image taps: im as w * h packed bytes.  *n_bytes = w * h; a null buf only asks for that size, a smaller cap is
+// FE_OVERFLOW.  FE_CUDA_ERROR leaves the copy's error to cudaGetLastError().
+inline int tap_image(const DevImage &im, void *buf, size_t cap, size_t *n_bytes) {
+  const size_t n = (size_t)im.w * im.h;
+  if (n_bytes) *n_bytes = n;
+  if (!buf) return FE_OK;
+  if (cap < n) return FE_OVERFLOW;
+  return cudaMemcpy2D(buf, im.w, im.p, im.pitch, im.w, im.h, cudaMemcpyDeviceToHost) == cudaSuccess ? FE_OK : FE_CUDA_ERROR;
+}
 
 constexpr int kMaxLevels = 8;       // pyramid images (maxLevel + 1)
 constexpr int kFastBandRows = 16;   // rows per FAST CTA band

@@ -15,9 +15,12 @@
 // The host glue of a single handle (fe_context.cu: filter_existing / grid_candidates / perform_detection / klt_feed /
 // lsd_feed) is the sequential statement of the same steps; here every loop whose iterations only interact through "the
 // first one in order wins" is run in parallel with an atomicMin on the order index plus an ordered compaction, which
-// gives the sequential result exactly.  Compiled with --fmad=false: float expressions round where the host's do.
+// gives the sequential result exactly.  The arithmetic both forms apply (undistortion, PointLineDistance, LineSimilar,
+// LineClassification) is defined once, in tracker_core.h.  Compiled with --fmad=false: float expressions round where the
+// host's do.
 #include "fe_group_dev.h"
 #include "ransac_core.h"
+#include "tracker_core.h"
 
 #include <cfloat>
 #include <climits>
@@ -559,56 +562,6 @@ void launch_group_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cuda
 }
 
 // ==================================================================================================== lines
-// TrackLSD::PointLineDistance (TrackLSD.cpp:794-814): float arithmetic, the last branch mixes in double (std::pow)
-__device__ __forceinline__ float point_line_distance(const float4 &line, float x0, float y0) {
-  const float x1 = line.x, y1 = line.y, x2 = line.z, y2 = line.w;
-  const float cross = (x2 - x1) * (x0 - x1) + (y2 - y1) * (y0 - y1);
-  if (cross <= 0) return sqrtf((x0 - x1) * (x0 - x1) + (y0 - y1) * (y0 - y1));
-  const float d = (x2 - x1) * (x2 - x1) + (y2 - y1) * (y2 - y1);
-  if (cross > d) return sqrtf((x0 - x2) * (x0 - x2) + (y0 - y2) * (y0 - y2));
-  const double dy = (double)(y2 - y1), dx = (double)(x1 - x2);
-  return (float)fabs((double)fabsf((y2 - y1) * x0 + (x1 - x2) * y0 + ((x2 * y1) - (x1 * y2))) / sqrt(dy * dy + dx * dx));
-}
-__device__ __forceinline__ bool line_similar(const float4 &line2, const float4 &line1) {   // :816-830
-  const float mx = (line1.x + line1.z) / 2, my = (line1.y + line1.w) / 2;
-  return point_line_distance(line2, mx, my) <= 6;
-}
-__device__ bool line_class(const float4 &line, double vx, double vy) {   // :335-366, atan(dy) / dx as written there
-  const double s[3] = {line.x, line.y, 1}, e[3] = {line.z, line.w, 1};
-  const double mid[3] = {(s[0] + e[0]) / 2, (s[1] + e[1]) / 2, (s[2] + e[2]) / 2};
-  const double v3[3] = {vx, vy, 1};
-  const double ln[3] = {mid[1] * v3[2] - mid[2] * v3[1], mid[2] * v3[0] - mid[0] * v3[2], mid[0] * v3[1] - mid[1] * v3[0]};
-  double dis_error = (fabs(ln[0] * s[0] + ln[1] * s[1] + ln[2] * s[2]) + fabs(ln[0] * e[0] + ln[1] * e[1] + ln[2] * e[2])) /
-                     (2 * sqrt(ln[0] * ln[0] + ln[1] * ln[1]));
-  dis_error = fabs(dis_error);
-  const double angle1 = atanf(line.y - line.w) / (line.x - line.z);   // float arithmetic
-  const double angle2 = atan(mid[1] - vy) / (mid[0] - vx);
-  const double angle_error = fabs(angle1 - angle2);
-  return dis_error <= 5.0 && angle_error <= 0.35;
-}
-__device__ int line_classification(const float4 &line, const double vp[6]) {   // :318-333
-  if (line_class(line, vp[4], vp[5])) return 3;
-  if (line_class(line, vp[2], vp[3])) return 2;
-  if (line_class(line, vp[0], vp[1])) return 1;
-  return 0;
-}
-// cv::undistortPoints on one point (SURVEY.md Appendix A6): 5 fixed-point iterations in double
-__device__ void undistort_pt(const double K[4], const double D[4], float u, float v, float &un, float &vn) {
-  const double x0 = ((double)u - K[2]) / K[0], y0 = ((double)v - K[3]) / K[1];
-  double x = x0, y = y0;
-#pragma unroll 1
-  for (int j = 0; j < 5; j++) {
-    const double r2 = x * x + y * y;
-    const double icdist = 1.0 / (1.0 + (D[1] * r2 + D[0]) * r2);
-    const double dx = 2 * D[2] * x * y + D[3] * (r2 + 2 * x * x);
-    const double dy = D[2] * (r2 + 2 * y * y) + 2 * D[3] * x * y;
-    x = (x0 - dx) * icdist;
-    y = (y0 - dy) * icdist;
-  }
-  un = (float)x;
-  vn = (float)y;
-}
-
 // AssignPointToLines' test of one (line, point) pair (:770-781): inside the mis-indexed bounding box and not farther than
 // 5 px from the SEGMENT
 __device__ __forceinline__ bool on_line(const float4 &l, float min_lx, float max_lx, float min_ly, float max_ly, float2 p, float &dist) {
@@ -809,8 +762,8 @@ __global__ void __launch_bounds__(kGT)
     memset(&r, 0, sizeof(r));
     r.id = id;
     r.line[0] = l.x; r.line[1] = l.y; r.line[2] = l.z; r.line[3] = l.w;
-    undistort_pt(job.K, job.D, l.x, l.y, r.line_n[0], r.line_n[1]);
-    undistort_pt(job.K, job.D, l.z, l.w, r.line_n[2], r.line_n[3]);
+    const float2 n0 = undistort_radtan(make_float2(l.x, l.y), job.K, job.D), n1 = undistort_radtan(make_float2(l.z, l.w), job.K, job.D);
+    r.line_n[0] = n0.x; r.line_n[1] = n0.y; r.line_n[2] = n1.x; r.line_n[3] = n1.y;
     r.D = line_classification(l, job.vp);
     r.n_pts = poff_new[i + 1] - poff_new[i];
     r.pt_offset = poff_new[i];

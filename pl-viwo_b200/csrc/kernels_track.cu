@@ -8,6 +8,7 @@
 //   CamRadtan::undistort_f -> cv::undistortPoints (one Mat per point)               cam/CamRadtan.h:99-120
 #include "fe_kernels.h"
 #include "fe_group_dev.h"
+#include "tracker_core.h"
 
 #include <algorithm>
 #include <mutex>
@@ -166,23 +167,6 @@ void launch_group_subpix(const GroupDev &g, const TrackJob *jobs, int n_jobs, cu
 }
 
 // ============================================================================================== undistort
-// cv::undistortPoints with a 4-coefficient radtan model: 5 fixed-point iterations in double (Appendix A6).
-__device__ __forceinline__ float2 undistort_radtan(float2 uv, const double *K, const double *D) {
-  double x0 = ((double)uv.x - K[2]) / K[0], y0 = ((double)uv.y - K[3]) / K[1];
-  double x = x0, y = y0;
-  const double k1 = D[0], k2 = D[1], p1 = D[2], p2 = D[3];
-#pragma unroll 1
-  for (int j = 0; j < 5; j++) {
-    double r2 = x * x + y * y;
-    double icdist = 1.0 / (1.0 + (k2 * r2 + k1) * r2);
-    double dx = 2 * p1 * x * y + p2 * (r2 + 2 * x * x);
-    double dy = p1 * (r2 + 2 * y * y) + 2 * p2 * x * y;
-    x = (x0 - dx) * icdist;
-    y = (y0 - dy) * icdist;
-  }
-  return make_float2((float)x, (float)y);
-}
-
 struct CalibArgs {
   double K[4], D[4];
 };

@@ -671,11 +671,12 @@ def test_capacity_and_boundary_guards(fe, synth):
         sizes = np.frombuffer(bytes(blob[off:off + 4 * n_lines]), np.int32).copy()
         sizes[0] += 5
         blob[off:off + 4 * n_lines] = sizes.tobytes()
-        with pytest.raises(fe.FrontEndError):
+        with pytest.raises(fe.FrontEndError, match="line sizes do not add up"):
             h.set_state(bytes(blob))
         assert h.get_state() == before
     bad = bytearray(before)
     bad[4:8] = np.uint32(7).tobytes()             # unknown version
-    with pytest.raises(fe.FrontEndError):
+    with pytest.raises(fe.FrontEndError, match="foreign blob"):
         h.set_state(bytes(bad))
+    assert h.get_state() == before
     h.close()

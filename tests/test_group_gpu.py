@@ -263,3 +263,31 @@ def test_group_bad_arguments(fe):
     with pytest.raises(fe.FrontEndError):
         g.set_state(5, b"\x00" * 128)
     g.close()
+
+
+def test_group_set_state_rejects_inconsistent_blobs(fe, synth):
+    """As a single handle (test_frontend_gpu.py test_capacity_and_boundary_guards): a blob whose per-line sizes do not add up
+    to its header's entry count, or of an unknown version, is refused with the reason and leaves the stream's state as it was."""
+    W, H = 1280, 560
+    seq = synth.SynthSequence(seed=3, width=W, height=H, n_frames=3, hard=False)
+    g = fe.GroupFrontEnd(fe.default_config(width=W, height=H, **CFG1), 2, calibs=[(seq.K, seq.D)] * 2)
+    for t in range(3):
+        g.feed([seq.timestamp(t)] * 2, [seq.frame(t)] * 2, vanishing_points=[seq.vanishing_points(t)] * 2)
+    before = g.get_state(0)
+    hdr = np.frombuffer(before[:56], fe._STATE_HDR, 1)[0]
+    n_pts, n_lines = int(hdr["n_pts"]), int(hdr["n_lines"])
+    assert n_lines > 0
+    blob = bytearray(before)
+    off = 56 + 16 * n_pts + 24 * n_lines          # the int32 sizes array
+    sizes = np.frombuffer(bytes(blob[off:off + 4 * n_lines]), np.int32).copy()
+    sizes[0] += 5
+    blob[off:off + 4 * n_lines] = sizes.tobytes()
+    with pytest.raises(fe.FrontEndError, match="line sizes do not add up"):
+        g.set_state(0, bytes(blob))
+    assert g.get_state(0) == before
+    bad = bytearray(before)
+    bad[4:8] = np.uint32(7).tobytes()             # unknown version
+    with pytest.raises(fe.FrontEndError, match="foreign blob"):
+        g.set_state(0, bytes(bad))
+    assert g.get_state(0) == before
+    g.close()

@@ -50,6 +50,62 @@ def test_no_cpu_fallback_stereo(fe):
     assert e.value.code == fe.FE_NO_DEVICE
 
 
+_SHARED_RULES = [
+    (dict(width=32), "image size must be in [64, 4095]"),
+    (dict(height=4096), "image size must be in [64, 4095]"),
+    (dict(win_size=16), "win_size must be odd and in [3, 31]"),
+    (dict(win_size=33), "win_size must be odd and in [3, 31]"),
+    (dict(pyr_levels=8), "pyr_levels must be in [0, 7]"),
+    (dict(grid_y=0), "bad grid / distance / feature count"),
+    (dict(min_px_dist=0), "bad grid / distance / feature count"),
+    (dict(num_features=0), "bad grid / distance / feature count"),
+    (dict(histogram_method=7), "bad histogram_method"),
+    (dict(width=642, height=281), "line tracker needs even (tracking) image dimensions (exact 2x decimation)"),
+    (dict(canny_th2=60.0), "canny_th1 != canny_th2: hysteresis pass is not implemented"),
+    (dict(fld_length_threshold=1), "bad fld_length_threshold"),
+]
+_CREATORS = ("handle", "group", "stereo")
+
+
+def _create(fe, creator, cfg, n_streams=2):
+    """rc and reason of a creation through the C ABI that is expected to be refused."""
+    import ctypes as C
+    L = fe.lib()
+    h = C.c_void_p()
+    if creator == "handle":
+        rc, why = L.plviwo_fe_create(C.byref(cfg), 0, C.byref(h)), L.plviwo_fe_last_error(None)
+    elif creator == "group":
+        rc, why = L.plviwo_fe_group_create(C.byref(cfg), n_streams, 0, C.byref(h)), L.plviwo_fe_group_last_error(None)
+    else:
+        K, D = (C.c_double * 4)(*cfg.K), (C.c_double * 4)(*cfg.D)
+        rc, why = L.plviwo_fe_stereo_create(C.byref(cfg), K, D, 0, C.byref(h)), L.plviwo_fe_stereo_last_error(None)
+    assert not h.value, "created a handle from a config that must be refused"
+    return rc, (why or b"").decode()
+
+
+@pytest.mark.parametrize("creator", _CREATORS)
+@pytest.mark.parametrize("kw,reason", _SHARED_RULES)
+def test_creators_refuse_bad_configs_before_the_device_query(fe, creator, kw, reason):
+    """Every creator checks the shared config rules before it looks for a device, so the refusal and its reason are the
+    same with and without a GPU."""
+    assert _create(fe, creator, fe.default_config(**kw)) == (fe.FE_BAD_ARG, reason)
+
+
+@pytest.mark.parametrize("creator,kw,reason", [
+    ("handle", dict(width=100, downsample=1), "downsampled image would be smaller than 64 pixels"),
+    ("handle", dict(width=1282, downsample=1), "line tracker needs even (tracking) image dimensions (exact 2x decimation)"),
+    ("group", dict(downsample=1), "cfg.downsample is not supported in a stream group"),
+    ("group", dict(grid_x=16, grid_y=17), "a stream group supports at most 256 grid cells"),
+])
+def test_creator_specific_config_rules(fe, creator, kw, reason):
+    assert _create(fe, creator, fe.default_config(**kw)) == (fe.FE_BAD_ARG, reason)
+
+
+@pytest.mark.parametrize("n_streams", [0, 4097])
+def test_group_refuses_bad_stream_count(fe, n_streams):
+    assert _create(fe, "group", fe.default_config(), n_streams) == (fe.FE_BAD_ARG, "n_streams must be in [1, 4096]")
+
+
 def test_stereo_state_blob_pack_unpack(fe):
     rng = np.random.default_rng(1)
     img = rng.integers(0, 255, (64, 96), np.uint8)
