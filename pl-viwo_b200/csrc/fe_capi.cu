@@ -543,14 +543,7 @@ static int op_lk(int device, const uint8_t *img0, const uint8_t *img1, int w, in
   if (d0.alloc(n) || d1.alloc(n) || dn0.alloc(n) || dn1.alloc(n) || ds.alloc(n)) return FE_CUDA_ERROR;
   OP_CUDA(cudaMemcpy(d0.p, pts0, (size_t)n * sizeof(float2), cudaMemcpyHostToDevice));
   OP_CUDA(cudaMemcpy(d1.p, pts1, (size_t)n * sizeof(float2), cudaMemcpyHostToDevice));
-  LkParams prm;
-  prm.win = win;
-  prm.max_level = max_level;
-  prm.max_count = 30;
-  prm.eps_sq = 0.01f * 0.01f;
-  prm.min_eig = 1e-4f;
-  prm.undistort = 0;
-  for (int i = 0; i < 4; i++) prm.K[i] = prm.D[i] = 0;
+  const LkParams prm = lk_params(win, max_level, nullptr, nullptr, false);
   if (!warp) launch_lk(p0.pyr, p1.pyr, d0.p, d1.p, ds.p, dn0.p, dn1.p, n, prm, 0);
   else if (!launch_lk_warp(p0.pyr, p1.pyr, d0.p, d1.p, ds.p, n, prm, 0)) return FE_BAD_ARG;
   OP_CUDA(cudaDeviceSynchronize());

@@ -197,7 +197,6 @@ int FeContext::init() {
     for (auto &e : s.ev_t) FE_CUDA(cudaEventCreate(&e));
   }
   for (auto &e : ev_pt_) FE_CUDA(cudaEventCreate(&e));
-  FE_CUDA(cudaEventCreateWithFlags(&ev_sync_, cudaEventDisableTiming));
   FE_CUDA(cudaMallocHost(&h_flag_lk_, 16 * sizeof(int)));
   std::memset(h_flag_lk_, 0, 16 * sizeof(int));
 
@@ -231,19 +230,12 @@ int FeContext::init() {
   }
   occ_bits_.assign((size_t)((W_ + 63) / 64) * H_, 0);
   layout_cells();
-  if (!external_) {
-    klt_thread_ = std::thread([this] { klt_main(); });
-    line_thread_ = std::thread([this] { line_main(); });
-  } else if (cfg_.use_lines) {
-    line_thread_ = std::thread([this] { line_main(); });   // the owner queues frames whose points are known (line_q_)
-  }
+  // an owner that tracks the frames itself (FeStereo) never queues work for the point tracker: that thread stays
+  // blocked on its empty queue
+  klt_thread_ = std::thread([this] { klt_main(); });
+  line_thread_ = std::thread([this] { line_main(); });
 
   max_pts_ = std::max(4096, 8 * cfg_.num_features) + 4096 * (cfg_.line_samples > 0 ? 8 : 0);
-  FE_CUDA(cudaMalloc(&d_pts0_, (size_t)max_pts_ * sizeof(float2)));
-  FE_CUDA(cudaMalloc(&d_pts1_, (size_t)max_pts_ * sizeof(float2)));
-  FE_CUDA(cudaMalloc(&d_p0n_, (size_t)max_pts_ * sizeof(float2)));
-  FE_CUDA(cudaMalloc(&d_p1n_, (size_t)max_pts_ * sizeof(float2)));
-  FE_CUDA(cudaMalloc(&d_status_, (size_t)max_pts_));
   FE_CUDA(cudaMalloc(&d_lk_done_, 4 * sizeof(unsigned)));   // [ordinary, speculative, candidates set 0, set 1]
   FE_CUDA(cudaMemset(d_lk_done_, 0, 4 * sizeof(unsigned)));
   FE_CUDA(cudaMallocHost(&h_sp_pts0_, (size_t)max_pts_ * sizeof(float2)));
@@ -308,7 +300,6 @@ FeContext::~FeContext() {
     for (auto &e : s.ev_t) if (e) cudaEventDestroy(e);
   }
   for (auto &e : ev_pt_) if (e) cudaEventDestroy(e);
-  if (ev_sync_) cudaEventDestroy(ev_sync_);
   cudaFreeHost(h_flag_lk_);
   cudaFree(d_cells_);
   cudaFree(d_lk_done_);
@@ -317,20 +308,8 @@ FeContext::~FeContext() {
     cudaFreeHost(s.h_sc_pts1); cudaFreeHost(s.h_sc_p0n); cudaFreeHost(s.h_sc_p1n); cudaFreeHost(s.h_sc_status);
     cudaFree(s.d_sc_done);
   }
-  cudaFree(d_pts0_); cudaFree(d_pts1_); cudaFree(d_p0n_); cudaFree(d_p1n_); cudaFree(d_status_);
   cudaFreeHost(h_pts0_); cudaFreeHost(h_pts1_); cudaFreeHost(h_p0n_); cudaFreeHost(h_p1n_); cudaFreeHost(h_status_);
   if (s_pt_) cudaStreamDestroy(s_pt_);
-}
-
-// Low-latency wait: poll an event instead of a blocking synchronise (the tracker thread has nothing else to do)
-int FeContext::spin_sync(cudaStream_t st) {
-  FE_CUDA(cudaEventRecord(ev_sync_, st));
-  while (true) {
-    cudaError_t e = cudaEventQuery(ev_sync_);
-    if (e == cudaSuccess) return FE_OK;
-    if (e != cudaErrorNotReady) return fail(e, "cudaEventQuery");
-    cpu_pause();
-  }
 }
 
 // Waits for a k_signal sequence number.  Polls memory only; every ~2M polls it asks the driver whether the stream
@@ -622,14 +601,7 @@ int FeContext::flush_line_batch() {
 int FeContext::track_candidates(FrameSlot &prev, FrameSlot &s) {
   s.sc_prev = -1;
   if (!use_spec_ || cfg_.line_samples > 0) return FE_OK;
-  LkParams prm;
-  prm.win = cfg_.win_size;
-  prm.max_level = cfg_.pyr_levels;
-  prm.max_count = 30;
-  prm.eps_sq = 0.01f * 0.01f;
-  prm.min_eig = 1e-4f;
-  prm.undistort = 1;
-  for (int i = 0; i < 4; i++) { prm.K[i] = s.K[i]; prm.D[i] = s.D[i]; }
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, s.K, s.D, true);
   const int ntab = prev.predet_ncell * prev.predet_nfg;
   if (ntab <= 0 || ntab > cand_cap_ || prev.predet_num_features != cfg_.num_features || !lk_table_mode_ok(prm, prev.pyr.n))
     return FE_OK;
@@ -647,26 +619,45 @@ int FeContext::track_candidates(FrameSlot &prev, FrameSlot &s) {
 int FeContext::submit(double t, const uint8_t *image, int stride, bool on_device, const uint8_t *mask, int mask_stride,
                       const double vp[6]) {
   int si = -1;
-  int rc = submit_impl(t, image, stride, on_device, mask, mask_stride, vp, &si);
+  int rc = stage_frame(t, image, stride, on_device, mask, mask_stride, vp, &si);
+  if (rc == FE_OK) {
+    HostTimer ht(&mst_.host_ms[FE_HOST_SUBMIT]);
+    if (prev_submit_slot_ >= 0) rc = track_candidates(slots_[prev_submit_slot_], slots_[si]);
+    if (rc == FE_OK) {
+      prev_submit_slot_ = si;
+      queue_.push_back(si);
+      slots_[si].stage.store(1, std::memory_order_release);
+      klt_q_.push(si);
+    }
+  }
   if (rc) {
     last_error = t_err;
-    if (si >= 0 && !external_) {   // a failed submit leaves no trace: the slot is free again, nothing of it is pending
-      FrameSlot &s = slots_[si];
-      cudaStreamSynchronize(s.s_a);
-      cudaStreamSynchronize(s.s_b);
-      if (s.s_line) cudaStreamSynchronize(s.s_line);
-      cudaGetLastError();
-      pending_lines_.erase(std::remove(pending_lines_.begin(), pending_lines_.end(), si), pending_lines_.end());
-      s.line_pending = false;
-      s.busy = false;
-    }
+    if (si >= 0) unstage_frame(si);   // a failed submit leaves no trace
   }
   flush_stats(mst_);
   return rc;
 }
 
-int FeContext::submit_impl(double t, const uint8_t *image, int stride, bool on_device, const uint8_t *mask, int mask_stride,
+// The slot is free again and nothing of the frame is pending: its streams are drained (the host-to-device copy may still
+// read h_raw), and a line path that never left the batch will never signal, so its sequence number is taken back.
+void FeContext::unstage_frame(int si) {
+  FrameSlot &s = slots_[si];
+  cudaStreamSynchronize(s.s_a);
+  cudaStreamSynchronize(s.s_b);
+  if (s.s_line) cudaStreamSynchronize(s.s_line);
+  cudaGetLastError();
+  if (s.line_pending) {
+    pending_lines_.erase(std::remove(pending_lines_.begin(), pending_lines_.end(), si), pending_lines_.end());
+    s.line_pending = false;
+    s.seq_lines--;
+  }
+  s.busy = false;
+}
+
+int FeContext::stage_frame(double t, const uint8_t *image, int stride, bool on_device, const uint8_t *mask, int mask_stride,
                            const double vp[6], int *slot_out) {
+  *slot_out = -1;
+  const int rc = [&]() -> int {
   HostTimer ht(&mst_.host_ms[FE_HOST_SUBMIT]);
   FE_CUDA(cudaSetDevice(device_));
   int si = -1;
@@ -674,7 +665,7 @@ int FeContext::submit_impl(double t, const uint8_t *image, int stride, bool on_d
     if (!slots_[i].busy && i != last_slot_) { si = i; break; }
   if (si < 0) return err(FE_BAD_ARG, "submit: lookahead window full (collect a frame first)");
   FrameSlot &s = slots_[si];
-  if (slot_out) *slot_out = si;
+  *slot_out = si;
   s.busy = true;
   s.timestamp = t;
   s.res.clear();
@@ -729,17 +720,17 @@ int FeContext::submit_impl(double t, const uint8_t *image, int stride, bool on_d
   rc = enqueue_frame_independent(s);
   if (rc) return rc;
   s.sc_prev = -1;
-  if (slot_out) *slot_out = si;
-  if (external_) return FE_OK;   // the owner (FeStereo) runs the state machine and releases the slot
-  if (prev_submit_slot_ >= 0) {
-    rc = track_candidates(slots_[prev_submit_slot_], s);
-    if (rc) return rc;
-  }
-  prev_submit_slot_ = si;
-  queue_.push_back(si);
-  s.stage.store(1, std::memory_order_release);
-  klt_q_.push(si);
   return FE_OK;
+  }();
+  flush_stats(mst_);
+  return rc;
+}
+
+void FeContext::queue_lines(int si, const std::vector<Pt> &pts, const std::vector<uint64_t> &ids) {
+  FrameSlot &s = slots_[si];
+  s.res.obs = pts;
+  s.res.obs_ids = ids;
+  line_q_.push(si);
 }
 
 // ------------------------------------------------------------------------------------------ pre-detection
@@ -1081,14 +1072,7 @@ int FeContext::speculate(FrameSlot &prev, const float2 *lk_pts, const uint8_t *l
   int nxt = -1;
   if (!klt_q_.peek(&nxt)) return FE_OK;          // the next frame has not been submitted yet
   FrameSlot &fn = slots_[nxt];
-  LkParams prm;
-  prm.win = cfg_.win_size;
-  prm.max_level = cfg_.pyr_levels;
-  prm.max_count = 30;
-  prm.eps_sq = 0.01f * 0.01f;
-  prm.min_eig = 1e-4f;
-  prm.undistort = 1;
-  for (int i = 0; i < 4; i++) { prm.K[i] = fn.K[i]; prm.D[i] = fn.D[i]; }
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, fn.K, fn.D, true);
   // ---- (A) the points tracked into `prev` whose KLT status is good: latency-critical stream
   int k = 0;
   for (int i = 0; i < n && k < max_pts_; i++)
@@ -1127,6 +1111,7 @@ void FeContext::filter_existing(const std::vector<uint8_t> &mask_test, std::vect
   const int d = cfg_.min_px_dist;
   const int cols = W_, rows = H_;
   const int close_w = (int)((float)cols / (float)d), close_h = (int)((float)rows / (float)d);
+  g.d = d;
   g.close_w = close_w;
   g.close_h = close_h;
   g.close.assign((size_t)close_w * close_h, 0);
@@ -1272,7 +1257,6 @@ int FeContext::perform_detection(const FrameSlot &img, std::vector<Pt> &pts0, st
   src.resize(pts0.size(), -1);   // per point: index into the speculative LK arrays, -1 none, -(2 + i) = candidate i
   HostTimer ht(&kst_.host_ms[FE_HOST_DETECTION]);
   FeFrameInfo *info = &res.info;
-  const int d = cfg_.min_px_dist;
   OccGrids g;
   filter_existing(img.mask, pts0, ids0, &src, nullptr, g);   // TrackKLT.cpp:411-464
   const double min_feat_percent = 0.50;
@@ -1287,10 +1271,7 @@ int FeContext::perform_detection(const FrameSlot &img, std::vector<Pt> &pts0, st
   int added = 0;
   for (size_t e = 0; e < ext.size(); e++) {
     const Pt &kp = ext[e];
-    int x_grid = (int)(kp.x / (float)d), y_grid = (int)(kp.y / (float)d);
-    if (x_grid < 0 || x_grid >= g.close_w || y_grid < 0 || y_grid >= g.close_h) continue;
-    if (g.close[(size_t)y_grid * g.close_w + x_grid] > 127) continue;
-    g.close[(size_t)y_grid * g.close_w + x_grid] = 255;
+    if (!g.take(kp)) continue;
     pts0.push_back(kp);
     ids0.push_back(++currid_);
     src.push_back(-(2 + ext_cand[e]));   // slot of the candidate in the frame's fixed-stride table
@@ -1359,14 +1340,7 @@ int FeContext::perform_matching(const FrameSlot &f0, FrameSlot &f1, std::vector<
     h_pts1_[k] = h_pts0_[k];   // OPTFLOW_USE_INITIAL_FLOW with pts1 = pts0 (:134-138)
   }
   for (int k = 0; k < ns; k++) h_pts1_[n2 + k] = h_pts0_[n2 + k];
-  LkParams prm;
-  prm.win = cfg_.win_size;
-  prm.max_level = cfg_.pyr_levels;
-  prm.max_count = 30;
-  prm.eps_sq = 0.01f * 0.01f;
-  prm.min_eig = 1e-4f;
-  prm.undistort = 1;
-  for (int i = 0; i < 4; i++) { prm.K[i] = f1.K[i]; prm.D[i] = f1.D[i]; }
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, f1.K, f1.D, true);
   // The feature arrays are a few KB: the kernel reads and writes them in pinned, device-mapped host memory directly
   // (no copy-engine operation queued behind the next frame's 700 KB upload, one synchronisation per frame).
   if (nt > 0) {
@@ -1457,6 +1431,35 @@ int FeContext::perform_matching(const FrameSlot &f0, FrameSlot &f1, std::vector<
   info->n_ransac_ok = n_in;
   return FE_OK;
 }
+
+// One LK launch in the pinned, device-mapped tracking buffers (zero-copy I/O, the kernel publishes its own completion
+// flag — see perform_matching)
+int FeContext::lk_launch(const Pyramid &p0, const Pyramid &p1, const std::vector<Pt> &pts, const double K[4], const double D[4],
+                         bool undistort) {
+  const int n = (int)pts.size();
+  if (n > max_pts_) return err(FE_INTERNAL, "stereo LK: more points than the tracking buffers hold");
+  for (int k = 0; k < n; k++) {
+    h_pts0_[k] = make_float2(pts[k].x, pts[k].y);
+    h_pts1_[k] = h_pts0_[k];   // OPTFLOW_USE_INITIAL_FLOW with pts1 = pts0
+  }
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, K, D, undistort);
+  const bool self_signal = launch_lk(p0, p1, h_pts0_, h_pts1_, h_status_, h_p0n_, h_p1n_, n, prm, s_pt_, h_flag_lk_, ++seq_lk_,
+                                     d_lk_done_);
+  if (!self_signal) launch_signal(h_flag_lk_, seq_lk_, s_pt_);
+  FE_CUDA(cudaGetLastError());
+  kst_.kernel_launches_total += self_signal ? 1 : 2;
+  kst_.h2d_bytes += (size_t)n * 2 * sizeof(float2);
+  kst_.d2h_bytes += (size_t)n * (3 * sizeof(float2) + 1);
+  return FE_OK;
+}
+
+int FeContext::lk_wait(LkTracks *out) {
+  if (wait_flag(h_flag_lk_, seq_lk_, s_pt_, &t_err)) return FE_CUDA_ERROR;
+  *out = LkTracks{h_pts1_, h_p0n_, h_p1n_, h_status_};
+  return FE_OK;
+}
+
+void FeContext::flush_tracker_stats() { flush_stats(kst_); }
 
 // -------------------------------------------------------------------------------------------- TrackLSD
 // TrackLSD::AssignPointToLines (:744-792): per line the points inside its (mis-indexed, :754-757) bounding box and within
@@ -1652,22 +1655,26 @@ int FeContext::get_state(void *buf, size_t cap, size_t *n_bytes) {
     last_error = "get_state: collect the pending frames first";
     return FE_BAD_ARG;
   }
+  return write_state(pts_last_, ids_last_, currid_, klt_last_slot_, buf, cap, n_bytes);
+}
+
+int FeContext::write_state(const std::vector<Pt> &pts, const std::vector<uint64_t> &ids, uint64_t currid, int image_slot, void *buf,
+                           size_t cap, size_t *n_bytes) {
   int rc = [&]() -> int {
   FE_CUDA(cudaSetDevice(device_));
-  const int last_slot_ = klt_last_slot_;
-  const bool has_image = last_slot_ >= 0;
-  const StateHeader hd = state_header(W_, H_, currid_, line_currid_, (int)pts_last_.size(), (int)lines_last_.size(), pol_last_,
-                                      has_image, has_image && !slots_[last_slot_].mask.empty());
+  const bool has_image = image_slot >= 0;
+  const StateHeader hd = state_header(W_, H_, currid, line_currid_, (int)pts.size(), (int)lines_last_.size(), pol_last_,
+                                      has_image, has_image && !slots_[image_slot].mask.empty());
   const StateLayout at = state_layout(hd);
   if (n_bytes) *n_bytes = at.size;
   if (!buf || cap < at.size) return buf ? FE_OVERFLOW : FE_OK;
   uint8_t *p = static_cast<uint8_t *>(buf);
-  state_write(p, hd, pts_last_.data(), ids_last_.data(), lines_last_.data(), line_ids_last_.data(), pol_last_);
+  state_write(p, hd, pts.data(), ids.data(), lines_last_.data(), line_ids_last_.data(), pol_last_);
   if (hd.has_image) {
-    const DevImage &l0 = slots_[last_slot_].pyr.lvl[0];
+    const DevImage &l0 = slots_[image_slot].pyr.lvl[0];
     FE_CUDA(cudaMemcpy2D(p + at.image, W_, l0.p, l0.pitch, W_, H_, cudaMemcpyDeviceToHost));
   }
-  if (hd.has_mask) std::memcpy(p + at.mask, slots_[last_slot_].mask.data(), (size_t)W_ * H_);
+  if (hd.has_mask) std::memcpy(p + at.mask, slots_[image_slot].mask.data(), (size_t)W_ * H_);
   return FE_OK;
   }();
   if (rc == FE_CUDA_ERROR) last_error = t_err;
@@ -1679,6 +1686,22 @@ int FeContext::set_state(const void *buf, size_t n_bytes) {
     last_error = "set_state: collect the pending frames first";
     return FE_BAD_ARG;
   }
+  int si = -1;
+  const int rc = load_state(buf, n_bytes, pts_last_, ids_last_, &currid_, &si);
+  if (rc == FE_BAD_ARG) return rc;   // rejected blob: nothing changed
+  last_slot_ = klt_last_slot_ = prev_submit_slot_ = si;
+  cur_slot_ = -1;
+  spec_valid_ = false;
+  last_src_.clear();
+  state_res_.clear();
+  state_res_.obs = pts_last_;
+  state_res_.obs_ids = ids_last_;
+  cur_res_ = &state_res_;
+  return rc;
+}
+
+int FeContext::load_state(const void *buf, size_t n_bytes, std::vector<Pt> &pts, std::vector<uint64_t> &ids, uint64_t *currid,
+                          int *image_slot) {
   // parse into temporaries: the tracker state is only replaced once the whole blob has been checked
   StateView v;
   if (const char *why = state_read(buf, n_bytes, W_, H_, v)) {
@@ -1688,14 +1711,14 @@ int FeContext::set_state(const void *buf, size_t n_bytes) {
   const StateHeader &hd = v.hd;
   int rc = [&]() -> int {
   FE_CUDA(cudaSetDevice(device_));
-  currid_ = hd.currid;
+  *currid = hd.currid;
   line_currid_ = hd.line_currid;
-  pts_last_.resize(hd.n_pts);
-  ids_last_.resize(hd.n_pts);
+  pts.resize(hd.n_pts);
+  ids.resize(hd.n_pts);
   lines_last_.resize(hd.n_lines);
   line_ids_last_.resize(hd.n_lines);
-  std::memcpy(pts_last_.data(), v.base + v.at.pts, (size_t)hd.n_pts * sizeof(Pt));
-  std::memcpy(ids_last_.data(), v.base + v.at.ids, (size_t)hd.n_pts * sizeof(uint64_t));
+  std::memcpy(pts.data(), v.base + v.at.pts, (size_t)hd.n_pts * sizeof(Pt));
+  std::memcpy(ids.data(), v.base + v.at.ids, (size_t)hd.n_pts * sizeof(uint64_t));
   std::memcpy(lines_last_.data(), v.base + v.at.lines, (size_t)hd.n_lines * sizeof(float4));
   std::memcpy(line_ids_last_.data(), v.base + v.at.line_ids, (size_t)hd.n_lines * sizeof(uint64_t));
   pol_last_.swap(v.pol);
@@ -1703,16 +1726,7 @@ int FeContext::set_state(const void *buf, size_t n_bytes) {
     s.busy = false;
   }
   FE_CUDA(cudaDeviceSynchronize());
-  last_slot_ = -1;
-  klt_last_slot_ = -1;
-  cur_slot_ = -1;
-  spec_valid_ = false;
-  prev_submit_slot_ = -1;
-  last_src_.clear();
-  state_res_.clear();
-  state_res_.obs = pts_last_;
-  state_res_.obs_ids = ids_last_;
-  cur_res_ = &state_res_;
+  *image_slot = -1;
   if (hd.has_image) {
     FrameSlot &s = slots_[0];
     s.busy = true;
@@ -1734,9 +1748,7 @@ int FeContext::set_state(const void *buf, size_t n_bytes) {
     }
     if (hd.has_mask) s.mask.assign(v.base + v.at.mask, v.base + v.at.mask + (size_t)W_ * H_);
     else s.mask.clear();
-    last_slot_ = 0;
-    klt_last_slot_ = 0;
-    prev_submit_slot_ = 0;
+    *image_slot = 0;
   }
   return FE_OK;
   }();

@@ -145,15 +145,29 @@ struct FrameSlot {
 // Occupancy bookkeeping of one top-off detection (TrackKLT.cpp:401-408): the min-distance grid, the per-cell counts and
 // the squares that mask0_updated gets around every kept point.
 struct OccGrids {
+  int d = 1;   // min_px_dist: the min-distance cell size
   int close_w = 0, close_h = 0;
   std::vector<uint8_t> close, grid;
   std::vector<std::pair<int, int>> rects;
+  // A new point is added only if its min-distance cell is inside the grid and free; the cell is then taken
+  // (TrackKLT.cpp:497-512; stereo: :631-645 left, :779-793 right)
+  bool take(const Pt &kp) {
+    const int x = (int)(kp.x / (float)d), y = (int)(kp.y / (float)d);
+    if (x < 0 || x >= close_w || y < 0 || y >= close_h) return false;
+    uint8_t &c = close[(size_t)y * close_w + x];
+    if (c > 127) return false;
+    c = 255;
+    return true;
+  }
 };
 
-class FeStereo;
+// Results of FeContext::lk_launch in the context's pinned tracking buffers, valid until its next launch
+struct LkTracks {
+  const float2 *pts1, *p0n, *p1n;
+  const uint8_t *status;
+};
 
 class FeContext {
-  friend class FeStereo;
  public:
   FeContext(const FeConfig &cfg, int device);
   ~FeContext();
@@ -190,22 +204,50 @@ class FeContext {
   FeStageTimes snapshot_times();
   void reset_times();
 
+  // ---- building blocks for an owner that runs its own point tracker on this context's frames (FeStereo).  Errors
+  // leave their text in thread_error() (write_state / load_state: in last_error).
+  // Takes a free slot (*slot_out; -1 if none) and enqueues the frame's frame-independent work.  If this fails after a
+  // slot was taken, unstage_frame() gives the slot back.
+  int stage_frame(double t, const uint8_t *image, int stride, bool on_device, const uint8_t *mask, int mask_stride,
+                  const double vp[6], int *slot_out);
+  void unstage_frame(int si);   // undoes a staged frame whose submit failed: nothing of it stays pending
+  void release_slot(int si) { slots_[si].busy = false; }
+  FrameSlot &slot(int si) { return slots_[si]; }
+  cudaStream_t track_stream() const { return s_pt_; }
+  int flush_line_batch();   // launches the line paths of the frames waiting in the line batch as ONE batch
+  // hands a tracked frame to the line tracker thread with the points it is associated against
+  void queue_lines(int si, const std::vector<Pt> &pts, const std::vector<uint64_t> &ids);
+  // LK of pts from p0 into p1 (initial guess: pts) on track_stream(), in the tracking buffers; lk_wait() waits for it.
+  // Launch and wait are separate so that the launches of several contexts run side by side.
+  int lk_launch(const Pyramid &p0, const Pyramid &p1, const std::vector<Pt> &pts, const double K[4], const double D[4],
+                bool undistort);
+  int lk_wait(LkTracks *out);
+  // the two halves of the top-off detection that the monocular and the stereo state machines share
+  void filter_existing(const std::vector<uint8_t> &mask_test, std::vector<Pt> &pts, std::vector<uint64_t> &ids, std::vector<int> *src,
+                       const std::vector<uint64_t> *stereo_ids, OccGrids &g) const;
+  int grid_candidates(FrameSlot &slot, const std::vector<uint8_t> &mask_resize, const std::vector<uint8_t> &mask_clone,
+                      const OccGrids &g, std::vector<Pt> &ext, std::vector<int> &ext_cand, FrameResult &res);
+  void flush_tracker_stats();   // thread that runs the point tracker: lk_launch / grid_candidates statistics
+  // State blob (state_blob.h) from point-tracker state passed in (image_slot: the slot holding the previous image, -1
+  // none) and this context's line-tracker state; load_state() loads one, the image into a slot, and hands the
+  // point-tracker state back.  Only legal while nothing is in flight.
+  int write_state(const std::vector<Pt> &pts, const std::vector<uint64_t> &ids, uint64_t currid, int image_slot, void *buf,
+                  size_t cap, size_t *n_bytes);
+  int load_state(const void *buf, size_t n_bytes, std::vector<Pt> &pts, std::vector<uint64_t> &ids, uint64_t *currid,
+                 int *image_slot);
+
  private:
   int fail(cudaError_t e, const char *what);
   int err(int code, const std::string &msg);
-  int submit_impl(double t, const uint8_t *image, int stride, bool on_device, const uint8_t *mask, int mask_stride,
-                  const double vp[6], int *slot_out = nullptr);
   int collect_impl(FeFrameInfo *info);
   void flush_stats(FeStageTimes &local);
   void klt_main();
   void line_main();
-  int spin_sync(cudaStream_t st);
   int wait_flag(volatile int *flag, int value, cudaStream_t st, std::string *err);
   int enqueue_frame_independent(FrameSlot &s);
   int record_image_path(FrameSlot &s, cudaStream_t st);
   int record_fast_path(FrameSlot &s, cudaStream_t st);
   int record_line_path(FrameSlot &s, cudaStream_t st);
-  int flush_line_batch();   // launches the line paths of the frames waiting in pending_lines_ as ONE batch
   int build_graphs(FrameSlot &s);
   void destroy_graphs(FrameSlot &s);
   void layout_cells();                       // all grid cells of the frame (Grider_GRID geometry)
@@ -215,11 +257,6 @@ class FeContext {
   int klt_feed(FrameSlot &cur);
   int perform_detection(const FrameSlot &img, std::vector<Pt> &pts, std::vector<uint64_t> &ids, std::vector<int> &src,
                         FrameResult &res);
-  // the two halves of the top-off detection that the monocular and the stereo state machines share
-  void filter_existing(const std::vector<uint8_t> &mask_test, std::vector<Pt> &pts, std::vector<uint64_t> &ids, std::vector<int> *src,
-                       const std::vector<uint64_t> *stereo_ids, OccGrids &g) const;
-  int grid_candidates(FrameSlot &slot, const std::vector<uint8_t> &mask_resize, const std::vector<uint8_t> &mask_clone,
-                      const OccGrids &g, std::vector<Pt> &ext, std::vector<int> &ext_cand, FrameResult &res);
   int perform_matching(const FrameSlot &f0, FrameSlot &f1, std::vector<Pt> &pts0, const std::vector<int> &src, bool spec,
                        std::vector<Pt> &pts1, std::vector<uint8_t> &mask_out, bool &mask_empty, FrameResult &res);
   int speculate(FrameSlot &prev, const float2 *lk_pts, const uint8_t *lk_status, int n);
@@ -228,7 +265,6 @@ class FeContext {
   int lsd_feed(FrameSlot &cur);
 
   FeConfig cfg_;
-  bool external_ = false;   // the frame-independent pipeline only: a FeStereo owns the tracker state and the slots
   int device_;
   int W_, H_;            // tracking size (= input size, or half of it with cfg.downsample)
   int Win_, Hin_;        // input size
@@ -275,8 +311,6 @@ class FeContext {
   std::vector<int> sc_shared_, sc_touched_;
   // ---- tracking scratch
   int max_pts_ = 0;
-  float2 *d_pts0_ = nullptr, *d_pts1_ = nullptr, *d_p0n_ = nullptr, *d_p1n_ = nullptr;
-  uint8_t *d_status_ = nullptr;
   unsigned *d_lk_done_ = nullptr;   // features finished in the running LK launches (completion signals) [ordinary, speculative]
   // ---- speculative tracking (FeContext::speculate): LK(t -> t+1) for every point that may be tracked, launched before
   // frame t's RANSAC gate
@@ -295,7 +329,6 @@ class FeContext {
   float2 *h_pts0_ = nullptr, *h_pts1_ = nullptr, *h_p0n_ = nullptr, *h_p1n_ = nullptr;
   uint8_t *h_status_ = nullptr;
   cudaEvent_t ev_pt_[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  cudaEvent_t ev_sync_ = nullptr;
   int *h_flag_lk_ = nullptr;
   int seq_lk_ = 0;
   int cur_slot_ = -1;

@@ -618,14 +618,7 @@ int FeGroup::launch_track(int tick) {
   TrackJob *hj = h_tjobs_ + (size_t)ring * S_, *dj = d_tjobs_ + (size_t)ring * S_;
   int nj = 0;
   for (int s = 0; s < S_; s++) nj += tr.cur_slot[s] >= 0 ? 1 : 0;
-  LkParams prm;
-  prm.win = cfg_.win_size;
-  prm.max_level = cfg_.pyr_levels;
-  prm.max_count = 30;
-  prm.eps_sq = 0.01f * 0.01f;
-  prm.min_eig = 1e-4f;
-  prm.undistort = 1;
-  for (int i = 0; i < 4; i++) prm.K[i] = prm.D[i] = 0;
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, nullptr, nullptr, true);
   const bool tm = timing_;
   // jobs are stored in stream order; lane l owns streams [S l / lanes, S (l + 1) / lanes) for the lifetime of the group
   // (a stream's frames are tracked in order on ONE CUDA stream), i.e. a contiguous range of the tick's jobs

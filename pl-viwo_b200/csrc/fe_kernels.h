@@ -137,6 +137,22 @@ struct LkParams {
   double K[4], D[4];
   int undistort;   // also write normalised coordinates of pts0 / pts1
 };
+// The reference's termination criteria and eigenvalue threshold (TrackKLT.cpp:855-858) with the given window, pyramid
+// depth and calibration (K / D null: zeros).  Host only.
+inline LkParams lk_params(int win, int max_level, const double *K, const double *D, bool undistort) {
+  LkParams prm;
+  prm.win = win;
+  prm.max_level = max_level;
+  prm.max_count = 30;
+  prm.eps_sq = 0.01f * 0.01f;
+  prm.min_eig = 1e-4f;
+  prm.undistort = undistort ? 1 : 0;
+  for (int i = 0; i < 4; i++) {
+    prm.K[i] = K ? K[i] : 0;
+    prm.D[i] = D ? D[i] : 0;
+  }
+  return prm;
+}
 // host_flag / flag_value / d_done_counter (optional): the kernel itself publishes flag_value to the pinned word when its
 // last feature is done (d_done_counter: one zeroed device word).  Returns true if the kernel will do so; false means
 // the caller has to queue its own completion signal (generic-window kernel).

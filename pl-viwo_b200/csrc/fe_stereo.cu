@@ -34,7 +34,6 @@ FeStereo::FeStereo(const FeConfig &cfg, const double K_right[4], const double D_
   }
   cam_[0].reset(new FeContext(cfg_, device));
   cam_[1].reset(new FeContext(cr, device));
-  cam_[0]->external_ = cam_[1]->external_ = true;
   currid_ = 4 * (uint64_t)cfg.numaruco + 1;   // TrackBase.cpp:34
 }
 
@@ -75,10 +74,15 @@ int FeStereo::set_calib(int cam, const double K[4], const double D[4]) {
 
 int FeStereo::set_num_features(int n) {
   if (!queue_.empty()) return err(FE_BAD_ARG, "set_num_features: collect the pending pairs first");
-  if (n < 1 || cam_[0]->cand_table_size(n) > cam_[0]->cand_cap_)
+  // both cameras have the same image size, grid and capacity: the right one accepts what the left one accepts
+  if (cam_[0]->set_num_features(n) || cam_[1]->set_num_features(n))
     return err(FE_BAD_ARG, "set_num_features: the candidate table of that feature count exceeds the capacity this rig was created with");
   cfg_.num_features = n;
-  cam_[0]->cfg_.num_features = cam_[1]->cfg_.num_features = n;
+  return FE_OK;
+}
+
+int FeStereo::classify_lines(const double vp[6]) {
+  for (FeLineRow &row : left_res_->line_rows) row.D = line_classification(make_float4(row.line[0], row.line[1], row.line[2], row.line[3]), vp);
   return FE_OK;
 }
 
@@ -104,21 +108,11 @@ int FeStereo::submit(double t, const uint8_t *const image[2], int stride, bool o
   if (ri < 0) return err(FE_BAD_ARG, "submit: lookahead window full (collect a pair first)");
   int slot[2] = {-1, -1};
   for (int c = 0; c < 2; c++) {
-    int rc = cam_[c]->submit_impl(t, image[c], stride, on_device, mask ? mask[c] : nullptr, mask_stride, c == 0 ? vp : nullptr,
+    int rc = cam_[c]->stage_frame(t, image[c], stride, on_device, mask ? mask[c] : nullptr, mask_stride, c == 0 ? vp : nullptr,
                                   &slot[c]);
-    cam_[c]->flush_stats(cam_[c]->mst_);
-    if (rc) {
-      if (c == 1 && slot[0] >= 0) {   // give the left image's slot back (and take it out of an unlaunched line batch)
-        FeContext &lc = *cam_[0];
-        auto &pl = lc.pending_lines_;
-        if (lc.slots_[slot[0]].line_pending) {
-          pl.erase(std::remove(pl.begin(), pl.end(), slot[0]), pl.end());
-          lc.slots_[slot[0]].line_pending = false;
-          lc.slots_[slot[0]].seq_lines--;   // its completion signal will never be queued
-        }
-        lc.slots_[slot[0]].busy = false;
-      }
-      if (slot[c] >= 0) cam_[c]->slots_[slot[c]].busy = false;
+    if (rc) {   // a failed submit leaves no trace: neither image stays staged
+      for (int k = 0; k <= c; k++)
+        if (slot[k] >= 0) cam_[k]->unstage_frame(slot[k]);
       return err(rc, FeContext::thread_error());
     }
   }
@@ -156,8 +150,6 @@ void FeStereo::track_main() {
   while (work_q_.pop(&ri)) {
     Pair &p = *ring_[ri];
     int rc = collect_impl(p);
-    FeContext &lc = *cam_[0];
-    FrameSlot &L = lc.slots_[p.slot[0]];
     for (int c = 0; c < 2; c++) {
       p.obs[c] = pts_last_[c];
       p.obs_ids[c] = ids_last_[c];
@@ -169,14 +161,11 @@ void FeStereo::track_main() {
     // thread (the association of pair t overlaps the tracking of pair t + 1).  Its line path was launched by the
     // caller's thread (at submit, or by collect() when the batch never filled).
     p.lines_queued = false;
-    if (rc == FE_OK && cfg_.use_lines && L.has_vp) {
-      L.res.obs = pts_last_[0];
-      L.res.obs_ids = ids_last_[0];
-      L.res.rc = FE_OK;
+    if (rc == FE_OK && cfg_.use_lines && cam_[0]->slot(p.slot[0]).has_vp) {
       p.lines_queued = true;
-      lc.line_q_.push(p.slot[0]);
+      cam_[0]->queue_lines(p.slot[0], pts_last_[0], ids_last_[0]);
     }
-    for (int c = 0; c < 2; c++) cam_[c]->flush_stats(cam_[c]->kst_);
+    for (int c = 0; c < 2; c++) cam_[c]->flush_tracker_stats();
     last_[0] = p.slot[0];   // move forward in time whatever happened (:366-378)
     last_[1] = p.slot[1];
     p.rc = rc;
@@ -190,10 +179,9 @@ int FeStereo::collect(FeStereoInfo *info) {
   if (queue_.empty()) return err(FE_BAD_ARG, "collect: nothing submitted");
   const int ri = queue_.front();
   Pair &p = *ring_[ri];
-  FeContext &lc = *cam_[0];
-  FrameSlot &L = lc.slots_[p.slot[0]];
+  FrameSlot &L = cam_[0]->slot(p.slot[0]);
   if (L.line_pending) {   // its line batch never filled up: launch what is there
-    int rc = lc.flush_line_batch();
+    int rc = cam_[0]->flush_line_batch();
     if (rc) return err(rc, FeContext::thread_error());
   }
   for (unsigned spins = 0; p.stage.load(std::memory_order_acquire) != 2; spins++) {
@@ -224,12 +212,11 @@ int FeStereo::collect(FeStereoInfo *info) {
     obs_[c].swap(p.obs[c]);
     obs_ids_[c].swap(p.obs_ids[c]);
   }
-  lc.cur_res_ = &L.res;   // line rows / line points of the left image (plviwo_fe_stereo_get_line_rows)
-  lc.cur_slot_ = p.slot[0];
+  left_res_ = &L.res;   // line rows / line points of the left image (plviwo_fe_stereo_get_line_rows)
   // the previous collected pair's slots become free: its pyramids are no longer the tracker's "last" pair (the tracker
   // finished THIS pair, which was the last one to read them)
   for (int c = 0; c < 2; c++) {
-    if (released_[c] >= 0) cam_[c]->slots_[released_[c]].busy = false;
+    if (released_[c] >= 0) cam_[c]->release_slot(released_[c]);
     released_[c] = p.slot[c];
   }
   st_.frames++;
@@ -238,43 +225,6 @@ int FeStereo::collect(FeStereoInfo *info) {
   if (rc) last_error = p.error;
   p.stage.store(0, std::memory_order_release);
   return rc;
-}
-
-// ------------------------------------------------------------------------------------------------ LK plumbing
-// One LK launch on camera `cam`'s tracking stream with that context's pinned, device-mapped feature arrays
-// (zero-copy I/O, the kernel publishes its own completion flag — see FeContext::perform_matching).
-int FeStereo::lk_launch(int cam, const Pyramid &p0, const Pyramid &p1, const std::vector<Pt> &pts, const double K[4],
-                        const double D[4], bool undistort) {
-  FeContext &c = *cam_[cam];
-  const int n = (int)pts.size();
-  if (n > c.max_pts_) return err(FE_INTERNAL, "stereo LK: more points than the tracking buffers hold");
-  for (int k = 0; k < n; k++) {
-    c.h_pts0_[k] = make_float2(pts[k].x, pts[k].y);
-    c.h_pts1_[k] = c.h_pts0_[k];   // OPTFLOW_USE_INITIAL_FLOW with pts1 = pts0
-  }
-  LkParams prm;
-  prm.win = cfg_.win_size;
-  prm.max_level = cfg_.pyr_levels;
-  prm.max_count = 30;
-  prm.eps_sq = 0.01f * 0.01f;
-  prm.min_eig = 1e-4f;
-  prm.undistort = undistort ? 1 : 0;
-  for (int i = 0; i < 4; i++) { prm.K[i] = K[i]; prm.D[i] = D[i]; }
-  const bool self_signal = launch_lk(p0, p1, c.h_pts0_, c.h_pts1_, c.h_status_, c.h_p0n_, c.h_p1n_, n, prm, c.s_pt_, c.h_flag_lk_,
-                                     ++c.seq_lk_, c.d_lk_done_);
-  if (!self_signal) launch_signal(c.h_flag_lk_, c.seq_lk_, c.s_pt_);
-  ST_CUDA(cudaGetLastError());
-  c.kst_.kernel_launches_total += self_signal ? 1 : 2;
-  c.kst_.h2d_bytes += (size_t)n * 2 * sizeof(float2);
-  c.kst_.d2h_bytes += (size_t)n * (3 * sizeof(float2) + 1);
-  return FE_OK;
-}
-
-int FeStereo::lk_wait(int cam) {
-  FeContext &c = *cam_[cam];
-  std::string e;
-  if (c.wait_flag(c.h_flag_lk_, c.seq_lk_, c.s_pt_, &e)) return err(FE_CUDA_ERROR, e);
-  return FE_OK;
 }
 
 // TrackKLT.cpp:829-868: the launch half ...
@@ -286,8 +236,8 @@ int FeStereo::matching_begin(int cam, FrameSlot &f0, FrameSlot &f1, const std::v
   m.mask_empty = false;
   m.mask.assign(m.n, 0);
   if (m.n < 10) return FE_OK;        // :848-852
-  int rc = lk_launch(cam, f0.pyr, f1.pyr, pts0, f1.K, f1.D, true);
-  if (rc) return rc;
+  int rc = cam_[cam]->lk_launch(f0.pyr, f1.pyr, pts0, f1.K, f1.D, true);
+  if (rc) return err(rc, FeContext::thread_error());
   m.launched = true;
   return FE_OK;
 }
@@ -296,21 +246,21 @@ int FeStereo::matching_begin(int cam, FrameSlot &f0, FrameSlot &f1, const std::v
 int FeStereo::matching_end(int cam, FrameSlot &f1, const std::vector<Pt> &pts0, Match &m, FeStereoInfo &info) {
   (void)pts0;
   if (!m.launched) return FE_OK;
-  int rc = lk_wait(cam);
-  if (rc) return rc;
-  FeContext &c = *cam_[cam];
+  LkTracks c;
+  int rc = cam_[cam]->lk_wait(&c);
+  if (rc) return err(rc, FeContext::thread_error());
   const int n = m.n;
   const double max_focal = std::max(f1.K[0], f1.K[1]);   // id0 == id1 for the temporal tracks
   std::vector<uint8_t> mask_rsc(n, 0);
   int mask_valid = 0;
-  const int n_in = ransac_fundamental(reinterpret_cast<const float *>(c.h_p0n_), reinterpret_cast<const float *>(c.h_p1n_), n,
+  const int n_in = ransac_fundamental(reinterpret_cast<const float *>(c.p0n), reinterpret_cast<const float *>(c.p1n), n,
                                       2.0 / max_focal, 0.999, mask_rsc.data(), &mask_valid);
-  m.p1n.assign(c.h_p1n_, c.h_p1n_ + n);
+  m.p1n.assign(c.p1n, c.p1n + n);
   int n_klt = 0;
   for (int i = 0; i < n; i++) {
-    m.mask[i] = (c.h_status_[i] && mask_valid && mask_rsc[i]) ? 1 : 0;
-    n_klt += c.h_status_[i] ? 1 : 0;
-    m.pts1[i] = Pt{c.h_pts1_[i].x, c.h_pts1_[i].y};
+    m.mask[i] = (c.status[i] && mask_valid && mask_rsc[i]) ? 1 : 0;
+    n_klt += c.status[i] ? 1 : 0;
+    m.pts1[i] = Pt{c.pts1[i].x, c.pts1[i].y};
   }
   info.n_lk_in[cam] = n;
   info.n_klt_ok[cam] = n_klt;
@@ -321,7 +271,6 @@ int FeStereo::matching_end(int cam, FrameSlot &f1, const std::vector<Pt> &pts0, 
 // ------------------------------------------------------------------------------------ perform_detection_stereo
 int FeStereo::detection_stereo(FrameSlot &L, FrameSlot &R, std::vector<Pt> &pts0, std::vector<Pt> &pts1, std::vector<uint64_t> &ids0,
                                std::vector<uint64_t> &ids1, FeStereoInfo &info) {
-  const int d = cfg_.min_px_dist;
   const int cols = cfg_.width, rows = cfg_.height;
   const int thr = std::min(20, (int)(0.50 * cfg_.num_features));
   std::vector<Pt> ext;
@@ -334,26 +283,20 @@ int FeStereo::detection_stereo(FrameSlot &L, FrameSlot &R, std::vector<Pt> &pts0
     int rc = cam_[0]->grid_candidates(L, L.mask, L.mask, g0, ext, ext_cand, scratch_res_);
     if (rc) return err(rc, FeContext::thread_error());
     std::vector<Pt> new0;
-    for (const Pt &kp : ext) {   // :631-645
-      int x_grid = (int)(kp.x / (float)d), y_grid = (int)(kp.y / (float)d);
-      if (x_grid < 0 || x_grid >= g0.close_w || y_grid < 0 || y_grid >= g0.close_h) continue;
-      if (g0.close[(size_t)y_grid * g0.close_w + x_grid] > 127) continue;
-      g0.close[(size_t)y_grid * g0.close_w + x_grid] = 255;
-      new0.push_back(kp);
-    }
+    for (const Pt &kp : ext)   // :631-645
+      if (g0.take(kp)) new0.push_back(kp);
     if (!new0.empty()) {
       // left -> right KLT of the new points, initial guess = the left position, no RANSAC gate (:658-666)
-      rc = lk_launch(0, L.pyr, R.pyr, new0, L.K, L.D, false);
-      if (rc) return rc;
-      rc = lk_wait(0);
-      if (rc) return rc;
-      const FeContext &c = *cam_[0];
+      LkTracks c;
+      rc = cam_[0]->lk_launch(L.pyr, R.pyr, new0, L.K, L.D, false);
+      if (rc == FE_OK) rc = cam_[0]->lk_wait(&c);
+      if (rc) return err(rc, FeContext::thread_error());
       for (size_t i = 0; i < new0.size(); i++) {   // :669-699
         const Pt p0 = new0[i];
-        const Pt p1 = Pt{c.h_pts1_[i].x, c.h_pts1_[i].y};
+        const Pt p1 = Pt{c.pts1[i].x, c.pts1[i].y};
         const bool oob_left = (int)p0.x < 0 || (int)p0.x >= cols || (int)p0.y < 0 || (int)p0.y >= rows;
         const bool oob_right = (int)p1.x < 0 || (int)p1.x >= cols || (int)p1.y < 0 || (int)p1.y >= rows;
-        if (!oob_left && !oob_right && c.h_status_[i] == 1) {
+        if (!oob_left && !oob_right && c.status[i] == 1) {
           const uint64_t id = ++currid_;
           pts0.push_back(p0);
           pts1.push_back(p1);
@@ -378,12 +321,9 @@ int FeStereo::detection_stereo(FrameSlot &L, FrameSlot &R, std::vector<Pt> &pts0
     int rc = cam_[1]->grid_candidates(R, R.mask, L.mask, g1, ext, ext_cand, scratch_res_);
     if (rc) return err(rc, FeContext::thread_error());
     for (const Pt &kp : ext) {   // :779-793
-      int x_grid = (int)(kp.x / (float)d), y_grid = (int)(kp.y / (float)d);
-      if (x_grid < 0 || x_grid >= g1.close_w || y_grid < 0 || y_grid >= g1.close_h) continue;
-      if (g1.close[(size_t)y_grid * g1.close_w + x_grid] > 127) continue;
+      if (!g1.take(kp)) continue;
       pts1.push_back(kp);
       ids1.push_back(++currid_);
-      g1.close[(size_t)y_grid * g1.close_w + x_grid] = 255;
       info.n_detected[1]++;
     }
   }
@@ -393,14 +333,14 @@ int FeStereo::detection_stereo(FrameSlot &L, FrameSlot &R, std::vector<Pt> &pts0
 // ------------------------------------------------------------------------------------------------ feed_stereo
 int FeStereo::collect_impl(Pair &pair) {
   FeStereoInfo *info = &pair.info;
-  FrameSlot &L = cam_[0]->slots_[pair.slot[0]], &R = cam_[1]->slots_[pair.slot[1]];
+  FrameSlot &L = cam_[0]->slot(pair.slot[0]), &R = cam_[1]->slot(pair.slot[1]);
   std::vector<FePointRow> *rows_out = pair.rows;
   rows_out[0].clear();
   rows_out[1].clear();
   // every tracking stream may read either image of the pair (the left->right launch runs on the left stream)
   for (int c = 0; c < 2; c++) {
-    ST_CUDA(cudaStreamWaitEvent(cam_[c]->s_pt_, L.ev_pyr, 0));
-    ST_CUDA(cudaStreamWaitEvent(cam_[c]->s_pt_, R.ev_pyr, 0));
+    ST_CUDA(cudaStreamWaitEvent(cam_[c]->track_stream(), L.ev_pyr, 0));
+    ST_CUDA(cudaStreamWaitEvent(cam_[c]->track_stream(), R.ev_pyr, 0));
   }
   const int cols = cfg_.width, rows = cfg_.height;
   // :221-241 — nothing tracked last time: detect on the CURRENT pair only
@@ -414,7 +354,7 @@ int FeStereo::collect_impl(Pair &pair) {
     info->first_frame = 1;
     return FE_OK;
   }
-  FrameSlot &L0 = cam_[0]->slots_[last_[0]], &R0 = cam_[1]->slots_[last_[1]];
+  FrameSlot &L0 = cam_[0]->slot(last_[0]), &R0 = cam_[1]->slot(last_[1]);
   // top-off on the PREVIOUS pair (:245-252)
   std::vector<Pt> pl_old = pts_last_[0], pr_old = pts_last_[1];
   std::vector<uint64_t> il_old = ids_last_[0], ir_old = ids_last_[1];
@@ -507,13 +447,8 @@ int FeStereo::get_state(void *buf, size_t cap, size_t *n_bytes) {
   if (!queue_.empty()) return err(FE_BAD_ARG, "get_state: collect the pending pairs first");
   size_t sz[2] = {0, 0};
   for (int c = 0; c < 2; c++) {
-    FeContext &x = *cam_[c];
-    x.pts_last_ = pts_last_[c];
-    x.ids_last_ = ids_last_[c];
-    x.currid_ = currid_;
-    x.klt_last_slot_ = last_[c];
-    int rc = x.get_state(nullptr, 0, &sz[c]);
-    if (rc) return err(rc, x.last_error);
+    int rc = cam_[c]->write_state(pts_last_[c], ids_last_[c], currid_, last_[c], nullptr, 0, &sz[c]);
+    if (rc) return err(rc, cam_[c]->last_error);
   }
   const size_t need = sizeof(StereoStateHeader) + sz[0] + sz[1];
   if (n_bytes) *n_bytes = need;
@@ -530,7 +465,7 @@ int FeStereo::get_state(void *buf, size_t cap, size_t *n_bytes) {
   p += sizeof(hd);
   for (int c = 0; c < 2; c++) {
     size_t got = 0;
-    int rc = cam_[c]->get_state(p, sz[c], &got);
+    int rc = cam_[c]->write_state(pts_last_[c], ids_last_[c], currid_, last_[c], p, sz[c], &got);
     if (rc) return err(rc, cam_[c]->last_error);
     p += sz[c];
   }
@@ -546,17 +481,14 @@ int FeStereo::set_state(const void *buf, size_t n_bytes) {
   if (hd.magic != 0x504c5653u || sizeof(hd) + hd.size[0] + hd.size[1] > n_bytes) return err(FE_BAD_ARG, "set_state: not a stereo state blob");
   for (int c = 0; c < 2; c++) {
     FeContext &x = *cam_[c];
-    int rc = x.set_state(p, hd.size[c]);
+    uint64_t cam_currid = 0;   // one id counter for both cameras: the envelope's
+    int rc = x.load_state(p, hd.size[c], pts_last_[c], ids_last_[c], &cam_currid, &last_[c]);
     if (rc) return err(rc, x.last_error.empty() ? "set_state: camera blob rejected" : x.last_error);
     p += hd.size[c];
-    pts_last_[c] = x.pts_last_;
-    ids_last_[c] = x.ids_last_;
-    obs_[c] = x.pts_last_;
-    obs_ids_[c] = x.ids_last_;
-    last_[c] = x.klt_last_slot_;
-    released_[c] = x.klt_last_slot_;   // the slot the image was loaded into is busy until the next pair has been collected
-    x.last_slot_ = -1;   // slot ownership is ours: the context must not keep its own "last collected" exclusion
-    x.flush_stats(x.mst_);
+    obs_[c] = pts_last_[c];
+    obs_ids_[c] = ids_last_[c];
+    released_[c] = last_[c];   // the slot the image was loaded into is busy until the next pair has been collected
+    left_res_ = &no_lines_;
   }
   currid_ = hd.currid;
   rows_[0].clear();

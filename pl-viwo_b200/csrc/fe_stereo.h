@@ -1,8 +1,8 @@
 // Stereo point tracker: ov_core::TrackKLT with use_stereo = true fed two images per message
 // (open_vins/ov_core/src/track/TrackKLT.cpp:202-393 feed_stereo, :530-827 perform_detection_stereo).
-// One FeStereo = one stereo rig on one device.  It owns two FeContext objects in "external" mode — each runs the
-// frame-independent pipeline of one camera (copy, equalise, pyramid, FAST on every cell, std::sort + top-k, cornerSubPix)
-// on its own streams at submit() — and runs the stereo state machine itself at collect().
+// One FeStereo = one stereo rig on one device.  It owns two FeContext objects and stages each camera's frames in one of
+// them — each runs the frame-independent pipeline of one camera (copy, equalise, pyramid, FAST on every cell, std::sort +
+// top-k, cornerSubPix) on its own streams at submit() — and runs the stereo state machine itself on its tracker thread.
 #pragma once
 #include <atomic>
 #include <deque>
@@ -38,8 +38,8 @@ class FeStereo {
   const std::vector<FePointRow> &rows(int cam) const { return rows_[cam]; }
   const std::vector<Pt> &last_obs(int cam) const { return obs_[cam]; }
   const std::vector<uint64_t> &last_ids(int cam) const { return obs_ids_[cam]; }
-  const FrameResult &left_result() const { return cam_[0]->result(); }   // line rows / line points of the left image
-  int classify_lines(const double vp[6]) { return cam_[0]->classify_lines(vp); }
+  const FrameResult &left_result() const { return *left_res_; }   // line rows / line points of the left image
+  int classify_lines(const double vp[6]);
   std::string last_error;
 
  private:
@@ -68,9 +68,6 @@ class FeStereo {
   int collect_impl(Pair &p);
   int detection_stereo(FrameSlot &L, FrameSlot &R, std::vector<Pt> &pts0, std::vector<Pt> &pts1, std::vector<uint64_t> &ids0,
                        std::vector<uint64_t> &ids1, FeStereoInfo &info);
-  int lk_launch(int cam, const Pyramid &p0, const Pyramid &p1, const std::vector<Pt> &pts, const double K[4], const double D[4],
-                bool undistort);
-  int lk_wait(int cam);
   int matching_begin(int cam, FrameSlot &f0, FrameSlot &f1, const std::vector<Pt> &pts0, Match &m);
   int matching_end(int cam, FrameSlot &f1, const std::vector<Pt> &pts0, Match &m, FeStereoInfo &info);
 
@@ -92,6 +89,8 @@ class FeStereo {
   std::vector<FePointRow> rows_[2];          // of the last collected pair
   std::vector<Pt> obs_[2];
   std::vector<uint64_t> obs_ids_[2];
+  FrameResult *left_res_ = &no_lines_;      // the left image's result of the last collected pair
+  FrameResult no_lines_;                     // ... before the first collect and after set_state
   FrameResult scratch_res_;
   FeStageTimes st_{};
 };
