@@ -359,6 +359,38 @@ int plviwo_fe_group_tap(FeGroupHandle *g, int stream, int what /* FE_TAP_PYR_LEV
 int plviwo_fe_group_enable_timing(FeGroupHandle *g, int on);
 int plviwo_fe_group_get_times(FeGroupHandle *g, FeGroupTimes *out, int reset);
 
+/* ---- stereo group: many stereo rigs of one device tracked together --------------------------------------- */
+/* Rig r of a stereo group is what one FeStereoHandle is — same point rows of both cameras, same pts_last / ids_last, same
+ * FeStereoInfo, same left-image line rows and state blob, bit for bit, when fed the same pairs — but the rigs of a tick share
+ * their kernel launches and the stereo state machine (top-off detection of both cameras with the left -> right KLT of the new
+ * points, temporal LK, the two RANSAC gates, the stereo row merge, the left image's line tracker) runs on the device.  Rig r is
+ * the group's camera streams 2r (left) and 2r + 1 (right).
+ * Calibration: cfg->K / cfg->D for every camera at creation, then per (rig, cam) from the next submitted tick.
+ * submit: per rig a left and a right image (both NULL: no pair this tick, its info timestamp is -1; exactly one NULL is
+ * FE_BAD_ARG and nothing is enqueued), masks per rig (both or neither; the mask arrays may be NULL), vps NULL (no line
+ * tracker) or 6 doubles per rig.  play: images[(t * n_rigs + r) * 2 + cam], one FePlayStats per rig (point rows of both
+ * cameras).  The state blob is the stereo rig's (plviwo_fe_stereo_get_state).  Each camera of a rig holds up to
+ * max(4096, 8 * num_features) points, as the stereo handle's tracking buffers; beyond that collect returns FE_INTERNAL.
+ * Not supported: cfg->downsample, cfg->line_samples (refused at creation), set_num_features / change_feat_id, taps, timing. */
+typedef struct FeStereoGroupHandle FeStereoGroupHandle;
+int plviwo_fe_stereo_group_create(const FeConfig *cfg, int n_rigs /* [1, 2048] */, int device, FeStereoGroupHandle **out);
+int plviwo_fe_stereo_group_destroy(FeStereoGroupHandle *g);
+const char *plviwo_fe_stereo_group_last_error(const FeStereoGroupHandle *g);   /* g may be NULL: last create() error */
+int plviwo_fe_stereo_group_set_calib(FeStereoGroupHandle *g, int rig, int cam, const double K[4], const double D[4]);
+int plviwo_fe_stereo_group_set_camera(FeStereoGroupHandle *g, int rig, int cam, int model, const double K[4], const double D[4]);
+int plviwo_fe_stereo_group_submit(FeStereoGroupHandle *g, const double *timestamps, const uint8_t *const *images_left,
+                                  const uint8_t *const *images_right, int stride, int on_device, const uint8_t *const *masks_left,
+                                  const uint8_t *const *masks_right, int mask_stride, const double *vps);
+int plviwo_fe_stereo_group_collect(FeStereoGroupHandle *g, FeStereoInfo *infos /* n_rigs or NULL */);
+int plviwo_fe_stereo_group_play(FeStereoGroupHandle *g, int n_ticks, const uint8_t *const *images, int stride, int on_device,
+                                const double *timestamps, const double *vps, FePlayStats *out /* n_rigs */);
+int plviwo_fe_stereo_group_get_point_rows(FeStereoGroupHandle *g, int rig, int cam, FePointRow *out, int cap, int *n_out);
+int plviwo_fe_stereo_group_get_last_obs(FeStereoGroupHandle *g, int rig, int cam, uint64_t *ids, float *uv, int cap, int *n_out);
+int plviwo_fe_stereo_group_get_line_rows(FeStereoGroupHandle *g, int rig, FeLineRow *out, int cap, int *n_out);
+int plviwo_fe_stereo_group_get_line_points(FeStereoGroupHandle *g, int rig, FeLinePoint *out, int cap, int *n_out);
+int plviwo_fe_stereo_group_get_state(FeStereoGroupHandle *g, int rig, void *buf, size_t cap, size_t *n_bytes);
+int plviwo_fe_stereo_group_set_state(FeStereoGroupHandle *g, int rig, const void *buf, size_t n_bytes);
+
 /* ---- stand-alone kernels (tests / micro-benchmarks; all pointers are HOST buffers) --------------------- */
 int plviwo_op_equalize_pyramid(int device, const uint8_t *img, int w, int h, int levels /* maxLevel */,
                                uint8_t *out_levels /* concatenated tight levels 0..maxLevel */, uint8_t *out_half);

@@ -125,6 +125,8 @@ EXPORTS = [
     "plviwo_fe_group_get_state", "plviwo_fe_group_set_state", "plviwo_fe_group_tap", "plviwo_fe_group_enable_timing",
     "plviwo_fe_group_get_times", "plviwo_fe_set_camera", "plviwo_fe_get_currid", "plviwo_fe_set_currid",
     "plviwo_fe_stereo_set_camera",
+    "plviwo_fe_stereo_group_create", "plviwo_fe_stereo_group_destroy", "plviwo_fe_stereo_group_last_error", "plviwo_fe_stereo_group_set_calib", "plviwo_fe_stereo_group_set_camera", "plviwo_fe_stereo_group_submit",
+    "plviwo_fe_stereo_group_collect", "plviwo_fe_stereo_group_play", "plviwo_fe_stereo_group_get_point_rows", "plviwo_fe_stereo_group_get_last_obs", "plviwo_fe_stereo_group_get_line_rows", "plviwo_fe_stereo_group_get_line_points", "plviwo_fe_stereo_group_get_state", "plviwo_fe_stereo_group_set_state",
 ]
 
 
@@ -226,6 +228,26 @@ def lib() -> C.CDLL:
         L.plviwo_fe_group_tap.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
         L.plviwo_fe_group_enable_timing.argtypes = [C.c_void_p, C.c_int]
         L.plviwo_fe_group_get_times.argtypes = [C.c_void_p, C.POINTER(FeGroupTimes), C.c_int]
+        L.plviwo_fe_stereo_group_last_error.restype = C.c_char_p
+        L.plviwo_fe_stereo_group_last_error.argtypes = [C.c_void_p]
+        L.plviwo_fe_stereo_group_create.argtypes = [C.POINTER(FeConfig), C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        L.plviwo_fe_stereo_group_destroy.argtypes = [C.c_void_p]
+        L.plviwo_fe_stereo_group_set_calib.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]
+        L.plviwo_fe_stereo_group_set_camera.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double),
+                                                        C.POINTER(C.c_double)]
+        L.plviwo_fe_stereo_group_submit.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
+                                                    C.c_int, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int,
+                                                    C.POINTER(C.c_double)]
+        L.plviwo_fe_stereo_group_collect.argtypes = [C.c_void_p, C.POINTER(FeStereoInfo)]
+        L.plviwo_fe_stereo_group_play.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_int, C.c_int,
+                                                  C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(FePlayStats)]
+        L.plviwo_fe_stereo_group_get_point_rows.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
+        L.plviwo_fe_stereo_group_get_last_obs.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
+                                                          C.POINTER(C.c_int)]
+        for name in ("plviwo_fe_stereo_group_get_line_rows", "plviwo_fe_stereo_group_get_line_points"):
+            getattr(L, name).argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
+        L.plviwo_fe_stereo_group_get_state.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
+        L.plviwo_fe_stereo_group_set_state.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]
         _lib = L
     return _lib
 
@@ -708,6 +730,136 @@ class GroupFrontEnd:
                 "frames_of": {k: int(t.frames[i]) for i, k in enumerate(GROUP_KERNELS)}, "ticks": int(t.ticks),
                 "frames": int(t.frames_total), "kernel_launches_total": int(t.kernel_launches_total),
                 "h2d_bytes": int(t.h2d_bytes), "d2h_bytes": int(t.d2h_bytes), "fast_cells": int(t.fast_cells)}
+
+
+class StereoGroupFrontEnd:
+    """Many stereo rigs of one device behind one FeStereoGroupHandle: rig r is what one StereoFrontEnd is (same rows, bit for
+    bit); a tick feeds one stereo pair of every rig.  Cameras: 0 left, 1 right."""
+
+    def __init__(self, cfg: FeConfig, n_rigs: int, device: int = 0, calibs=None):
+        """calibs: per rig ((K_left, D_left), (K_right, D_right)), or None (cfg.K / cfg.D for every camera)."""
+        self.cfg = cfg
+        self.n = int(n_rigs)
+        self._h = C.c_void_p()
+        self._lib = lib()
+        rc = self._lib.plviwo_fe_stereo_group_create(C.byref(cfg), self.n, device, C.byref(self._h))
+        if rc != FE_OK:
+            raise FrontEndError(rc, (self._lib.plviwo_fe_stereo_group_last_error(None) or b"").decode())
+        self.infos = (FeStereoInfo * self.n)()
+        if calibs is not None:
+            for r, cams in enumerate(calibs):
+                for cam, (K, D) in enumerate(cams):
+                    self.set_calib(r, cam, K, D)
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            self._lib.plviwo_fe_stereo_group_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _check(self, rc):
+        if rc != FE_OK:
+            raise FrontEndError(rc, (self._lib.plviwo_fe_stereo_group_last_error(self._h) or b"").decode())
+
+    def set_calib(self, rig: int, cam: int, K, D):
+        self._check(self._lib.plviwo_fe_stereo_group_set_calib(self._h, rig, cam, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
+
+    def set_camera(self, rig: int, cam: int, model: int, K, D):
+        """Calibration with the camera model stated (0 radtan, 1 equidistant: refused, cam/CamEqui.h is not implemented)."""
+        self._check(self._lib.plviwo_fe_stereo_group_set_camera(self._h, rig, cam, model, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
+
+    def _ptrs(self, arrays, keep, on_device=False):
+        out = (C.c_void_p * self.n)()
+        stride = 0
+        for r, im in enumerate(arrays):
+            if im is None:
+                out[r] = None
+            elif on_device:
+                out[r] = int(im)
+            else:
+                a = im if (im.dtype == np.uint8 and im.strides[1] == 1) else np.ascontiguousarray(im, np.uint8)
+                keep.append(a)
+                out[r] = a.ctypes.data
+                stride = a.strides[0]
+        return out, stride
+
+    def submit(self, timestamps, pairs, stride: int = 0, on_device: bool = False, vanishing_points=None, masks=None):
+        """pairs: per rig (left, right) 2-D uint8 arrays / device pointers (on_device), or None (no pair for that rig in this
+        tick); vanishing_points: per rig 3 x (x, y), or None (line tracker not fed); masks: per rig (left, right) or None."""
+        keep = []
+        pl, s0 = self._ptrs([None if p is None else p[0] for p in pairs], keep, on_device)
+        pr, s1 = self._ptrs([None if p is None else p[1] for p in pairs], keep, on_device)
+        stride = stride or s0 or s1
+        ts = (C.c_double * self.n)(*[float(t) for t in (timestamps if hasattr(timestamps, "__len__") else [timestamps] * self.n)])
+        vp = None
+        if vanishing_points is not None:
+            vp = (C.c_double * (6 * self.n))(*[float(v) for f in vanishing_points for p in f for v in p])
+        ml = mr = None
+        mstride = 0
+        if masks is not None:
+            ml, mstride = self._ptrs([None if m is None else m[0] for m in masks], keep)
+            mr, _ = self._ptrs([None if m is None else m[1] for m in masks], keep)
+        self._check(self._lib.plviwo_fe_stereo_group_submit(self._h, ts, pl, pr, stride, 1 if on_device else 0, ml, mr, mstride, vp))
+
+    def collect(self):
+        self._check(self._lib.plviwo_fe_stereo_group_collect(self._h, self.infos))
+        return self.infos
+
+    def feed(self, timestamps, pairs, vanishing_points=None, masks=None):
+        self.submit(timestamps, pairs, vanishing_points=vanishing_points, masks=masks)
+        return self.collect()
+
+    def play(self, timestamps, ptr_table, stride: int, on_device: bool, vanishing_points=None):
+        """ptr_table: ctypes array of n_ticks * n_rigs * 2 pointers, [(t * n_rigs + r) * 2 + cam]; vanishing_points: per rig."""
+        n_ticks = len(timestamps)
+        ts = (C.c_double * n_ticks)(*[float(t) for t in timestamps])
+        vp = None
+        if vanishing_points is not None:
+            vp = (C.c_double * (6 * self.n))(*[float(v) for f in vanishing_points for p in f for v in p])
+        st = (FePlayStats * self.n)()
+        self._check(self._lib.plviwo_fe_stereo_group_play(self._h, n_ticks, ptr_table, stride, 1 if on_device else 0, ts, vp, st))
+        return st
+
+    def _rows(self, fn, args, dtype):
+        n = C.c_int(0)
+        self._check(fn(self._h, *args, None, 0, C.byref(n)))
+        out = np.zeros((n.value,), dtype)
+        if n.value:
+            self._check(fn(self._h, *args, out.ctypes.data, n.value, C.byref(n)))
+        return out
+
+    def point_rows(self, rig: int, cam: int) -> np.ndarray:
+        return self._rows(self._lib.plviwo_fe_stereo_group_get_point_rows, (rig, cam), POINT_ROW_DTYPE)
+
+    def line_rows(self, rig: int):
+        """Line rows and line points of the rig's left image."""
+        return (self._rows(self._lib.plviwo_fe_stereo_group_get_line_rows, (rig,), LINE_ROW_DTYPE),
+                self._rows(self._lib.plviwo_fe_stereo_group_get_line_points, (rig,), LINE_POINT_DTYPE))
+
+    def last_obs(self, rig: int, cam: int):
+        n = C.c_int(0)
+        self._check(self._lib.plviwo_fe_stereo_group_get_last_obs(self._h, rig, cam, None, None, 0, C.byref(n)))
+        ids = np.zeros((n.value,), np.uint64)
+        uv = np.zeros((n.value, 2), np.float32)
+        if n.value:
+            self._check(self._lib.plviwo_fe_stereo_group_get_last_obs(self._h, rig, cam, ids.ctypes.data, uv.ctypes.data, n.value,
+                                                                      C.byref(n)))
+        return ids, uv
+
+    def get_state(self, rig: int) -> bytes:
+        n = C.c_size_t(0)
+        self._check(self._lib.plviwo_fe_stereo_group_get_state(self._h, rig, None, 0, C.byref(n)))
+        buf = C.create_string_buffer(n.value)
+        self._check(self._lib.plviwo_fe_stereo_group_get_state(self._h, rig, buf, n.value, C.byref(n)))
+        return buf.raw[:n.value]
+
+    def set_state(self, rig: int, blob: bytes):
+        self._check(self._lib.plviwo_fe_stereo_group_set_state(self._h, rig, blob, len(blob)))
 
 
 class GroupEngine:

@@ -24,6 +24,10 @@ struct FeGroupHandle {
   FeGroup *grp;
 };
 
+struct FeStereoGroupHandle {
+  FeGroup *grp;
+};
+
 static thread_local std::string g_create_error;
 
 // See bench.py / INTEGRATION.md: one hardware queue per stream.  Only effective if no CUDA context exists yet.
@@ -923,6 +927,131 @@ int plviwo_fe_group_get_times(FeGroupHandle *g, FeGroupTimes *out, int reset) {
   if (!g || !out) return FE_BAD_ARG;
   *out = g->grp->times(reset != 0);
   return FE_OK;
+}
+
+// ---- stereo group (many stereo rigs of one device, csrc/fe_group.h) ---------------------------------------------
+int plviwo_fe_stereo_group_create(const FeConfig *cfg, int n_rigs, int device, FeStereoGroupHandle **out) {
+  API_BEGIN
+  if (!cfg || !out) return FE_BAD_ARG;
+  *out = nullptr;
+  if (n_rigs < 1 || n_rigs > 2048) return create_error(FE_BAD_ARG, "n_rigs must be in [1, 2048] (2 camera streams per rig, at most 4096)");
+  if (const char *why = check_config(*cfg, cfg->width, cfg->height)) return create_error(FE_BAD_ARG, why);
+  if (cfg->grid_x * cfg->grid_y > 256) return create_error(FE_BAD_ARG, "a stream group supports at most 256 grid cells");
+  // the stereo handle ignores both; a stereo group refuses them rather than run something else than asked
+  if (cfg->downsample) return create_error(FE_BAD_ARG, "cfg.downsample is not supported in a stereo group");
+  if (cfg->line_samples) return create_error(FE_BAD_ARG, "cfg.line_samples is not supported in a stereo group");
+  if (int rc = check_device(device)) return rc;
+  FeGroup *grp = new FeGroup(*cfg, 2 * n_rigs, device, true);
+  int rc = grp->init();
+  if (rc != FE_OK) {
+    g_create_error = grp->last_error;
+    delete grp;
+    return rc;
+  }
+  *out = new FeStereoGroupHandle{grp};
+  return FE_OK;
+  API_END
+}
+
+int plviwo_fe_stereo_group_destroy(FeStereoGroupHandle *g) {
+  API_BEGIN
+  if (!g) return FE_BAD_ARG;
+  delete g->grp;
+  delete g;
+  return FE_OK;
+  API_END
+}
+
+const char *plviwo_fe_stereo_group_last_error(const FeStereoGroupHandle *g) { return g ? g->grp->last_error.c_str() : g_create_error.c_str(); }
+
+// stream of (rig, cam), or -1 with the reason in last_error
+static int rig_stream(FeStereoGroupHandle *g, int rig, int cam) {
+  if (rig < 0 || rig >= g->grp->n_streams() / 2 || cam < 0 || cam > 1) {
+    g->grp->last_error = "rig or cam out of range (cam: 0 left, 1 right)";
+    return -1;
+  }
+  return 2 * rig + cam;
+}
+
+int plviwo_fe_stereo_group_set_calib(FeStereoGroupHandle *g, int rig, int cam, const double K[4], const double D[4]) {
+  if (!g) return FE_BAD_ARG;
+  const int s = rig_stream(g, rig, cam);
+  if (s < 0) return FE_BAD_ARG;
+  return g->grp->set_calib(s, K, D);
+}
+
+int plviwo_fe_stereo_group_set_camera(FeStereoGroupHandle *g, int rig, int cam, int model, const double K[4], const double D[4]) {
+  if (!g) return FE_BAD_ARG;
+  if (model != FE_CAM_RADTAN) {   // as plviwo_fe_set_camera
+    g->grp->last_error = "set_camera: only the radtan model is implemented (cam/CamEqui.h:108-129 is not)";
+    return FE_BAD_ARG;
+  }
+  return plviwo_fe_stereo_group_set_calib(g, rig, cam, K, D);
+}
+
+int plviwo_fe_stereo_group_submit(FeStereoGroupHandle *g, const double *timestamps, const uint8_t *const *images_left,
+                                  const uint8_t *const *images_right, int stride, int on_device, const uint8_t *const *masks_left,
+                                  const uint8_t *const *masks_right, int mask_stride, const double *vps) {
+  API_BEGIN
+  if (!g) return FE_BAD_ARG;
+  return g->grp->stereo_submit(timestamps, images_left, images_right, stride, on_device != 0, masks_left, masks_right, mask_stride, vps);
+  API_END
+}
+
+int plviwo_fe_stereo_group_collect(FeStereoGroupHandle *g, FeStereoInfo *infos) {
+  API_BEGIN
+  if (!g) return FE_BAD_ARG;
+  return g->grp->stereo_collect(infos);
+  API_END
+}
+
+int plviwo_fe_stereo_group_play(FeStereoGroupHandle *g, int n_ticks, const uint8_t *const *images, int stride, int on_device,
+                                const double *timestamps, const double *vps, FePlayStats *out) {
+  API_BEGIN
+  if (!g || n_ticks < 0 || !images || !timestamps) return FE_BAD_ARG;
+  return g->grp->play(n_ticks, images, stride, on_device != 0, timestamps, vps, out);
+  API_END
+}
+
+int plviwo_fe_stereo_group_get_point_rows(FeStereoGroupHandle *g, int rig, int cam, FePointRow *out, int cap, int *n_out) {
+  if (!g) return FE_BAD_ARG;
+  const int s = rig_stream(g, rig, cam);
+  const GroupOutHeader *h = s < 0 ? nullptr : g->grp->header(s);
+  if (!h) return FE_BAD_ARG;
+  return copy_rows(g->grp->point_rows(s), h->info.n_point_rows, sizeof(FePointRow), out, cap, n_out);
+}
+int plviwo_fe_stereo_group_get_last_obs(FeStereoGroupHandle *g, int rig, int cam, uint64_t *ids, float *uv, int cap, int *n_out) {
+  if (!g) return FE_BAD_ARG;
+  const int s = rig_stream(g, rig, cam);
+  if (s < 0) return FE_BAD_ARG;
+  FeGroupHandle view{g->grp};   // the group's getter on the rig's stream
+  return plviwo_fe_group_get_last_obs(&view, s, ids, uv, cap, n_out);
+}
+int plviwo_fe_stereo_group_get_line_rows(FeStereoGroupHandle *g, int rig, FeLineRow *out, int cap, int *n_out) {
+  if (!g) return FE_BAD_ARG;
+  const int s = rig_stream(g, rig, 0);
+  if (s < 0) return FE_BAD_ARG;
+  FeGroupHandle view{g->grp};   // the group's getter on the rig's stream
+  return plviwo_fe_group_get_line_rows(&view, s, out, cap, n_out);
+}
+int plviwo_fe_stereo_group_get_line_points(FeStereoGroupHandle *g, int rig, FeLinePoint *out, int cap, int *n_out) {
+  if (!g) return FE_BAD_ARG;
+  const int s = rig_stream(g, rig, 0);
+  if (s < 0) return FE_BAD_ARG;
+  FeGroupHandle view{g->grp};   // the group's getter on the rig's stream
+  return plviwo_fe_group_get_line_points(&view, s, out, cap, n_out);
+}
+int plviwo_fe_stereo_group_get_state(FeStereoGroupHandle *g, int rig, void *buf, size_t cap, size_t *n_bytes) {
+  API_BEGIN
+  if (!g) return FE_BAD_ARG;
+  return g->grp->stereo_get_state(rig, buf, cap, n_bytes);
+  API_END
+}
+int plviwo_fe_stereo_group_set_state(FeStereoGroupHandle *g, int rig, const void *buf, size_t n_bytes) {
+  API_BEGIN
+  if (!g) return FE_BAD_ARG;
+  return g->grp->stereo_set_state(rig, buf, n_bytes);
+  API_END
 }
 
 // ---- stereo rig (TrackKLT with use_stereo = true) -----------------------------------------------------------

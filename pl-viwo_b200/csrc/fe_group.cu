@@ -24,7 +24,8 @@ namespace plviwo {
 static inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
 static inline size_t align_up_sz(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-FeGroup::FeGroup(const FeConfig &cfg, int n_streams, int device) : cfg_(cfg), S_(n_streams), device_(device), W_(cfg.width), H_(cfg.height) {}
+FeGroup::FeGroup(const FeConfig &cfg, int n_streams, int device, bool stereo)
+    : cfg_(cfg), S_(n_streams), device_(device), W_(cfg.width), H_(cfg.height), stereo_(stereo) {}
 
 int FeGroup::fail(cudaError_t e, const char *what) {
   last_error = std::string(what) + ": " + cudaGetErrorString(e);
@@ -68,7 +69,7 @@ int FeGroup::init() {
     // chain; the chain is latency bound (~0.4 ms per tick whatever the number of streams), so lanes overlap
     e = std::getenv("PLVIWO_GROUP_LANES");
     lanes_ = e ? std::atoi(e) : 4;
-    lanes_ = std::max(1, std::min(lanes_, S_));
+    lanes_ = std::max(1, std::min(lanes_, stereo_ ? S_ / 2 : S_));   // a rig's two streams share a lane
   }
   K_.resize(4 * (size_t)S_);
   D_.resize(4 * (size_t)S_);
@@ -98,6 +99,9 @@ int FeGroup::init() {
   const int ncell = g_.n_cells, nfg = g_.nfg;
   g_.cand_cap = std::max(ncell * nfg, 1);
   g_.pts_cap = align_up(cfg_.num_features + ncell * nfg + 32, 32);
+  // a stereo rig's right list is not bounded by its own top-off (it also receives the new stereo points of the left): hold
+  // as many points per camera as the stereo handle's tracking buffers (fe_context.cu, max_pts without line samples)
+  if (stereo_) g_.pts_cap = align_up(std::max(g_.pts_cap, std::max(4096, 8 * cfg_.num_features)), 32);
   g_.lines_cap = 1024;
   g_.pol_cap = 8192;
   g_.segs_cap = 4096;
@@ -222,9 +226,14 @@ int FeGroup::init() {
     g_.off_sp1 = g_.off_sp0 + (size_t)g_.sample_cap * sizeof(float2);
     g_.off_sst = g_.off_sp1 + (size_t)g_.sample_cap * sizeof(float2);
     g_.out_stride = align_up_sz(g_.off_sst + (size_t)g_.sample_cap, 256);
+  } else if (stereo_) {
+    g_.off_sinfo = align_up_sz(end_lpts, 64);
+    g_.out_stride = align_up_sz(g_.off_sinfo + sizeof(FeStereoInfo), 256);
   } else {
     g_.out_stride = align_up_sz(end_lpts, 256);
   }
+  if (stereo_ && stereo_rows_smem(g_.pts_cap) > 227 * 1024)
+    return err(FE_BAD_ARG, "stereo group: the id table of num_features + the grid's candidates exceeds shared memory");
   FG_CUDA(cudaHostAlloc((void **)&h_out_, g_.out_stride * (size_t)RB_ * S_, cudaHostAllocMapped));
   host_allocs_.push_back(h_out_);
   std::memset(h_out_, 0, g_.out_stride * (size_t)RB_ * S_);
@@ -459,7 +468,7 @@ int FeGroup::submit(const double *timestamps, const uint8_t *const *images, int 
       fj.flags |= 1;
     }
     b.jobs.push_back(fj);
-    const bool lines = cfg_.use_lines && vps != nullptr;
+    const bool lines = cfg_.use_lines && vps != nullptr && !(stereo_ && (s & 1));   // stereo: the left image only
     if (lines) b.line_slots.push_back(slot);
     TrackJob &j = tj[nj++];
     std::memset(&j, 0, sizeof(j));
@@ -475,7 +484,7 @@ int FeGroup::submit(const double *timestamps, const uint8_t *const *images, int 
       j.K[i] = K_[4 * s + i];
       j.D[i] = D_[4 * s + i];
     }
-    if (vps) std::memcpy(j.vp, vps + 6 * (size_t)s, 6 * sizeof(double));
+    if (vps) std::memcpy(j.vp, vps + 6 * (size_t)(stereo_ ? s / 2 : s), 6 * sizeof(double));
     tr.cur_slot[s] = slot;
     prev_slot_[s] = slot;
     frame_count_[s]++;
@@ -519,6 +528,11 @@ int FeGroup::launch_front(FrontBatch &b, int buf) {
   cudaStream_t st = timing_ ? s_front_[0] : s_front_[buf % s_front_.size()];
   FrontJob *hj = h_fjobs_ + (size_t)buf * B_ * S_, *dj = d_fjobs_ + (size_t)buf * B_ * S_;
   int *hl = h_ljobs_ + (size_t)buf * B_ * S_, *dl = d_ljobs_ + (size_t)buf * B_ * S_;
+  int n_half = cfg_.use_lines ? nj : 0;   // jobs [0, n_half) get the half-resolution image of the line front work
+  if (stereo_ && cfg_.use_lines) {        // ... in a stereo group the left images only (TrackLSD.cpp:57-60): left jobs first
+    auto right_image = [this](const FrontJob &j) { return (j.slot / R_) & 1; };
+    n_half = (int)(std::stable_partition(b.jobs.begin(), b.jobs.end(), [&](const FrontJob &j) { return !right_image(j); }) - b.jobs.begin());
+  }
   std::memcpy(hj, b.jobs.data(), nj * sizeof(FrontJob));
   if (nl) std::memcpy(hl, b.line_slots.data(), nl * sizeof(int));
   // the frames (and masks) of the batch are on their way on the copy stream
@@ -567,8 +581,14 @@ int FeGroup::launch_front(FrontBatch &b, int buf) {
     launches_++;
     if (tm) e0 = mark();
   }
-  launch_eq_pyr1_batch(d_slots_, dj, nj, fg_, cfg_.use_lines != 0, st);
-  launches_++;
+  if (n_half > 0) {
+    launch_eq_pyr1_batch(d_slots_, dj, n_half, fg_, true, st);
+    launches_++;
+  }
+  if (n_half < nj) {
+    launch_eq_pyr1_batch(d_slots_, dj + n_half, nj - n_half, fg_, false, st);
+    launches_++;
+  }
   step(FE_GK_EQ_PYR1, nj);
   const SlotRec &s0 = slots_[0];
   for (int l = 2; l < s0.n_lvl; l++) {
@@ -612,6 +632,7 @@ int FeGroup::launch_front(FrontBatch &b, int buf) {
 }
 
 int FeGroup::launch_track(int tick) {
+  if (stereo_) return launch_track_stereo(tick);
   const int ring = tick % RB_;
   TickRec &tr = ticks_[ring];
   tr.track_launched = true;
@@ -726,8 +747,8 @@ int FeGroup::collect(FeFrameInfo *infos) {
     if (h->status != FE_OK && status == FE_OK) {
       status = h->status;
       static const char *what[] = {"?", "points", "lines", "point / line pairs", "candidates"};
-      last_error = std::string("stream ") + std::to_string(s) + ": more " + what[std::min(std::max(h->overflow_what, 0), 4)] +
-                   " than the group's buffers hold";
+      last_error = (stereo_ ? "rig " + std::to_string(s / 2) + (s & 1 ? " right" : " left") : "stream " + std::to_string(s)) + ": more " +
+                   what[std::min(std::max(h->overflow_what, 0), 4)] + " than the group's buffers hold";
     }
   }
   if (timing_ && submitted_ == collected_) {   // everything launched has finished: read the stage events
@@ -787,7 +808,11 @@ int FeGroup::line_samples(int s, float *uv01, uint8_t *status, int cap, int *n_o
 int FeGroup::play(int n_ticks, const uint8_t *const *images, int stride, bool on_device, const double *timestamps, const double *vps,
                   FePlayStats *out) {
   if (submitted_ != collected_) return err(FE_BAD_ARG, "play: ticks submitted with submit are still pending");
-  std::vector<FePlayStats> st(S_);
+  if (stereo_)
+    for (size_t k = 0; k < (size_t)n_ticks * S_; k += 2)
+      if (!images[k] != !images[k + 1]) return err(FE_BAD_ARG, "play: a rig's pair has exactly one image");
+  const int per = stereo_ ? 2 : 1, U = S_ / per;   // a stereo rig's statistics cover both cameras' point rows
+  std::vector<FePlayStats> st(U);
   for (auto &x : st) std::memset(&x, 0, sizeof(x));
   std::vector<double> ts(S_);
   int sub = 0;
@@ -803,18 +828,20 @@ int FeGroup::play(int n_ticks, const uint8_t *const *images, int stride, bool on
     for (int s = 0; s < S_; s++) {
       const GroupOutHeader *h = header(s);
       if (!images[(size_t)i * S_ + s]) continue;
-      FePlayStats &x = st[s];
-      x.frames++;
+      FePlayStats &x = st[s / per];
+      if (s % per == 0) {
+        x.frames++;
+        x.resets += (stereo_ ? stereo_info(s / 2).reset : h->info.reset) ? 1 : 0;
+      }
       x.point_rows += (uint64_t)h->info.n_point_rows;
       x.line_rows += (uint64_t)h->info.n_line_rows;
-      x.resets += h->info.reset ? 1 : 0;
       const FePointRow *pr = point_rows(s);
       for (int k = 0; k < h->info.n_point_rows; k++) x.checksum += (double)pr[k].id + pr[k].u + pr[k].v;
       const FeLineRow *lr = line_rows(s);
       for (int k = 0; k < h->info.n_line_rows; k++) x.checksum += (double)lr[k].id + lr[k].line[0] + lr[k].line[1] + lr[k].line[2] + lr[k].line[3];
     }
   }
-  if (out) std::memcpy(out, st.data(), S_ * sizeof(FePlayStats));
+  if (out) std::memcpy(out, st.data(), U * sizeof(FePlayStats));
   return FE_OK;
 }
 
@@ -876,16 +903,21 @@ int FeGroup::get_state(int s, void *buf, size_t cap, size_t *n_bytes) {
   return FE_OK;
 }
 
+const char *FeGroup::check_state(const void *buf, size_t n_bytes, StateView &v) const {
+  if (const char *why = state_read(buf, n_bytes, W_, H_, v)) return why;
+  if (v.hd.n_pts > g_.pts_cap || v.hd.n_lines > g_.lines_cap || v.hd.n_pol_entries > g_.pol_cap)
+    return "set_state: more points / lines than the group's buffers hold";
+  return nullptr;
+}
+
 int FeGroup::set_state(int s, const void *buf, size_t n_bytes) {
   FG_CUDA(cudaSetDevice(device_));
   if (s < 0 || s >= S_) return err(FE_BAD_ARG, "set_state: bad stream");
   if (submitted_ != collected_) return err(FE_BAD_ARG, "set_state: collect the pending ticks first");
   // ---- parse and validate everything before any of it is applied
   StateView v;
-  if (const char *why = state_read(buf, n_bytes, W_, H_, v)) return err(FE_BAD_ARG, why);
+  if (const char *why = check_state(buf, n_bytes, v)) return err(FE_BAD_ARG, why);
   const StateHeader &hd = v.hd;
-  if (hd.n_pts > g_.pts_cap || hd.n_lines > g_.lines_cap || hd.n_pol_entries > g_.pol_cap)
-    return err(FE_BAD_ARG, "set_state: more points / lines than the group's buffers hold");
   std::vector<int> poff(hd.n_lines + 1, 0), ppid;
   std::vector<float> pdist;
   for (int i = 0; i < hd.n_lines; i++) {
@@ -936,7 +968,7 @@ int FeGroup::set_state(int s, const void *buf, size_t n_bytes) {
     cudaStream_t st = s_front_[0];
     FG_CUDA(cudaMemcpy(d_fjobs_, &fj, sizeof(fj), cudaMemcpyHostToDevice));
     launch_hist_batch(d_slots_, d_fjobs_, 1, fg_, d_slot_flags_, st);
-    launch_eq_pyr1_batch(d_slots_, d_fjobs_, 1, fg_, cfg_.use_lines != 0, st);
+    launch_eq_pyr1_batch(d_slots_, d_fjobs_, 1, fg_, cfg_.use_lines != 0 && !(stereo_ && (s & 1)), st);
     for (int l = 2; l < sl.n_lvl; l++) launch_pyr_level_batch(d_slots_, d_fjobs_, 1, l, sl.lvl[l].w, sl.lvl[l].h, st);
     FG_CUDA(cudaGetLastError());
     FG_CUDA(cudaStreamSynchronize(st));
@@ -958,6 +990,170 @@ int FeGroup::tap(int s, int what, void *buf, size_t cap, size_t *n_bytes) {
   if (!im) return err(FE_BAD_ARG, "tap: not available");
   const int rc = tap_image(*im, buf, cap, n_bytes);
   return rc == FE_CUDA_ERROR ? fail(cudaGetLastError(), "tap: cudaMemcpy2D") : rc;
+}
+
+// ------------------------------------------------------------------------------------------------ stereo rigs
+// The tracking phase of a tick for the rigs of each lane (fe_group_dev.h has the sequence and the job layout).
+int FeGroup::launch_track_stereo(int tick) {
+  const int ring = tick % RB_;
+  TickRec &tr = ticks_[ring];
+  tr.track_launched = true;
+  TrackJob *hj = h_tjobs_ + (size_t)ring * S_, *dj = d_tjobs_ + (size_t)ring * S_;
+  int nj = 0;
+  for (int s = 0; s < S_; s++) nj += tr.cur_slot[s] >= 0 ? 1 : 0;
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, nullptr, nullptr, true);
+  const int n_rigs = S_ / 2;
+  std::vector<TrackJob> pairs;
+  int jpos = 0;
+  for (int l = 0; l < lanes_; l++) {
+    const int s_end = 2 * (int)((long long)n_rigs * (l + 1) / lanes_);
+    const int j0 = jpos;
+    while (jpos < nj && hj[jpos].stream < s_end) jpos++;
+    const int n = (jpos - j0) / 2;   // rigs with a pair in this tick: their left and right jobs are adjacent (stream order)
+    cudaStream_t st = s_track_[l];
+    if (n == 0) {
+      FG_CUDA(cudaEventRecord(ev_done_[(size_t)ring * lanes_ + l], st));
+      continue;
+    }
+    pairs.assign(hj + j0, hj + j0 + 2 * n);
+    for (int k = 0; k < n; k++) {
+      hj[j0 + k] = pairs[2 * k];
+      hj[j0 + n + k] = pairs[2 * k + 1];
+    }
+    FG_CUDA(cudaStreamWaitEvent(st, ev_pyr_[tr.batch], 0));
+    FG_CUDA(cudaMemcpyAsync(dj + j0, hj + j0, (size_t)2 * n * sizeof(TrackJob), cudaMemcpyHostToDevice, st));
+    const TrackJob *jl = dj + j0, *jr = dj + j0 + n;
+    auto detect_tail = [&](const TrackJob *jobs, bool right) {   // FAST .. accept of one camera of the lane's rigs
+      if (fg_.n_cells > 0) {
+        launch_group_fast(g_, jobs, n, fg_, st);
+        launch_group_fast_select(g_, jobs, n, fg_, st);
+        launches_ += 2;
+      }
+      if (right) launch_stereo_cands_right(g_, jobs, n, st);
+      else launch_group_cands(g_, jobs, n, st);
+      launch_group_subpix(g_, jobs, n, st);
+      launch_group_accept(g_, jobs, n, st);
+      launches_ += 3;
+    };
+    launch_stereo_detect(g_, jl, n, false, st);
+    detect_tail(jl, false);
+    launch_stereo_lr_lk(g_, jl, n, prm, st);
+    launch_stereo_pair(g_, jl, n, st);
+    launch_stereo_detect(g_, jr, n, true, st);
+    detect_tail(jr, true);
+    launch_group_lk(g_, jl, 2 * n, prm, st);
+    launch_stereo_gate(g_, jl, 2 * n, st);
+    launch_stereo_rows(g_, jl, n, st);
+    launches_ += 7;
+    cudaStream_t sl = st;
+    if (cfg_.use_lines) {   // the left image's line tracker, against the left points the rig has just produced
+      sl = s_lines_[l];
+      FG_CUDA(cudaEventRecord(ev_gate_[(size_t)ring * lanes_ + l], st));
+      FG_CUDA(cudaStreamWaitEvent(sl, ev_gate_[(size_t)ring * lanes_ + l], 0));
+      FG_CUDA(cudaStreamWaitEvent(sl, ev_front_[tr.batch], 0));
+      launch_group_lines(g_, jl, n, sl);
+      launches_++;
+    }
+    FG_CUDA(cudaGetLastError());
+    FG_CUDA(cudaEventRecord(ev_done_[(size_t)ring * lanes_ + l], sl));
+  }
+  return FE_OK;
+}
+
+int FeGroup::stereo_submit(const double *timestamps, const uint8_t *const *left, const uint8_t *const *right, int stride, bool on_device,
+                           const uint8_t *const *masks_left, const uint8_t *const *masks_right, int mask_stride, const double *vps) {
+  if (!stereo_ || !timestamps || !left || !right) return err(FE_BAD_ARG, "submit: bad arguments");
+  if (!masks_left != !masks_right) return err(FE_BAD_ARG, "submit: masks are given for both cameras or for neither");
+  const int n_rigs = S_ / 2;
+  std::vector<const uint8_t *> img(S_), msk(masks_left ? S_ : 0);
+  std::vector<double> ts(S_);
+  for (int r = 0; r < n_rigs; r++) {
+    if (!left[r] != !right[r]) return err(FE_BAD_ARG, "submit: rig " + std::to_string(r) + " has exactly one image of its pair");
+    img[2 * r] = left[r];
+    img[2 * r + 1] = right[r];
+    ts[2 * r] = ts[2 * r + 1] = timestamps[r];
+    if (masks_left) {
+      if (!masks_left[r] != !masks_right[r]) return err(FE_BAD_ARG, "submit: rig " + std::to_string(r) + " has exactly one mask");
+      if (masks_left[r] && left[r] && mask_stride < W_) return err(FE_BAD_ARG, "submit: bad mask stride");
+      msk[2 * r] = masks_left[r];
+      msk[2 * r + 1] = masks_right[r];
+    }
+  }
+  return submit(ts.data(), img.data(), stride, on_device, masks_left ? msk.data() : nullptr, mask_stride, vps);
+}
+
+FeStereoInfo FeGroup::stereo_info(int rig) const {
+  FeStereoInfo si;
+  std::memset(&si, 0, sizeof(si));
+  si.timestamp = -1.0;
+  const GroupOutHeader *h = header(2 * rig);
+  if (!stereo_ || !h || ticks_[(int)(last_collected_ % RB_)].cur_slot[2 * rig] < 0) return si;   // no pair in the tick
+  std::memcpy(&si, reinterpret_cast<const uint8_t *>(h) + g_.off_sinfo, sizeof(si));
+  si.n_line_rows = h->info.n_line_rows;   // k_group_lines writes the left record's header
+  si.n_lines_detected = h->info.n_lines_detected;
+  si.n_line_matches = h->info.n_line_matches;
+  return si;
+}
+
+int FeGroup::stereo_collect(FeStereoInfo *infos) {
+  if (!stereo_) return err(FE_BAD_ARG, "collect: not a stereo group");
+  const int rc = collect(nullptr);
+  if (infos && last_collected_ >= 0)
+    for (int r = 0; r < S_ / 2; r++) infos[r] = stereo_info(r);
+  return rc;
+}
+
+int FeGroup::stereo_get_state(int rig, void *buf, size_t cap, size_t *n_bytes) {
+  if (!stereo_ || rig < 0 || rig >= S_ / 2) return err(FE_BAD_ARG, "get_state: bad rig");
+  size_t sz[2] = {0, 0};
+  for (int c = 0; c < 2; c++) {
+    int rc = get_state(2 * rig + c, nullptr, 0, &sz[c]);
+    if (rc) return rc;
+  }
+  const size_t need = sizeof(StereoStateHeader) + sz[0] + sz[1];
+  if (n_bytes) *n_bytes = need;
+  if (!buf) return FE_OK;
+  if (cap < need) return FE_OVERFLOW;
+  StereoStateHeader hd;
+  hd.magic = kStereoStateMagic;
+  hd.version = kStereoStateVersion;
+  FG_CUDA(cudaMemcpy(&hd.currid, g_.currid + 2 * rig, sizeof(uint64_t), cudaMemcpyDeviceToHost));   // the rig's counter
+  hd.size[0] = sz[0];
+  hd.size[1] = sz[1];
+  uint8_t *p = static_cast<uint8_t *>(buf);
+  std::memcpy(p, &hd, sizeof(hd));
+  p += sizeof(hd);
+  for (int c = 0; c < 2; c++) {
+    int rc = get_state(2 * rig + c, p, sz[c], nullptr);
+    if (rc) return rc;
+    p += sz[c];
+  }
+  return FE_OK;
+}
+
+int FeGroup::stereo_set_state(int rig, const void *buf, size_t n_bytes) {
+  if (!stereo_ || rig < 0 || rig >= S_ / 2) return err(FE_BAD_ARG, "set_state: bad rig");
+  if (submitted_ != collected_) return err(FE_BAD_ARG, "set_state: collect the pending ticks first");
+  // ---- both cameras' blobs are checked before either is applied
+  StereoStateHeader hd;
+  if (!buf || n_bytes < sizeof(hd)) return err(FE_BAD_ARG, "set_state: blob shorter than the stereo header");
+  std::memcpy(&hd, buf, sizeof(hd));
+  if (hd.magic != kStereoStateMagic) return err(FE_BAD_ARG, "set_state: not a stereo state blob (magic)");
+  if (hd.version != kStereoStateVersion) return err(FE_BAD_ARG, "set_state: unknown stereo state version");
+  if (hd.size[0] > n_bytes || hd.size[1] > n_bytes || sizeof(hd) + hd.size[0] + hd.size[1] > n_bytes)
+    return err(FE_BAD_ARG, "set_state: truncated stereo blob (its camera blobs end past its size)");
+  const uint8_t *cam[2] = {static_cast<const uint8_t *>(buf) + sizeof(hd), static_cast<const uint8_t *>(buf) + sizeof(hd) + hd.size[0]};
+  for (int c = 0; c < 2; c++) {
+    StateView v;
+    if (const char *why = check_state(cam[c], hd.size[c], v)) return err(FE_BAD_ARG, std::string(c ? "right camera: " : "left camera: ") + why);
+  }
+  // ---- apply
+  for (int c = 0; c < 2; c++) {
+    int rc = set_state(2 * rig + c, cam[c], hd.size[c]);
+    if (rc) return rc;
+    FG_CUDA(cudaMemcpy(g_.currid + 2 * rig + c, &hd.currid, sizeof(uint64_t), cudaMemcpyHostToDevice));   // one counter per rig
+  }
+  return FE_OK;
 }
 
 }  // namespace plviwo

@@ -9,6 +9,11 @@
 //     streams (kernels_glue.cu, kernels_fast.cu, k_lk15w_g) — no host thread sees a feature before the
 //     rows of the frame are complete in pinned host memory.
 // The caller's thread only enqueues launches (submit) and waits for a tick's completion event (collect).
+//
+// Created for stereo rigs (FeGroup(cfg, 2 * n_rigs, device, true)), rig r is streams 2r (left) and 2r + 1 (right), and is what
+// one FeStereo is (TrackKLT::feed_stereo, same rows bit for bit): the front batch builds both images' pyramids and runs the
+// line front work on the left images only (TrackLSD.cpp:57-60), and the tracking phase of a tick runs the stereo state machine
+// of fe_group_dev.h for every rig of a lane in one set of launches.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -18,13 +23,14 @@
 
 #include "../../include/plviwo_fe.h"
 #include "fe_group_dev.h"
+#include "state_blob.h"
 #include "tracker_core.h"
 
 namespace plviwo {
 
 class FeGroup {
  public:
-  FeGroup(const FeConfig &cfg, int n_streams, int device);
+  FeGroup(const FeConfig &cfg, int n_streams, int device, bool stereo = false);
   ~FeGroup();
   int init();
 
@@ -54,6 +60,17 @@ class FeGroup {
   int set_state(int stream, const void *buf, size_t n_bytes);
   int tap(int stream, int what, void *buf, size_t cap, size_t *n_bytes);
 
+  // ---- stereo rigs (created with stereo = true; n_streams() = 2 * rigs).  submit / collect / play work per stream as above
+  // with the rig's images at 2r, 2r + 1 and vps of 6 doubles per RIG; these add the rig's view.
+  bool stereo() const { return stereo_; }
+  int stereo_submit(const double *timestamps, const uint8_t *const *left, const uint8_t *const *right, int stride, bool on_device,
+                    const uint8_t *const *masks_left, const uint8_t *const *masks_right, int mask_stride, const double *vps);
+  int stereo_collect(FeStereoInfo *infos);   // n_rigs entries or null
+  FeStereoInfo stereo_info(int rig) const;   // of the last collected tick
+  // the rig's blob in FeStereo's format (state_blob.h: StereoStateHeader + one stream blob per camera)
+  int stereo_get_state(int rig, void *buf, size_t cap, size_t *n_bytes);
+  int stereo_set_state(int rig, const void *buf, size_t n_bytes);
+
   void enable_timing(bool on) { timing_ = on; }
   FeGroupTimes times(bool reset);
   std::string last_error;
@@ -77,11 +94,14 @@ class FeGroup {
   int flush_front();                     // launches the pending front batch and the tracking of its ticks
   int launch_front(FrontBatch &b, int buf);
   int launch_track(int tick);
+  int launch_track_stereo(int tick);
+  const char *check_state(const void *buf, size_t n_bytes, StateView &v) const;   // nullptr: set_state accepts the blob
   int ensure_mask_buffer(int slot);
   void account(int k, cudaEvent_t a, cudaEvent_t b, int frames);
 
   FeConfig cfg_;
   int S_, device_, W_, H_;
+  bool stereo_ = false;
   int la_ = 0, R_ = 2, RB_ = 2, B_ = 1, lanes_ = 1;
   std::vector<double> K_, D_;            // per stream, 4 each
   // ---- device data

@@ -95,6 +95,8 @@ struct GroupDev {
   // truncates them, and the record's sample region: sample_cap positions p0, p1 (float2) and status bytes
   int line_samples, sample_max_pts, sample_cap;
   size_t off_sp0, off_sp1, off_sst;
+  // stereo group only: the rig's FeStereoInfo, in the record of its left stream
+  size_t off_sinfo;
 };
 
 // tracking launches (kernels_glue.cu, kernels_track.cu)
@@ -113,5 +115,21 @@ void launch_group_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cuda
 // frames whose point LK ran; reads the header the gate wrote and lnew before this tick's k_group_lines rewrites it
 void launch_group_line_samples(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s);
 void launch_group_lines(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
+
+// ---- stereo group (FeGroup created for stereo rigs): rig r is streams 2r (left) and 2r + 1 (right).  A lane's jobs are laid
+// out as its n rigs' left jobs followed by their n right jobs, so a kernel launched on the left half finds the right job of
+// its rig at jobs[blockIdx + n] and one launched on the right half the left job at jobs[blockIdx - n] (n = the launch's
+// grid size).  The steps of TrackKLT::feed_stereo / perform_detection_stereo (TrackKLT.cpp:202-393, 530-827), in order:
+//   launch_stereo_detect(left) -> FAST / select / cands / cornerSubPix / accept (left) -> launch_stereo_lr_lk ->
+//   launch_stereo_pair -> launch_stereo_detect(right) -> FAST / select / launch_stereo_cands_right / cornerSubPix /
+//   accept (right) -> launch_group_lk (both halves) -> launch_stereo_gate (both halves) -> launch_stereo_rows ->
+//   launch_group_lines (left half)
+void launch_stereo_detect(const GroupDev &g, const TrackJob *jobs, int n_rigs, bool right, cudaStream_t s);
+void launch_stereo_cands_right(const GroupDev &g, const TrackJob *jobs, int n_rigs, cudaStream_t s);
+void launch_stereo_lr_lk(const GroupDev &g, const TrackJob *jobs, int n_rigs, const LkParams &prm, cudaStream_t s);   // kernels_track.cu
+void launch_stereo_pair(const GroupDev &g, const TrackJob *jobs, int n_rigs, cudaStream_t s);
+void launch_stereo_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
+void launch_stereo_rows(const GroupDev &g, const TrackJob *jobs, int n_rigs, cudaStream_t s);
+size_t stereo_rows_smem(int pts_cap);   // dynamic shared memory of launch_stereo_rows
 
 }  // namespace plviwo

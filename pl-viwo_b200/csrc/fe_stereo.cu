@@ -9,6 +9,7 @@
 // left->right LK launch for the new points, then right), the two temporal LK launches side by side on two streams,
 // the two RANSAC gates, and the left/right merge.
 #include "fe_stereo.h"
+#include "state_blob.h"
 
 #include <algorithm>
 #include <cmath>
@@ -435,13 +436,6 @@ int FeStereo::collect_impl(Pair &pair) {
 }
 
 // ------------------------------------------------------------------------------------------------ state
-namespace {
-struct StereoStateHeader {
-  uint32_t magic, version;
-  uint64_t currid;
-  uint64_t size[2];
-};
-}  // namespace
 
 int FeStereo::get_state(void *buf, size_t cap, size_t *n_bytes) {
   if (!queue_.empty()) return err(FE_BAD_ARG, "get_state: collect the pending pairs first");
@@ -455,8 +449,8 @@ int FeStereo::get_state(void *buf, size_t cap, size_t *n_bytes) {
   if (!buf) return FE_OK;
   if (cap < need) return FE_OVERFLOW;
   StereoStateHeader hd;
-  hd.magic = 0x504c5653u;
-  hd.version = 1;
+  hd.magic = kStereoStateMagic;
+  hd.version = kStereoStateVersion;
   hd.currid = currid_;
   hd.size[0] = sz[0];
   hd.size[1] = sz[1];
@@ -478,7 +472,7 @@ int FeStereo::set_state(const void *buf, size_t n_bytes) {
   const uint8_t *p = static_cast<const uint8_t *>(buf);
   std::memcpy(&hd, p, sizeof(hd));
   p += sizeof(hd);
-  if (hd.magic != 0x504c5653u || sizeof(hd) + hd.size[0] + hd.size[1] > n_bytes) return err(FE_BAD_ARG, "set_state: not a stereo state blob");
+  if (hd.magic != kStereoStateMagic || sizeof(hd) + hd.size[0] + hd.size[1] > n_bytes) return err(FE_BAD_ARG, "set_state: not a stereo state blob");
   for (int c = 0; c < 2; c++) {
     FeContext &x = *cam_[c];
     uint64_t cam_currid = 0;   // one id counter for both cameras: the envelope's

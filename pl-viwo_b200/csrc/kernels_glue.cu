@@ -62,32 +62,97 @@ __device__ __forceinline__ GroupOutHeader *out_header(const GroupDev &g, const T
 }
 
 // ======================================================================================== top-off detection
-__global__ void __launch_bounds__(kGT)
-    k_group_detect(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+// The rig's FeStereoInfo (stereo group): in the record of the left stream
+__device__ __forceinline__ FeStereoInfo *stereo_info(const GroupDev &g, const TrackJob &left_job) {
+  return reinterpret_cast<FeStereoInfo *>(g.out + (size_t)left_job.out * g.out_stride + g.off_sinfo);
+}
+
+// Id lookups of the stereo kernels: an open-addressing table in shared memory of 2^hbits indices into an id list (-1 empty);
+// an id maps to the first index holding it.  stereo_id_hbits sizes it for a list of up to pts_cap ids (load <= 2/3).
+__device__ __forceinline__ unsigned stereo_id_hash(uint64_t id, int hbits) {
+  return (unsigned)((id * 0x9E3779B97F4A7C15ull) >> (64 - hbits));
+}
+// all threads of the CTA; the table is complete when it returns
+__device__ __forceinline__ void id_table_build(int *table, int hbits, const uint64_t *__restrict__ ids, int n) {
+  const int H = 1 << hbits;
+  for (int j = threadIdx.x; j < H; j += kGT) table[j] = -1;
+  __syncthreads();
+  for (int i = threadIdx.x; i < n; i += kGT) {
+    const uint64_t id = ids[i];
+    unsigned h = stereo_id_hash(id, hbits);
+    while (true) {
+      const int prev = atomicCAS(&table[h], -1, i);
+      if (prev < 0) break;
+      if (ids[prev] == id) {
+        atomicMin(&table[h], i);
+        break;
+      }
+      h = (h + 1) & (unsigned)(H - 1);
+    }
+  }
+  __syncthreads();
+}
+__device__ __forceinline__ int id_table_find(const int *table, int hbits, const uint64_t *__restrict__ ids, uint64_t id) {
+  unsigned h = stereo_id_hash(id, hbits);
+  while (true) {
+    const int v = table[h];
+    if (v < 0 || ids[v] == id) return v;
+    h = (h + 1) & (unsigned)((1 << hbits) - 1);
+  }
+}
+static int stereo_id_hbits(int pts_cap) {
+  int b = 1;
+  while ((1 << b) < pts_cap + pts_cap / 2) b++;
+  return b;
+}
+
+// kDetMono: the monocular frame (:395-528).  Stereo (:530-827): kDetLeft on the left job of a rig, kDetRight on the right
+// one, after k_stereo_pair has put the right camera's points (pts_last plus the new stereo points) in its working list.
+enum { kDetMono = 0, kDetLeft = 1, kDetRight = 2 };
+
+template <int Mode>
+__device__ __forceinline__ void group_detect_body(const GroupDev &g, const TrackJob *__restrict__ jobs, int hbits) {
   __shared__ BlockScan bs;
   __shared__ int grid_cnt[256];
   const TrackJob &job = jobs[blockIdx.x];
   const int s = job.stream, tid = threadIdx.x;
   const int cols = g.W, rows = g.H, d = g.min_px_dist, gx = g.grid_x, gy = g.grid_y;
   const int close_w = g.close_w, close_h = g.close_h, close_n = close_w * close_h;
-  const int n0 = g.n_pts[job.prev_rec];
-  // TrackKLT.cpp:110-123 — nothing tracked last time (or no previous image): detect on the CURRENT image only
-  const bool first = n0 == 0 || job.prev_slot < 0;
+  // stereo: the rig's left job (kDetRight: the left half of the launch precedes this one, signed index)
+  const TrackJob *left_job = Mode == kDetRight ? &jobs[(int)blockIdx.x - (int)gridDim.x] : &job;
+  // kDetRight: the working list is compacted in place, every thread reads its point before the ordered write
+  const int n0 = Mode == kDetRight ? g.wn[s] : g.n_pts[job.prev_rec];
+  const bool first = [&]() -> bool {
+    // TrackKLT.cpp:110-123 — nothing tracked last time (or no previous image): detect on the CURRENT image only
+    if constexpr (Mode == kDetMono) return n0 == 0 || job.prev_slot < 0;
+    // :221-241 — nothing tracked last time in either camera (or no previous pair): detect on the CURRENT pair only
+    if constexpr (Mode == kDetLeft) {
+      const TrackJob &rj = jobs[blockIdx.x + gridDim.x];
+      return (n0 == 0 && g.n_pts[rj.prev_rec] == 0) || job.prev_slot < 0 || rj.prev_slot < 0;
+    }
+    return g.wmode[left_job->stream] == 1;
+  }();
   const int islot = first ? job.cur_slot : job.prev_slot;
   const SlotRec &sl = g.slots[islot];
   const uint8_t *__restrict__ mask = (g.slot_flags[islot] & 1) ? sl.mask : nullptr;
   const size_t o = (size_t)s * g.pts_cap;
-  const float2 *__restrict__ pts = g.pts + (size_t)job.prev_rec * g.pts_cap;
-  const uint64_t *__restrict__ ids = g.ids + (size_t)job.prev_rec * g.pts_cap;
+  const float2 *__restrict__ pts = Mode == kDetRight ? g.wpts + o : g.pts + (size_t)job.prev_rec * g.pts_cap;
+  const uint64_t *__restrict__ ids = Mode == kDetRight ? g.wids + o : g.ids + (size_t)job.prev_rec * g.pts_cap;
   float2 *__restrict__ wpts = g.wpts + o;
   uint64_t *__restrict__ wids = g.wids + o;
   int *__restrict__ close = g.close + (size_t)s * close_n;
-  const int np = first ? 0 : n0;
+  const int np = (Mode == kDetRight || !first) ? n0 : 0;
   const float size_x = (float)cols / (float)gx, size_y = (float)rows / (float)gy;
 
   for (int i = tid; i < close_n; i += kGT) close[i] = INT_MAX;
   grid_cnt[tid] = 0;
   __syncthreads();
+  int *ltab = nullptr;   // kDetRight: the left list's ids (:720-726)
+  if constexpr (Mode == kDetRight) {
+    extern __shared__ int det_smem[];
+    ltab = det_smem;
+    id_table_build(ltab, hbits, g.wids + (size_t)left_job->stream * g.pts_cap, g.wn[left_job->stream]);
+  }
 
   // ---- first loop (:411-464).  A point is kept iff it passes the tests that do not depend on the other points (border,
   // grids, mask) and no EARLIER such point sits in its min-distance cell: first in order per cell wins.
@@ -114,15 +179,23 @@ __global__ void __launch_bounds__(kGT)
     const int k = base + tid;
     int cell = 0, gcell = 0;
     float2 kp = make_float2(0.f, 0.f);
+    uint64_t kid = 0;
     bool keep = false;
     if (k < np) {
       kp = pts[k];
       keep = classify(kp, cell, gcell) && close[cell] == k;
+      if constexpr (Mode == kDetRight) {
+        // :720-726 — a right point on an occupied cell survives if its id is also one of the left image's points
+        kid = ids[k];
+        if (!keep && classify(kp, cell, gcell))
+          keep = id_table_find(ltab, hbits, g.wids + (size_t)left_job->stream * g.pts_cap, kid) >= 0;
+      }
     }
     const int e = block_excl(keep ? 1 : 0, bs);
     if (keep) {
       wpts[nk + e] = kp;
-      wids[nk + e] = ids[k];
+      if constexpr (Mode == kDetRight) wids[nk + e] = kid;
+      else wids[nk + e] = ids[k];
       atomicAdd(&grid_cnt[gcell], 1);   // the reference saturates at 255; only "< required" is ever asked
     }
     nk += bs.total;
@@ -134,7 +207,7 @@ __global__ void __launch_bounds__(kGT)
   const int need = g.num_features - nk;
   const int need_min = min(20, (int)(min_feat_percent * g.num_features));
   int *__restrict__ valid = g.valid + (size_t)s * kValidStride;
-  if (need >= need_min) {   // :468-471
+  if (Mode == kDetMono ? need >= need_min : need > need_min) {   // :468-471 (stereo :606, :753: strictly greater)
     detection_ran = 1;
     // ---- valid cells in x-major order (:479-492)
     if (tid == 0) {
@@ -166,14 +239,38 @@ __global__ void __launch_bounds__(kGT)
     g.winfo[4 * s + 1] = 0;
     g.winfo[4 * s + 2] = 0;
     g.winfo[4 * s + 3] = 0;             // candidates waiting for cornerSubPix: k_group_cands
+    if constexpr (Mode == kDetLeft) {
+      FeStereoInfo *si = stereo_info(g, job);
+      int *w = reinterpret_cast<int *>(si);
+      for (int k = 0; k < (int)(sizeof(FeStereoInfo) / sizeof(int)); k++) w[k] = 0;
+      si->timestamp = job.timestamp;
+      si->detection_ran[0] = detection_ran;
+    } else if constexpr (Mode == kDetRight) {
+      stereo_info(g, *left_job)->detection_ran[1] = detection_ran;
+    }
   }
+}
+__global__ void __launch_bounds__(kGT)
+    k_group_detect(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+  group_detect_body<kDetMono>(g, jobs, 0);
+}
+// __maxnreg__ instead of __launch_bounds__(kGT): under the launch bound ptxas holds this instance to 32 registers and spills
+// 12 bytes to local memory; 256 threads x 64 registers still fit an SM
+__global__ void __maxnreg__(64)
+    k_stereo_detect_left(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+  group_detect_body<kDetLeft>(g, jobs, 0);
+}
+__global__ void __launch_bounds__(kGT)
+    k_stereo_detect_right(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, int hbits) {
+  group_detect_body<kDetRight>(g, jobs, hbits);
 }
 
 // Grider_GRID.h:133-149 on the candidate table of the valid cells (k_fast_g + k_fast_select_g have just filled it): bounds and
 // mask0_updated (caller mask, or inside the (2d+1)^2 square of a kept point whose square lies inside the image,
 // TrackKLT.cpp:457-461), in (cell, rank) order.
-__global__ void __launch_bounds__(kGT)
-    k_group_cands(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+// StereoRight: the right image of a rig, whose working mask is a clone of the LEFT image's mask (:691)
+template <bool StereoRight>
+__device__ __forceinline__ void group_cands_body(const GroupDev &g, const TrackJob *__restrict__ jobs) {
   __shared__ BlockScan bs;
   const TrackJob &job = jobs[blockIdx.x];
   const int s = job.stream, tid = threadIdx.x;
@@ -182,7 +279,14 @@ __global__ void __launch_bounds__(kGT)
   const bool first = g.wmode[s] == 1;
   const int islot = first ? job.cur_slot : job.prev_slot;
   const SlotRec &sl = g.slots[islot];
-  const uint8_t *__restrict__ mask = (g.slot_flags[islot] & 1) ? sl.mask : nullptr;
+  const uint8_t *__restrict__ mask;
+  if constexpr (StereoRight) {
+    const TrackJob &lj = jobs[(int)blockIdx.x - (int)gridDim.x];
+    const int lslot = first ? lj.cur_slot : lj.prev_slot;
+    mask = (g.slot_flags[lslot] & 1) ? g.slots[lslot].mask : nullptr;
+  } else {
+    mask = (g.slot_flags[islot] & 1) ? sl.mask : nullptr;
+  }
   const float2 *__restrict__ wpts = g.wpts + (size_t)s * g.pts_cap;
   const int *__restrict__ valid = g.valid + (size_t)s * kValidStride;
   const int nk = g.wn[s];
@@ -233,6 +337,14 @@ __global__ void __launch_bounds__(kGT)
     __syncthreads();
   }
   if (tid == 0) g.winfo[4 * s + 3] = next;
+}
+__global__ void __launch_bounds__(kGT)
+    k_group_cands(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+  group_cands_body<false>(g, jobs);
+}
+__global__ void __launch_bounds__(kGT)
+    k_stereo_cands_right(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+  group_cands_body<true>(g, jobs);
 }
 
 // Second half of the top-off detection, after cornerSubPix of the surviving candidates (Grider_GRID.h:163-179).
@@ -298,10 +410,29 @@ void launch_group_detect(const GroupDev &g, const TrackJob *jobs, int n_jobs, cu
   PLVIWO_CARVEOUT(k_group_detect);
   k_group_detect<<<n_jobs, kGT, 0, s>>>(g, jobs);
 }
+void launch_stereo_detect(const GroupDev &g, const TrackJob *jobs, int n_rigs, bool right, cudaStream_t s) {
+  if (n_rigs <= 0) return;
+  if (right) {
+    const int hbits = stereo_id_hbits(g.pts_cap);
+    const size_t smem = ((size_t)1 << hbits) * sizeof(int);
+    static SmemOptIn optin;
+    optin.ensure(k_stereo_detect_right, smem);
+    PLVIWO_CARVEOUT(k_stereo_detect_right);
+    k_stereo_detect_right<<<n_rigs, kGT, smem, s>>>(g, jobs, hbits);
+  } else {
+    PLVIWO_CARVEOUT(k_stereo_detect_left);
+    k_stereo_detect_left<<<n_rigs, kGT, 0, s>>>(g, jobs);
+  }
+}
 void launch_group_cands(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s) {
   if (n_jobs <= 0) return;
   PLVIWO_CARVEOUT(k_group_cands);
   k_group_cands<<<n_jobs, kGT, 0, s>>>(g, jobs);
+}
+void launch_stereo_cands_right(const GroupDev &g, const TrackJob *jobs, int n_rigs, cudaStream_t s) {
+  if (n_rigs <= 0) return;
+  PLVIWO_CARVEOUT(k_stereo_cands_right);
+  k_stereo_cands_right<<<n_rigs, kGT, 0, s>>>(g, jobs);
 }
 void launch_group_accept(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s) {
   if (n_jobs <= 0) return;
@@ -364,8 +495,11 @@ __device__ int lmeds_gate(const float2 *m1, const float2 *m2, int count, uint8_t
   return good;
 }
 
-__global__ void __launch_bounds__(kGT)
-    k_group_gate(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+// Stereo: the RANSAC of one camera of a rig only (perform_matching, :862-885, as FeStereo::matching_end): lk_status becomes
+// mask_out = mask_klt && mask_rsc in place and the counts go to the rig's FeStereoInfo; k_stereo_rows builds the rows
+// (k_stereo_gate).
+template <bool Stereo>
+__device__ __forceinline__ void group_gate_body(const GroupDev &g, const TrackJob *__restrict__ jobs) {
   extern __shared__ uint8_t gate_smem[];   // two inlier masks of pts_cap bytes
   __shared__ BlockScan bs;
   __shared__ float s_ms1[kRounds][14], s_ms2[kRounds][14];
@@ -386,7 +520,9 @@ __global__ void __launch_bounds__(kGT)
   FePointRow *rows = reinterpret_cast<FePointRow *>(rec + g.off_rows);
   uint64_t *obs_ids = reinterpret_cast<uint64_t *>(rec + g.off_obs_ids);
   float2 *obs_uv = reinterpret_cast<float2 *>(rec + g.off_obs_uv);
-  if (tid == 0) {
+  if (Stereo) {
+    if (mode == 1 || n < 10) return;   // detection-only pair / no LK launch (:848-852)
+  } else if (tid == 0) {
     GroupOutHeader h;
     memset(&h, 0, sizeof(h));
     h.info.timestamp = job.timestamp;
@@ -511,6 +647,24 @@ __global__ void __launch_bounds__(kGT)
     }
   }
   __syncthreads();
+  if constexpr (Stereo) {
+    uint8_t *__restrict__ st_out = g.lk_status + o;
+    int n_klt = 0;
+    for (int i = tid; i < n; i += kGT) {
+      const uint8_t k = st[i];
+      n_klt += k ? 1 : 0;
+      st_out[i] = (k && mask_valid && mbest[i]) ? 1 : 0;
+    }
+    n_klt = block_sum(n_klt, bs);
+    if (tid == 0) {
+      const int nr = gridDim.x / 2, cam = (int)blockIdx.x >= nr ? 1 : 0;
+      FeStereoInfo *si = stereo_info(g, jobs[(int)blockIdx.x - cam * nr]);
+      si->n_lk_in[cam] = n;
+      si->n_klt_ok[cam] = n_klt;
+      si->n_ransac_ok[cam] = n_in;
+    }
+    return;
+  }
   // ---- mask_out = mask_klt && mask_rsc (:876-879), then feed_monocular's filter (:159-173) and the rows (:176-179)
   const uint8_t *__restrict__ cmask = (g.slot_flags[job.cur_slot] & 1) ? g.slots[job.cur_slot].mask : nullptr;
   int n_good = 0, n_klt = 0;
@@ -554,11 +708,273 @@ __global__ void __launch_bounds__(kGT)
     hdr->n_obs = n_good;
   }
 }
+__global__ void __launch_bounds__(kGT)
+    k_group_gate(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+  group_gate_body<false>(g, jobs);
+}
+// __maxnreg__ instead of __launch_bounds__(kGT): under the launch bound ptxas holds this instance to 128 registers and
+// spills 272 bytes; 184 is about what the monocular instance takes (170), and 256 x 184 registers fit an SM
+__global__ void __maxnreg__(184)
+    k_stereo_gate(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+  group_gate_body<true>(g, jobs);
+}
 
 void launch_group_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s) {
   if (n_jobs <= 0) return;
   PLVIWO_CARVEOUT(k_group_gate);
   k_group_gate<<<n_jobs, kGT, 2 * (size_t)g.pts_cap, s>>>(g, jobs);
+}
+void launch_stereo_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s) {
+  if (n_jobs <= 0) return;
+  PLVIWO_CARVEOUT(k_stereo_gate);
+  k_stereo_gate<<<n_jobs, kGT, 2 * (size_t)g.pts_cap, s>>>(g, jobs);
+}
+
+// ============================================================================================ stereo glue
+// perform_detection_stereo :669-699 after the left -> right KLT of the new left points (k_lk15w_lr_g / k_lk_lr_g wrote
+// their right positions and status into the RIGHT stream's LK arrays): a new left point inside the image gets the next id
+// of the rig's counter; if its right position is inside the image and tracked too, it joins the right camera's working
+// list with the same id.  The right list is the right camera's pts_last (empty on a detection-only pair) followed by those
+// points.  One CTA per rig, launched on the left half of the lane's jobs.
+__global__ void __launch_bounds__(kGT)
+    k_stereo_pair(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs) {
+  __shared__ BlockScan bs;
+  const TrackJob &lj = jobs[blockIdx.x], &rj = jobs[blockIdx.x + gridDim.x];
+  const int sl = lj.stream, sr = rj.stream, tid = threadIdx.x;
+  const int cols = g.W, rows = g.H, cap = g.pts_cap;
+  float2 *__restrict__ lp = g.wpts + (size_t)sl * cap;
+  uint64_t *__restrict__ li = g.wids + (size_t)sl * cap;
+  float2 *__restrict__ rp = g.wpts + (size_t)sr * cap;
+  uint64_t *__restrict__ ri = g.wids + (size_t)sr * cap;
+  const int nr0 = g.wmode[sl] == 1 ? 0 : g.n_pts[rj.prev_rec];
+  {
+    const float2 *__restrict__ pp = g.pts + (size_t)rj.prev_rec * cap;
+    const uint64_t *__restrict__ pi = g.ids + (size_t)rj.prev_rec * cap;
+    for (int i = tid; i < nr0; i += kGT) {
+      rp[i] = pp[i];
+      ri[i] = pi[i];
+    }
+  }
+  const int n_new = g.winfo[4 * sl + 1];            // k_group_accept's new points, appended to the left list
+  const int start = g.wn[sl] - n_new;
+  const uint64_t base = g.currid[sl] - (uint64_t)n_new;   // ... which it numbered: the ids are handed out again here
+  const float2 *__restrict__ q1 = g.lk_pts1 + (size_t)sr * cap;
+  const uint8_t *__restrict__ st1 = g.lk_status + (size_t)sr * cap;
+  int nl = 0, np = 0;
+  for (int b = 0; b < n_new; b += kGT) {
+    const int i = b + tid;
+    bool kl = false, kp = false;
+    float2 p0 = make_float2(0.f, 0.f), q = p0;
+    if (i < n_new) {
+      p0 = lp[start + i];
+      q = q1[i];
+      const bool oob_left = (int)p0.x < 0 || (int)p0.x >= cols || (int)p0.y < 0 || (int)p0.y >= rows;
+      const bool oob_right = (int)q.x < 0 || (int)q.x >= cols || (int)q.y < 0 || (int)q.y >= rows;
+      kl = !oob_left;
+      kp = kl && !oob_right && st1[i] == 1;
+    }
+    const int el = block_excl(kl ? 1 : 0, bs), tl = bs.total;
+    const int ep = block_excl(kp ? 1 : 0, bs), tp = bs.total;
+    const uint64_t id = base + 1 + (uint64_t)(nl + el);
+    if (kl) {
+      lp[start + nl + el] = p0;
+      li[start + nl + el] = id;
+    }
+    if (kp && nr0 + np + ep < cap) {
+      rp[nr0 + np + ep] = q;
+      ri[nr0 + np + ep] = id;
+    }
+    nl += tl;
+    np += tp;
+  }
+  if (tid == 0) {
+    g.wn[sl] = start + nl;
+    g.wn[sr] = min(nr0 + np, cap);
+    // the right camera's overflow flag: k_stereo_detect_right and the right accept rewrite its own winfo, the left's
+    // candidate count (winfo[3]) is no longer read once the left accept has run
+    g.winfo[4 * sl + 3] = nr0 + np > cap ? 1 : 0;
+    g.currid[sl] = base + (uint64_t)nl;
+    g.currid[sr] = base + (uint64_t)nl;   // the right detection continues the rig's counter (k_group_accept on the right job)
+    g.winfo[4 * sl + 1] = nl;
+    FeStereoInfo *si = stereo_info(g, lj);
+    si->n_detected[0] = nl;
+    si->n_stereo_new = np;
+  }
+}
+
+void launch_stereo_pair(const GroupDev &g, const TrackJob *jobs, int n_rigs, cudaStream_t s) {
+  if (n_rigs <= 0) return;
+  PLVIWO_CARVEOUT(k_stereo_pair);
+  k_stereo_pair<<<n_rigs, kGT, 0, s>>>(g, jobs);
+}
+
+// feed_stereo :286-349 after the two gates, one CTA per rig (left half of the lane's jobs): the reset when both masks are
+// empty, the left rows with their right partner looked up by id (the left bound test uses '>', the right one '>='), the
+// right rows not added already, pts_last / ids_last of both cameras, the records' headers and the rig's counters.  The id
+// lookups go through an id table of the right list in shared memory.
+
+__global__ void __launch_bounds__(kGT)
+    k_stereo_rows(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, int hbits) {
+  extern __shared__ int rows_smem[];
+  __shared__ BlockScan bs;
+  const int H = 1 << hbits, cap = g.pts_cap;
+  int *table = rows_smem;                                           // H entries: index into the right list, -1 empty
+  int *first_pass = table + H;                                      // cap: per first index, the first passing right index
+  uint8_t *added = reinterpret_cast<uint8_t *>(first_pass + cap);   // cap: per first index, added by the left loop
+  const TrackJob &lj = jobs[blockIdx.x], &rj = jobs[blockIdx.x + gridDim.x];
+  const int sl = lj.stream, sr = rj.stream, tid = threadIdx.x;
+  const int cols = g.W, rows = g.H;
+  const int nL = g.wn[sl], nR = g.wn[sr];
+  const bool first = g.wmode[sl] == 1;
+  const size_t oL = (size_t)sl * cap, oR = (size_t)sr * cap;
+  const float2 *__restrict__ wpL = g.wpts + oL, *__restrict__ wpR = g.wpts + oR;
+  const uint64_t *__restrict__ wiL = g.wids + oL, *__restrict__ wiR = g.wids + oR;
+  uint8_t *const recL = g.out + (size_t)lj.out * g.out_stride, *const recR = g.out + (size_t)rj.out * g.out_stride;
+  float2 *__restrict__ ptsL = g.pts + (size_t)lj.out * cap, *__restrict__ ptsR = g.pts + (size_t)rj.out * cap;
+  uint64_t *__restrict__ idsL = g.ids + (size_t)lj.out * cap, *__restrict__ idsR = g.ids + (size_t)rj.out * cap;
+  FePointRow *rowsL = reinterpret_cast<FePointRow *>(recL + g.off_rows), *rowsR = reinterpret_cast<FePointRow *>(recR + g.off_rows);
+  uint64_t *oiL = reinterpret_cast<uint64_t *>(recL + g.off_obs_ids), *oiR = reinterpret_cast<uint64_t *>(recR + g.off_obs_ids);
+  float2 *ouL = reinterpret_cast<float2 *>(recL + g.off_obs_uv), *ouR = reinterpret_cast<float2 *>(recR + g.off_obs_uv);
+  int nrL = 0, nrR = 0, n_stereo = 0, reset = 0;
+  auto put = [&](float2 *pts, uint64_t *ids, uint64_t *oi, float2 *ou, int k, uint64_t id, float2 p) {
+    if (k >= cap) return;   // only reachable with duplicate ids in a loaded state
+    pts[k] = p;
+    ids[k] = id;
+    oi[k] = id;
+    ou[k] = p;
+  };
+  auto row = [&](FePointRow *r, int k, uint64_t id, float2 p, float2 pn) {
+    if (k >= cap) return;
+    FePointRow x;
+    x.id = id;
+    x.u = p.x;
+    x.v = p.y;
+    x.un = pn.x;
+    x.vn = pn.y;
+    r[k] = x;
+  };
+  int nobsL = 0, nobsR = 0;
+  if (first) {   // :221-241: the detection's points are pts_last; no rows
+    for (int i = tid; i < nL; i += kGT) put(ptsL, idsL, oiL, ouL, i, wiL[i], wpL[i]);
+    for (int i = tid; i < nR; i += kGT) put(ptsR, idsR, oiR, ouR, i, wiR[i], wpR[i]);
+    nobsL = nL;
+    nobsR = nR;
+  } else if (nL == 0 && nR == 0) {   // :286-300
+    reset = 1;
+  } else {
+    // perform_matching without an LK launch (fewer than 10 points) leaves pts1 = pts0 and an all-zero mask
+    const bool lkL = nL >= 10, lkR = nR >= 10;
+    const float2 *__restrict__ p1L = lkL ? g.lk_pts1 + oL : wpL, *__restrict__ p1R = lkR ? g.lk_pts1 + oR : wpR;
+    const float2 *__restrict__ pnL = g.lk_p1n + oL, *__restrict__ pnR = g.lk_p1n + oR;
+    const uint8_t *__restrict__ mkL = g.lk_status + oL, *__restrict__ mkR = g.lk_status + oR;   // mask_out (k_stereo_gate)
+    for (int i = tid; i < nR; i += kGT) {
+      first_pass[i] = INT_MAX;
+      added[i] = 0;
+    }
+    id_table_build(table, hbits, wiR, nR);   // (its barriers also order the two stores above)
+    auto lookup = [&](uint64_t id) -> int { return id_table_find(table, hbits, wiR, id); };
+    // ---- left points in order (:298-334)
+    for (int b = 0; b < nL; b += kGT) {
+      const int i = b + tid;
+      bool kl = false, kp = false;
+      int f = -1;
+      float2 p = make_float2(0.f, 0.f), q = p;
+      if (i < nL) {
+        p = p1L[i];
+        if (!(p.x < 0 || p.y < 0 || (int)p.x > cols || (int)p.y > rows)) {
+          const bool mL = lkL && mkL[i];
+          f = lookup(wiL[i]);
+          if (mL && f >= 0 && lkR && mkR[f]) {
+            q = p1R[f];
+            if (!(q.x < 0 || q.y < 0 || (int)q.x >= cols || (int)q.y >= rows)) kl = kp = true;
+          } else {
+            kl = mL;
+          }
+        }
+      }
+      const int el = block_excl(kl ? 1 : 0, bs), tl = bs.total;
+      const int ep = block_excl(kp ? 1 : 0, bs), tp = bs.total;
+      if (kl) {
+        put(ptsL, idsL, oiL, ouL, nrL + el, wiL[i], p);
+        row(rowsL, nrL + el, wiL[i], p, pnL[i]);
+      }
+      if (kp) {
+        put(ptsR, idsR, oiR, ouR, nrR + ep, wiR[f], q);
+        row(rowsR, nrR + ep, wiR[f], q, pnR[f]);
+        added[f] = 1;
+      }
+      nrL += tl;
+      nrR += tp;
+    }
+    n_stereo = nrR;
+    __syncthreads();
+    // ---- right points not added already (:337-349): an id joins the rows once, at its first passing index
+    auto passes = [&](int i, int &f, float2 &q) -> bool {
+      q = p1R[i];
+      if (q.x < 0 || q.y < 0 || (int)q.x >= cols || (int)q.y >= rows || !(lkR && mkR[i])) return false;
+      f = lookup(wiR[i]);
+      return !added[f];
+    };
+    for (int i = tid; i < nR; i += kGT) {
+      int f;
+      float2 q;
+      if (passes(i, f, q)) atomicMin(&first_pass[f], i);
+    }
+    __syncthreads();
+    for (int b = 0; b < nR; b += kGT) {
+      const int i = b + tid;
+      int f = -1;
+      float2 q = make_float2(0.f, 0.f);
+      const bool k = i < nR && passes(i, f, q) && first_pass[f] == i;
+      const int e = block_excl(k ? 1 : 0, bs);
+      if (k) {
+        put(ptsR, idsR, oiR, ouR, nrR + e, wiR[i], q);
+        row(rowsR, nrR + e, wiR[i], q, pnR[i]);
+      }
+      nrR += bs.total;
+    }
+    nobsL = nrL = min(nrL, cap);
+    nobsR = nrR = min(nrR, cap);
+  }
+  if (tid == 0) {
+    const TrackJob *cj[2] = {&lj, &rj};
+    const int nrow[2] = {nrL, nrR}, nobs[2] = {nobsL, nobsR};
+    uint8_t *recs[2] = {recL, recR};
+    FeStereoInfo *si = stereo_info(g, lj);
+    for (int c = 0; c < 2; c++) {
+      const int s = cj[c]->stream;
+      GroupOutHeader h;
+      memset(&h, 0, sizeof(h));
+      h.info.timestamp = cj[c]->timestamp;
+      h.info.n_point_rows = nrow[c];
+      h.info.n_last_obs = nobs[c];
+      h.n_obs = nobs[c];
+      if (g.winfo[4 * s + 2] || (c == 1 && g.winfo[4 * sl + 3])) {
+        h.status = FE_INTERNAL;
+        h.overflow_what = 1;
+      }
+      *reinterpret_cast<GroupOutHeader *>(recs[c]) = h;
+      g.n_pts[cj[c]->out] = nobs[c];
+      si->n_point_rows[c] = nrow[c];
+      si->n_last_obs[c] = nobs[c];
+    }
+    si->reset = reset;
+    si->first_frame = first ? 1 : 0;
+    si->n_detected[1] = g.winfo[4 * sr + 1];
+    si->n_stereo_rows = n_stereo;
+    g.currid[sl] = g.currid[sr];
+  }
+}
+
+size_t stereo_rows_smem(int pts_cap) { return ((size_t)1 << stereo_id_hbits(pts_cap)) * sizeof(int) + (size_t)pts_cap * 5; }
+
+void launch_stereo_rows(const GroupDev &g, const TrackJob *jobs, int n_rigs, cudaStream_t s) {
+  if (n_rigs <= 0) return;
+  const size_t smem = stereo_rows_smem(g.pts_cap);
+  static SmemOptIn optin;
+  optin.ensure(k_stereo_rows, smem);
+  PLVIWO_CARVEOUT(k_stereo_rows);
+  k_stereo_rows<<<n_rigs, kGT, smem, s>>>(g, jobs, stereo_id_hbits(g.pts_cap));
 }
 
 // ==================================================================================================== lines

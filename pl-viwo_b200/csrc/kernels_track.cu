@@ -1164,6 +1164,69 @@ void launch_group_lk(const GroupDev &g, const TrackJob *jobs, int n_jobs, const 
   k_lk_g<<<dim3((g.pts_cap + kLkWarps - 1) / kLkWarps, n_jobs), kLkWarps * 32, smem, s>>>(g, jobs, prm);
 }
 
+// ---- stereo group: the left -> right KLT of the new left points of a rig's detection (perform_detection_stereo :658-666,
+// FeStereo's lk_launch(L.pyr, R.pyr, new0, ..., false)): previous image = the left image of the detection pair, next image =
+// its right image, initial flow = the left position, no undistortion.  The new points are the tail k_group_accept appended
+// to the left working list; the results go to the RIGHT stream's LK arrays (k_stereo_pair reads them).  grid.y = rig, on
+// the left half of the lane's jobs.
+__device__ __forceinline__ int stereo_lr_setup(LkArgs &sa, const GroupDev &g, const TrackJob *jobs, const LkParams &prm, int first_pt,
+                                               int *start) {
+  const TrackJob &lj = jobs[blockIdx.y], &rj = jobs[blockIdx.y + gridDim.y];
+  const int n = g.winfo[4 * lj.stream + 1];
+  *start = g.wn[lj.stream] - n;
+  if (first_pt < n) {
+    const bool first = g.wmode[lj.stream] == 1;
+    TrackJob j = lj;
+    j.prev_slot = first ? lj.cur_slot : lj.prev_slot;
+    j.cur_slot = first ? rj.cur_slot : rj.prev_slot;
+    group_lk_args(sa, g, j, prm);
+    sa.undistort = 0;
+  }
+  return n;
+}
+
+__global__ void __launch_bounds__(kLkWarps * 32)
+    k_lk_lr_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
+  __shared__ LkArgs sa;
+  __shared__ int s_n, s_start;
+  if (threadIdx.x == 0) s_n = stereo_lr_setup(sa, g, jobs, prm, (int)blockIdx.x * kLkWarps, &s_start);
+  __syncthreads();
+  const int pi = blockIdx.x * kLkWarps + (threadIdx.x >> 5);
+  if (pi >= s_n) return;
+  const size_t ol = (size_t)jobs[blockIdx.y].stream * g.pts_cap, orr = (size_t)jobs[blockIdx.y + gridDim.y].stream * g.pts_cap;
+  lk_body(sa, g.wpts + ol + s_start, g.lk_pts1 + orr, g.lk_status + orr, nullptr, nullptr, pi);
+}
+
+__global__ void __launch_bounds__(kLkwWarps * 32, 5)
+    k_lk15w_lr_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
+  __shared__ LkArgs sa;
+  __shared__ LkwSmem sm[kLkwWarps];
+  __shared__ int s_n, s_start;
+  if (threadIdx.x == 0) s_n = stereo_lr_setup(sa, g, jobs, prm, (int)blockIdx.x * kLkwWarps, &s_start);
+  __syncthreads();
+  const int warp = threadIdx.x >> 5;
+  const int pi = blockIdx.x * kLkwWarps + warp;
+  if (pi >= s_n) return;
+  const size_t ol = (size_t)jobs[blockIdx.y].stream * g.pts_cap, orr = (size_t)jobs[blockIdx.y + gridDim.y].stream * g.pts_cap;
+  lk15w_body(sa, g.wpts + ol + s_start, g.lk_pts1 + orr, g.lk_status + orr, nullptr, nullptr, pi, sm[warp]);
+}
+
+void launch_stereo_lr_lk(const GroupDev &g, const TrackJob *jobs, int n_rigs, const LkParams &prm, cudaStream_t s) {
+  if (n_rigs <= 0) return;
+  if (prm.win == kW15 && prm.max_level + 1 <= kLk15MaxLevels) {
+    PLVIWO_CARVEOUT(k_lk15w_lr_g);
+    k_lk15w_lr_g<<<dim3((g.pts_cap + kLkwWarps - 1) / kLkwWarps, n_rigs), kLkwWarps * 32, 0, s>>>(g, jobs, prm);
+    return;
+  }
+  const int win = prm.win, np = win + 3, nd = win + 1, nw = win * win;
+  const int per_warp = ((np * np + 15) & ~15) + 2 * ((nd * nd * 2 + 15) & ~15) + 3 * ((nw * 2 + 15) & ~15);
+  const size_t smem = (size_t)per_warp * kLkWarps;
+  static SmemOptIn optin;
+  optin.ensure(k_lk_lr_g, smem);
+  PLVIWO_CARVEOUT(k_lk_lr_g);
+  k_lk_lr_g<<<dim3((g.pts_cap + kLkWarps - 1) / kLkWarps, n_rigs), kLkWarps * 32, smem, s>>>(g, jobs, prm);
+}
+
 // ---- stream group, cfg.line_samples: the samples a handle appends to its point LK launch (fe_context.cu perform_matching),
 // one warp per sample, grid.y = job.  Samples exist when the frame's point LK ran — the gate then wrote n_lk_in = n >= 10
 // into the frame's header, 0 otherwise — and lie along the stream's last detected segments (lnew, n_lnew: k_group_lines of

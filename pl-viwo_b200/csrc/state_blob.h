@@ -53,4 +53,14 @@ struct StateView {
 // reason and leaves v unspecified.
 const char *state_read(const void *buf, size_t n_bytes, int w, int h, StateView &v);
 
+// A stereo rig's blob (plviwo_fe_stereo_get_state, plviwo_fe_stereo_group_get_state): this header, then the left and the right
+// camera's blob of the format above (size[0] and size[1] bytes).  currid is the rig's id counter, shared by both cameras.
+struct StereoStateHeader {
+  uint32_t magic, version;
+  uint64_t currid;
+  uint64_t size[2];
+};
+constexpr uint32_t kStereoStateMagic = 0x504c5653u;   // 'PLVS'
+constexpr uint32_t kStereoStateVersion = 1;
+
 }  // namespace plviwo
