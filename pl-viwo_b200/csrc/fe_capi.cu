@@ -381,12 +381,13 @@ int build_pyramid(const uint8_t *img, int w, int h, int levels, int win, int equ
                   TmpImage *half) {
   if (raw.alloc(w, h) || raw.upload(img) || pyr.alloc(w, h, levels, win)) return 1;
   DevBuf<unsigned> hist, counters;
-  if (hist.alloc(256) || counters.alloc(4)) return 1;
+  DevBuf<uint8_t> lut;
+  if (hist.alloc(256) || counters.alloc(4) || lut.alloc(256)) return 1;
   cudaMemset(hist.p, 0, 256 * sizeof(unsigned));
   cudaMemset(counters.p, 0, 4 * sizeof(unsigned));
-  if (equalize) launch_hist(raw.im, hist.p, 0);
+  if (equalize) launch_hist(raw.im, hist.p, counters.p, lut.p, 0);
   DevImage l1 = pyr.pyr.n > 1 ? pyr.pyr.lvl[1] : DevImage();
-  launch_eq_pyr1(raw.im, hist.p, counters.p, equalize, pyr.pyr.lvl[0], l1, half ? half->im : DevImage(), 0);
+  launch_eq_pyr1(raw.im, lut.p, equalize, pyr.pyr.lvl[0], l1, half ? half->im : DevImage(), 0);
   launch_pyr_rest(pyr.pyr, counters.p + 1, 0);
   return cudaDeviceSynchronize() == cudaSuccess ? 0 : 1;
 }
@@ -399,11 +400,9 @@ int plviwo_op_clahe(int device, const uint8_t *img, int w, int h, uint8_t *out) 
   OP_CUDA(cudaSetDevice(device));
   TmpImage raw, l0;
   DevBuf<uint8_t> luts;
-  DevBuf<unsigned> hist, counters;
-  if (raw.alloc(w, h) || raw.upload(img) || l0.alloc(w, h) || luts.alloc(64 * 256) || hist.alloc(256) || counters.alloc(4))
-    return FE_CUDA_ERROR;
+  if (raw.alloc(w, h) || raw.upload(img) || l0.alloc(w, h) || luts.alloc(64 * 256)) return FE_CUDA_ERROR;
   launch_clahe_lut(raw.im, luts.p, 0);
-  launch_eq_pyr1(raw.im, hist.p, counters.p, 2, l0.im, DevImage(), DevImage(), 0, luts.p);
+  launch_eq_pyr1(raw.im, nullptr, 2, l0.im, DevImage(), DevImage(), 0, luts.p);
   OP_CUDA(cudaDeviceSynchronize());
   OP_CUDA(cudaMemcpy2D(out, w, l0.im.p, l0.im.pitch, w, h, cudaMemcpyDeviceToHost));
   return FE_OK;
@@ -661,6 +660,7 @@ int plviwo_op_image_kernels_time(int device, int w, int h, int iters, float ms[4
   OP_CUDA(cudaSetDevice(device));
   TmpImage raw, l0, l1, half;
   DevBuf<unsigned> hist, counters, total, kps;
+  DevBuf<uint8_t> eq_lut;
   DevBuf<int> off, cnt;
   DevBuf<FastCell> cells;
   TmpFld f;
@@ -669,7 +669,7 @@ int plviwo_op_image_kernels_time(int device, int w, int h, int iters, float ms[4
   const int nb = (ch + kFastBandRows - 1) / kFastBandRows;
   const int kcap = 1 << 22;
   if (raw.alloc(w, h) || l0.alloc(w, h) || l1.alloc((w + 1) / 2, (h + 1) / 2) || half.alloc(w / 2, h / 2) || hist.alloc(256) ||
-      counters.alloc(4) || total.alloc(2) || kps.alloc(kcap) || off.alloc((size_t)ncell * nb) || cnt.alloc((size_t)ncell * nb) ||
+      counters.alloc(4) || eq_lut.alloc(256) || total.alloc(2) || kps.alloc(kcap) || off.alloc((size_t)ncell * nb) || cnt.alloc((size_t)ncell * nb) ||
       cells.alloc(std::max(ncell, 1)) || f.alloc(w / 2, h / 2, 20, 16))
     return FE_CUDA_ERROR;
   {  // synthetic texture: smooth ramps + hash noise (uploaded once)
@@ -698,8 +698,8 @@ int plviwo_op_image_kernels_time(int device, int w, int h, int iters, float ms[4
       if (which == 0) cudaMemsetAsync(hist.p, 0, 256 * sizeof(unsigned), 0);
       if (which == 2) cudaMemsetAsync(total.p, 0, 2 * sizeof(unsigned), 0);
       cudaEventRecord(e0, 0);
-      if (which == 0) launch_hist(raw.im, hist.p, 0);
-      if (which == 1) launch_eq_pyr1(raw.im, hist.p, counters.p, 0, l0.im, l1.im, half.im, 0);
+      if (which == 0) launch_hist(raw.im, hist.p, counters.p, eq_lut.p, 0);
+      if (which == 1) launch_eq_pyr1(raw.im, eq_lut.p, 0, l0.im, l1.im, half.im, 0);
       if (which == 2) launch_fast(l0.im, cells.p, ncell, nb, cw, 20, total.p, off.p, cnt.p, kps.p, kcap, 0);
       if (which == 3) launch_canny(half.im, 50.f, 50.f, f.fb, 0);
       cudaEventRecord(e1, 0);

@@ -188,6 +188,7 @@ int FeContext::init() {
     FE_CUDA(cudaMalloc(&s.d_hist, 256 * sizeof(unsigned)));
     FE_CUDA(cudaMemset(s.d_hist, 0, 256 * sizeof(unsigned)));
     FE_CUDA(cudaMalloc(&s.d_clahe, 64 * 256));
+    FE_CUDA(cudaMalloc(&s.d_eq_lut, 256));
     FE_CUDA(cudaMalloc(&s.d_counters, 4 * sizeof(unsigned)));
     FE_CUDA(cudaMemset(s.d_counters, 0, 4 * sizeof(unsigned)));
     FE_CUDA(cudaMalloc(&s.d_seq, 4 * sizeof(int)));
@@ -291,7 +292,7 @@ FeContext::~FeContext() {
     for (auto &e : s.ev_fast_t) if (e) cudaEventDestroy(e);
     for (auto &e : s.ev_sp_t) if (e) cudaEventDestroy(e);
     destroy_graphs(s);
-    cudaFree(s.d_hist); cudaFree(s.d_counters); cudaFree(s.d_seq); cudaFree(s.d_clahe);
+    cudaFree(s.d_hist); cudaFree(s.d_counters); cudaFree(s.d_eq_lut); cudaFree(s.d_seq); cudaFree(s.d_clahe);
     if (s.s_a) cudaStreamDestroy(s.s_a);
     if (s.s_b) cudaStreamDestroy(s.s_b);
     if (s.s_line) cudaStreamDestroy(s.s_line);
@@ -398,11 +399,11 @@ int FeContext::set_currid(uint64_t id) {
 // the paths, so timings can be read whether or not the graphs are used.
 int FeContext::record_image_path(FrameSlot &s, cudaStream_t st) {
   const int eq = cfg_.histogram_method == FE_HIST_HISTOGRAM ? 1 : (cfg_.histogram_method == FE_HIST_CLAHE ? 2 : 0);
-  if (eq == 1) launch_hist(s.raw, s.d_hist, st);
+  if (eq == 1) launch_hist(s.raw, s.d_hist, s.d_counters, s.d_eq_lut, st);
   if (eq == 2) launch_clahe_lut(s.raw, s.d_clahe, st);
   if (timing) cudaEventRecord(s.ev_t[2], st);
   DevImage half = cfg_.use_lines ? s.half : DevImage();
-  launch_eq_pyr1(s.raw, s.d_hist, s.d_counters, eq, s.pyr.lvl[0], s.pyr.n > 1 ? s.pyr.lvl[1] : DevImage(), half, st, s.d_clahe);
+  launch_eq_pyr1(s.raw, s.d_eq_lut, eq, s.pyr.lvl[0], s.pyr.n > 1 ? s.pyr.lvl[1] : DevImage(), half, st, s.d_clahe);
   if (timing) cudaEventRecord(s.ev_t[3], st);
   if (s.pyr.n > 2) launch_pyr_rest(s.pyr, s.d_counters + 1, st);
   if (timing) cudaEventRecord(s.ev_t[4], st);
@@ -1732,7 +1733,7 @@ int FeContext::load_state(const void *buf, size_t n_bytes, std::vector<Pt> &pts,
     s.busy = true;
     FE_CUDA(cudaMemcpy2DAsync(s.raw.p, s.raw.pitch, v.base + v.at.image, W_, W_, H_, cudaMemcpyHostToDevice, s.s_a));
     // the stored image is already equalised: rebuild the pyramid from it without a LUT
-    launch_eq_pyr1(s.raw, s.d_hist, s.d_counters, 0, s.pyr.lvl[0], s.pyr.n > 1 ? s.pyr.lvl[1] : DevImage(),
+    launch_eq_pyr1(s.raw, s.d_eq_lut, 0, s.pyr.lvl[0], s.pyr.n > 1 ? s.pyr.lvl[1] : DevImage(),
                    cfg_.use_lines ? s.half : DevImage(), s.s_a);
     if (s.pyr.n > 2) launch_pyr_rest(s.pyr, s.d_counters + 1, s.s_a);
     FE_CUDA(cudaEventRecord(s.ev_pyr, s.s_a));

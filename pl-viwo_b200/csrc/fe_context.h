@@ -104,6 +104,7 @@ struct FrameSlot {
   cudaStream_t s_line = nullptr;   // per-slot streams: the frame-independent work of different frames overlaps
   cudaStream_t s_a = nullptr, s_b = nullptr;
   unsigned *d_hist = nullptr, *d_counters = nullptr;
+  uint8_t *d_eq_lut = nullptr;     // cv::equalizeHist LUT of this frame (launch_hist -> launch_eq_pyr1)
   uint8_t *d_clahe = nullptr;      // CLAHE: 64 tile LUTs of this frame
   int *d_seq = nullptr;            // device-side sequence numbers of the completion signals [fast, -, lines]
   cudaGraphExec_t g_image = nullptr, g_fast = nullptr, g_lines = nullptr;

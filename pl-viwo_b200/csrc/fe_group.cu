@@ -142,6 +142,7 @@ int FeGroup::init() {
     sl.mask = nullptr;
     FG_CUDA(dev_alloc(dev_allocs_, &sl.hist, 256));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.counters, 4));
+    FG_CUDA(dev_alloc(dev_allocs_, &sl.eq_lut, 256));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.clahe, cfg_.histogram_method == FE_HIST_CLAHE ? 64 * 256 : 1));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.fast_total, 2));
     FG_CUDA(dev_alloc(dev_allocs_, &sl.kps, kps_cap, false));

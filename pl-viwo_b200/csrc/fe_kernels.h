@@ -85,12 +85,12 @@ struct Pyramid {
 };
 
 // ---- image kernels (kernels_image.cu) -------------------------------------------------------------------
-// hist[256] must be zero on entry (the equalise kernel re-zeroes it when it is done with it).
-void launch_hist(const DevImage &src, unsigned *d_hist, cudaStream_t s);
-// LUT from hist (cv::equalizeHist), level 0 = lut[src] (or a plain copy when equalize == 0), level 1 = pyrDown,
-// half = exact 2x2 INTER_AREA of level 0 (may be null).  d_hist is cleared for the next frame by the last CTA.
-// equalize: 0 copy, 1 cv::equalizeHist LUT from d_hist, 2 CLAHE blend of the 64 tile LUTs in d_clahe_luts.
-void launch_eq_pyr1(const DevImage &src, unsigned *d_hist, unsigned *d_counter, int equalize, const DevImage &l0,
+// hist[256] and counter[0] must be zero on entry; the kernel's last CTA writes the frame's cv::equalizeHist LUT (256 bytes)
+// to d_lut and zeroes both again for the next frame.
+void launch_hist(const DevImage &src, unsigned *d_hist, unsigned *d_counter, uint8_t *d_lut, cudaStream_t s);
+// level 0 = lut[src] (or a plain copy when equalize == 0), level 1 = pyrDown, half = exact 2x2 INTER_AREA of level 0
+// (may be null).  equalize: 0 copy, 1 the LUT launch_hist wrote to d_lut, 2 CLAHE blend of the 64 tile LUTs in d_clahe_luts.
+void launch_eq_pyr1(const DevImage &src, const uint8_t *d_lut, int equalize, const DevImage &l0,
                     const DevImage &l1, const DevImage &half, cudaStream_t s, const uint8_t *d_clahe_luts = nullptr);
 // cv::createCLAHE(10.0, 8x8): the 64 tile LUTs (64 * 256 bytes) of the frame
 void launch_clahe_lut(const DevImage &src, uint8_t *d_luts, cudaStream_t s);
@@ -225,6 +225,7 @@ struct SlotRec {
   DevImage half;                 // half-resolution equalised frame (line detector input)
   uint8_t *mask;                 // caller mask of the frame (w * h bytes, tight); valid iff the slot's flag bit 0 is set
   unsigned *hist, *counters;     // 256 bins (zero between frames), 4 counters
+  uint8_t *eq_lut;               // the frame's cv::equalizeHist LUT (written by k_hist_b's last CTA)
   uint8_t *clahe;                // 64 tile LUTs
   unsigned *fast_total;          // [0] corners [1] scratch cursor
   unsigned *kps, *sort_scratch;

@@ -42,9 +42,53 @@ __device__ __forceinline__ void hist_add16(unsigned *my, const uint4 &v) {
   }
 }
 
-__device__ __forceinline__ void hist_body(const uint8_t *__restrict__ src, int w, int h, int pitch,
-                                          unsigned *__restrict__ hist, int block, int n_blocks) {
+// The frame's 256-byte cv::equalizeHist LUT (Appendix A1) from its complete histogram, one bin per thread.
+__device__ __forceinline__ void equalize_lut(const unsigned *__restrict__ hist, unsigned total, uint8_t *__restrict__ lut) {
+  __shared__ unsigned warp_tot[kHistWarps];
+  __shared__ int s_i0;
+  __shared__ unsigned s_h0;
+  const int tid = threadIdx.x;
+  if (tid == 0) s_i0 = 256;
+  __syncthreads();
+  const unsigned hv = __ldcg(hist + tid);   // other CTAs' atomics: read at L2
+  if (hv) atomicMin(&s_i0, tid);
+  // inclusive scan over 256 bins
+  unsigned v = hv;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    unsigned t = __shfl_up_sync(0xffffffffu, v, d);
+    if ((tid & 31) >= d) v += t;
+  }
+  if ((tid & 31) == 31) warp_tot[tid >> 5] = v;
+  __syncthreads();
+  unsigned base = 0;
+  for (int k = 0; k < (tid >> 5); k++) base += warp_tot[k];
+  const unsigned cum = v + base;  // sum hist[0..tid]
+  const int i0 = s_i0;
+  if (tid == i0) s_h0 = hv;
+  __syncthreads();
+  const unsigned hist0 = s_h0;
+  uint8_t out;
+  if (hist0 == total) {
+    out = (uint8_t)i0;  // single-valued image: dst.setTo(i0)
+  } else if (tid <= i0) {
+    out = 0;
+  } else {
+    float scale = __fdiv_rn(255.f, (float)(total - hist0));
+    int sum = (int)(cum - hist0);  // bins i0+1..tid (bins below i0 are empty)
+    int r = __float2int_rn(__fmul_rn((float)sum, scale));
+    out = (uint8_t)min(max(r, 0), 255);
+  }
+  lut[tid] = out;
+}
+
+// hist (zero on entry) accumulates the frame; the last of the n_blocks CTAs to finish (counter: zero on entry) turns it into
+// the LUT and leaves hist and counter zeroed for the next frame.  k_eq_pyr1 then only loads the 256 bytes.
+__device__ __forceinline__ void hist_body(const uint8_t *__restrict__ src, int w, int h, int pitch, unsigned *__restrict__ hist,
+                                          unsigned *__restrict__ counter, uint8_t *__restrict__ lut, int block, int n_blocks) {
+  static_assert(kHistThreads == 256, "one LUT bin per thread");
   __shared__ unsigned sh[kHistWarps][256];
+  __shared__ unsigned s_last;
   for (int i = threadIdx.x; i < kHistWarps * 256; i += kHistThreads) (&sh[0][0])[i] = 0;
   __syncthreads();
   unsigned *my = sh[threadIdx.x >> 5];
@@ -83,11 +127,23 @@ __device__ __forceinline__ void hist_body(const uint8_t *__restrict__ src, int w
     for (int k = 0; k < kHistWarps; k++) s += sh[k][b];
     if (s) atomicAdd(&hist[b], s);
   }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    s_last = (atomicAdd(counter, 1u) == (unsigned)n_blocks - 1) ? 1u : 0u;
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  equalize_lut(hist, (unsigned)w * (unsigned)h, lut);
+  hist[threadIdx.x] = 0;
+  if (threadIdx.x == 0) *counter = 0;
 }
 
 __global__ void __launch_bounds__(kHistThreads) k_hist(const uint8_t *__restrict__ src, int w, int h, int pitch,
-                                                       unsigned *__restrict__ hist) {
-  hist_body(src, w, h, pitch, hist, blockIdx.x, gridDim.x);
+                                                       unsigned *__restrict__ hist, unsigned *__restrict__ counter,
+                                                       uint8_t *__restrict__ lut) {
+  hist_body(src, w, h, pitch, hist, counter, lut, blockIdx.x, gridDim.x);
 }
 
 // grid.z = job.  Block 0 of a job also publishes the frame's flags and zeroes the FAST counters of its slot (every later
@@ -102,7 +158,7 @@ __global__ void __launch_bounds__(kHistThreads)
     sl.fast_total[1] = 0;
   }
   if (job.eq_mode != 1) return;
-  hist_body(job.src, w, h, job.src_pitch, sl.hist, blockIdx.x, gridDim.x);
+  hist_body(job.src, w, h, job.src_pitch, sl.hist, sl.counters, sl.eq_lut, blockIdx.x, gridDim.x);
 }
 
 void launch_hist_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, const FrontGeom &g, int *slot_flags, cudaStream_t s) {
@@ -114,13 +170,13 @@ void launch_hist_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs, c
   k_hist_b<<<dim3(grid, 1, n_jobs), kHistThreads, 0, s>>>(slots, jobs, g.w, g.h, slot_flags);
 }
 
-void launch_hist(const DevImage &src, unsigned *d_hist, cudaStream_t s) {
+void launch_hist(const DevImage &src, unsigned *d_hist, unsigned *d_counter, uint8_t *d_lut, cudaStream_t s) {
   int chunks = ((src.w + 15) >> 4) * src.h;
   int grid = (chunks + kHistThreads * 2 - 1) / (kHistThreads * 2);  // ~2 chunks per thread for one frame
   if (grid < 1) grid = 1;
   if (grid > 148 * 8) grid = 148 * 8;                               // 8 KB of shared memory per CTA: 8 CTAs per SM
   PLVIWO_CARVEOUT(k_hist);
-  k_hist<<<grid, kHistThreads, 0, s>>>(src.p, src.w, src.h, src.pitch, d_hist);
+  k_hist<<<grid, kHistThreads, 0, s>>>(src.p, src.w, src.h, src.pitch, d_hist, d_counter, d_lut);
 }
 
 // ------------------------------------------------------------------------------------------------ CLAHE
@@ -254,25 +310,48 @@ constexpr int kTileCols = kT0W + 8;            // staged columns: [2*tx0 - 4, 2*
 constexpr int kTileRows = kT0H + 4;            // staged rows:    [2*ty0 - 2, 2*ty0 + 34)
 constexpr int kEqThreads = 256;
 // Interior tiles (no reflected row or column, the 16-byte aligned span inside the row) are staged by the TMA unit: one
-// bulk copy per tile row of the span [2*tx0 - 16, 2*tx0 + 144), issued before the LUT is built so that the copy overlaps
-// the histogram scan.  Border tiles take the per-thread path with BORDER_REFLECT_101.
+// bulk copy per tile row of the span [2*tx0 - 16, 2*tx0 + 144), issued before the LUT is loaded so that the copy overlaps
+// the load.  Border tiles take the per-thread path with BORDER_REFLECT_101.
 constexpr int kBulkCols = kT0W + 32;           // 160 bytes per row
 constexpr int kBulkLead = 12;                  // bulk column of tile column 0: (2*tx0 - 4) - (2*tx0 - 16)
 
-__device__ __forceinline__ void eq_pyr1_body(const uint8_t *__restrict__ src, int w, int h, int spitch, unsigned *__restrict__ hist,
-              unsigned *__restrict__ counter, int equalize, const uint8_t *__restrict__ clahe_luts, const ClaheGeom &cg,
+// Packed 16-bit lanes.  A word of 4 consecutive pixels (b0 b1 b2 b3) splits into Ev = (b0, b2) and Od = (b1, b3), low lane
+// first.  With pixel c0 at the first byte of wd[0], hpyr_words gives in hs[m] the [1 4 6 4 1] sums centred on pixels
+// 4m + 4 and 4m + 6 (taps 4m + 2 .. 4m + 8): two horizontally adjacent pyrDown columns per word, each lane <= 16 * 255.
+// Bytes c0, c1 and the last two of wd[N + 1] do not enter any sum.
+template <int N>
+__device__ __forceinline__ void hpyr_words(const unsigned (&wd)[N + 2], unsigned (&hs)[N]) {
+  unsigned ev[N + 2], od[N + 1];
+#pragma unroll
+  for (int k = 0; k < N + 2; k++) ev[k] = __byte_perm(wd[k], 0, 0x4240);
+#pragma unroll
+  for (int k = 0; k < N + 1; k++) od[k] = __byte_perm(wd[k], 0, 0x4341);
+#pragma unroll
+  for (int m = 0; m < N; m++) {
+    const unsigned e_m2 = __byte_perm(ev[m], ev[m + 1], 0x5432);       // pixels 4m + 2, 4m + 4
+    const unsigned e_p2 = __byte_perm(ev[m + 1], ev[m + 2], 0x5432);   // 4m + 6, 4m + 8
+    const unsigned o_m1 = __byte_perm(od[m], od[m + 1], 0x5432);       // 4m + 3, 4m + 5
+    hs[m] = e_m2 + e_p2 + 4 * (o_m1 + od[m + 1]) + 6 * ev[m + 1];
+  }
+}
+// Vertical [1 4 6 4 1] of five packed horizontal sums, rounded: each lane <= 16 * 4080 + 128 = 65408, so no carry crosses
+// into the next lane and (s + 128) >> 8 is the lane's high byte.
+__device__ __forceinline__ unsigned vpyr_words(unsigned a, unsigned b, unsigned c, unsigned d, unsigned e) {
+  return a + e + 4 * (b + d) + 6 * c + 0x00800080u;
+}
+// The four output bytes of two vpyr_words results (lo lane, hi lane of v0, then of v1).
+__device__ __forceinline__ unsigned pack_hi_bytes(unsigned v0, unsigned v1) { return __byte_perm(v0, v1, 0x7531); }
+
+__device__ __forceinline__ void eq_pyr1_body(const uint8_t *__restrict__ src, int w, int h, int spitch,
+              const uint8_t *__restrict__ eq_lut, int equalize, const uint8_t *__restrict__ clahe_luts, const ClaheGeom &cg,
               uint8_t *__restrict__ l0, int l0pitch,
               uint8_t *__restrict__ l1, int w1, int h1, int l1pitch, uint8_t *__restrict__ half, int wh, int hh,
               int hpitch) {
   __shared__ __align__(16) uint8_t tile[kTileRows][kTileCols];
   __shared__ __align__(16) uint8_t rawt[kTileRows][kBulkCols];
   __shared__ __align__(8) unsigned long long bulk_bar;
-  __shared__ unsigned short hbuf[kTileRows][kT1W];
+  __shared__ __align__(16) unsigned hbuf[kTileRows][kT1W / 2];   // packed horizontal sums, level-1 columns (2j, 2j + 1)
   __shared__ uint8_t lut[256];
-  __shared__ unsigned warp_tot[kEqThreads / 32];
-  __shared__ int s_i0;
-  __shared__ unsigned s_h0;
-  __shared__ unsigned s_last;
 
   const int tid = threadIdx.x;
   const int tx0 = blockIdx.x * kT1W, ty0 = blockIdx.y * kT1H;
@@ -288,44 +367,8 @@ __device__ __forceinline__ void eq_pyr1_body(const uint8_t *__restrict__ src, in
 #pragma unroll 4
     for (int r = 0; r < kTileRows; r++) bulk_g2s(smem_u32(&rawt[r][0]), g + (size_t)r * spitch, kBulkCols, bar);
   }
-  // ---- LUT (cv::equalizeHist, Appendix A1): every CTA rebuilds it from the 1 KB histogram
-  if (equalize == 1) {
-    if (tid == 0) s_i0 = 256;
-    __syncthreads();
-    unsigned hv = hist[tid];
-    if (hv) atomicMin(&s_i0, tid);
-    // inclusive scan over 256 bins
-    unsigned v = hv;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      unsigned t = __shfl_up_sync(0xffffffffu, v, d);
-      if ((tid & 31) >= d) v += t;
-    }
-    if ((tid & 31) == 31) warp_tot[tid >> 5] = v;
-    __syncthreads();
-    unsigned base = 0;
-    for (int k = 0; k < (tid >> 5); k++) base += warp_tot[k];
-    unsigned cum = v + base;  // sum hist[0..tid]
-    int i0 = s_i0;
-    unsigned total = (unsigned)w * (unsigned)h;
-    if (tid == i0) s_h0 = hv;
-    __syncthreads();
-    unsigned hist0 = s_h0;
-    uint8_t out;
-    if (hist0 == total) {
-      out = (uint8_t)i0;  // single-valued image: dst.setTo(i0)
-    } else if (tid <= i0) {
-      out = 0;
-    } else {
-      float scale = __fdiv_rn(255.f, (float)(total - hist0));
-      int sum = (int)(cum - hist0);  // bins i0+1..tid (bins below i0 are empty)
-      int r = __float2int_rn(__fmul_rn((float)sum, scale));
-      out = (uint8_t)min(max(r, 0), 255);
-    }
-    lut[tid] = out;
-  } else {
-    lut[tid] = (uint8_t)tid;
-  }
+  // ---- LUT (cv::equalizeHist, Appendix A1): built once per frame by the histogram's last CTA
+  lut[tid] = equalize == 1 ? eq_lut[tid] : (uint8_t)tid;
   __syncthreads();
 
   // ---- stage the raw window through the LUT
@@ -394,26 +437,31 @@ __device__ __forceinline__ void eq_pyr1_body(const uint8_t *__restrict__ src, in
     }
   }
 
-  // ---- horizontal [1 4 6 4 1] on all staged rows
-  for (int i = tid; i < kTileRows * kT1W; i += kEqThreads) {
-    int r = i / kT1W, c = i - r * kT1W;
-    const uint8_t *p = &tile[r][2 * c + 2];
-    hbuf[r][c] = (unsigned short)(p[0] + 4 * p[1] + 6 * p[2] + 4 * p[3] + p[4]);
+  // ---- horizontal [1 4 6 4 1] on all staged rows, packed: a task is 4 words of hbuf (level-1 columns 8g .. 8g + 7)
+  // from tile words 4g .. 4g + 5 of one row
+  constexpr int kHGroups = kT1W / 8;
+  for (int t = tid; t < kTileRows * kHGroups; t += kEqThreads) {
+    const int r = t / kHGroups, g = t - r * kHGroups;
+    const uint2 *p = reinterpret_cast<const uint2 *>(&tile[r][16 * g]);   // rows are 8-byte aligned (kTileCols = 136)
+    const uint2 a = p[0], b = p[1], c = p[2];
+    const unsigned wd[6] = {a.x, a.y, b.x, b.y, c.x, c.y};
+    unsigned hs[4];
+    hpyr_words<4>(wd, hs);
+    *reinterpret_cast<uint4 *>(&hbuf[r][4 * g]) = make_uint4(hs[0], hs[1], hs[2], hs[3]);
   }
   __syncthreads();
 
-  // ---- vertical pass -> level 1, and the 2x2 mean -> half-resolution image; 4 outputs per thread, one word store
+  // ---- vertical pass -> level 1, and the 2x2 mean -> half-resolution image; one output word of each per thread
   {
-    int r = tid / (kT1W / 4), c4 = (tid - r * (kT1W / 4)) * 4;
-    int oy = ty0 + r, ox = tx0 + c4;
+    static_assert(kT1H * (kT1W / 4) == kEqThreads, "one level-1 word per thread");
+    const int r = tid / (kT1W / 4), q = tid - r * (kT1W / 4);
+    const int oy = ty0 + r, ox = tx0 + 4 * q;
     if (oy < h1 && ox < w1) {
-      unsigned packed = 0;
+      uint2 hv[5];
 #pragma unroll
-      for (int k = 0; k < 4; k++) {
-        int c = c4 + k;
-        int s = hbuf[2 * r][c] + 4 * hbuf[2 * r + 1][c] + 6 * hbuf[2 * r + 2][c] + 4 * hbuf[2 * r + 3][c] + hbuf[2 * r + 4][c];
-        packed |= (unsigned)((s + 128) >> 8) << (8 * k);
-      }
+      for (int j = 0; j < 5; j++) hv[j] = *reinterpret_cast<const uint2 *>(&hbuf[2 * r + j][2 * q]);
+      const unsigned packed = pack_hi_bytes(vpyr_words(hv[0].x, hv[1].x, hv[2].x, hv[3].x, hv[4].x),
+                                            vpyr_words(hv[0].y, hv[1].y, hv[2].y, hv[3].y, hv[4].y));
       uint8_t *dst = l1 + (size_t)oy * l1pitch + ox;
       if (ox + 4 <= w1) {
         *reinterpret_cast<unsigned *>(dst) = packed;
@@ -422,13 +470,15 @@ __device__ __forceinline__ void eq_pyr1_body(const uint8_t *__restrict__ src, in
       }
     }
     if (half != nullptr && oy < hh && ox < wh) {
-      unsigned packed = 0;
-#pragma unroll
-      for (int k = 0; k < 4; k++) {
-        const uint8_t *p0 = &tile[2 * r + 2][2 * (c4 + k) + 4];
-        const uint8_t *p1 = &tile[2 * r + 3][2 * (c4 + k) + 4];
-        packed |= (unsigned)((p0[0] + p0[1] + p1[0] + p1[1] + 2) >> 2) << (8 * k);
-      }
+      // (a + b + c + d + 2) >> 2 per lane: Ev + Od of a word are the sums of its two pixel pairs; each lane <= 1022
+      const unsigned *p0 = reinterpret_cast<const unsigned *>(&tile[2 * r + 2][8 * q + 4]);
+      const unsigned *p1 = reinterpret_cast<const unsigned *>(&tile[2 * r + 3][8 * q + 4]);
+      const unsigned a0 = p0[0], a1 = p0[1], b0 = p1[0], b1 = p1[1];
+      const unsigned s0 = __byte_perm(a0, 0, 0x4240) + __byte_perm(a0, 0, 0x4341) + __byte_perm(b0, 0, 0x4240) +
+                          __byte_perm(b0, 0, 0x4341) + 0x00020002u;
+      const unsigned s1 = __byte_perm(a1, 0, 0x4240) + __byte_perm(a1, 0, 0x4341) + __byte_perm(b1, 0, 0x4240) +
+                          __byte_perm(b1, 0, 0x4341) + 0x00020002u;
+      const unsigned packed = __byte_perm(s0 >> 2, s1 >> 2, 0x6420);
       uint8_t *dst = half + (size_t)oy * hpitch + ox;
       if (ox + 4 <= wh) {
         *reinterpret_cast<unsigned *>(dst) = packed;
@@ -437,29 +487,15 @@ __device__ __forceinline__ void eq_pyr1_body(const uint8_t *__restrict__ src, in
       }
     }
   }
-
-  // ---- the last CTA to finish clears the histogram for the next frame
-  if (equalize == 1) {
-    __syncthreads();
-    if (tid == 0) {
-      __threadfence();
-      s_last = (atomicAdd(counter, 1u) == gridDim.x * gridDim.y - 1) ? 1u : 0u;
-    }
-    __syncthreads();
-    if (s_last) {
-      hist[tid] = 0;
-      if (tid == 0) *counter = 0;
-    }
-  }
 }
 
 __global__ void __launch_bounds__(kEqThreads)
-    k_eq_pyr1(const uint8_t *__restrict__ src, int w, int h, int spitch, unsigned *__restrict__ hist,
-              unsigned *__restrict__ counter, int equalize, const uint8_t *__restrict__ clahe_luts, ClaheGeom cg,
+    k_eq_pyr1(const uint8_t *__restrict__ src, int w, int h, int spitch, const uint8_t *__restrict__ eq_lut, int equalize,
+              const uint8_t *__restrict__ clahe_luts, ClaheGeom cg,
               uint8_t *__restrict__ l0, int l0pitch,
               uint8_t *__restrict__ l1, int w1, int h1, int l1pitch, uint8_t *__restrict__ half, int wh, int hh,
               int hpitch) {
-  eq_pyr1_body(src, w, h, spitch, hist, counter, equalize, clahe_luts, cg, l0, l0pitch, l1, w1, h1, l1pitch, half, wh, hh, hpitch);
+  eq_pyr1_body(src, w, h, spitch, eq_lut, equalize, clahe_luts, cg, l0, l0pitch, l1, w1, h1, l1pitch, half, wh, hh, hpitch);
 }
 __global__ void __launch_bounds__(kEqThreads)
     k_eq_pyr1_b(const SlotRec *__restrict__ slots, const FrontJob *__restrict__ jobs, int w, int h, ClaheGeom cg, int want_half) {
@@ -467,7 +503,7 @@ __global__ void __launch_bounds__(kEqThreads)
   const SlotRec &sl = slots[job.slot];
   const DevImage &l1 = sl.lvl[1];
   const bool has1 = sl.n_lvl > 1;
-  eq_pyr1_body(job.src, w, h, job.src_pitch, sl.hist, sl.counters, job.eq_mode, sl.clahe, cg, sl.lvl[0].p, sl.lvl[0].pitch,
+  eq_pyr1_body(job.src, w, h, job.src_pitch, sl.eq_lut, job.eq_mode, sl.clahe, cg, sl.lvl[0].p, sl.lvl[0].pitch,
                has1 ? l1.p : nullptr, has1 ? l1.w : 0, has1 ? l1.h : 0, l1.pitch, want_half ? sl.half.p : nullptr, sl.half.w, sl.half.h,
                sl.half.pitch);
 }
@@ -480,13 +516,13 @@ void launch_eq_pyr1_batch(const SlotRec *slots, const FrontJob *jobs, int n_jobs
   k_eq_pyr1_b<<<grid, kEqThreads, 0, s>>>(slots, jobs, g.w, g.h, clahe_geom(g.w, g.h), want_half ? 1 : 0);
 }
 
-void launch_eq_pyr1(const DevImage &src, unsigned *d_hist, unsigned *d_counter, int equalize, const DevImage &l0,
+void launch_eq_pyr1(const DevImage &src, const uint8_t *d_lut, int equalize, const DevImage &l0,
                     const DevImage &l1, const DevImage &half, cudaStream_t s, const uint8_t *d_clahe_luts) {
   // tiles are laid over the level-1 footprint of the frame even when level 1 itself is not wanted (l1.p == null)
   const int w1 = (src.w + 1) / 2, h1 = (src.h + 1) / 2;
   dim3 grid((w1 + kT1W - 1) / kT1W, (h1 + kT1H - 1) / kT1H);
   PLVIWO_CARVEOUT(k_eq_pyr1);
-  k_eq_pyr1<<<grid, kEqThreads, 0, s>>>(src.p, src.w, src.h, src.pitch, d_hist, d_counter, equalize, d_clahe_luts,
+  k_eq_pyr1<<<grid, kEqThreads, 0, s>>>(src.p, src.w, src.h, src.pitch, d_lut, equalize, d_clahe_luts,
                                         clahe_geom(src.w, src.h), l0.p, l0.pitch, l1.p,
                                         l1.p ? l1.w : 0, l1.p ? l1.h : 0, l1.pitch, half.p, half.w, half.h, half.pitch);
 }
