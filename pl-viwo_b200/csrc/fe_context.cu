@@ -604,7 +604,7 @@ int FeContext::track_candidates(FrameSlot &prev, FrameSlot &s) {
   if (!use_spec_ || cfg_.line_samples > 0) return FE_OK;
   const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, s.K, s.D, true);
   const int ntab = prev.predet_ncell * prev.predet_nfg;
-  if (ntab <= 0 || ntab > cand_cap_ || prev.predet_num_features != cfg_.num_features || !lk_table_mode_ok(prm, prev.pyr.n))
+  if (ntab <= 0 || ntab > cand_cap_ || prev.predet_num_features != cfg_.num_features || !lk_w15_form(prm.win, prev.pyr.n))
     return FE_OK;
   FE_CUDA(cudaStreamWaitEvent(s.s_b, prev.ev_fast, 0));   // the candidate table of the previous frame
   launch_lk(prev.pyr, s.pyr, prev.d_cand_ref, s.h_sc_pts1, s.h_sc_status, s.h_sc_p0n, s.h_sc_p1n, ntab, prm, s.s_b, &s.h_flags[3],
@@ -1088,7 +1088,7 @@ int FeContext::speculate(FrameSlot &prev, const float2 *lk_pts, const uint8_t *l
     FE_CUDA(cudaStreamWaitEvent(s_pt_, fn.ev_pyr, 0));
     spec_timed_ = fn.timed;
     if (spec_timed_) cudaEventRecord(ev_pt_[2], s_pt_);
-    const bool flow0 = lk_table_mode_ok(prm, prev.pyr.n);   // pts1 = pts0 is implicit for the 15 x 15 kernel
+    const bool flow0 = lk_w15_form(prm.win, prev.pyr.n);   // pts1 = pts0 is implicit for the 15 x 15 kernel
     if (!flow0) std::memcpy(h_sp_pts1_, h_sp_pts0_, (size_t)k * sizeof(float2));
     const bool self_signal = launch_lk(prev.pyr, fn.pyr, h_sp_pts0_, h_sp_pts1_, h_sp_status_, h_sp_p0n_, h_sp_p1n_, k, prm, s_pt_,
                                        &h_flag_lk_[1], ++seq_sp_, d_lk_done_ + 1, nullptr, 0, flow0);

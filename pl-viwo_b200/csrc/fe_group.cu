@@ -162,6 +162,9 @@ int FeGroup::init() {
   FG_CUDA(dev_alloc(dev_allocs_, &d_slot_flags_, nslots));
   g_.slots = d_slots_;
   g_.slot_flags = d_slot_flags_;
+  // every slot's pyramid holds n_lvl images: LK tracks through all of them (cv::calcOpticalFlowPyrLK on a prebuilt pyramid),
+  // and the body of its launches is chosen by that count, as a handle chooses it (fe_kernels.h lk_w15_form)
+  lk_prm_ = lk_params(cfg_.win_size, slots_[0].n_lvl - 1, nullptr, nullptr, true);
 
   // ---- tracker state and work arrays
   const size_t P = (size_t)S_ * g_.pts_cap;
@@ -640,7 +643,7 @@ int FeGroup::launch_track(int tick) {
   TrackJob *hj = h_tjobs_ + (size_t)ring * S_, *dj = d_tjobs_ + (size_t)ring * S_;
   int nj = 0;
   for (int s = 0; s < S_; s++) nj += tr.cur_slot[s] >= 0 ? 1 : 0;
-  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, nullptr, nullptr, true);
+  const LkParams &prm = lk_prm_;
   const bool tm = timing_;
   // jobs are stored in stream order; lane l owns streams [S l / lanes, S (l + 1) / lanes) for the lifetime of the group
   // (a stream's frames are tracked in order on ONE CUDA stream), i.e. a contiguous range of the tick's jobs
@@ -1002,7 +1005,7 @@ int FeGroup::launch_track_stereo(int tick) {
   TrackJob *hj = h_tjobs_ + (size_t)ring * S_, *dj = d_tjobs_ + (size_t)ring * S_;
   int nj = 0;
   for (int s = 0; s < S_; s++) nj += tr.cur_slot[s] >= 0 ? 1 : 0;
-  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, nullptr, nullptr, true);
+  const LkParams &prm = lk_prm_;
   const int n_rigs = S_ / 2;
   std::vector<TrackJob> pairs;
   int jpos = 0;

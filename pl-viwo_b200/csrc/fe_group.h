@@ -6,7 +6,7 @@
 //   * the tracker state (pts_last / ids_last / currid, lines_last / point_on_lines_last) lives in device memory and the
 //     state machine of a frame (top-off detection on the previous image, with FAST + std::sort / top-k + cornerSubPix on
 //     the cells it leaves open, LK, RANSAC gate, row filter, line association) is one set of launches per tick for all
-//     streams (kernels_glue.cu, kernels_fast.cu, k_lk15w_g) — no host thread sees a feature before the
+//     streams (kernels_glue.cu, kernels_fast.cu, k_lk15w_g<GroupPoints>) — no host thread sees a feature before the
 //     rows of the frame are complete in pinned host memory.
 // The caller's thread only enqueues launches (submit) and waits for a tick's completion event (collect).
 //
@@ -107,6 +107,7 @@ class FeGroup {
   // ---- device data
   GroupDev g_{};
   FrontGeom fg_{};
+  LkParams lk_prm_{};                    // LK of every launch: max_level = the images the slots' pyramids hold - 1
   std::vector<SlotRec> slots_;           // host copy of the table (S * R entries, stream-major)
   SlotRec *d_slots_ = nullptr;
   int *d_slot_flags_ = nullptr;

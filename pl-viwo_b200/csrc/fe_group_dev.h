@@ -109,6 +109,8 @@ void launch_group_fast_select(const GroupDev &g, const TrackJob *jobs, int n_job
 void launch_group_cands(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
 void launch_group_subpix(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);   // kernels_track.cu
 void launch_group_accept(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
+// the LK launches (kernels_track.cu; also launch_group_line_samples, launch_stereo_lr_lk): prm.max_level + 1 = the images
+// every slot's pyramid holds (SlotRec::n_lvl)
 void launch_group_lk(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s);
 void launch_group_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cudaStream_t s);
 // cfg.line_samples: LK of the samples along the stream's last detected segments (lnew), previous -> current pyramid, for the

@@ -153,19 +153,21 @@ inline LkParams lk_params(int win, int max_level, const double *K, const double 
   }
   return prm;
 }
+// The one rule for the LK body: true if a win x win window over pyramid_images images (those the pyramid holds, at most
+// max_level + 1) runs the 15 x 15 bodies (k_lk15, k_lk15w_g), false if it runs the generic one (k_lk_g).
+bool lk_w15_form(int win, int pyramid_images);
 // host_flag / flag_value / d_done_counter (optional): the kernel itself publishes flag_value to the pinned word when its
 // last feature is done (d_done_counter: one zeroed device word).  Returns true if the kernel will do so; false means
 // the caller has to queue its own completion signal (generic-window kernel).
+// table mode (lk_w15_form only): d_pts0 is a fixed-stride candidate table (slot i belongs to cell i / tab_stride, live iff
+// i % tab_stride < d_tab_cnt[cell]); flow_is_zero: the initial guess is the previous position, d_pts1 is written only;
+// cell_mask (8 words, optional): only cells whose bit is set are tracked.
 bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status,
                float2 *d_p0n, float2 *d_p1n, int n, const LkParams &prm, cudaStream_t s, int *host_flag = nullptr,
                int flag_value = 0, unsigned *d_done_counter = nullptr, const int *d_tab_cnt = nullptr, int tab_stride = 0,
                bool flow_is_zero = false, const unsigned *cell_mask = nullptr);
-// table mode (15 x 15 window, <= 6 pyramid images only — lk_table_mode_ok): d_pts0 is a fixed-stride candidate table (slot i
-// belongs to cell i / tab_stride, live iff i % tab_stride < d_tab_cnt[cell]); flow_is_zero: the initial guess is the
-// previous position, d_pts1 is written only; cell_mask (8 words, optional): only cells whose bit is set are tracked.
-bool lk_table_mode_ok(const LkParams &prm, int pyramid_images);
-// k_lk15w_g's one-warp-per-feature body on n points over one pyramid pair (15 x 15 window, <= 6 pyramid images, no
-// undistortion; false otherwise): the same results as launch_lk's k_lk15, bit for bit
+// k_lk15w_g's one-warp-per-feature body on n points over one pyramid pair (lk_w15_form and no undistortion; false
+// otherwise): the same results as launch_lk's k_lk15, bit for bit
 bool launch_lk_warp(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status, int n,
                     const LkParams &prm, cudaStream_t s);
 void launch_undistort(const float2 *d_pts, float2 *d_out, int n, const double K[4], const double D[4], cudaStream_t s);

@@ -731,7 +731,7 @@ void launch_stereo_gate(const GroupDev &g, const TrackJob *jobs, int n_jobs, cud
 }
 
 // ============================================================================================ stereo glue
-// perform_detection_stereo :669-699 after the left -> right KLT of the new left points (k_lk15w_lr_g / k_lk_lr_g wrote
+// perform_detection_stereo :669-699 after the left -> right KLT of the new left points (k_lk15w_g / k_lk_g<StereoLr> wrote
 // their right positions and status into the RIGHT stream's LK arrays): a new left point inside the image gets the next id
 // of the rig's counter; if its right position is inside the image and tracked too, it joins the right camera's working
 // list with the same id.  The right list is the right camera's pts_last (empty on a detection-only pair) followed by those

@@ -192,8 +192,7 @@ void launch_undistort(const float2 *d_pts, float2 *d_out, int n, const double K[
 //   3. builds the fixed-point (W_BITS = 14) bilinear patches I, Ix, Iy (int16) and the 2x2 normal matrix,
 //   4. iterates <= 30 times: bilinear J patch, mismatch vector b (shuffle-reduced), 2x2 solve.
 // Nothing but the two 8-bit pyramids is read from HBM: no derivative planes, no padded copies.
-constexpr int kLkWarps = 4;
-constexpr int kLkMaxPatch = (kMaxWin + 3) * (kMaxWin + 3);
+constexpr int kLkWarps = 4;   // features (warps) per CTA of the warp-per-feature kernels
 
 struct LkArgs {
   const uint8_t *p0[kMaxLevels];
@@ -206,6 +205,41 @@ struct LkArgs {
   CalibArgs calib;
 };
 
+// The arguments of one pair of pyramids: `levels` images of l0 (previous) and l1 (next), prm's window and criteria,
+// calibration K / D (undistort: also write the undistorted positions), cell_mask null = every cell.
+__host__ __device__ inline void lk_args(LkArgs &a, const DevImage *l0, const DevImage *l1, int levels, const LkParams &prm,
+                                        const double *K, const double *D, int undistort, int flow_is_zero, const unsigned *cell_mask) {
+  for (int l = 0; l < levels; l++) {
+    a.p0[l] = l0[l].p;
+    a.p1[l] = l1[l].p;
+    a.w[l] = l0[l].w;
+    a.h[l] = l0[l].h;
+    a.pitch0[l] = l0[l].pitch;
+    a.pitch1[l] = l1[l].pitch;
+  }
+  a.win = prm.win;
+  a.max_level = levels - 1;
+  a.max_count = prm.max_count;
+  a.eps_sq = prm.eps_sq;
+  a.min_eig = prm.min_eig;
+  a.undistort = undistort;
+  a.flow_is_zero = flow_is_zero;
+  for (int i = 0; i < 8; i++) a.cell_mask[i] = cell_mask ? cell_mask[i] : 0xffffffffu;
+  for (int i = 0; i < 4; i++) {
+    a.calib.K[i] = K[i];
+    a.calib.D[i] = D[i];
+  }
+}
+
+// lk_body's shared memory per warp: raw[np*np] u8 | dx[nd*nd] s16 | dy[nd*nd] s16 | Iw[nw] s16 | Ix[nw] s16 | Iy[nw] s16,
+// each part rounded up to 16 bytes.  Its launches size their dynamic shared memory with it.
+struct LkLayout {
+  int raw, d, w, per_warp;   // bytes of the raw patch, of one derivative plane, of one window patch, of a warp's slice
+  __host__ __device__ explicit LkLayout(int win)
+      : raw(((win + 3) * (win + 3) + 15) & ~15), d(((win + 1) * (win + 1) * 2 + 15) & ~15), w((win * win * 2 + 15) & ~15),
+        per_warp(raw + 2 * d + 3 * w) {}
+};
+
 // feature pi of the warp's launch; the warp's shared memory is its slice of the dynamic buffer
 template <class Args>
 __device__ __forceinline__ void lk_body(const Args &a, const float2 *__restrict__ pts0, float2 *__restrict__ pts1,
@@ -216,12 +250,9 @@ __device__ __forceinline__ void lk_body(const Args &a, const float2 *__restrict_
   const int np = win + 3;        // raw patch side
   const int nd = win + 1;        // derivative grid side
   const int nw = win * win;
-  // per-warp shared layout: raw[np*np] u8 | dx[nd*nd] s16 | dy[nd*nd] s16 | Iw[nw] s16 | Ix[nw] s16 | Iy[nw] s16
-  const int raw_bytes = (np * np + 15) & ~15;
-  const int d_bytes = (nd * nd * 2 + 15) & ~15;
-  const int w_bytes = (nw * 2 + 15) & ~15;
-  const int per_warp = raw_bytes + 2 * d_bytes + 3 * w_bytes;
-  uint8_t *base = lk_smem + warp * per_warp;
+  const LkLayout lay(win);
+  const int raw_bytes = lay.raw, d_bytes = lay.d, w_bytes = lay.w;
+  uint8_t *base = lk_smem + warp * lay.per_warp;
   uint8_t *raw = base;
   short *ddx = reinterpret_cast<short *>(base + raw_bytes);
   short *ddy = reinterpret_cast<short *>(base + raw_bytes + d_bytes);
@@ -384,14 +415,6 @@ __device__ __forceinline__ void lk_body(const Args &a, const float2 *__restrict_
   }
 }
 
-__global__ void __launch_bounds__(kLkWarps * 32)
-    k_lk(LkArgs a, const float2 *__restrict__ pts0, float2 *__restrict__ pts1, uint8_t *__restrict__ status,
-         float2 *__restrict__ p0n, float2 *__restrict__ p1n, int n) {
-  const int pi = blockIdx.x * kLkWarps + (threadIdx.x >> 5);
-  if (pi >= n) return;
-  lk_body(a, pts0, pts1, status, p0n, p1n, pi);
-}
-
 // ------------------------------------------------------------------------------------------ LK, 15 x 15 window
 // Specialisation for the reference's window (TrackKLT.h:144): ONE CTA PER FEATURE, one warp per pyramid level.
 //
@@ -413,7 +436,7 @@ __global__ void __launch_bounds__(kLkWarps * 32)
 // The per-pixel arithmetic is that of the generic kernel above; the only difference is that it accumulates the integer
 // products in float32 while this kernel sums them exactly.
 constexpr int kW15 = 15;
-constexpr int kLk15MaxLevels = 6;   // pyr_levels <= 5 (the reference uses 5); deeper pyramids take the generic kernel
+constexpr int kLk15MaxLevels = 6;   // pyramid images (the reference's pyr_levels 5); deeper pyramids take the generic body
 constexpr int kJMargin = 4;         // the staged region of the next image extends this far around a window
 constexpr int kJSpan = kW15 + 2;    // rows / columns a window touches: 15 + 1 (bilinear) + 1 (the lanes' masked 16th row)
 constexpr int kJR = kJSpan + 2 * kJMargin;   // 25
@@ -729,7 +752,6 @@ __global__ void __launch_bounds__(kLk15MaxLevels * 32)
 // — and moves on to level l - 1.  The mismatch sums are exact integers (per-lane 32-bit, warp reductions on 16-bit halves),
 // so the split of the window over lanes cannot change a bit: results are identical to k_lk15's (tests/test_group_gpu.py
 // compares a group, which runs this kernel, with single handles, which run k_lk15).  An SM holds 32+ features.
-constexpr int kLkwWarps = 4;
 // Staged rows of the previous image (18 x 18 pixels) and of the region of the next image (25 x 25) are kept with a row
 // stride that is a multiple of 4 bytes and their first word aligned like the image's (it holds the region's first column,
 // x0 & 3 bytes in).  Rows are reflected through their row pointer; a word that lies inside the image row is one 32-bit
@@ -1086,308 +1108,216 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
   }
 }
 
-// ---- stream group: the points of every stream of a tracking launch in ONE launch (grid.y = job).  The arguments of a job
-// (pyramids of its previous and current slot, calibration in force) are assembled in shared memory; the per-feature work is
-// the body above, so a stream's tracks are bit-identical to those of a single handle.
-__device__ __forceinline__ void group_lk_args(LkArgs &a, const GroupDev &g, const TrackJob &job, const LkParams &prm) {
-  const SlotRec &s0 = g.slots[job.prev_slot], &s1 = g.slots[job.cur_slot];
-  int levels = prm.max_level + 1;
-  if (levels > s0.n_lvl) levels = s0.n_lvl;
-  for (int l = 0; l < levels; l++) {
-    a.p0[l] = s0.lvl[l].p;
-    a.p1[l] = s1.lvl[l].p;
-    a.w[l] = s0.lvl[l].w;
-    a.h[l] = s0.lvl[l].h;
-    a.pitch0[l] = s0.lvl[l].pitch;
-    a.pitch1[l] = s1.lvl[l].pitch;
+// ------------------------------------------------------------------------------------- LK, one warp per feature
+// Two kernel templates, one per body — k_lk_g (lk_body, any window) and k_lk15w_g (lk15w_body) — over a point source that
+// gives CTA (blockIdx.x, blockIdx.y) its job (grid.y) and features blockIdx.x * kLkWarps + warp of that job:
+//   Cta                  the source's shared per-CTA state
+//   setup(c, first)      thread 0, once per CTA: the job's feature count; c is set up when feature `first` is below it
+//   track(c, pi, body)   runs body(args, pts0, pts1, status, p0n, p1n, i) on feature pi of the job and stores what it leaves
+
+// n points in explicit arrays over one pyramid pair (launch_lk's generic form, launch_lk_warp)
+struct LkArrays {
+  LkArgs a;
+  const float2 *pts0;
+  float2 *pts1;
+  uint8_t *status;
+  float2 *p0n, *p1n;
+  int n;
+  struct Cta {};
+  __device__ int setup(Cta &, int) const { return n; }
+  template <class Body>
+  __device__ void track(Cta &, int pi, Body body) const { body(a, pts0, pts1, status, p0n, p1n, pi); }
+};
+
+// The group sources assemble a job's LkArgs in shared memory from the slot table, through the prm.max_level + 1 images every
+// slot's pyramid holds (FeGroup clamps max_level to them), so a stream's tracks are bit-identical to those of a single handle.
+struct GroupSrc {
+  GroupDev g;
+  const TrackJob *jobs;
+  LkParams prm;
+  // previous image = slot s0, next image = slot s1, calibration of `cal`, initial guess = the previous position
+  __device__ void args(LkArgs &a, int s0, int s1, const TrackJob &cal, int undistort) const {
+    lk_args(a, g.slots[s0].lvl, g.slots[s1].lvl, prm.max_level + 1, prm, cal.K, cal.D, undistort, 1, nullptr);
   }
-  a.win = prm.win;
-  a.max_level = levels - 1;
-  a.max_count = prm.max_count;
-  a.eps_sq = prm.eps_sq;
-  a.min_eig = prm.min_eig;
-  a.undistort = 1;
-  a.flow_is_zero = 1;   // pts_new = pts_old (TrackKLT.cpp:134)
-  for (int i = 0; i < 8; i++) a.cell_mask[i] = 0xffffffffu;
-  for (int i = 0; i < 4; i++) {
-    a.calib.K[i] = job.K[i];
-    a.calib.D[i] = job.D[i];
+};
+
+// Stream group: the working list of every stream of a tracking launch, previous -> current image (pts_new = pts_old,
+// TrackKLT.cpp:134); a stream with fewer than 10 points runs no LK (TrackKLT.cpp:848-852).
+struct GroupPoints : GroupSrc {
+  struct Cta {
+    LkArgs a;
+  };
+  __device__ int setup(Cta &c, int first) const {
+    const TrackJob &job = jobs[blockIdx.y];
+    const int n = g.wn[job.stream];
+    if (g.wmode[job.stream] != 0 || n < 10) return 0;
+    if (first < n) args(c.a, job.prev_slot, job.cur_slot, job, 1);
+    return n;
   }
-}
-
-__global__ void __launch_bounds__(kLkWarps * 32)
-    k_lk_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
-  __shared__ LkArgs sa;
-  const TrackJob &job = jobs[blockIdx.y];
-  const int s = job.stream;
-  const int n = g.wn[s];
-  if (g.wmode[s] != 0 || n < 10 || (int)blockIdx.x * kLkWarps >= n) return;
-  if (threadIdx.x == 0) group_lk_args(sa, g, job, prm);
-  __syncthreads();
-  const int pi = blockIdx.x * kLkWarps + (threadIdx.x >> 5);
-  if (pi >= n) return;
-  const size_t o = (size_t)s * g.pts_cap;
-  lk_body(sa, g.wpts + o, g.lk_pts1 + o, g.lk_status + o, g.lk_p0n + o, g.lk_p1n + o, pi);
-}
-
-// 5 resident CTAs per SM: 94 registers, no spills
-__global__ void __launch_bounds__(kLkwWarps * 32, 5)
-    k_lk15w_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
-  __shared__ LkArgs sa;
-  __shared__ LkwSmem sm[kLkwWarps];
-  const TrackJob &job = jobs[blockIdx.y];
-  const int s = job.stream;
-  const int n = g.wn[s];
-  if (g.wmode[s] != 0 || n < 10 || (int)blockIdx.x * kLkwWarps >= n) return;   // TrackKLT.cpp:848-852
-  if (threadIdx.x == 0) group_lk_args(sa, g, job, prm);
-  __syncthreads();
-  const int warp = threadIdx.x >> 5;
-  const int pi = blockIdx.x * kLkwWarps + warp;
-  if (pi >= n) return;
-  const size_t o = (size_t)s * g.pts_cap;
-  lk15w_body(sa, g.wpts + o, g.lk_pts1 + o, g.lk_status + o, g.lk_p0n + o, g.lk_p1n + o, pi, sm[warp]);
-}
-
-void launch_group_lk(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s) {
-  if (n_jobs <= 0) return;
-  if (prm.win == kW15 && prm.max_level + 1 <= kLk15MaxLevels) {
-    PLVIWO_CARVEOUT(k_lk15w_g);
-    k_lk15w_g<<<dim3((g.pts_cap + kLkwWarps - 1) / kLkwWarps, n_jobs), kLkwWarps * 32, 0, s>>>(g, jobs, prm);
-    return;
+  template <class Body>
+  __device__ void track(Cta &c, int pi, Body body) const {
+    const size_t o = (size_t)jobs[blockIdx.y].stream * g.pts_cap;
+    body(c.a, g.wpts + o, g.lk_pts1 + o, g.lk_status + o, g.lk_p0n + o, g.lk_p1n + o, pi);
   }
-  const int win = prm.win, np = win + 3, nd = win + 1, nw = win * win;
-  const int per_warp = ((np * np + 15) & ~15) + 2 * ((nd * nd * 2 + 15) & ~15) + 3 * ((nw * 2 + 15) & ~15);
-  const size_t smem = (size_t)per_warp * kLkWarps;
-  static SmemOptIn optin;
-  optin.ensure(k_lk_g, smem);
-  PLVIWO_CARVEOUT(k_lk_g);
-  k_lk_g<<<dim3((g.pts_cap + kLkWarps - 1) / kLkWarps, n_jobs), kLkWarps * 32, smem, s>>>(g, jobs, prm);
-}
+};
 
-// ---- stereo group: the left -> right KLT of the new left points of a rig's detection (perform_detection_stereo :658-666,
+// Stereo group: the left -> right KLT of the new left points of a rig's detection (perform_detection_stereo :658-666,
 // FeStereo's lk_launch(L.pyr, R.pyr, new0, ..., false)): previous image = the left image of the detection pair, next image =
 // its right image, initial flow = the left position, no undistortion.  The new points are the tail k_group_accept appended
 // to the left working list; the results go to the RIGHT stream's LK arrays (k_stereo_pair reads them).  grid.y = rig, on
 // the left half of the lane's jobs.
-__device__ __forceinline__ int stereo_lr_setup(LkArgs &sa, const GroupDev &g, const TrackJob *jobs, const LkParams &prm, int first_pt,
-                                               int *start) {
-  const TrackJob &lj = jobs[blockIdx.y], &rj = jobs[blockIdx.y + gridDim.y];
-  const int n = g.winfo[4 * lj.stream + 1];
-  *start = g.wn[lj.stream] - n;
-  if (first_pt < n) {
-    const bool first = g.wmode[lj.stream] == 1;
-    TrackJob j = lj;
-    j.prev_slot = first ? lj.cur_slot : lj.prev_slot;
-    j.cur_slot = first ? rj.cur_slot : rj.prev_slot;
-    group_lk_args(sa, g, j, prm);
-    sa.undistort = 0;
+struct StereoLr : GroupSrc {
+  struct Cta {
+    LkArgs a;
+    int start;   // the first new point in the left working list
+  };
+  __device__ int setup(Cta &c, int first) const {
+    const TrackJob &lj = jobs[blockIdx.y], &rj = jobs[blockIdx.y + gridDim.y];
+    const int n = g.winfo[4 * lj.stream + 1];
+    c.start = g.wn[lj.stream] - n;
+    if (first < n) {
+      const bool first_frame = g.wmode[lj.stream] == 1;
+      args(c.a, first_frame ? lj.cur_slot : lj.prev_slot, first_frame ? rj.cur_slot : rj.prev_slot, lj, 0);
+    }
+    return n;
   }
-  return n;
-}
+  template <class Body>
+  __device__ void track(Cta &c, int pi, Body body) const {
+    const size_t ol = (size_t)jobs[blockIdx.y].stream * g.pts_cap, orr = (size_t)jobs[blockIdx.y + gridDim.y].stream * g.pts_cap;
+    body(c.a, g.wpts + ol + c.start, g.lk_pts1 + orr, g.lk_status + orr, nullptr, nullptr, pi);
+  }
+};
 
-__global__ void __launch_bounds__(kLkWarps * 32)
-    k_lk_lr_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
-  __shared__ LkArgs sa;
-  __shared__ int s_n, s_start;
-  if (threadIdx.x == 0) s_n = stereo_lr_setup(sa, g, jobs, prm, (int)blockIdx.x * kLkWarps, &s_start);
+// Stream group, cfg.line_samples: the samples a handle appends to its point LK launch (fe_context.cu perform_matching),
+// grid.y = job.  Samples exist when the frame's point LK ran — the gate then wrote n_lk_in = n >= 10 into the frame's
+// header, 0 otherwise — and lie along the stream's last detected segments (lnew, n_lnew: k_group_lines of the latest frame
+// fed with vanishing points), k = 0..S-1 per segment, cut where the handle's LK buffer ends: ns = min(S * L, max_pts - n).
+// Same LK parameters and pyramids as the points, initial guess = the sample itself, no undistortion (the handle computes
+// the samples' undistorted positions and discards them).  CTAs past the job's samples read nothing but n_lnew.
+struct LineSamples : GroupSrc {
+  struct Cta {
+    LkArgs a;
+    float2 p1[kLkWarps];   // the body's result, stored to the record afterwards (no record pointer held through it)
+    uint8_t st[kLkWarps];
+  };
+  __device__ int setup(Cta &c, int first) const {
+    const TrackJob &job = jobs[blockIdx.y];
+    const long long all = (long long)g.line_samples * g.n_lnew[job.stream];
+    if (first >= all) return 0;
+    GroupOutHeader *hdr = reinterpret_cast<GroupOutHeader *>(g.out + (size_t)job.out * g.out_stride);
+    const int n = hdr->info.n_lk_in;
+    if (n < 10) return 0;
+    const int ns = (int)max(0ll, min(all, (long long)(g.sample_max_pts - n)));
+    if (blockIdx.x == 0) hdr->n_samples = ns;
+    if (first < ns) args(c.a, job.prev_slot, job.cur_slot, job, 0);
+    return ns;
+  }
+  // sample pi: a = k / (S - 1) (0.5 for S = 1) along segment pi / S, rounded as the host rounds it (no contraction)
+  template <class Body>
+  __device__ void track(Cta &c, int pi, Body body) const {
+    const TrackJob &job = jobs[blockIdx.y];
+    const int warp = threadIdx.x >> 5, S = g.line_samples, k = pi % S;
+    const float4 l = g.lnew[(size_t)job.stream * g.lines_cap + pi / S];
+    const float a = S > 1 ? (float)k / (float)(S - 1) : 0.5f;
+    const float2 p0 = make_float2(l.x + (l.z - l.x) * a, l.y + (l.w - l.y) * a);
+    body(c.a, &p0, &c.p1[warp], &c.st[warp], nullptr, nullptr, 0);
+    if ((threadIdx.x & 31) == 0) {   // the lane that wrote the result
+      uint8_t *const rec = g.out + (size_t)job.out * g.out_stride;
+      reinterpret_cast<float2 *>(rec + g.off_sp0)[pi] = p0;
+      reinterpret_cast<float2 *>(rec + g.off_sp1)[pi] = c.p1[warp];
+      rec[g.off_sst + pi] = c.st[warp];
+    }
+  }
+};
+
+template <class Src>
+__global__ void __launch_bounds__(kLkWarps * 32) k_lk_g(const __grid_constant__ Src src) {
+  __shared__ typename Src::Cta c;
+  __shared__ int s_n;
+  if (threadIdx.x == 0) s_n = src.setup(c, blockIdx.x * kLkWarps);
   __syncthreads();
   const int pi = blockIdx.x * kLkWarps + (threadIdx.x >> 5);
   if (pi >= s_n) return;
-  const size_t ol = (size_t)jobs[blockIdx.y].stream * g.pts_cap, orr = (size_t)jobs[blockIdx.y + gridDim.y].stream * g.pts_cap;
-  lk_body(sa, g.wpts + ol + s_start, g.lk_pts1 + orr, g.lk_status + orr, nullptr, nullptr, pi);
+  src.track(c, pi, [&](const LkArgs &a, const float2 *p0, float2 *p1, uint8_t *st, float2 *p0n, float2 *p1n, int i) {
+    lk_body(a, p0, p1, st, p0n, p1n, i);
+  });
 }
 
-__global__ void __launch_bounds__(kLkwWarps * 32, 5)
-    k_lk15w_lr_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
-  __shared__ LkArgs sa;
-  __shared__ LkwSmem sm[kLkwWarps];
-  __shared__ int s_n, s_start;
-  if (threadIdx.x == 0) s_n = stereo_lr_setup(sa, g, jobs, prm, (int)blockIdx.x * kLkwWarps, &s_start);
+// 5 resident CTAs per SM: 96 registers, no spills
+template <class Src>
+__global__ void __launch_bounds__(kLkWarps * 32, 5) k_lk15w_g(const __grid_constant__ Src src) {
+  __shared__ typename Src::Cta c;
+  __shared__ LkwSmem sm[kLkWarps];
+  __shared__ int s_n;
+  if (threadIdx.x == 0) s_n = src.setup(c, blockIdx.x * kLkWarps);
   __syncthreads();
   const int warp = threadIdx.x >> 5;
-  const int pi = blockIdx.x * kLkwWarps + warp;
+  const int pi = blockIdx.x * kLkWarps + warp;
   if (pi >= s_n) return;
-  const size_t ol = (size_t)jobs[blockIdx.y].stream * g.pts_cap, orr = (size_t)jobs[blockIdx.y + gridDim.y].stream * g.pts_cap;
-  lk15w_body(sa, g.wpts + ol + s_start, g.lk_pts1 + orr, g.lk_status + orr, nullptr, nullptr, pi, sm[warp]);
+  src.track(c, pi, [&](const LkArgs &a, const float2 *p0, float2 *p1, uint8_t *st, float2 *p0n, float2 *p1n, int i) {
+    lk15w_body(a, p0, p1, st, p0n, p1n, i, sm[warp]);
+  });
+}
+
+bool lk_w15_form(int win, int pyramid_images) { return win == kW15 && pyramid_images <= kLk15MaxLevels; }
+
+// src's features, at most per_job of each of n_jobs jobs: the 15 x 15 body where lk_w15_form allows it, the generic body
+// otherwise.  `images`: the pyramid images the source's LkArgs hold.
+template <class Src>
+static void launch_lk_warps(const Src &src, int win, int images, int per_job, int n_jobs, cudaStream_t s) {
+  const dim3 grid((per_job + kLkWarps - 1) / kLkWarps, n_jobs);
+  if (lk_w15_form(win, images)) {
+    PLVIWO_CARVEOUT(k_lk15w_g<Src>);
+    k_lk15w_g<Src><<<grid, kLkWarps * 32, 0, s>>>(src);
+    return;
+  }
+  const size_t smem = (size_t)LkLayout(win).per_warp * kLkWarps;
+  static SmemOptIn optin;
+  optin.ensure(k_lk_g<Src>, smem);
+  PLVIWO_CARVEOUT(k_lk_g<Src>);
+  k_lk_g<Src><<<grid, kLkWarps * 32, smem, s>>>(src);
+}
+
+void launch_group_lk(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s) {
+  if (n_jobs > 0) launch_lk_warps(GroupPoints{{g, jobs, prm}}, prm.win, prm.max_level + 1, g.pts_cap, n_jobs, s);
 }
 
 void launch_stereo_lr_lk(const GroupDev &g, const TrackJob *jobs, int n_rigs, const LkParams &prm, cudaStream_t s) {
-  if (n_rigs <= 0) return;
-  if (prm.win == kW15 && prm.max_level + 1 <= kLk15MaxLevels) {
-    PLVIWO_CARVEOUT(k_lk15w_lr_g);
-    k_lk15w_lr_g<<<dim3((g.pts_cap + kLkwWarps - 1) / kLkwWarps, n_rigs), kLkwWarps * 32, 0, s>>>(g, jobs, prm);
-    return;
-  }
-  const int win = prm.win, np = win + 3, nd = win + 1, nw = win * win;
-  const int per_warp = ((np * np + 15) & ~15) + 2 * ((nd * nd * 2 + 15) & ~15) + 3 * ((nw * 2 + 15) & ~15);
-  const size_t smem = (size_t)per_warp * kLkWarps;
-  static SmemOptIn optin;
-  optin.ensure(k_lk_lr_g, smem);
-  PLVIWO_CARVEOUT(k_lk_lr_g);
-  k_lk_lr_g<<<dim3((g.pts_cap + kLkWarps - 1) / kLkWarps, n_rigs), kLkWarps * 32, smem, s>>>(g, jobs, prm);
-}
-
-// ---- stream group, cfg.line_samples: the samples a handle appends to its point LK launch (fe_context.cu perform_matching),
-// one warp per sample, grid.y = job.  Samples exist when the frame's point LK ran — the gate then wrote n_lk_in = n >= 10
-// into the frame's header, 0 otherwise — and lie along the stream's last detected segments (lnew, n_lnew: k_group_lines of
-// the latest frame fed with vanishing points), k = 0..S-1 per segment, cut where the handle's LK buffer ends:
-// ns = min(S * L, max_pts - n).  Same LK parameters and pyramids as the points, initial guess = the sample itself.
-// Thread 0 of a CTA: the job's sample count (CTAs past it read nothing but n_lnew) and the job's LK arguments.
-__device__ __forceinline__ int group_samples_setup(LkArgs &sa, const GroupDev &g, const TrackJob &job, const LkParams &prm,
-                                                   int first) {
-  const long long all = (long long)g.line_samples * g.n_lnew[job.stream];
-  if (first >= all) return 0;
-  GroupOutHeader *hdr = reinterpret_cast<GroupOutHeader *>(g.out + (size_t)job.out * g.out_stride);
-  const int n = hdr->info.n_lk_in;
-  if (n < 10) return 0;
-  const int ns = (int)max(0ll, min(all, (long long)(g.sample_max_pts - n)));
-  if (blockIdx.x == 0) hdr->n_samples = ns;
-  if (first < ns) {
-    group_lk_args(sa, g, job, prm);
-    sa.undistort = 0;   // the handle computes the samples' undistorted positions and discards them
-  }
-  return ns;
-}
-
-// sample pi of the job: a = k / (S - 1) (0.5 for S = 1) along segment pi / S, rounded as the host rounds it (no contraction)
-__device__ __forceinline__ float2 group_sample_pos(const GroupDev &g, const TrackJob &job, int pi) {
-  const int S = g.line_samples, k = pi % S;
-  const float4 l = g.lnew[(size_t)job.stream * g.lines_cap + pi / S];
-  const float a = S > 1 ? (float)k / (float)(S - 1) : 0.5f;
-  return make_float2(l.x + (l.z - l.x) * a, l.y + (l.w - l.y) * a);
-}
-
-__global__ void __launch_bounds__(kLkwWarps * 32, 5)
-    k_lk15w_samples_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
-  __shared__ LkArgs sa;
-  __shared__ LkwSmem sm[kLkwWarps];
-  __shared__ float2 s_p1[kLkwWarps];   // the body's result, stored to the record afterwards (no record pointer held through it)
-  __shared__ uint8_t s_st[kLkwWarps];
-  __shared__ int s_ns;
-  const TrackJob &job = jobs[blockIdx.y];
-  const int warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) s_ns = group_samples_setup(sa, g, job, prm, (int)blockIdx.x * kLkwWarps);
-  __syncthreads();
-  const int pi = blockIdx.x * kLkwWarps + warp;
-  if (pi >= s_ns) return;
-  const float2 p0 = group_sample_pos(g, job, pi);
-  lk15w_body(sa, &p0, &s_p1[warp], &s_st[warp], nullptr, nullptr, 0, sm[warp]);
-  if ((threadIdx.x & 31) == 0) {   // the lane that wrote the result
-    uint8_t *const rec = g.out + (size_t)jobs[blockIdx.y].out * g.out_stride;
-    reinterpret_cast<float2 *>(rec + g.off_sp0)[pi] = p0;
-    reinterpret_cast<float2 *>(rec + g.off_sp1)[pi] = s_p1[warp];
-    rec[g.off_sst + pi] = s_st[warp];
-  }
-}
-
-__global__ void __launch_bounds__(kLkWarps * 32)
-    k_lk_samples_g(const __grid_constant__ GroupDev g, const TrackJob *__restrict__ jobs, const __grid_constant__ LkParams prm) {
-  __shared__ LkArgs sa;
-  __shared__ float2 s_p1[kLkWarps];
-  __shared__ uint8_t s_st[kLkWarps];
-  __shared__ int s_ns;
-  const TrackJob &job = jobs[blockIdx.y];
-  const int warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) s_ns = group_samples_setup(sa, g, job, prm, (int)blockIdx.x * kLkWarps);
-  __syncthreads();
-  const int pi = blockIdx.x * kLkWarps + warp;
-  if (pi >= s_ns) return;
-  const float2 p0 = group_sample_pos(g, job, pi);
-  lk_body(sa, &p0, &s_p1[warp], &s_st[warp], nullptr, nullptr, 0);
-  if ((threadIdx.x & 31) == 0) {
-    uint8_t *const rec = g.out + (size_t)jobs[blockIdx.y].out * g.out_stride;
-    reinterpret_cast<float2 *>(rec + g.off_sp0)[pi] = p0;
-    reinterpret_cast<float2 *>(rec + g.off_sp1)[pi] = s_p1[warp];
-    rec[g.off_sst + pi] = s_st[warp];
-  }
+  if (n_rigs > 0) launch_lk_warps(StereoLr{{g, jobs, prm}}, prm.win, prm.max_level + 1, g.pts_cap, n_rigs, s);
 }
 
 void launch_group_line_samples(const GroupDev &g, const TrackJob *jobs, int n_jobs, const LkParams &prm, cudaStream_t s) {
-  if (n_jobs <= 0 || g.sample_cap <= 0) return;
-  if (prm.win == kW15 && prm.max_level + 1 <= kLk15MaxLevels) {
-    PLVIWO_CARVEOUT(k_lk15w_samples_g);
-    k_lk15w_samples_g<<<dim3((g.sample_cap + kLkwWarps - 1) / kLkwWarps, n_jobs), kLkwWarps * 32, 0, s>>>(g, jobs, prm);
-    return;
-  }
-  const int win = prm.win, np = win + 3, nd = win + 1, nw = win * win;
-  const int per_warp = ((np * np + 15) & ~15) + 2 * ((nd * nd * 2 + 15) & ~15) + 3 * ((nw * 2 + 15) & ~15);
-  const size_t smem = (size_t)per_warp * kLkWarps;
-  static SmemOptIn optin;
-  optin.ensure(k_lk_samples_g, smem);
-  PLVIWO_CARVEOUT(k_lk_samples_g);
-  k_lk_samples_g<<<dim3((g.sample_cap + kLkWarps - 1) / kLkWarps, n_jobs), kLkWarps * 32, smem, s>>>(g, jobs, prm);
-}
-
-bool lk_table_mode_ok(const LkParams &prm, int pyramid_images) {
-  return prm.win == kW15 && std::min(prm.max_level + 1, pyramid_images) <= kLk15MaxLevels;
-}
-
-static LkArgs lk_args(const Pyramid &prev, const Pyramid &next, const LkParams &prm, bool flow_is_zero, const unsigned *cell_mask) {
-  LkArgs a;
-  int levels = prm.max_level + 1;
-  if (levels > prev.n) levels = prev.n;
-  for (int l = 0; l < levels; l++) {
-    a.p0[l] = prev.lvl[l].p;
-    a.p1[l] = next.lvl[l].p;
-    a.w[l] = prev.lvl[l].w;
-    a.h[l] = prev.lvl[l].h;
-    a.pitch0[l] = prev.lvl[l].pitch;
-    a.pitch1[l] = next.lvl[l].pitch;
-  }
-  a.win = prm.win;
-  a.max_level = levels - 1;
-  a.max_count = prm.max_count;
-  a.eps_sq = prm.eps_sq;
-  a.min_eig = prm.min_eig;
-  a.undistort = prm.undistort;
-  a.flow_is_zero = flow_is_zero ? 1 : 0;
-  for (int i = 0; i < 8; i++) a.cell_mask[i] = cell_mask ? cell_mask[i] : 0xffffffffu;
-  for (int i = 0; i < 4; i++) { a.calib.K[i] = prm.K[i]; a.calib.D[i] = prm.D[i]; }
-  return a;
+  if (n_jobs > 0 && g.sample_cap > 0) launch_lk_warps(LineSamples{{g, jobs, prm}}, prm.win, prm.max_level + 1, g.sample_cap, n_jobs, s);
 }
 
 bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status,
                float2 *d_p0n, float2 *d_p1n, int n, const LkParams &prm, cudaStream_t s, int *host_flag, int flag_value,
                unsigned *d_done_counter, const int *d_tab_cnt, int tab_stride, bool flow_is_zero, const unsigned *cell_mask) {
   if (n <= 0) return false;
-  const LkArgs a = lk_args(prev, next, prm, flow_is_zero, cell_mask);
-  const int levels = a.max_level + 1;
-  if (prm.win == kW15 && levels <= kLk15MaxLevels) {   // one CTA per feature, one warp per level
+  const int levels = std::min(prm.max_level + 1, prev.n);
+  LkArgs a;
+  lk_args(a, prev.lvl, next.lvl, levels, prm, prm.K, prm.D, prm.undistort, flow_is_zero ? 1 : 0, cell_mask);
+  if (lk_w15_form(prm.win, levels)) {   // one CTA per feature, one warp per level
     PLVIWO_CARVEOUT(k_lk15);
     k_lk15<<<n, std::max(levels, kChainWarps) * 32, 0, s>>>(a, d_pts0, d_pts1, d_status, d_p0n, d_p1n, n, host_flag, flag_value, d_done_counter,
                                      d_tab_cnt, tab_stride);
     return host_flag != nullptr;
   }
   if (d_tab_cnt != nullptr || flow_is_zero) return false;   // table mode exists for the 15 x 15 kernel only (caller checks)
-  const int win = prm.win, np = win + 3, nd = win + 1, nw = win * win;
-  const int per_warp = ((np * np + 15) & ~15) + 2 * ((nd * nd * 2 + 15) & ~15) + 3 * ((nw * 2 + 15) & ~15);
-  size_t smem = (size_t)per_warp * kLkWarps;
-  static SmemOptIn optin;
-  optin.ensure(k_lk, smem);
-  PLVIWO_CARVEOUT(k_lk);
-  k_lk<<<(n + kLkWarps - 1) / kLkWarps, kLkWarps * 32, smem, s>>>(a, d_pts0, d_pts1, d_status, d_p0n, d_p1n, n);
+  launch_lk_warps(LkArrays{a, d_pts0, d_pts1, d_status, d_p0n, d_p1n, n}, prm.win, levels, n, 1, s);
   return false;
 }
 
-
-// k_lk15w_g's per-feature body (one warp per feature) on arbitrary points over one image pair: lets tests reach the border
-// paths of the group kernel with points a tracker would not produce
-__global__ void __launch_bounds__(kLkwWarps * 32, 5)
-    k_lk15w(const __grid_constant__ LkArgs a, const float2 *__restrict__ pts0, float2 *__restrict__ pts1,
-            uint8_t *__restrict__ status, int n) {
-  __shared__ LkwSmem sm[kLkwWarps];
-  const int pi = blockIdx.x * kLkwWarps + (threadIdx.x >> 5);
-  if (pi >= n) return;
-  lk15w_body(a, pts0, pts1, status, nullptr, nullptr, pi, sm[threadIdx.x >> 5]);
-}
-
+// k_lk15w_g on arbitrary points over one image pair: lets tests reach the border paths of the group kernel with points a
+// tracker would not produce
 bool launch_lk_warp(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status, int n,
                     const LkParams &prm, cudaStream_t s) {
-  if (prm.win != kW15 || std::min(prm.max_level + 1, prev.n) > kLk15MaxLevels || prm.undistort) return false;
+  const int levels = std::min(prm.max_level + 1, prev.n);
+  if (!lk_w15_form(prm.win, levels) || prm.undistort) return false;
   if (n <= 0) return true;
-  const LkArgs a = lk_args(prev, next, prm, false, nullptr);
-  PLVIWO_CARVEOUT(k_lk15w);
-  k_lk15w<<<(n + kLkwWarps - 1) / kLkwWarps, kLkwWarps * 32, 0, s>>>(a, d_pts0, d_pts1, d_status, n);
+  LkArgs a;
+  lk_args(a, prev.lvl, next.lvl, levels, prm, prm.K, prm.D, 0, 0, nullptr);
+  launch_lk_warps(LkArrays{a, d_pts0, d_pts1, d_status, nullptr, nullptr, n}, prm.win, levels, n, 1, s);
   return true;
 }
 

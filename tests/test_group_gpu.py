@@ -16,6 +16,7 @@ CFG1 = dict(num_features=200, fast_threshold=20, grid_x=5, grid_y=5, min_px_dist
 CFG2 = dict(num_features=400, fast_threshold=20, grid_x=5, grid_y=5, min_px_dist=10, pyr_levels=4, win_size=15)
 CFG_KAIST = dict(num_features=1500, fast_threshold=30, grid_x=15, grid_y=15, min_px_dist=15, pyr_levels=5, win_size=15)
 CFG4 = dict(num_features=1000, fast_threshold=20, grid_x=10, grid_y=6, min_px_dist=15, pyr_levels=5, win_size=21)
+CFG_DEEP = dict(CFG_KAIST, pyr_levels=6)   # at 1280 x 560 the pyramid stops at 6 images (40 x 18): the 15 x 15 bodies
 
 
 def _single_rows(fe, seq, kw, n_frames, W, H, lines=True, masks=False, hist=1):
@@ -74,8 +75,9 @@ def test_group_equals_single_handles(fe, synth, kw, lookahead, n_streams):
 
 
 def test_group_kaist_yaml_and_wide_window(fe, synth):
-    """KAIST yaml (1500 points, 15 x 15 grid) and config 4 (1920 x 1080, 21 x 21 window: the generic LK kernel)."""
-    for kw, W, H, n_frames in ((CFG_KAIST, 1280, 560, 8), (CFG4, 1920, 1080, 6)):
+    """KAIST yaml (1500 points, 15 x 15 grid), config 4 (1920 x 1080, 21 x 21 window: the generic LK kernel) and pyr_levels
+    6 at 1280 x 560 (a pyramid of 6 images: the 15 x 15 kernels, as in a handle)."""
+    for kw, W, H, n_frames in ((CFG_KAIST, 1280, 560, 8), (CFG4, 1920, 1080, 6), (CFG_DEEP, 1280, 560, 8)):
         seqs = [synth.SynthSequence(seed=1010 + s, width=W, height=H, n_frames=n_frames) for s in range(2)]
         ref = [_single_rows(fe, q, kw, n_frames, W, H) for q in seqs]
         g = fe.GroupFrontEnd(fe.default_config(width=W, height=H, lookahead=2, **kw), 2, calibs=[(q.K, q.D) for q in seqs])

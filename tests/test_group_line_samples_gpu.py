@@ -119,14 +119,16 @@ def test_group_line_samples_cut_at_the_lk_buffer(fe, synth):
         assert 200 * n_seg > max_pts - n_pts and len(ref[t]["su"]) == max_pts - n_pts, (t, n_pts, n_seg, len(ref[t]["su"]))
 
 
-@pytest.mark.parametrize("line_samples,win", [(1, 15), (2, 15), (3, 21)])
-def test_group_line_samples_per_segment_and_window(fe, synth, line_samples, win):
-    """S = 1 (a = 0.5), S = 2 (the end points) and a 21 x 21 window (the generic LK kernel), 2 streams, 2 ticks ahead."""
+@pytest.mark.parametrize("line_samples,win,pyr_levels", [(1, 15, 3), (2, 15, 3), (3, 21, 3), (3, 15, 6)],
+                         ids=["1-15", "2-15", "3-21", "3-15-6"])
+def test_group_line_samples_per_segment_and_window(fe, synth, line_samples, win, pyr_levels):
+    """S = 1 (a = 0.5), S = 2 (the end points), a 21 x 21 window (the generic LK kernel) and pyr_levels 6 (a pyramid of 6
+    images at 1280 x 560: the 15 x 15 kernels, as in a handle), 2 streams, 2 ticks ahead."""
     n = 8
     seqs = [synth.SynthSequence(seed=1050 + s, width=W, height=H, n_frames=n) for s in range(2)]
     frames = [[q.frame(t) for t in range(n)] for q in seqs]
     vps = [[q.vanishing_points(t) for q in seqs] for t in range(n)]
-    ref = _run(fe, seqs, dict(CFG1, win_size=win, line_samples=line_samples), frames, vps, 2)
+    ref = _run(fe, seqs, dict(CFG1, win_size=win, pyr_levels=pyr_levels, line_samples=line_samples), frames, vps, 2)
     assert all(len(ref[s][t]["su"]) > 0 for s in range(2) for t in range(1, n))
 
 

@@ -19,6 +19,7 @@ CFG1 = dict(num_features=200, fast_threshold=20, grid_x=5, grid_y=5, min_px_dist
 CFG2 = dict(num_features=400, fast_threshold=20, grid_x=5, grid_y=5, min_px_dist=10, pyr_levels=4, win_size=15)
 CFG_KAIST = dict(num_features=1500, fast_threshold=30, grid_x=15, grid_y=15, min_px_dist=15, pyr_levels=5, win_size=15)
 CFG4 = dict(num_features=1000, fast_threshold=20, grid_x=10, grid_y=6, min_px_dist=15, pyr_levels=5, win_size=21)
+CFG_DEEP = dict(CFG_KAIST, pyr_levels=6)   # at 1280 x 560 the pyramid stops at 6 images (40 x 18): the 15 x 15 bodies
 
 
 def _info_bytes(info):
@@ -118,9 +119,10 @@ def test_stereo_group_equals_stereo_handles(fe, synth, lookahead):
     assert sum(len(x["lr"]) for r in ref for x in r if x) > 30
 
 
-@pytest.mark.parametrize("kw,W,H,n", [(CFG_KAIST, 1280, 560, 6), (CFG4, 1920, 1080, 5)])
+@pytest.mark.parametrize("kw,W,H,n", [(CFG_KAIST, 1280, 560, 6), (CFG4, 1920, 1080, 5), (CFG_DEEP, 1280, 560, 6)])
 def test_stereo_group_kaist_yaml_and_wide_window(fe, synth, kw, W, H, n):
-    """KAIST yaml knobs (1500 points, 15 x 15 grid) and config 4 (1920 x 1080, 21 x 21 window: the generic LK kernel)."""
+    """KAIST yaml knobs (1500 points, 15 x 15 grid), config 4 (1920 x 1080, 21 x 21 window: the generic LK kernel) and
+    pyr_levels 6 at 1280 x 560 (a pyramid of 6 images: the 15 x 15 kernels, as in a handle)."""
     _run_group(fe, synth, kw, 2, n, W=W, H=H, seed0=2100)
 
 
