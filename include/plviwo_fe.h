@@ -78,7 +78,7 @@ typedef struct FeConfig {
                                 /* image and mask to (width/2, height/2) before tracking; width/height above are the    */
                                 /* INPUT size, K is the (already halved, OptionsCamera.cpp:123-126) tracking calibration */
   double K[4];                  /* fx fy cx cy                                                          */
-  double D[4];                  /* radtan k1 k2 p1 p2                                                   */
+  double D[4];                  /* radtan k1 k2 p1 p2, or equidistant k1 k2 k3 k4 (the handle's camera model) */
 } FeConfig;
 
 /* One FeatureDatabase::update_feature call (TrackKLT.cpp:176-179). */
@@ -151,16 +151,21 @@ typedef struct FeStageTimes {
 int plviwo_fe_abi_version(void);
 void plviwo_fe_default_config(FeConfig *cfg);                 /* reference defaults, KAIST cam0 calibration */
 int plviwo_fe_device_count(int *n);
-int plviwo_fe_create(const FeConfig *cfg, int device, FeHandle **out);
+int plviwo_fe_create(const FeConfig *cfg, int device, FeHandle **out);   /* = _create_model with FE_CAM_RADTAN */
+/* Camera models: the ov_core::CamBase subclasses (cam/CamRadtan.h, cam/CamEqui.h).  A CamBase object's class is chosen when
+ * the camera is built and never changes (the estimator refines K and D only, StateHelper.cpp:166), so the model is fixed when
+ * a handle, rig or group is created.  FE_CAM_EQUI undistorts as CamEqui::undistort_f (cv::fisheye::undistortPoints,
+ * cam/CamEqui.h:108-129) with D = k1 k2 k3 k4.  Any other value is FE_BAD_ARG. */
+enum FeCameraModel { FE_CAM_RADTAN = 0, FE_CAM_EQUI = 1 };
+int plviwo_fe_create_model(const FeConfig *cfg, int model, int device, FeHandle **out);
 int plviwo_fe_destroy(FeHandle *h);
 const char *plviwo_fe_last_error(const FeHandle *h);          /* h may be NULL: last create() error         */
 
 /* ---- per-frame ---------------------------------------------------------------------------------------- */
 /* Intrinsics are refined online by the estimator (StateHelper.cpp:166): call before feed whenever they change. */
 int plviwo_fe_set_calib(FeHandle *h, const double K[4], const double D[4]);
-/* The same with the camera model named (ov_core::CamBase subclasses, cam/CamRadtan.h / cam/CamEqui.h).  Only the radtan
- * model is implemented: FE_CAM_EQUI is rejected with FE_BAD_ARG instead of being undistorted with the wrong formula. */
-enum FeCameraModel { FE_CAM_RADTAN = 0, FE_CAM_EQUI = 1 };
+/* The same with the camera model named (ov_core::CamBase subclasses, cam/CamRadtan.h / cam/CamEqui.h): the model the handle
+ * was created with updates K / D, any other model is FE_BAD_ARG (the model is fixed at creation). */
 int plviwo_fe_set_camera(FeHandle *h, int model, const double K[4], const double D[4]);
 /* TrackBase::currid (TrackBase.h:192) is one counter per tracker object, shared by all its cameras: a caller that owns
  * several handles hands the counter from handle to handle around every feed (between frames only). */
@@ -266,11 +271,14 @@ typedef struct FeStereoInfo {
 } FeStereoInfo;
 
 int plviwo_fe_stereo_create(const FeConfig *cfg, const double K_right[4], const double D_right[4], int device,
-                            FeStereoHandle **out);
+                            FeStereoHandle **out);   /* = _create_model with FE_CAM_RADTAN */
+/* one camera model for both cameras of the rig (FeCameraModel) */
+int plviwo_fe_stereo_create_model(const FeConfig *cfg, int model, const double K_right[4], const double D_right[4], int device,
+                                  FeStereoHandle **out);
 int plviwo_fe_stereo_destroy(FeStereoHandle *h);
 const char *plviwo_fe_stereo_last_error(const FeStereoHandle *h);
 int plviwo_fe_stereo_set_calib(FeStereoHandle *h, int cam, const double K[4], const double D[4]);
-int plviwo_fe_stereo_set_camera(FeStereoHandle *h, int cam, int model, const double K[4], const double D[4]);
+int plviwo_fe_stereo_set_camera(FeStereoHandle *h, int cam, int model, const double K[4], const double D[4]);   /* model: the rig's */
 int plviwo_fe_stereo_set_num_features(FeStereoHandle *h, int num_features);
 int plviwo_fe_stereo_change_feat_id(FeStereoHandle *h, uint64_t id_old, uint64_t id_new);
 /* Synchronous drop-in for feed_new_camera with two images (HOST buffers, 8UC1, same stride; masks may be NULL). */
@@ -325,12 +333,14 @@ typedef struct FeGroupTimes {
   uint64_t fast_cells;       /* grid cells FAST ran on (the valid cells of the detections, Grider_GRID.h:108-125)  */
 } FeGroupTimes;
 
-int plviwo_fe_group_create(const FeConfig *cfg, int n_streams, int device, FeGroupHandle **out);
+int plviwo_fe_group_create(const FeConfig *cfg, int n_streams, int device, FeGroupHandle **out);   /* FE_CAM_RADTAN */
+/* one camera model for every stream of the group (FeCameraModel) */
+int plviwo_fe_group_create_model(const FeConfig *cfg, int n_streams, int model, int device, FeGroupHandle **out);
 int plviwo_fe_group_destroy(FeGroupHandle *g);
 const char *plviwo_fe_group_last_error(const FeGroupHandle *g);
 int plviwo_fe_group_set_calib(FeGroupHandle *g, int stream, const double K[4], const double D[4]);
 /* as plviwo_fe_set_camera (CamBase::camera_k_OPENCV / camera_d_OPENCV + the model of the CamBase subclass, cam/CamBase.h:47-60):
- * FE_CAM_EQUI is refused with FE_BAD_ARG */
+ * a model other than the group's is refused with FE_BAD_ARG */
 int plviwo_fe_group_set_camera(FeGroupHandle *g, int stream, int model, const double K[4], const double D[4]);
 /* One tick: images[s] = frame of stream s (host or device pointer, NULL: no frame for that stream), timestamps[s] its
  * time; masks = NULL or per-stream host pointers (NULL entries allowed); vps = NULL (line tracker not fed) or 6 doubles per
@@ -374,6 +384,8 @@ int plviwo_fe_group_get_times(FeGroupHandle *g, FeGroupTimes *out, int reset);
  * Not supported: cfg->downsample, cfg->line_samples (refused at creation), set_num_features / change_feat_id, taps, timing. */
 typedef struct FeStereoGroupHandle FeStereoGroupHandle;
 int plviwo_fe_stereo_group_create(const FeConfig *cfg, int n_rigs /* [1, 2048] */, int device, FeStereoGroupHandle **out);
+/* one camera model for every camera of every rig (FeCameraModel); the _create form above uses FE_CAM_RADTAN */
+int plviwo_fe_stereo_group_create_model(const FeConfig *cfg, int n_rigs, int model, int device, FeStereoGroupHandle **out);
 int plviwo_fe_stereo_group_destroy(FeStereoGroupHandle *g);
 const char *plviwo_fe_stereo_group_last_error(const FeStereoGroupHandle *g);   /* g may be NULL: last create() error */
 int plviwo_fe_stereo_group_set_calib(FeStereoGroupHandle *g, int rig, int cam, const double K[4], const double D[4]);
@@ -409,6 +421,9 @@ int plviwo_op_lk(int device, const uint8_t *img0, const uint8_t *img1, int w, in
 int plviwo_op_lk_warp(int device, const uint8_t *img0, const uint8_t *img1, int w, int h, int win, int max_level,
                       const float *pts0, float *pts1 /* in: initial flow, out */, uint8_t *status, int n);
 int plviwo_op_undistort(int device, const float *pts, int n, const double K[4], const double D[4], float *out);
+/* cv::fisheye::undistortPoints (FE_CAM_EQUI, D = k1 k2 k3 k4) of n points (2 floats each).  device < 0: the host instantiation
+ * of the same arithmetic (the handle's line rows use it); device >= 0: the kernel. */
+int plviwo_op_undistort_equi(int device, const float *pts, int n, const double K[4], const double D[4], float *out);
 int plviwo_op_canny_half(int device, const uint8_t *img, int w, int h, float th, uint8_t *edges /* w*h bytes */);
 /* Connected components (8-connected) of every 64 x 16 tile of a bit-packed edge map on its own, as the line detector's first
    labelling step computes them.  edge_words: (w + 31) / 32 words per row, bit x % 32 of word x / 32 = pixel x.  For every

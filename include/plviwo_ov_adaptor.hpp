@@ -22,6 +22,7 @@
 #include <vector>
 
 #include "cam/CamBase.h"
+#include "cam/CamEqui.h"
 #include "cam/CamRadtan.h"
 #include "feat/FeatureDatabase.h"
 #include "plviwo_fe.h"
@@ -81,8 +82,8 @@ class TrackB200 : public ov_core::TrackBase {
     if (it != handles_.end()) return it->second;
     FeConfig cfg = make_config(img);
     FeHandle *h = nullptr;
-    if (plviwo_fe_create(&cfg, device_, &h) != FE_OK)
-      throw std::runtime_error(std::string("plviwo_fe_create: ") + plviwo_fe_last_error(nullptr));
+    if (plviwo_fe_create_model(&cfg, camera_model(cam_id), device_, &h) != FE_OK)
+      throw std::runtime_error(std::string("plviwo_fe_create_model: ") + plviwo_fe_last_error(nullptr));
     handles_[cam_id] = h;
     return h;
   }
@@ -103,22 +104,26 @@ class TrackB200 : public ov_core::TrackBase {
     return cfg;
   }
   int numaruco_of_currid() const { return (int)((currid.load() - 1) / 4); }   // TrackBase.cpp:34: currid = 4 * numaruco + 1
-  // only the radtan model is implemented: any other CamBase subclass (cam/CamEqui.h) is refused, not mis-undistorted
-  void require_radtan(size_t cam_id) const {
-    if (!std::dynamic_pointer_cast<ov_core::CamRadtan>(camera_calib.at(cam_id)))
-      throw std::invalid_argument("plviwo::TrackB200: camera " + std::to_string(cam_id) + " is not an ov_core::CamRadtan (only radtan is implemented)");
+  // the FeCameraModel of a camera's CamBase subclass (fixed for the camera's lifetime); any other subclass is refused, not
+  // undistorted with the wrong formula
+  int camera_model(size_t cam_id) const {
+    const std::shared_ptr<ov_core::CamBase> &cam = camera_calib.at(cam_id);
+    if (std::dynamic_pointer_cast<ov_core::CamRadtan>(cam)) return FE_CAM_RADTAN;
+    if (std::dynamic_pointer_cast<ov_core::CamEqui>(cam)) return FE_CAM_EQUI;
+    throw std::invalid_argument("plviwo::TrackB200: camera " + std::to_string(cam_id) +
+                                " is neither an ov_core::CamRadtan nor an ov_core::CamEqui");
   }
 
   void feed_monocular(const ov_core::CameraData &message, size_t msg_id) {
     const size_t cam_id = (size_t)message.sensor_ids.at(msg_id);
     const cv::Mat &img = message.images.at(msg_id);
     const cv::Mat &mask = message.masks.at(msg_id);
-    require_radtan(cam_id);
+    const int model = camera_model(cam_id);
     FeHandle *h = handle_for(cam_id, img);
     // intrinsics are refined online (StateHelper.cpp:166): hand over the current values every frame
     const Eigen::MatrixXd calib = camera_calib.at(cam_id)->get_value();
     const double K[4] = {calib(0), calib(1), calib(2), calib(3)}, D[4] = {calib(4), calib(5), calib(6), calib(7)};
-    if (plviwo_fe_set_camera(h, FE_CAM_RADTAN, K, D) != FE_OK) throw std::runtime_error(std::string("plviwo_fe_set_camera: ") + plviwo_fe_last_error(h));
+    if (plviwo_fe_set_camera(h, model, K, D) != FE_OK) throw std::runtime_error(std::string("plviwo_fe_set_camera: ") + plviwo_fe_last_error(h));
     int &last_nf = last_num_features_[cam_id];   // per handle: every camera's handle follows set_num_features
     if (num_features != last_nf) {
       if (plviwo_fe_set_num_features(h, num_features) != FE_OK)
@@ -169,6 +174,10 @@ class TrackB200 : public ov_core::TrackBase {
     const cv::Mat *mask[2] = {&message.masks.at(msg_id_left), &message.masks.at(msg_id_right)};
     if (img[0]->cols != img[1]->cols || img[0]->rows != img[1]->rows || img[0]->step != img[1]->step)
       throw std::invalid_argument("plviwo::TrackB200: stereo images must have the same size and step");
+    // one camera model per rig
+    const int model = camera_model(cam[0]);
+    if (camera_model(cam[1]) != model)
+      throw std::invalid_argument("plviwo::TrackB200: the two cameras of a stereo pair must have the same camera model");
     double K[2][4], D[2][4];
     for (int c = 0; c < 2; c++) {
       const Eigen::MatrixXd calib = camera_calib.at(cam[c])->get_value();
@@ -183,13 +192,12 @@ class TrackB200 : public ov_core::TrackBase {
         cfg.K[i] = K[0][i];
         cfg.D[i] = D[0][i];
       }
-      if (plviwo_fe_stereo_create(&cfg, K[1], D[1], device_, &stereo_) != FE_OK)
-        throw std::runtime_error(std::string("plviwo_fe_stereo_create: ") + plviwo_fe_stereo_last_error(nullptr));
+      if (plviwo_fe_stereo_create_model(&cfg, model, K[1], D[1], device_, &stereo_) != FE_OK)
+        throw std::runtime_error(std::string("plviwo_fe_stereo_create_model: ") + plviwo_fe_stereo_last_error(nullptr));
     }
-    for (int c = 0; c < 2; c++) {
-      require_radtan(cam[c]);
-      plviwo_fe_stereo_set_camera(stereo_, c, FE_CAM_RADTAN, K[c], D[c]);
-    }
+    for (int c = 0; c < 2; c++)
+      if (plviwo_fe_stereo_set_camera(stereo_, c, model, K[c], D[c]) != FE_OK)
+        throw std::runtime_error(std::string("plviwo_fe_stereo_set_camera: ") + plviwo_fe_stereo_last_error(stereo_));
     if (num_features != last_num_features_stereo_) {
       if (plviwo_fe_stereo_set_num_features(stereo_, num_features) != FE_OK)
         throw std::runtime_error(std::string("plviwo_fe_stereo_set_num_features: ") + plviwo_fe_stereo_last_error(stereo_));

@@ -22,6 +22,9 @@ LIB_PATH = os.path.join(_HERE, "libplviwo_fe.so")
 
 FE_OK, FE_BAD_ARG, FE_NO_DEVICE, FE_CUDA_ERROR, FE_OVERFLOW, FE_INTERNAL = range(6)
 HIST_NONE, HIST_HISTOGRAM, HIST_CLAHE = 0, 1, 2
+# camera models (FeCameraModel): ov_core's CamRadtan and CamEqui, fixed when a front end is created
+CAM_RADTAN, CAM_EQUI = 0, 1
+FE_CAM_RADTAN, FE_CAM_EQUI = CAM_RADTAN, CAM_EQUI
 _STATUS = {0: "FE_OK", 1: "FE_BAD_ARG", 2: "FE_NO_DEVICE", 3: "FE_CUDA_ERROR", 4: "FE_OVERFLOW", 5: "FE_INTERNAL"}
 HOST_STAGES = ["submit", "detection", "matching", "ransac", "lines", "collect", "line_wait", "predet_wait",
                "speculate", "assemble", "line_assign", "spec_launch", "lk_launch", "lk_wait", "line_match", "line_rows"]
@@ -126,6 +129,8 @@ EXPORTS = [
     "plviwo_fe_group_get_times", "plviwo_fe_set_camera", "plviwo_fe_get_currid", "plviwo_fe_set_currid",
     "plviwo_fe_stereo_set_camera",
     "plviwo_fe_stereo_group_create", "plviwo_fe_stereo_group_destroy", "plviwo_fe_stereo_group_last_error", "plviwo_fe_stereo_group_set_calib", "plviwo_fe_stereo_group_set_camera", "plviwo_fe_stereo_group_submit",
+    "plviwo_fe_create_model", "plviwo_fe_stereo_create_model", "plviwo_fe_group_create_model", "plviwo_fe_stereo_group_create_model",
+    "plviwo_op_undistort_equi",
     "plviwo_fe_stereo_group_collect", "plviwo_fe_stereo_group_play", "plviwo_fe_stereo_group_get_point_rows", "plviwo_fe_stereo_group_get_last_obs", "plviwo_fe_stereo_group_get_line_rows", "plviwo_fe_stereo_group_get_line_points", "plviwo_fe_stereo_group_get_state", "plviwo_fe_stereo_group_set_state",
 ]
 
@@ -141,6 +146,13 @@ def lib() -> C.CDLL:
         L.plviwo_fe_last_error.restype = C.c_char_p
         L.plviwo_fe_last_error.argtypes = [C.c_void_p]
         L.plviwo_fe_create.argtypes = [C.POINTER(FeConfig), C.c_int, C.POINTER(C.c_void_p)]
+        L.plviwo_fe_create_model.argtypes = [C.POINTER(FeConfig), C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        L.plviwo_fe_stereo_create_model.argtypes = [C.POINTER(FeConfig), C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double),
+                                                    C.c_int, C.POINTER(C.c_void_p)]
+        L.plviwo_fe_group_create_model.argtypes = [C.POINTER(FeConfig), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        L.plviwo_fe_stereo_group_create_model.argtypes = [C.POINTER(FeConfig), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        L.plviwo_op_undistort_equi.argtypes = [C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double),
+                                               C.c_void_p]
         L.plviwo_fe_destroy.argtypes = [C.c_void_p]
         L.plviwo_fe_set_calib.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double)]
         L.plviwo_fe_set_camera.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]
@@ -365,11 +377,13 @@ class LineFeatureDatabase:
 class FrontEnd:
     """One camera stream: TrackKLT + TrackLSD behind one FeHandle."""
 
-    def __init__(self, cfg: Optional[FeConfig] = None, device: int = 0, **kw):
+    def __init__(self, cfg: Optional[FeConfig] = None, device: int = 0, camera_model: int = CAM_RADTAN, **kw):
+        """camera_model: CAM_RADTAN or CAM_EQUI (cfg.D = k1 k2 k3 k4), fixed for the handle's lifetime."""
         self.cfg = cfg if cfg is not None else default_config(**kw)
+        self.camera_model = camera_model
         self._h = C.c_void_p()
         self._lib = lib()
-        _check(self._lib.plviwo_fe_create(C.byref(self.cfg), device, C.byref(self._h)))
+        _check(self._lib.plviwo_fe_create_model(C.byref(self.cfg), camera_model, device, C.byref(self._h)))
         self.database = FeatureDatabase()
         self.line_database = LineFeatureDatabase()
         self.cam_id = 0
@@ -394,7 +408,7 @@ class FrontEnd:
         _check(self._lib.plviwo_fe_set_num_features(self._h, n), self._h)
 
     def set_camera(self, model: int, K: Sequence[float], D: Sequence[float]):
-        """CamBase model + calibration (0 radtan, 1 equidistant: rejected, not implemented)."""
+        """CamBase model + calibration: the model the handle was created with updates K / D, any other is refused."""
         _check(self._lib.plviwo_fe_set_camera(self._h, model, (C.c_double * 4)(*K), (C.c_double * 4)(*D)), self._h)
 
     def get_currid(self) -> int:
@@ -579,12 +593,14 @@ class GroupFrontEnd:
     """Many camera streams of one device behind one FeGroupHandle (BASELINE.json configs[4]): stream s is one TrackKLT + one
     TrackLSD; a tick feeds one frame of every stream."""
 
-    def __init__(self, cfg: FeConfig, n_streams: int, device: int = 0, calibs=None):
+    def __init__(self, cfg: FeConfig, n_streams: int, device: int = 0, calibs=None, camera_model: int = CAM_RADTAN):
+        """camera_model: CAM_RADTAN or CAM_EQUI, one model for every stream, fixed for the group's lifetime."""
         self.cfg = cfg
         self.n = int(n_streams)
+        self.camera_model = camera_model
         self._h = C.c_void_p()
         self._lib = lib()
-        rc = self._lib.plviwo_fe_group_create(C.byref(cfg), self.n, device, C.byref(self._h))
+        rc = self._lib.plviwo_fe_group_create_model(C.byref(cfg), self.n, camera_model, device, C.byref(self._h))
         if rc != FE_OK:
             raise FrontEndError(rc, (self._lib.plviwo_fe_group_last_error(None) or b"").decode())
         self.infos = (FeFrameInfo * self.n)()
@@ -611,7 +627,7 @@ class GroupFrontEnd:
         self._check(self._lib.plviwo_fe_group_set_calib(self._h, stream, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
 
     def set_camera(self, stream: int, model: int, K, D):
-        """Calibration with the camera model stated (0 radtan, 1 equidistant: refused, cam/CamEqui.h is not implemented)."""
+        """Calibration with the camera model stated: the group's model updates K / D, any other is refused."""
         self._check(self._lib.plviwo_fe_group_set_camera(self._h, stream, model, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
 
     def submit(self, timestamps, images, stride: int = 0, on_device: bool = False, vanishing_points=None, masks=None):
@@ -736,13 +752,15 @@ class StereoGroupFrontEnd:
     """Many stereo rigs of one device behind one FeStereoGroupHandle: rig r is what one StereoFrontEnd is (same rows, bit for
     bit); a tick feeds one stereo pair of every rig.  Cameras: 0 left, 1 right."""
 
-    def __init__(self, cfg: FeConfig, n_rigs: int, device: int = 0, calibs=None):
-        """calibs: per rig ((K_left, D_left), (K_right, D_right)), or None (cfg.K / cfg.D for every camera)."""
+    def __init__(self, cfg: FeConfig, n_rigs: int, device: int = 0, calibs=None, camera_model: int = CAM_RADTAN):
+        """calibs: per rig ((K_left, D_left), (K_right, D_right)), or None (cfg.K / cfg.D for every camera).  camera_model:
+        CAM_RADTAN or CAM_EQUI, one model for every camera, fixed for the group's lifetime."""
         self.cfg = cfg
         self.n = int(n_rigs)
+        self.camera_model = camera_model
         self._h = C.c_void_p()
         self._lib = lib()
-        rc = self._lib.plviwo_fe_stereo_group_create(C.byref(cfg), self.n, device, C.byref(self._h))
+        rc = self._lib.plviwo_fe_stereo_group_create_model(C.byref(cfg), self.n, camera_model, device, C.byref(self._h))
         if rc != FE_OK:
             raise FrontEndError(rc, (self._lib.plviwo_fe_stereo_group_last_error(None) or b"").decode())
         self.infos = (FeStereoInfo * self.n)()
@@ -770,7 +788,7 @@ class StereoGroupFrontEnd:
         self._check(self._lib.plviwo_fe_stereo_group_set_calib(self._h, rig, cam, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
 
     def set_camera(self, rig: int, cam: int, model: int, K, D):
-        """Calibration with the camera model stated (0 radtan, 1 equidistant: refused, cam/CamEqui.h is not implemented)."""
+        """Calibration with the camera model stated: the group's model updates K / D, any other is refused."""
         self._check(self._lib.plviwo_fe_stereo_group_set_camera(self._h, rig, cam, model, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
 
     def _ptrs(self, arrays, keep, on_device=False):
@@ -918,13 +936,16 @@ _STATE_HDR = np.dtype([("magic", "<u4"), ("version", "<u4"), ("w", "<i4"), ("h",
 class StereoFrontEnd:
     """One stereo rig: ov_core::TrackKLT with use_stereo = true behind one FeStereoHandle (camera 0 = left, 1 = right)."""
 
-    def __init__(self, cfg: Optional[FeConfig] = None, K_right=None, D_right=None, device: int = 0, **kw):
+    def __init__(self, cfg: Optional[FeConfig] = None, K_right=None, D_right=None, device: int = 0, camera_model: int = CAM_RADTAN,
+                 **kw):
+        """camera_model: CAM_RADTAN or CAM_EQUI for both cameras, fixed for the rig's lifetime."""
         self.cfg = cfg if cfg is not None else default_config(**kw)
+        self.camera_model = camera_model
         self._h = C.c_void_p()
         self._lib = lib()
         kr = None if K_right is None else (C.c_double * 4)(*K_right)
         dr = None if D_right is None else (C.c_double * 4)(*D_right)
-        rc = self._lib.plviwo_fe_stereo_create(C.byref(self.cfg), kr, dr, device, C.byref(self._h))
+        rc = self._lib.plviwo_fe_stereo_create_model(C.byref(self.cfg), camera_model, kr, dr, device, C.byref(self._h))
         if rc != FE_OK:
             raise FrontEndError(rc, (self._lib.plviwo_fe_stereo_last_error(None) or b"").decode())
         self.database = FeatureDatabase()      # one database shared by both cameras (UpdaterCamera.cpp:47-56)
@@ -948,6 +969,10 @@ class StereoFrontEnd:
 
     def set_calib(self, cam: int, K, D):
         self._check(self._lib.plviwo_fe_stereo_set_calib(self._h, cam, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
+
+    def set_camera(self, cam: int, model: int, K, D):
+        """Calibration with the camera model stated: the rig's model updates K / D, any other is refused."""
+        self._check(self._lib.plviwo_fe_stereo_set_camera(self._h, cam, model, (C.c_double * 4)(*K), (C.c_double * 4)(*D)))
 
     def set_num_features(self, n: int):
         self._check(self._lib.plviwo_fe_stereo_set_num_features(self._h, n))
@@ -1230,6 +1255,14 @@ def op_undistort(pts, K, D, device: int = 0) -> np.ndarray:
     p = np.ascontiguousarray(pts, np.float32).reshape(-1, 2)
     out = np.zeros_like(p)
     _check(lib().plviwo_op_undistort(device, p.ctypes.data, len(p), (C.c_double * 4)(*K), (C.c_double * 4)(*D), out.ctypes.data))
+    return out
+
+
+def op_undistort_equi(pts, K, D, device: int = 0) -> np.ndarray:
+    """cv::fisheye::undistortPoints of (n, 2) points; device < 0 runs the host instantiation of the same arithmetic."""
+    p = np.ascontiguousarray(pts, np.float32).reshape(-1, 2)
+    out = np.zeros_like(p)
+    _check(lib().plviwo_op_undistort_equi(device, p.ctypes.data, len(p), (C.c_double * 4)(*K), (C.c_double * 4)(*D), out.ctypes.data))
     return out
 
 

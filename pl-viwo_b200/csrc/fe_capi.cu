@@ -70,6 +70,18 @@ static const char *check_config(const FeConfig &c, int tw, int th) {
   return nullptr;
 }
 
+// The camera model of a creator (FeCameraModel): nullptr when it is one the library implements, otherwise the reason.
+static const char *check_model(int model) {
+  if (model != FE_CAM_RADTAN && model != FE_CAM_EQUI) return "camera model must be FE_CAM_RADTAN (0) or FE_CAM_EQUI (1)";
+  return nullptr;
+}
+static const char *model_name(int model) { return model == FE_CAM_EQUI ? "equidistant" : "radtan"; }
+// set_camera's refusal of a model other than the one the object was created with (a CamBase keeps its class for life)
+static std::string model_mismatch(int created) {
+  return std::string("set_camera: created with the ") + model_name(created) +
+         " model; the model is fixed at creation (use the _create_model functions to pick it)";
+}
+
 // After the config checks: the device a creator is asked for exists.
 static int check_device(int device) {
   int ndev = 0;
@@ -135,14 +147,19 @@ int plviwo_fe_device_count(int *n) {
 }
 
 int plviwo_fe_create(const FeConfig *cfg, int device, FeHandle **out) {
+  return plviwo_fe_create_model(cfg, FE_CAM_RADTAN, device, out);
+}
+
+int plviwo_fe_create_model(const FeConfig *cfg, int model, int device, FeHandle **out) {
   API_BEGIN
   if (!cfg || !out) return FE_BAD_ARG;
   *out = nullptr;
+  if (const char *why = check_model(model)) return create_error(FE_BAD_ARG, why);
   const int tw = cfg->downsample ? (int)(cfg->width / 2.0) : cfg->width, th = cfg->downsample ? (int)(cfg->height / 2.0) : cfg->height;
   if (cfg->downsample && (tw < 64 || th < 64)) return create_error(FE_BAD_ARG, "downsampled image would be smaller than 64 pixels");
   if (const char *why = check_config(*cfg, tw, th)) return create_error(FE_BAD_ARG, why);
   if (int rc = check_device(device)) return rc;
-  FeContext *ctx = new FeContext(*cfg, device);
+  FeContext *ctx = new FeContext(*cfg, device, model);
   int rc = ctx->init();
   if (rc != FE_OK) {
     g_create_error = ctx->last_error;
@@ -173,9 +190,8 @@ int plviwo_fe_set_calib(FeHandle *h, const double K[4], const double D[4]) {
 
 int plviwo_fe_set_camera(FeHandle *h, int model, const double K[4], const double D[4]) {
   if (!h || !K || !D) return FE_BAD_ARG;
-  if (model != FE_CAM_RADTAN) {
-    h->ctx->last_error = "set_camera: only the radtan model is implemented (an equidistant camera, cam/CamEqui.h:108-129, would be "
-                         "undistorted with the wrong formula)";
+  if (model != h->ctx->model()) {
+    h->ctx->last_error = model_mismatch(h->ctx->model());
     return FE_BAD_ARG;
   }
   return h->ctx->set_calib(K, D);
@@ -573,7 +589,29 @@ int plviwo_op_undistort(int device, const float *pts, int n, const double K[4], 
   DevBuf<float2> a, b;
   if (a.alloc(n) || b.alloc(n)) return FE_CUDA_ERROR;
   OP_CUDA(cudaMemcpy(a.p, pts, (size_t)n * sizeof(float2), cudaMemcpyHostToDevice));
-  launch_undistort(a.p, b.p, n, K, D, 0);
+  launch_undistort(a.p, b.p, n, FE_CAM_RADTAN, K, D, 0);
+  OP_CUDA(cudaDeviceSynchronize());
+  OP_CUDA(cudaMemcpy(out, b.p, (size_t)n * sizeof(float2), cudaMemcpyDeviceToHost));
+  return FE_OK;
+  API_END
+}
+
+int plviwo_op_undistort_equi(int device, const float *pts, int n, const double K[4], const double D[4], float *out) {
+  API_BEGIN
+  if (!pts || !out || !K || !D || n < 0) return FE_BAD_ARG;
+  if (device < 0) {   // host instantiation of tracker_core.h's undistort_equi
+    for (int i = 0; i < n; i++) {
+      const float2 r = undistort_equi(make_float2(pts[2 * i], pts[2 * i + 1]), K, D);
+      out[2 * i] = r.x;
+      out[2 * i + 1] = r.y;
+    }
+    return FE_OK;
+  }
+  OP_CUDA(cudaSetDevice(device));
+  DevBuf<float2> a, b;
+  if (a.alloc(n) || b.alloc(n)) return FE_CUDA_ERROR;
+  OP_CUDA(cudaMemcpy(a.p, pts, (size_t)n * sizeof(float2), cudaMemcpyHostToDevice));
+  launch_undistort(a.p, b.p, n, FE_CAM_EQUI, K, D, 0);
   OP_CUDA(cudaDeviceSynchronize());
   OP_CUDA(cudaMemcpy(out, b.p, (size_t)n * sizeof(float2), cudaMemcpyDeviceToHost));
   return FE_OK;
@@ -798,15 +836,20 @@ int plviwo_op_line_match(int n_last, const int32_t *last_off, const int32_t *las
 
 // ---- stream group (many camera streams of one device, csrc/fe_group.h) ---------------------------------------------
 int plviwo_fe_group_create(const FeConfig *cfg, int n_streams, int device, FeGroupHandle **out) {
+  return plviwo_fe_group_create_model(cfg, n_streams, FE_CAM_RADTAN, device, out);
+}
+
+int plviwo_fe_group_create_model(const FeConfig *cfg, int n_streams, int model, int device, FeGroupHandle **out) {
   API_BEGIN
   if (!cfg || !out) return FE_BAD_ARG;
   *out = nullptr;
+  if (const char *why = check_model(model)) return create_error(FE_BAD_ARG, why);
   if (n_streams < 1 || n_streams > 4096) return create_error(FE_BAD_ARG, "n_streams must be in [1, 4096]");
   if (cfg->downsample) return create_error(FE_BAD_ARG, "cfg.downsample is not supported in a stream group");
   if (const char *why = check_config(*cfg, cfg->width, cfg->height)) return create_error(FE_BAD_ARG, why);
   if (cfg->grid_x * cfg->grid_y > 256) return create_error(FE_BAD_ARG, "a stream group supports at most 256 grid cells");
   if (int rc = check_device(device)) return rc;
-  FeGroup *grp = new FeGroup(*cfg, n_streams, device);
+  FeGroup *grp = new FeGroup(*cfg, n_streams, device, false, model);
   int rc = grp->init();
   if (rc != FE_OK) {
     g_create_error = grp->last_error;
@@ -836,8 +879,8 @@ int plviwo_fe_group_set_calib(FeGroupHandle *g, int stream, const double K[4], c
 
 int plviwo_fe_group_set_camera(FeGroupHandle *g, int stream, int model, const double K[4], const double D[4]) {
   if (!g) return FE_BAD_ARG;
-  if (model != FE_CAM_RADTAN) {   // as plviwo_fe_set_camera: an equidistant camera is refused, not undistorted with the radtan formula
-    g->grp->last_error = "set_camera: only the radtan model is implemented (cam/CamEqui.h:108-129 is not)";
+  if (model != g->grp->model()) {   // as plviwo_fe_set_camera
+    g->grp->last_error = model_mismatch(g->grp->model());
     return FE_BAD_ARG;
   }
   return g->grp->set_calib(stream, K, D);
@@ -931,9 +974,14 @@ int plviwo_fe_group_get_times(FeGroupHandle *g, FeGroupTimes *out, int reset) {
 
 // ---- stereo group (many stereo rigs of one device, csrc/fe_group.h) ---------------------------------------------
 int plviwo_fe_stereo_group_create(const FeConfig *cfg, int n_rigs, int device, FeStereoGroupHandle **out) {
+  return plviwo_fe_stereo_group_create_model(cfg, n_rigs, FE_CAM_RADTAN, device, out);
+}
+
+int plviwo_fe_stereo_group_create_model(const FeConfig *cfg, int n_rigs, int model, int device, FeStereoGroupHandle **out) {
   API_BEGIN
   if (!cfg || !out) return FE_BAD_ARG;
   *out = nullptr;
+  if (const char *why = check_model(model)) return create_error(FE_BAD_ARG, why);
   if (n_rigs < 1 || n_rigs > 2048) return create_error(FE_BAD_ARG, "n_rigs must be in [1, 2048] (2 camera streams per rig, at most 4096)");
   if (const char *why = check_config(*cfg, cfg->width, cfg->height)) return create_error(FE_BAD_ARG, why);
   if (cfg->grid_x * cfg->grid_y > 256) return create_error(FE_BAD_ARG, "a stream group supports at most 256 grid cells");
@@ -941,7 +989,7 @@ int plviwo_fe_stereo_group_create(const FeConfig *cfg, int n_rigs, int device, F
   if (cfg->downsample) return create_error(FE_BAD_ARG, "cfg.downsample is not supported in a stereo group");
   if (cfg->line_samples) return create_error(FE_BAD_ARG, "cfg.line_samples is not supported in a stereo group");
   if (int rc = check_device(device)) return rc;
-  FeGroup *grp = new FeGroup(*cfg, 2 * n_rigs, device, true);
+  FeGroup *grp = new FeGroup(*cfg, 2 * n_rigs, device, true, model);
   int rc = grp->init();
   if (rc != FE_OK) {
     g_create_error = grp->last_error;
@@ -982,8 +1030,8 @@ int plviwo_fe_stereo_group_set_calib(FeStereoGroupHandle *g, int rig, int cam, c
 
 int plviwo_fe_stereo_group_set_camera(FeStereoGroupHandle *g, int rig, int cam, int model, const double K[4], const double D[4]) {
   if (!g) return FE_BAD_ARG;
-  if (model != FE_CAM_RADTAN) {   // as plviwo_fe_set_camera
-    g->grp->last_error = "set_camera: only the radtan model is implemented (cam/CamEqui.h:108-129 is not)";
+  if (model != g->grp->model()) {   // as plviwo_fe_set_camera
+    g->grp->last_error = model_mismatch(g->grp->model());
     return FE_BAD_ARG;
   }
   return plviwo_fe_stereo_group_set_calib(g, rig, cam, K, D);
@@ -1057,13 +1105,19 @@ int plviwo_fe_stereo_group_set_state(FeStereoGroupHandle *g, int rig, const void
 // ---- stereo rig (TrackKLT with use_stereo = true) -----------------------------------------------------------
 int plviwo_fe_stereo_create(const FeConfig *cfg, const double K_right[4], const double D_right[4], int device,
                             FeStereoHandle **out) {
+  return plviwo_fe_stereo_create_model(cfg, FE_CAM_RADTAN, K_right, D_right, device, out);
+}
+
+int plviwo_fe_stereo_create_model(const FeConfig *cfg, int model, const double K_right[4], const double D_right[4], int device,
+                                  FeStereoHandle **out) {
   API_BEGIN
   if (!cfg || !out) return FE_BAD_ARG;
   *out = nullptr;
+  if (const char *why = check_model(model)) return create_error(FE_BAD_ARG, why);
   // the rig tracks at the raw size: it zeroes cfg.downsample
   if (const char *why = check_config(*cfg, cfg->width, cfg->height)) return create_error(FE_BAD_ARG, why);
   if (int rc = check_device(device)) return rc;
-  FeStereo *st = new FeStereo(*cfg, K_right, D_right, device);
+  FeStereo *st = new FeStereo(*cfg, K_right, D_right, device, model);
   int rc = st->init();
   if (rc != FE_OK) {
     g_create_error = st->last_error;
@@ -1092,8 +1146,8 @@ int plviwo_fe_stereo_set_calib(FeStereoHandle *h, int cam, const double K[4], co
 }
 int plviwo_fe_stereo_set_camera(FeStereoHandle *h, int cam, int model, const double K[4], const double D[4]) {
   if (!h || !K || !D) return FE_BAD_ARG;
-  if (model != FE_CAM_RADTAN) {
-    h->st->last_error = "set_camera: only the radtan model is implemented";
+  if (model != h->st->model()) {
+    h->st->last_error = model_mismatch(h->st->model());
     return FE_BAD_ARG;
   }
   return plviwo_fe_stereo_set_calib(h, cam, K, D);

@@ -101,8 +101,8 @@ void WorkQueue::stop() {
   cv_.notify_all();
 }
 
-FeContext::FeContext(const FeConfig &cfg, int device)
-    : cfg_(cfg), device_(device), W_(cfg.width), H_(cfg.height), Win_(cfg.width), Hin_(cfg.height) {
+FeContext::FeContext(const FeConfig &cfg, int device, int model)
+    : cfg_(cfg), device_(device), model_(model), W_(cfg.width), H_(cfg.height), Win_(cfg.width), Hin_(cfg.height) {
   if (cfg.downsample) {   // cv::Size(img.cols / 2.0, img.rows / 2.0): truncation (UpdaterCamera.cpp:91)
     W_ = (int)(cfg.width / 2.0);
     H_ = (int)(cfg.height / 2.0);
@@ -602,7 +602,7 @@ int FeContext::flush_line_batch() {
 int FeContext::track_candidates(FrameSlot &prev, FrameSlot &s) {
   s.sc_prev = -1;
   if (!use_spec_ || cfg_.line_samples > 0) return FE_OK;
-  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, s.K, s.D, true);
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, s.K, s.D, true, model_);
   const int ntab = prev.predet_ncell * prev.predet_nfg;
   if (ntab <= 0 || ntab > cand_cap_ || prev.predet_num_features != cfg_.num_features || !lk_w15_form(prm.win, prev.pyr.n))
     return FE_OK;
@@ -1073,7 +1073,7 @@ int FeContext::speculate(FrameSlot &prev, const float2 *lk_pts, const uint8_t *l
   int nxt = -1;
   if (!klt_q_.peek(&nxt)) return FE_OK;          // the next frame has not been submitted yet
   FrameSlot &fn = slots_[nxt];
-  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, fn.K, fn.D, true);
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, fn.K, fn.D, true, model_);
   // ---- (A) the points tracked into `prev` whose KLT status is good: latency-critical stream
   int k = 0;
   for (int i = 0; i < n && k < max_pts_; i++)
@@ -1341,7 +1341,7 @@ int FeContext::perform_matching(const FrameSlot &f0, FrameSlot &f1, std::vector<
     h_pts1_[k] = h_pts0_[k];   // OPTFLOW_USE_INITIAL_FLOW with pts1 = pts0 (:134-138)
   }
   for (int k = 0; k < ns; k++) h_pts1_[n2 + k] = h_pts0_[n2 + k];
-  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, f1.K, f1.D, true);
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, f1.K, f1.D, true, model_);
   // The feature arrays are a few KB: the kernel reads and writes them in pinned, device-mapped host memory directly
   // (no copy-engine operation queued behind the next frame's 700 KB upload, one synchronisation per frame).
   if (nt > 0) {
@@ -1443,7 +1443,7 @@ int FeContext::lk_launch(const Pyramid &p0, const Pyramid &p1, const std::vector
     h_pts0_[k] = make_float2(pts[k].x, pts[k].y);
     h_pts1_[k] = h_pts0_[k];   // OPTFLOW_USE_INITIAL_FLOW with pts1 = pts0
   }
-  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, K, D, undistort);
+  const LkParams prm = lk_params(cfg_.win_size, cfg_.pyr_levels, K, D, undistort, model_);
   const bool self_signal = launch_lk(p0, p1, h_pts0_, h_pts1_, h_status_, h_p0n_, h_p1n_, n, prm, s_pt_, h_flag_lk_, ++seq_lk_,
                                      d_lk_done_);
   if (!self_signal) launch_signal(h_flag_lk_, seq_lk_, s_pt_);
@@ -1618,7 +1618,8 @@ int FeContext::lsd_feed(FrameSlot &cur) {
     r.id = good_ids[i];
     const float4 &l = filt_lines[i];
     r.line[0] = l.x; r.line[1] = l.y; r.line[2] = l.z; r.line[3] = l.w;
-    const float2 n0 = undistort_radtan(make_float2(l.x, l.y), cur.K, cur.D), n1 = undistort_radtan(make_float2(l.z, l.w), cur.K, cur.D);
+    const float2 n0 = undistort_point(model_, make_float2(l.x, l.y), cur.K, cur.D),
+                 n1 = undistort_point(model_, make_float2(l.z, l.w), cur.K, cur.D);
     r.line_n[0] = n0.x; r.line_n[1] = n0.y; r.line_n[2] = n1.x; r.line_n[3] = n1.y;
     r.D = line_classification(l, cur.vp);
     r.n_pts = (int)pol_new[i].size();

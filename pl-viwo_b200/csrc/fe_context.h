@@ -170,7 +170,8 @@ struct LkTracks {
 
 class FeContext {
  public:
-  FeContext(const FeConfig &cfg, int device);
+  // model: the FeCameraModel of the camera (ov_core's CamBase subclass), fixed for the context's lifetime
+  FeContext(const FeConfig &cfg, int device, int model = FE_CAM_RADTAN);
   ~FeContext();
   int init();  // allocates; returns FeStatus
 
@@ -198,6 +199,7 @@ class FeContext {
   int tap(int what, void *buf, size_t cap, size_t *n_bytes);
 
   const FeConfig &cfg() const { return cfg_; }
+  int model() const { return model_; }
   static std::string &thread_error();   // error text of the calling thread (what last_error is filled from)
   std::string last_error;
   std::atomic<bool> timing{false};
@@ -267,6 +269,7 @@ class FeContext {
 
   FeConfig cfg_;
   int device_;
+  int model_;            // FeCameraModel (undistortion of the LK epilogue and of the line rows)
   int W_, H_;            // tracking size (= input size, or half of it with cfg.downsample)
   int Win_, Hin_;        // input size
   cudaStream_t s_pt_ = nullptr;

@@ -24,8 +24,8 @@ namespace plviwo {
 static inline int align_up(int v, int a) { return (v + a - 1) / a * a; }
 static inline size_t align_up_sz(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-FeGroup::FeGroup(const FeConfig &cfg, int n_streams, int device, bool stereo)
-    : cfg_(cfg), S_(n_streams), device_(device), W_(cfg.width), H_(cfg.height), stereo_(stereo) {}
+FeGroup::FeGroup(const FeConfig &cfg, int n_streams, int device, bool stereo, int model)
+    : cfg_(cfg), S_(n_streams), device_(device), W_(cfg.width), H_(cfg.height), stereo_(stereo), model_(model) {}
 
 int FeGroup::fail(cudaError_t e, const char *what) {
   last_error = std::string(what) + ": " + cudaGetErrorString(e);
@@ -95,6 +95,7 @@ int FeGroup::init() {
   g_.close_h = (int)((float)H_ / (float)cfg_.min_px_dist);
   g_.line_min_length = cfg_.line_min_length;
   g_.use_lines = cfg_.use_lines;
+  g_.cam_model = model_;
   layout_cells();
   const int ncell = g_.n_cells, nfg = g_.nfg;
   g_.cand_cap = std::max(ncell * nfg, 1);
@@ -164,7 +165,7 @@ int FeGroup::init() {
   g_.slot_flags = d_slot_flags_;
   // every slot's pyramid holds n_lvl images: LK tracks through all of them (cv::calcOpticalFlowPyrLK on a prebuilt pyramid),
   // and the body of its launches is chosen by that count, as a handle chooses it (fe_kernels.h lk_w15_form)
-  lk_prm_ = lk_params(cfg_.win_size, slots_[0].n_lvl - 1, nullptr, nullptr, true);
+  lk_prm_ = lk_params(cfg_.win_size, slots_[0].n_lvl - 1, nullptr, nullptr, true, model_);
 
   // ---- tracker state and work arrays
   const size_t P = (size_t)S_ * g_.pts_cap;

@@ -30,12 +30,14 @@ namespace plviwo {
 
 class FeGroup {
  public:
-  FeGroup(const FeConfig &cfg, int n_streams, int device, bool stereo = false);
+  // model: the FeCameraModel of every stream's camera, fixed for the group's lifetime
+  FeGroup(const FeConfig &cfg, int n_streams, int device, bool stereo = false, int model = FE_CAM_RADTAN);
   ~FeGroup();
   int init();
 
   int n_streams() const { return S_; }
   const FeConfig &cfg() const { return cfg_; }
+  int model() const { return model_; }
   int set_calib(int stream, const double K[4], const double D[4]);
   // One tick: a frame of every stream whose images[s] is not null.  vps: 6 doubles per stream (all streams) or null (the line
   // tracker is not fed); masks: per-stream host pointers or null.
@@ -102,6 +104,7 @@ class FeGroup {
   FeConfig cfg_;
   int S_, device_, W_, H_;
   bool stereo_ = false;
+  int model_ = FE_CAM_RADTAN;
   int la_ = 0, R_ = 2, RB_ = 2, B_ = 1, lanes_ = 1;
   std::vector<double> K_, D_;            // per stream, 4 each
   // ---- device data

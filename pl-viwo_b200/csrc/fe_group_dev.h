@@ -46,6 +46,7 @@ struct GroupDev {
   int close_w, close_h;
   float line_min_length;
   int use_lines;
+  int cam_model;                 // FeCameraModel of every stream, fixed at creation
   // ---- capacities
   int pts_cap, lines_cap, pol_cap, cand_cap, segs_cap;
   // ---- slot table

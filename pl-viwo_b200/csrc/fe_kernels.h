@@ -136,10 +136,11 @@ struct LkParams {
   float min_eig;   // 1e-4
   double K[4], D[4];
   int undistort;   // also write normalised coordinates of pts0 / pts1
+  int model;       // FeCameraModel of K / D
 };
 // The reference's termination criteria and eigenvalue threshold (TrackKLT.cpp:855-858) with the given window, pyramid
-// depth and calibration (K / D null: zeros).  Host only.
-inline LkParams lk_params(int win, int max_level, const double *K, const double *D, bool undistort) {
+// depth and calibration (K / D null: zeros) of camera model `model`.  Host only.
+inline LkParams lk_params(int win, int max_level, const double *K, const double *D, bool undistort, int model = FE_CAM_RADTAN) {
   LkParams prm;
   prm.win = win;
   prm.max_level = max_level;
@@ -147,6 +148,7 @@ inline LkParams lk_params(int win, int max_level, const double *K, const double 
   prm.eps_sq = 0.01f * 0.01f;
   prm.min_eig = 1e-4f;
   prm.undistort = undistort ? 1 : 0;
+  prm.model = model;
   for (int i = 0; i < 4; i++) {
     prm.K[i] = K ? K[i] : 0;
     prm.D[i] = D ? D[i] : 0;
@@ -170,7 +172,7 @@ bool launch_lk(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, f
 // otherwise): the same results as launch_lk's k_lk15, bit for bit
 bool launch_lk_warp(const Pyramid &prev, const Pyramid &next, const float2 *d_pts0, float2 *d_pts1, uint8_t *d_status, int n,
                     const LkParams &prm, cudaStream_t s);
-void launch_undistort(const float2 *d_pts, float2 *d_out, int n, const double K[4], const double D[4], cudaStream_t s);
+void launch_undistort(const float2 *d_pts, float2 *d_out, int n, int model, const double K[4], const double D[4], cudaStream_t s);
 
 // ---- lines (kernels_lines.cu) -------------------------------------------------------------------------------
 struct FldBuffers {

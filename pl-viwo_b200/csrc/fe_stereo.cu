@@ -23,7 +23,7 @@ namespace plviwo {
     if (e__ != cudaSuccess) return err(FE_CUDA_ERROR, std::string(#call) + ": " + cudaGetErrorString(e__)); \
   } while (0)
 
-FeStereo::FeStereo(const FeConfig &cfg, const double K_right[4], const double D_right[4], int device)
+FeStereo::FeStereo(const FeConfig &cfg, const double K_right[4], const double D_right[4], int device, int model)
     : cfg_(cfg), device_(device) {
   cfg_.line_samples = 0;
   cfg_.downsample = 0;
@@ -33,8 +33,8 @@ FeStereo::FeStereo(const FeConfig &cfg, const double K_right[4], const double D_
     if (K_right) cr.K[i] = K_right[i];
     if (D_right) cr.D[i] = D_right[i];
   }
-  cam_[0].reset(new FeContext(cfg_, device));
-  cam_[1].reset(new FeContext(cr, device));
+  cam_[0].reset(new FeContext(cfg_, device, model));
+  cam_[1].reset(new FeContext(cr, device, model));
   currid_ = 4 * (uint64_t)cfg.numaruco + 1;   // TrackBase.cpp:34
 }
 

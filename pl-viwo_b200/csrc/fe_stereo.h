@@ -18,9 +18,11 @@ namespace plviwo {
 
 class FeStereo {
  public:
-  FeStereo(const FeConfig &cfg, const double K_right[4], const double D_right[4], int device);
+  // model: the FeCameraModel of both cameras, fixed for the rig's lifetime
+  FeStereo(const FeConfig &cfg, const double K_right[4], const double D_right[4], int device, int model = FE_CAM_RADTAN);
   ~FeStereo();
   int init();
+  int model() const { return cam_[0]->model(); }
 
   int set_calib(int cam, const double K[4], const double D[4]);
   int set_num_features(int n);

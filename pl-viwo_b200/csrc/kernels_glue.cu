@@ -1178,7 +1178,8 @@ __global__ void __launch_bounds__(kGT)
     memset(&r, 0, sizeof(r));
     r.id = id;
     r.line[0] = l.x; r.line[1] = l.y; r.line[2] = l.z; r.line[3] = l.w;
-    const float2 n0 = undistort_radtan(make_float2(l.x, l.y), job.K, job.D), n1 = undistort_radtan(make_float2(l.z, l.w), job.K, job.D);
+    const float2 n0 = undistort_point(g.cam_model, make_float2(l.x, l.y), job.K, job.D),
+                 n1 = undistort_point(g.cam_model, make_float2(l.z, l.w), job.K, job.D);
     r.line_n[0] = n0.x; r.line_n[1] = n0.y; r.line_n[2] = n1.x; r.line_n[3] = n1.y;
     r.D = line_classification(l, job.vp);
     r.n_pts = poff_new[i + 1] - poff_new[i];

@@ -1,11 +1,12 @@
 // Per-feature kernels (sm_100a): sub-pixel corner refinement, pyramidal Lucas-Kanade with on-the-fly Scharr
-// derivatives, and radtan undistortion.  One warp per feature; compiled with --fmad=false so that float
+// derivatives, and undistortion (radtan or equidistant).  One warp per feature; compiled with --fmad=false so that float
 // expressions round exactly where the reference's SSE build rounds.
 //
 // Reference ops replaced (SURVEY.md Appendix A3, A5, A6):
 //   cv::cornerSubPix(img, pts, (5,5), (-1,-1), {COUNT+EPS, 20, 0.001})             Grider_GRID.h:163-174
 //   cv::calcOpticalFlowPyrLK(.., win, maxLevel, {COUNT|EPS, 30, 0.01}, USE_INITIAL_FLOW)  TrackKLT.cpp:855-858
 //   CamRadtan::undistort_f -> cv::undistortPoints (one Mat per point)               cam/CamRadtan.h:99-120
+//   CamEqui::undistort_f -> cv::fisheye::undistortPoints (one Mat per point)        cam/CamEqui.h:108-129
 #include "fe_kernels.h"
 #include "fe_group_dev.h"
 #include "tracker_core.h"
@@ -171,17 +172,32 @@ struct CalibArgs {
   double K[4], D[4];
 };
 
-__global__ void k_undistort(const float2 *__restrict__ pts, float2 *__restrict__ out, int n, CalibArgs c) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = undistort_radtan(pts[i], c.K, c.D);
+// The equidistant model out of line: its Newton loop and tan stay out of the register budget of the LK kernels, whose
+// epilogue calls it for one point per lane at most.  The calibration goes by value (registers): a pointer into a kernel's
+// parameter block would make the caller copy the whole block to its stack.
+__device__ __noinline__ float2 undistort_equi_call(float2 uv, double fx, double fy, double cx, double cy, double k1, double k2,
+                                                   double k3, double k4) {
+  const double K[4] = {fx, fy, cx, cy}, D[4] = {k1, k2, k3, k4};
+  return undistort_equi(uv, K, D);
+}
+// undistort_point of the kernels: `model` is uniform per launch
+__device__ __forceinline__ float2 undistort_dev(int model, float2 uv, const CalibArgs &c) {
+  if (model == FE_CAM_EQUI)
+    return undistort_equi_call(uv, c.K[0], c.K[1], c.K[2], c.K[3], c.D[0], c.D[1], c.D[2], c.D[3]);
+  return undistort_radtan(uv, c.K, c.D);
 }
 
-void launch_undistort(const float2 *d_pts, float2 *d_out, int n, const double K[4], const double D[4], cudaStream_t s) {
+__global__ void k_undistort(const float2 *__restrict__ pts, float2 *__restrict__ out, int n, int model, CalibArgs c) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = undistort_point(model, pts[i], c.K, c.D);
+}
+
+void launch_undistort(const float2 *d_pts, float2 *d_out, int n, int model, const double K[4], const double D[4], cudaStream_t s) {
   if (n <= 0) return;
   CalibArgs c;
   for (int i = 0; i < 4; i++) { c.K[i] = K[i]; c.D[i] = D[i]; }
   PLVIWO_CARVEOUT(k_undistort);
-  k_undistort<<<(n + 127) / 128, 128, 0, s>>>(d_pts, d_out, n, c);
+  k_undistort<<<(n + 127) / 128, 128, 0, s>>>(d_pts, d_out, n, model, c);
 }
 
 // ===================================================================================================== LK
@@ -202,6 +218,7 @@ struct LkArgs {
   int flow_is_zero;   // the initial guess is the previous position itself: pts1 is output only
   unsigned cell_mask[8];   // table mode: cells whose candidates are tracked at all (bit c of word c / 32)
   float eps_sq, min_eig;
+  int model;          // FeCameraModel of calib (in the padding before it: LkArgs keeps its size)
   CalibArgs calib;
 };
 
@@ -223,6 +240,7 @@ __host__ __device__ inline void lk_args(LkArgs &a, const DevImage *l0, const Dev
   a.eps_sq = prm.eps_sq;
   a.min_eig = prm.min_eig;
   a.undistort = undistort;
+  a.model = prm.model;
   a.flow_is_zero = flow_is_zero;
   for (int i = 0; i < 8; i++) a.cell_mask[i] = cell_mask ? cell_mask[i] : 0xffffffffu;
   for (int i = 0; i < 4; i++) {
@@ -410,8 +428,8 @@ __device__ __forceinline__ void lk_body(const Args &a, const float2 *__restrict_
     status[pi] = ok ? 1 : 0;
   }
   if (a.undistort) {
-    if (lane == 0) p0n[pi] = undistort_radtan(prev_in, a.calib.K, a.calib.D);
-    if (lane == 1) p1n[pi] = undistort_radtan(next, a.calib.K, a.calib.D);
+    if (lane == 0) p0n[pi] = undistort_dev(a.model, prev_in, a.calib);
+    if (lane == 1) p1n[pi] = undistort_dev(a.model, next, a.calib);
   }
 }
 
@@ -718,8 +736,8 @@ __device__ __forceinline__ void lk15_body(const Args &a, const float2 *__restric
     status[pi] = ok ? 1 : 0;
   }
   if (a.undistort) {
-    if (lane == 0) p0n[pi] = undistort_radtan(prev_in, a.calib.K, a.calib.D);
-    if (lane == 1) p1n[pi] = undistort_radtan(next, a.calib.K, a.calib.D);
+    if (lane == 0) p0n[pi] = undistort_dev(a.model, prev_in, a.calib);
+    if (lane == 1) p1n[pi] = undistort_dev(a.model, next, a.calib);
   }
   // ---- completion signal: the last feature to finish publishes the sequence number (results first, system-wide)
   if (host_flag != nullptr) {
@@ -1103,8 +1121,8 @@ __device__ __forceinline__ void lk15w_body(const Args &a, const float2 *__restri
     status[pi] = ok ? 1 : 0;
   }
   if (a.undistort) {
-    if (lane == 0) p0n[pi] = undistort_radtan(prev_in, a.calib.K, a.calib.D);
-    if (lane == 1) p1n[pi] = undistort_radtan(next, a.calib.K, a.calib.D);
+    if (lane == 0) p0n[pi] = undistort_dev(a.model, prev_in, a.calib);
+    if (lane == 1) p1n[pi] = undistort_dev(a.model, next, a.calib);
   }
 }
 
